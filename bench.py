@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DAVO pose forward path (BASELINE.json metric: frame pairs / second).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A step is one pass of the hot path (attention front end -> dilated PoseNN -> 6-DoF
 head) over one batch of synthetic 128x416 samples: 128 samples = 256 frame pairs
@@ -22,6 +22,12 @@ BASELINE.json north_star); under N > 1 the per-step gather is the library's own
 [N*B,2,6] equals, bit for bit, what rank 0 computes alone from every rank's
 seeded inputs.  ``stream_4541`` is BASELINE configs[2]: the 4541-frame stream
 sharded over the N ranks (strong scaling), gathered and composed.
+
+``--dump-outputs DIR`` writes (rank 0) what the last timed step returned to its
+caller as ``DIR/pose.npy``: the CUDA path's [N*B,2,6] float32 poses (gathered
+over the N ranks), or under ``--impl reference`` the oracle's [16,2,6] float64
+poses of its CPU sample.  Inputs and weights are seeded, so two builds run with
+the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -169,6 +175,15 @@ def parity_block(ref, **got):
     return out
 
 
+def dump_outputs(out_dir, **arrays):
+    """Writes each array as ``out_dir/<name>.npy``, float64 kept, anything else as float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 def run_reference(args):
     """--impl reference: the reference graph's CPU restatement (oracle port) on host cores.
 
@@ -183,7 +198,9 @@ def run_reference(args):
     for _ in range(max(args.warmup, 1) - 1):
         cpu_oracle_rate(batch, 1, cores)
     steps = max(1, args.steps)                   # a step = 16 samples: ~0.2 s of CPU work
-    rate, dt, thr, steps, _ = cpu_oracle_rate(batch, steps, cores)
+    rate, dt, thr, steps, poses = cpu_oracle_rate(batch, steps, cores)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pose=poses)
     sample = "%d steps x %d samples (%d frame pairs each) of the 128-sample batch, fp32 torch-CPU" % (
         steps, batch, 2 * batch)
     line = {
@@ -321,6 +338,8 @@ def run_ours(args):
     clocks = sampler.stop()
     launches = system.last_launch_count() * args.steps
     timed_out = timed_out.cpu().numpy()          # [world*B,2,6] under N > 1 (gathered), [B,2,6] at N = 1
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pose=timed_out)
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -545,7 +564,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=128, help="samples per GPU per step (2 frame pairs each)")
     ap.add_argument("--micro-batch", type=int, default=0, help="frame pairs per pass of the conv stack")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the poses of the last timed step to DIR/pose.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # started as plain `python bench.py --gpus N`: become the N-rank launch the contract describes
         # (torch.distributed.run, one rank per GPU, rendezvous on 127.0.0.1)

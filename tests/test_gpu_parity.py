@@ -1121,3 +1121,28 @@ def test_front_pipeline_experiment_gives_the_same_bits(monkeypatch):
                            env=dict(os.environ, DAVO_B200_FRONT_PIPE="1"))
         assert r.returncode == 0, r.stderr[-2000:]
         assert np.array_equal(np.load(os.path.join(d, "p.npy")), ref)
+
+
+def test_bench_dump_outputs_repeats_and_is_what_the_timed_path_returns(tmp_path):
+    """`bench.py --dump-outputs DIR` run twice with the same arguments writes the same DIR/pose.npy ([B,2,6] float32),
+    and that is what DAVO.inference returns for bench's seeded inputs (seed 1234 on rank 0) and weights."""
+    _need_gpu()
+    import subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = {k: v for k, v in os.environ.items() if k not in ("WORLD_SIZE", "RANK", "LOCAL_RANK")}
+    env["DAVO_BENCH_SKIP_STREAM"] = "1"                                  # the 4541-frame stream is not what is dumped
+    B = 16
+    dumps = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+                            "--batch", str(B), "--dump-outputs", str(tmp_path / run)],
+                           capture_output=True, text=True, timeout=600, env=env)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert sorted(os.listdir(tmp_path / run)) == ["pose.npy"]
+        dumps.append(np.load(tmp_path / run / "pose.npy"))
+    a, b = dumps
+    assert a.shape == (B, 2, 6) and a.dtype == np.float32 and np.all(np.isfinite(a))
+    assert np.array_equal(a, b)
+    import bench
+    sysm, _ = _system(bench.VERSION, B, S.init_weights(bench.VERSION), S.make_inputs(B, bench.H, bench.W, seed=1234))
+    assert np.array_equal(sysm.inference(None, "pose")["pose"], a)

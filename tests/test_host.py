@@ -70,38 +70,38 @@ def _mat2euler(r):
     return np.arctan2(-r[0, 1], r[0, 0]), np.arctan2(r[0, 2], cy), np.arctan2(-r[1, 2], r[2, 2])
 
 
-def _gt_trajectory():
-    path = "/root/reference/kitti_benchmark/data/odometry/poses/00.txt"
-    if os.path.exists(path):                          # real KITTI motion when the checkout is present
-        rows = np.loadtxt(path)[:300].reshape(-1, 3, 4)
-        gt = np.tile(np.eye(4), (rows.shape[0], 1, 1))
-        gt[:, :3, :] = rows
-        return gt
+def _gt_trajectory(turn=0.0):
+    """300 frames of seeded random motion, translation steps up to about a metre.  turn = 0: small rotation steps;
+    turn > 0: a steady yaw of `turn` rad per frame and larger rotation noise, so that the heading sweeps several full
+    turns (every yaw in -pi..pi) and the steps' Euler angles reach a few tenths of a radian."""
     rng = np.random.default_rng(2)
+    std = [0.005, 0.02, 0.005, 0.03, 0.02, 0.8] if turn == 0.0 else [0.03, 0.1, 0.03, 0.03, 0.02, 0.8]
     gt = [np.eye(4)]
     for _ in range(299):
-        step = geo_utils.pose_vec2mat(rng.normal(0, [0.005, 0.02, 0.005, 0.03, 0.02, 0.8], size=(1, 6)))[0]
+        step = geo_utils.pose_vec2mat(rng.normal([0.0, turn, 0.0, 0.0, 0.0, 0.0], std, size=(1, 6)))[0]
         gt.append(gt[-1] @ step.astype(np.float64))
     return np.stack(gt)
 
 
 def test_ground_truth_round_trip_through_pose_vectors():
-    """encode GT steps as the network's [rz,ry,rx,t] vectors -> compose -> the GT trajectory again."""
-    gt = _gt_trajectory()
-    n = gt.shape[0] - 2                               # samples for a stream of n+2 frames
-    poses = np.zeros((n, 2, 6), np.float32)
-    for s in range(n):
-        # pose[s,1] is tgt->src1 with tgt = frame s+1: inv(step s+1 -> s+2) (test_kitti_pose.py:145)
-        t_fwd = np.linalg.inv(gt[s + 1]) @ gt[s + 2]
-        m = np.linalg.inv(t_fwd)
-        poses[s, 1, :3] = _mat2euler(m[:3, :3])
-        poses[s, 1, 3:] = m[:3, 3]
-    first = np.linalg.inv(gt[0]) @ gt[1]              # pose[0,0] = tgt->src0 of the first sample
-    poses[0, 0, :3] = _mat2euler(first[:3, :3])
-    poses[0, 0, 3:] = first[:3, 3]
-    traj = geo_utils.compose_trajectory(poses)
-    assert traj.shape == gt.shape
-    assert O.ate(traj, gt) < 2e-3 * max(1.0, np.abs(gt[:, :3, 3]).max() / 100)
+    """encode GT steps as the network's [rz,ry,rx,t] vectors -> compose -> the GT trajectory again, for gentle motion
+    and for a trajectory that turns through every heading."""
+    for turn in (0.0, 0.05):
+        gt = _gt_trajectory(turn)
+        n = gt.shape[0] - 2                           # samples for a stream of n+2 frames
+        poses = np.zeros((n, 2, 6), np.float32)
+        for s in range(n):
+            # pose[s,1] is tgt->src1 with tgt = frame s+1: inv(step s+1 -> s+2) (test_kitti_pose.py:145)
+            t_fwd = np.linalg.inv(gt[s + 1]) @ gt[s + 2]
+            m = np.linalg.inv(t_fwd)
+            poses[s, 1, :3] = _mat2euler(m[:3, :3])
+            poses[s, 1, 3:] = m[:3, 3]
+        first = np.linalg.inv(gt[0]) @ gt[1]          # pose[0,0] = tgt->src0 of the first sample
+        poses[0, 0, :3] = _mat2euler(first[:3, :3])
+        poses[0, 0, 3:] = first[:3, 3]
+        traj = geo_utils.compose_trajectory(poses)
+        assert traj.shape == gt.shape
+        assert O.ate(traj, gt) < 2e-3 * max(1.0, np.abs(gt[:, :3, 3]).max() / 100), turn
 
 
 # ------------------------------------------------------------------ sharding --
@@ -529,15 +529,15 @@ def test_data_loader_mirrors_load_test_batch_flow(tmp_path):
         loader.load_test_batch_flow(names, poses, flows, depths, segs, decode="nvjpeg")      # needs a DAVO handle
 
 
-def test_bench_reference_arm_prints_one_contract_line_also_when_started_plainly_with_gpus_2():
+def test_bench_reference_arm_prints_one_contract_line_also_when_started_plainly_with_gpus_2(tmp_path):
     """`python bench.py --impl reference --gpus 2` (no torchrun around it): bench.py becomes the 2-rank launch itself
     (127.0.0.1 rendezvous), rank 0 alone times the CPU port and prints ONE JSON line with the contract's keys; the other
-    rank exits 0 without work."""
+    rank exits 0 without work.  --dump-outputs writes the poses of the last timed step, the same ones on every run."""
     import json, subprocess, sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     env = {k: v for k, v in os.environ.items() if k not in ("WORLD_SIZE", "RANK", "LOCAL_RANK")}
-    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "1"],
-                       capture_output=True, text=True, timeout=600, env=env)
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "1",
+                        "--dump-outputs", str(tmp_path / "a")], capture_output=True, text=True, timeout=600, env=env)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1, r.stdout
@@ -546,3 +546,10 @@ def test_bench_reference_arm_prints_one_contract_line_also_when_started_plainly_
     for key in ("metric", "value", "unit", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data", "config", "cpu_baseline", "e2e"):
         assert key in d, key
     assert d["cpu_baseline"]["kind"] == "port" and d["e2e"]["h2d_bytes_per_step"] == 0 and d["value"] > 0
+    assert sorted(os.listdir(tmp_path / "a")) == ["pose.npy"]
+    pose = np.load(tmp_path / "a" / "pose.npy")
+    assert pose.shape == (16, 2, 6) and pose.dtype == np.float64 and np.all(np.isfinite(pose))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                        "--dump-outputs", str(tmp_path / "b")], capture_output=True, text=True, timeout=600, env=env)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert np.array_equal(np.load(tmp_path / "b" / "pose.npy"), pose)

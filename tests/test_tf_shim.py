@@ -199,21 +199,23 @@ def test_committed_fixture_is_what_the_reference_code_produces(key):
         np.testing.assert_array_equal(gold[key + "/" + name], a, err_msg=name)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference checkout not on this box")
 def test_reference_rejects_the_version_strings_the_parser_rejects():
-    """davo_b200.version raises the same exception type as the reference's graph code for unbuildable strings."""
-    from davo_b200 import synthetic as S
+    """davo_b200.version raises the same exception type as the reference's graph code for unbuildable strings: the
+    types stored in make_golden.REFERENCE_RAISES (which the generator checks against the reference), and, where the
+    checkout exists, a fresh run of the reference."""
     from davo_b200 import version as V
+    for ver, exc in G.REFERENCE_RAISES.items():
+        with pytest.raises(Exception) as ours:
+            V.parse_version(ver)
+        assert type(ours.value).__name__ == exc, (ver, ours.value)
+    if not HAVE_REF:
+        return
     img, flow, seg, depth = G.golden_inputs()
     with G.reference_on_path():
         for ver, exc in G.REFERENCE_RAISES.items():
-            with pytest.raises(Exception) as ours:
-                V.parse_version(ver)
-            assert type(ours.value).__name__ == exc, (ver, ours.value)
             with pytest.raises(Exception) as theirs:
                 G.run_reference(ver, img[:1, :32, :96 * 3], flow[:1, :, :32, :96], seg[:1, :, :32, :96], depth[:1, :, :32, :96], {})
             assert type(theirs.value).__name__ == exc, (ver, theirs.value)
-    del S
 
 
 @pytest.mark.skipif(not HAVE_REF, reason="reference checkout not on this box")

@@ -1,5 +1,5 @@
 import os, sys, time
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from davo_b200 import synthetic as S
 from davo_b200.davo import DAVO
