@@ -23,6 +23,7 @@ SYMBOLS = (
     "davo_compose_trajectory", "davo_kitti_errors", "davo_decode_jpeg_batch",
     "davo_forward_host_pairs_async", "davo_forward_host_compact_async", "davo_host_wait",
     "davo_comm_unique_id", "davo_comm_create", "davo_comm_world", "davo_allgather_poses",
+    "davo_forward_sequence", "davo_forward_sequence_host",
     "davo_last_error",
     "davo_destroy", "davo_build_info", "davo_config_bytes",
 )
@@ -80,6 +81,8 @@ def load() -> C.CDLL:
     lib.davo_forward_host_pairs_async.argtypes = [vp, ip, ip, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_longlong)]
     lib.davo_forward_host_compact_async.argtypes = [vp, ip, ip, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_longlong)]
     lib.davo_host_wait.argtypes = [vp, C.c_longlong]
+    lib.davo_forward_sequence.argtypes = [vp, ip, ip, vp, vp, vp, vp, vp, vp, vp]
+    lib.davo_forward_sequence_host.argtypes = [vp, ip, ip, vp, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_longlong)]
     lib.davo_get_intermediate.argtypes = [vp, C.c_char_p, ip, vp, C.c_int64, C.POINTER(C.c_int64)]
     lib.davo_last_launch_count.argtypes = [vp]
     lib.davo_last_host_copy_bytes.argtypes = [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
@@ -101,7 +104,7 @@ def load() -> C.CDLL:
     if lib.davo_config_bytes() != C.sizeof(DavoConfigC):
         raise ImportError("%s: davo_config is %d bytes in the library, %d in this binding (rebuild: python davo_b200/build.py --force)"
                           % (path, lib.davo_config_bytes(), C.sizeof(DavoConfigC)))
-    for s in SYMBOLS[:27]:
+    for s in SYMBOLS[:SYMBOLS.index("davo_last_error")]:
         getattr(lib, s).restype = ip
     _LIB = lib
     return lib

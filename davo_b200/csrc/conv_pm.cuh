@@ -248,9 +248,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       uint8_t* raw = raw0 + (c & 1) * fg.raw_bytes;
       const uint32_t raw_u = smem_u32(raw);
       const int b = s.b, k = s.k, y0 = s.y0, X0 = s.X0;
-      const uint8_t* img_b = f.img + (size_t)b * f.H * 3 * f.W * 3;
-      const size_t seg_src = ((size_t)b * 3 + (k == 0 ? 0 : 2)) * hw, seg_tgt = ((size_t)b * 3 + 1) * hw;
-      const int src_col0 = (k == 0) ? 0 : 2 * f.W;
+      const size_t seg_src = frame_plane(f.in, b, k == 0 ? 0 : 2, hw), seg_tgt = frame_plane(f.in, b, 1, hw);
       if ((c & 1) == 0 && ptid < 2 * kNumClasses) {               // the tile's class weights
         const bool se = f.att_src == 1 || f.att_src >= 3;
         const int fr = ptid / kNumClasses, cl = ptid - fr * kNumClasses;
@@ -258,11 +256,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             (se && (fr == 0 || !f.att_tgt_ones)) ? __ldcg(f.att_w + ((size_t)s.n * kAttFrames + fr) * kAttStride + cl)
             : f.att_src == 2 ? f.static_w[cl] : 1.0f;
       }
-      const bool flow_plain = use_flow && !f.flow_f16 && b >= f.n_flow16;       // float32 flow used as it is
+      const bool flow_plain = use_flow && !f.flow_f16 && b >= f.in.n_flow16;    // float32 flow used as it is
       if (flow_plain) {
         const int RF = kFusedThreads / NF, r0 = ptid / NF, e = ptid - r0 * NF, x = X0 + 2 * e;      // two pixels of flow
         if (r0 < RF && x >= 0 && x < f.W) {
-          const float* fsrc = f.flow + (((size_t)b * 4 + k) * hw + x) * 2;
+          const float* fsrc = flow_plane(f.in, b, k) + (size_t)x * 2;
           for (int rr = r0; rr < Hp; rr += RF) {
             const int y = y0 + 2 * rr;
             if (y >= 0 && y < f.H) cp_async_16(raw_u + (rr * NFP + e) * 16, fsrc + (size_t)y * f.W * 2);
@@ -275,11 +273,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int x = X0 + (wd / 3) * 4;                                 // the quad the word belongs to
         if (r0 < RI && x >= 0 && x < f.W) {
           // (16-byte copies of the aligned middle of a row were tried: slower than word copies, 0.371 against 0.348 ms)
-          const uint8_t* isrc = img_b + ((size_t)(fr ? src_col0 : f.W) + X0) * 3 + wd * 4;
+          const uint8_t* isrc = frame_img(f.in, b, fr ? (k == 0 ? 0 : 2) : 1) + (size_t)X0 * 3 + wd * 4;
           const uint32_t dst0 = raw_u + (fr ? fg.off_src : fg.off_tgt) + wd * 4;
           for (int rr = r0; rr < Hp; rr += RI) {
             const int y = y0 + 2 * rr;
-            if (y >= 0 && y < f.H) cp_async_4(dst0 + rr * NT * 4, isrc + (size_t)y * 3 * f.W * 3);
+            if (y >= 0 && y < f.H) cp_async_4(dst0 + rr * NT * 4, isrc + (size_t)y * f.in.img_row);
           }
         }
       }
@@ -307,24 +305,24 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (r0 < RL && x >= 0 && x < f.W) {
           const size_t plane = (fr ? seg_tgt : seg_src) + x;
           const int dst0 = (fr ? fg.off_lab_t : fg.off_lab_s) + qd * 4;
-          if (f.seg8) {
+          if (f.in.seg8) {
             for (int rr = r0; rr < Hp; rr += RL) {
               const int y = y0 + 2 * rr;
-              if (y >= 0 && y < f.H) cp_async_4(raw_u + dst0 + rr * NL * 4, f.seg8 + plane + (size_t)y * f.W);
+              if (y >= 0 && y < f.H) cp_async_4(raw_u + dst0 + rr * NL * 4, f.in.seg8 + plane + (size_t)y * f.W);
             }
           } else {
 #pragma unroll
             for (int u = 0; u < kLabRegs; ++u) {                         // the loads only: their values are first used in stage_finish
               const int rr = r0 + u * RL, y = y0 + 2 * rr;
               if (rr < Hp && y >= 0 && y < f.H) {
-                lab_v[u] = __ldg(reinterpret_cast<const float4*>(f.seg + plane + (size_t)y * f.W));
+                lab_v[u] = __ldg(reinterpret_cast<const float4*>(f.in.seg + plane + (size_t)y * f.W));
                 lab_mask |= 1u << u;
               }
             }
             for (int rr = r0 + kLabRegs * RL; rr < Hp; rr += RL) {        // more rows than registers (target labels too): on the spot
               const int y = y0 + 2 * rr;
               if (y >= 0 && y < f.H)
-                *reinterpret_cast<uint32_t*>(raw + dst0 + rr * NL * 4) = narrow4(__ldg(reinterpret_cast<const float4*>(f.seg + plane + (size_t)y * f.W)));
+                *reinterpret_cast<uint32_t*>(raw + dst0 + rr * NL * 4) = narrow4(__ldg(reinterpret_cast<const float4*>(f.in.seg + plane + (size_t)y * f.W)));
             }
           }
         }

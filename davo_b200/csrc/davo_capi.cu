@@ -239,15 +239,9 @@ struct davo_ctx {
   float *d_bn_mean = nullptr, *d_bn_rstd = nullptr;
   void* d_traj_scratch = nullptr;         // davo_compose_trajectory / davo_kitti_errors: relative motions, distances, segments
   size_t traj_scratch_bytes = 0;
-  const uint16_t* cur_flow16 = nullptr;   // binary16 flow of the chunk being enqueued (NULL: float flow) ...
-  int cur_n16 = 0;                        // ... for its first cur_n16 samples; the rest of the chunk crosses as float32
-  const uint16_t* last_flow16 = nullptr;
-  int last_n16 = 0;
   float flow16_frac = 0.75f;              // share of a chunk's samples converted on the CPU (the rest keeps the copy engine busy)
   HostPool* pool = nullptr;
   bool host_seg8 = true;
-  const uint8_t* cur_seg8 = nullptr; // byte labels of the chunk being enqueued (NULL: float labels)
-  const uint8_t* last_seg8 = nullptr;
   int s_chunk = 0;                  // samples per staging buffer
   cudaStream_t copy_stream = nullptr;
   cudaEvent_t ev_copied[kStage] = {}, ev_consumed[kStage] = {}, ev_start = nullptr;
@@ -258,9 +252,13 @@ struct davo_ctx {
   // last forward
   int last_launches = 0;
   int last_npairs_mb = 0;
-  const uint8_t* last_img = nullptr; const float* last_flow = nullptr; const float* last_seg = nullptr;
+  InputView last_in{};              // inputs of the last forward's last micro-batch (davo_profile_layers runs on them)
   float* last_pose = nullptr; int last_B = 0; int last_pairs = 0;
-  const float* cur_depth = nullptr; // depth planes of the batch (chunk) being enqueued; se_depth sources only
+  // davo_forward_sequence_host: the frames of a call (images, labels, depth) staged at their final place, so that a
+  // frame shared by two chunks crosses PCIe once; two sets, so that a call's copies can run under the previous call
+  uint8_t* q_img[2] = {}; uint8_t* q_seg8[2] = {}; float *q_seg[2] = {}, *q_depth[2] = {};
+  cudaEvent_t ev_q_done[2] = {};    // the call that last used set i has finished reading it
+  long long q_calls = 0;
   // Function attributes are per device: what this context has already raised, by kernel.
   std::map<const void*, int> smem_attr;
   std::map<std::pair<const void*, int>, int> max_clusters;   // by (kernel, dynamic shared memory)
@@ -1078,8 +1076,7 @@ int pack8_blocks(int npairs) {
   return npairs >= 64 ? kPack8Blocks / 4 : kPack8Blocks;
 }
 
-int launch_front(davo_ctx* ctx, int pair_mode, int pair0, int npairs, const uint8_t* img, const float* flow,
-                 const float* seg, cudaStream_t st, int* launches) {
+int launch_front(davo_ctx* ctx, int pair_mode, int pair0, int npairs, const InputView& in, cudaStream_t st, int* launches) {
   const davo_config& c = ctx->cfg;
   FrontParams fp;
   memset(&fp, 0, sizeof fp);
@@ -1090,10 +1087,7 @@ int launch_front(davo_ctx* ctx, int pair_mode, int pair0, int npairs, const uint
   fp.mask_rgb = c.mask_mode != 0;
   fp.mask_flow = c.mask_mode == 2;
   fp.se_act = c.se_act; fp.flow_abs = c.flow_abs; fp.flow_norm = c.flow_norm;
-  fp.img = img; fp.flow = flow; fp.seg = seg; fp.depth = ctx->cur_depth; fp.depth_norm = c.depth_norm;
-  fp.seg8 = seg ? nullptr : ctx->cur_seg8;       // the host entry point passes seg = NULL with byte labels
-  fp.flow16 = reinterpret_cast<const __half*>(ctx->cur_flow16);   // host entry point: the first cur_n16 samples of the chunk
-  fp.n_flow16 = ctx->cur_flow16 ? ctx->cur_n16 : 0;
+  fp.in = in; fp.depth_norm = c.depth_norm;
   fp.flow_f16 = c.flow_f16;
   fp.se_w = ctx->d_sew; fp.static_w = ctx->d_staticw;
   fp.pool_part = ctx->d_pool; fp.pool_count = ctx->d_poolcnt; fp.att_w = ctx->d_attw; fp.packed = ctx->d_packed;
@@ -1173,9 +1167,9 @@ Layer& pick_layer(davo_ctx* ctx, size_t li, int npairs) {
   return B;
 }
 
-int run_microbatch(davo_ctx* ctx, int pair_mode, int pair0, int npairs, const uint8_t* img, const float* flow,
-                   const float* seg, float* pose_out, cudaStream_t st, int* launches) {
-  if (int rc = launch_front(ctx, pair_mode, pair0, npairs, img, flow, seg, st, launches)) return rc;
+int run_microbatch(davo_ctx* ctx, int pair_mode, int pair0, int npairs, const InputView& in, float* pose_out,
+                   cudaStream_t st, int* launches) {
+  if (int rc = launch_front(ctx, pair_mode, pair0, npairs, in, st, launches)) return rc;
   for (size_t li = 0; li < ctx->layers.size(); ++li) {
     Layer& L = pick_layer(ctx, li, npairs);
     const int pse = ctx->cfg.posenn_se;
@@ -1367,6 +1361,13 @@ extern "C" void davo_destroy(davo_ctx* ctx) {
     if (ctx->ev_seg8[i]) cudaEventDestroy(ctx->ev_seg8[i]);
     if (ctx->ev_copied[i]) cudaEventDestroy(ctx->ev_copied[i]);
     if (ctx->ev_consumed[i]) cudaEventDestroy(ctx->ev_consumed[i]);
+  }
+  for (int i = 0; i < 2; ++i) {
+    if (ctx->q_img[i]) cudaFree(ctx->q_img[i]);
+    if (ctx->q_seg8[i]) cudaFree(ctx->q_seg8[i]);
+    if (ctx->q_seg[i]) cudaFree(ctx->q_seg[i]);
+    if (ctx->q_depth[i]) cudaFree(ctx->q_depth[i]);
+    if (ctx->ev_q_done[i]) cudaEventDestroy(ctx->ev_q_done[i]);
   }
   delete ctx->pool;
   if (ctx->comm) davo_comm::api().CommDestroy(ctx->comm);
@@ -1744,43 +1745,108 @@ extern "C" int davo_forward(davo_ctx* ctx, int B, const uint8_t* img, const floa
   return davo_forward_pairs(ctx, B, DAVO_PAIRS_ALL, img, flow, seg, depth, pose_out, stream);
 }
 
+// The passes of a device-buffer forward of B samples, on either input layout.  `who` names the entry point in errors.
+static int forward_device(davo_ctx* ctx, const char* who, int B, int pairs, const InputView& in, float* pose_out, void* stream) {
+  CU_OK(cudaSetDevice(ctx->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (ctx->cfg.batch_norm && !ctx->unit_sample && pairs != DAVO_PAIRS_ALL)
+    return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm normalises with the statistics of a whole PoseNN call: every pair must be computed (DAVO_PAIRS_ALL)", who);
+  if (ctx->unit_sample) pairs = kUnitsAreSamples;        // both poses come out of one evaluation
+  int launches = 0;
+  const int total = pairs_selected(pairs, B);
+  if (ctx->cfg.batch_norm && total > ctx->mb)
+    return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm needs the whole batch in one pass (%d units > micro_batch %d)", who, total, ctx->mb);
+  int last_n = 0;
+  if (pairs == DAVO_PAIRS_TRAJECTORY || pairs == DAVO_PAIRS_TRAJECTORY_FIRST)
+    CU_OK(cudaMemsetAsync(pose_out, 0, (size_t)B * 12 * sizeof(float), st));
+  for (int p0 = 0; p0 < total; p0 += ctx->mb) {
+    const int n = (total - p0) < ctx->mb ? (total - p0) : ctx->mb;
+    if (int rc = run_microbatch(ctx, pairs, p0, n, in, pose_out, st, &launches)) return rc;
+    last_n = n;
+  }
+  ctx->last_launches = launches;
+  ctx->last_npairs_mb = last_n;
+  ctx->last_in = in; ctx->last_pose = pose_out; ctx->last_B = B;
+  ctx->last_pairs = pairs;
+  return 0;
+}
+
 extern "C" int davo_forward_pairs(davo_ctx* ctx, int B, int pairs, const uint8_t* img, const float* flow,
                                   const float* seg, const float* depth, float* pose_out, void* stream) {
   if (!ctx) return DAVO_ERR_ARG;
   if (pairs < DAVO_PAIRS_ALL || pairs > DAVO_PAIRS_TRAJECTORY_FIRST)
     return fail(ctx, DAVO_ERR_ARG, "davo_forward: pair selection %d unknown", pairs);
   if ((ctx->cfg.att_src == 5 || ctx->cfg.depth_split) && !depth) return fail(ctx, DAVO_ERR_ARG, "davo_forward: this variant reads input_depth; got NULL");
-  ctx->cur_depth = depth;
-  ctx->cur_seg8 = nullptr;
-  ctx->cur_flow16 = nullptr; ctx->cur_n16 = 0;
   if (!ctx->finalized) return fail(ctx, DAVO_ERR_STATE, "davo_forward: weights not finalized");
   if (B <= 0 || B > ctx->cfg.max_batch) return fail(ctx, DAVO_ERR_ARG, "davo_forward: B=%d outside 1..%d", B, ctx->cfg.max_batch);
   if (!img || !pose_out || (ctx->cfg.att_src != 0 && !seg) || ((ctx->cfg.in_mode == 1 || ctx->cfg.att_src == 1 || ctx->cfg.att_src == 6 || ctx->cfg.pixel_map == 2) && !flow))
     return fail(ctx, DAVO_ERR_ARG, "davo_forward: null input buffer");
-  CU_OK(cudaSetDevice(ctx->device));
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (ctx->cfg.batch_norm && !ctx->unit_sample && pairs != DAVO_PAIRS_ALL)
-    return fail(ctx, DAVO_ERR_ARG, "davo_forward: -batch_norm normalises with the statistics of a whole PoseNN call: every pair must be computed (DAVO_PAIRS_ALL)");
-  if (ctx->unit_sample) pairs = kUnitsAreSamples;        // both poses come out of one evaluation
-  int launches = 0;
-  const int total = pairs_selected(pairs, B);
-  if (ctx->cfg.batch_norm && total > ctx->mb)
-    return fail(ctx, DAVO_ERR_ARG, "davo_forward: -batch_norm needs the whole batch in one pass (%d units > micro_batch %d)", total, ctx->mb);
-  int last_n = 0;
-  if (pairs == DAVO_PAIRS_TRAJECTORY || pairs == DAVO_PAIRS_TRAJECTORY_FIRST)
-    CU_OK(cudaMemsetAsync(pose_out, 0, (size_t)B * 12 * sizeof(float), st));
-  for (int p0 = 0; p0 < total; p0 += ctx->mb) {
-    const int n = (total - p0) < ctx->mb ? (total - p0) : ctx->mb;
-    if (int rc = run_microbatch(ctx, pairs, p0, n, img, flow, seg, pose_out, st, &launches)) return rc;
-    last_n = n;
+  return forward_device(ctx, "davo_forward", B, pairs, triplet_view(ctx->cfg.H, ctx->cfg.W, img, flow, seg, nullptr, depth, nullptr, 0),
+                        pose_out, stream);
+}
+
+namespace {
+
+// What a sequence call of n frames reads (include/davo_b200.h: davo_forward_sequence).  Sample s computes the pair
+// tgt -> src1 always and tgt -> src0 when k0(s); a frame is read as the target of sample f - 1, as src1 of f - 2 and as
+// src0 of f.
+struct SeqReads {
+  bool flow = false, labels = false, tgt_labels = false, depth = false;
+  int pairs = 0;                  // the selection as the passes run it (kUnitsAreSamples for the non-shared nets)
+  bool k0(int s) const { return pairs == DAVO_PAIRS_ALL || pairs == kUnitsAreSamples || (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && s == 0); }
+  bool fwd(int s) const { return flow && k0(s); }                              // flow_fwd[s]
+  bool img(int f, int n) const {                                               // image (and depth) of frame f
+    return (f >= 1 && f - 1 < n - 2) || (f >= 2) || (f < n - 2 && k0(f));
   }
-  ctx->last_launches = launches;
-  ctx->last_npairs_mb = last_n;
-  ctx->last_img = img; ctx->last_flow = flow; ctx->last_seg = seg; ctx->last_pose = pose_out; ctx->last_B = B;
-  ctx->last_seg8 = nullptr;
-  ctx->last_flow16 = nullptr; ctx->last_n16 = 0;
-  ctx->last_pairs = pairs;
+  bool lab(int f, int n) const {
+    if (!labels) return false;
+    return f >= 2 || (f < n - 2 && k0(f)) || (tgt_labels && f >= 1 && f - 1 < n - 2);
+  }
+};
+SeqReads seq_reads(const davo_ctx* ctx, int pairs) {
+  const davo_config& c = ctx->cfg;
+  SeqReads r;
+  r.pairs = ctx->unit_sample ? kUnitsAreSamples : pairs;
+  r.flow = c.in_mode == 1 || c.att_src == 1 || c.att_src == 6 || c.pixel_map == 2;
+  r.labels = c.att_src != 0 && (!c.pixel_map || c.att_src == 6);     // the per-pixel rgb / depth sources gather no class weight
+  r.tgt_labels = r.labels && !c.att_tgt_ones;
+  r.depth = c.att_src == 5 || c.depth_split;
+  return r;
+}
+
+// Argument checks shared by the two sequence entry points.
+int check_sequence(davo_ctx* ctx, const char* who, int n_frames, int pairs, const void* img, const void* flow_fwd,
+                   const void* flow_bwd, const void* seg, const void* depth, const void* pose_out) {
+  if (pairs < DAVO_PAIRS_ALL || pairs > DAVO_PAIRS_TRAJECTORY_FIRST) return fail(ctx, DAVO_ERR_ARG, "%s: pair selection %d unknown", who, pairs);
+  if (!ctx->finalized) return fail(ctx, DAVO_ERR_STATE, "%s: weights not finalized", who);
+  if (n_frames < 3) return fail(ctx, DAVO_ERR_ARG, "%s: n_frames=%d: a sample needs 3 frames", who, n_frames);
+  if (n_frames - 2 > ctx->cfg.max_batch)
+    return fail(ctx, DAVO_ERR_ARG, "%s: n_frames=%d is %d samples, more than max_batch %d", who, n_frames, n_frames - 2, ctx->cfg.max_batch);
+  const SeqReads r = seq_reads(ctx, pairs);
+  const davo_config& c = ctx->cfg;
+  struct { const void* p; bool needed; const char* name; } in[] = {
+      {img, true, "img"}, {pose_out, true, "pose_out"}, {seg, c.att_src != 0, "seg"}, {depth, r.depth, "depth"},
+      {flow_bwd, r.flow, "flow_bwd"}, {flow_fwd, r.flow && r.k0(0), "flow_fwd"}};
+  for (const auto& x : in) {
+    if (x.needed && !x.p) return fail(ctx, DAVO_ERR_ARG, "%s: %s is NULL; this variant and pair selection read it", who, x.name);
+    if (x.p && (reinterpret_cast<uintptr_t>(x.p) & 15)) return fail(ctx, DAVO_ERR_ARG, "%s: %s is not 16-byte aligned", who, x.name);
+  }
   return 0;
+}
+
+}  // namespace
+
+extern "C" int davo_forward_sequence(davo_ctx* ctx, int n_frames, int pairs, const uint8_t* img, const float* flow_fwd,
+                                     const float* flow_bwd, const float* seg, const float* depth, float* pose_out, void* stream) {
+  if (!ctx) return DAVO_ERR_ARG;
+  if (int rc = check_sequence(ctx, "davo_forward_sequence", n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
+  const davo_config& c = ctx->cfg;
+  const size_t hw = (size_t)c.H * c.W;
+  // plane 1 of sample s is flow_bwd[s + 1]; a flow_fwd nobody reads stands in as flow_bwd, so that a front end re-run
+  // over every pair (davo_profile_layers) still reads mapped memory
+  const float* bwd1 = flow_bwd ? flow_bwd + 2 * hw : nullptr;
+  const InputView in = sequence_view(c.H, c.W, img, flow_fwd ? flow_fwd : flow_bwd, bwd1, seg, nullptr, depth, nullptr, nullptr, 0);
+  return forward_device(ctx, "davo_forward_sequence", n_frames - 2, pairs, in, pose_out, stream);
 }
 
 // Host-buffer entry point: the batch is cut into micro-batch chunks; chunk i+1 is copied
@@ -1847,6 +1913,133 @@ extern "C" int davo_forward_host_compact_async(davo_ctx* ctx, int B, int pairs, 
                            depth, pose_out, stream, uses_flow ? flow_f16 : nullptr, c.att_src != 0 ? seg_u8 : nullptr, ticket);
 }
 
+namespace {
+
+// Staging of the host entry points: kStage chunk slots of `cs` samples, pinned buffers for the CPU narrowing, the
+// private copy stream.  Allocated by the first host call; returns the chunk size, or an error code (< 0).
+int host_setup(davo_ctx* ctx, const char* who) {
+  const davo_config& c = ctx->cfg;
+  const size_t hw = (size_t)c.H * c.W;
+  const size_t n_img = hw * 9, n_flow = hw * 8, n_seg = hw * 3;   // elements per sample
+  const bool uses_flow = (c.in_mode == 1 || c.att_src == 1 || c.att_src == 6 || c.pixel_map == 2);
+  // Host inputs arrive over PCIe more slowly than the stack computes, so what matters is how soon
+  // compute can start behind the copy: chunks of 16 samples (8 chunks per 128-sample batch).
+  const int ups = ctx->unit_sample ? 1 : 2;                        // units of a pass per sample
+  int cs = std::max(1, std::min(ctx->mb / ups, 16));               // samples per chunk
+  if (const char* e = getenv("DAVO_B200_HOST_CHUNK"))              // experiment knob
+    cs = std::max(1, std::min(atoi(e), std::max(1, ctx->mb / ups)));
+  if (ctx->s_img[0] && ctx->s_chunk != cs) return fail(ctx, DAVO_ERR_STATE, "%s: chunk size changed", who);
+  if (ctx->s_img[0]) return cs;
+  ctx->s_chunk = cs;
+  // A slot also holds a sequence chunk: its cs + 2 frames, cs flow_fwd and cs flow_bwd entries take less room than cs
+  // triplets (davo_forward_sequence_host).
+  for (int i = 0; i < davo_ctx::kStage; ++i) {
+    CU_OK(cudaMalloc((void**)&ctx->s_img[i], n_img * cs));
+    CU_OK(cudaMalloc((void**)&ctx->s_flow[i], n_flow * 4 * cs));
+    CU_OK(cudaMalloc((void**)&ctx->s_seg[i], n_seg * 4 * cs));
+    CU_OK(cudaMemset(ctx->s_flow[i], 0, n_flow * 4 * cs));
+    CU_OK(cudaMemset(ctx->s_seg[i], 0, n_seg * 4 * cs));
+    if (c.att_src == 5 || c.depth_split) CU_OK(cudaMalloc((void**)&ctx->s_depth[i], n_seg * 4 * cs));
+    if (c.att_src != 0) {
+      CU_OK(cudaMalloc((void**)&ctx->s_seg8[i], n_seg * cs));
+      if (ctx->host_seg8) CU_OK(cudaHostAlloc((void**)&ctx->h_seg8[i], n_seg * cs, cudaHostAllocDefault));
+    }
+    if (uses_flow) {
+      CU_OK(cudaMalloc((void**)&ctx->s_flow16[i], n_flow / 2 * sizeof(uint16_t) * cs));
+      if (ctx->host_flow16) CU_OK(cudaHostAlloc((void**)&ctx->h_flow16[i], n_flow / 2 * sizeof(uint16_t) * cs, cudaHostAllocDefault));
+    }
+    CU_OK(cudaEventCreateWithFlags(&ctx->ev_seg8[i], cudaEventDisableTiming));
+    CU_OK(cudaEventCreateWithFlags(&ctx->ev_copied[i], cudaEventDisableTiming));
+    CU_OK(cudaEventCreateWithFlags(&ctx->ev_consumed[i], cudaEventDisableTiming));
+  }
+  CU_OK(cudaMalloc((void**)&ctx->s_pose, (size_t)12 * 4 * c.max_batch));
+  if ((ctx->host_seg8 && c.att_src != 0) || (ctx->host_flow16 && uses_flow)) {
+    // conversion threads: the host's hardware threads shared among the ranks of the box (torchrun sets
+    // LOCAL_WORLD_SIZE), at most 16: one thread streams ~9 GB/s and a chunk is ~30 MB of traffic
+    int ranks_here = 1;
+    if (const char* e = getenv("LOCAL_WORLD_SIZE")) ranks_here = std::max(1, atoi(e));
+    int nthreads = std::max(2, std::min(16, (int)std::thread::hardware_concurrency() / ranks_here));
+    if (const char* e = getenv("DAVO_B200_HOST_THREADS")) nthreads = std::max(1, std::min(atoi(e), 32));
+    // Narrowing the flow only pays when this process has the host's cores and memory system to
+    // itself: with 16 threads it is +10 % on one GPU; with the 4 threads per rank of an 8-GPU box
+    // (32 host threads) it costs 35 % (profiles/r1_e2e_n8_flow_transport.log), and ranks that share
+    // a host share its memory bandwidth too, which the conversion doubles.  So: a single rank with
+    // >= 16 threads, unless an explicit fraction says otherwise.
+    if ((nthreads < 16 || ranks_here > 1) && !getenv("DAVO_B200_HOST_FLOW16_FRAC")) ctx->flow16_frac = 0.0f;
+    ctx->pool = new HostPool(nthreads - 1);
+  }
+  CU_OK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+  CU_OK(cudaEventCreateWithFlags(&ctx->ev_start, cudaEventDisableTiming));
+  return cs;
+}
+
+// The copy stream must not run ahead of work already queued on the caller's stream.  (Staging buffers are protected
+// by their own events, so consecutive calls may overlap: the copies of call k+1 run under the compute of call k.  Only
+// the first use of the copy stream is ordered behind the caller's stream.)
+int host_order_first_call(davo_ctx* ctx, cudaStream_t st) {
+  if (ctx->host_calls++ == 0) {
+    CU_OK(cudaEventRecord(ctx->ev_start, st));
+    CU_OK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_start, 0));
+  }
+  return 0;
+}
+
+// One piece of CPU narrowing: n float32 flow values -> binary16, or n float labels -> bytes.
+struct NarrowJob { const float* src; void* dst; size_t n; bool flow; };
+
+// Runs the jobs on the handle's thread pool (flow jobs first); returns false when some flow value has no finite half.
+bool host_narrow(davo_ctx* ctx, const std::vector<NarrowJob>& jobs) {
+  std::atomic<int> flow_bad{0};
+  ctx->pool->run([&](int part, int parts) {
+    // Work units are pieces of a plane: `sub` pieces per plane so that every thread gets a few
+    // long contiguous streams (a label plane costs half a flow plane: 4 bytes read per pixel vs 8).
+    const size_t sub = jobs.size() >= (size_t)4 * parts ? 1 : (size_t)parts;
+    const size_t units = jobs.size() * sub;
+    for (size_t u = part; u < units; u += parts) {
+      const NarrowJob& jb = jobs[u / sub];
+      const size_t piece = u % sub, n = jb.n;
+      const size_t beg = (n * piece / sub) & ~(size_t)15, end = piece + 1 == sub ? n : ((n * (piece + 1) / sub) & ~(size_t)15);
+      if (jb.flow) {
+        if (!davo_host::flows_to_half(jb.src + beg, static_cast<uint16_t*>(jb.dst) + beg, end - beg))
+          flow_bad.store(1, std::memory_order_relaxed);
+      } else {
+        davo_host::labels_to_bytes(jb.src + beg, static_cast<uint8_t*>(jb.dst) + beg, end - beg);
+      }
+    }
+  });
+  return flow_bad.load() == 0;
+}
+
+// Poses of a host call back to the caller's memory; blocking, or the asynchronous form's ticket.
+int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket) {
+  CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
+  if (ticket) {
+    const long long t = ++ctx->host_tickets;
+    cudaEvent_t& ev = ctx->ev_host_done[t % davo_ctx::kTickets];
+    if (!ev) CU_OK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    CU_OK(cudaEventRecord(ev, st));
+    *ticket = t;
+  } else {
+    CU_OK(cudaStreamSynchronize(st));
+  }
+  ctx->last_d2h = (long long)12 * 4 * B;
+  return 0;
+}
+
+// The passes of one chunk: `chunk_pairs` over its `ns` samples, poses to s_pose from sample s0 on.
+int host_run_chunk(davo_ctx* ctx, int chunk_pairs, int s0, int ns, const InputView& in, cudaStream_t st, int* launches,
+                   int* last_n) {
+  const int np_chunk = pairs_selected(chunk_pairs, ns);
+  const bool copy_only = getenv("DAVO_B200_HOST_COPY_ONLY") != nullptr;   // measurement: the copies alone (bench.py e2e.copy_only)
+  for (int q0 = 0; q0 < np_chunk && !copy_only; q0 += ctx->mb)
+    if (int rc = run_microbatch(ctx, chunk_pairs, q0, std::min(ctx->mb, np_chunk - q0), in, ctx->s_pose + (size_t)12 * s0, st, launches))
+      return rc;
+  *last_n = np_chunk;
+  return 0;
+}
+
+}  // namespace
+
 static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img, const float* flow,
                              const float* seg, const float* depth, float* pose_out, void* stream,
                              const uint16_t* flow16_in, const uint8_t* seg8_in, long long* ticket) {
@@ -1865,62 +2058,11 @@ static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img
   const size_t hw = (size_t)c.H * c.W;
   const size_t n_img = hw * 9, n_flow = hw * 8, n_seg = hw * 3;   // elements per sample
   const bool uses_flow = (c.in_mode == 1 || c.att_src == 1 || c.att_src == 6 || c.pixel_map == 2);
-  // Host inputs arrive over PCIe more slowly than the stack computes, so what matters is how soon
-  // compute can start behind the copy: chunks of 16 samples (8 chunks per 128-sample batch).
-  const int ups = ctx->unit_sample ? 1 : 2;                        // units of a pass per sample
-  int cs = std::max(1, std::min(ctx->mb / ups, 16));               // samples per chunk
-  if (const char* e = getenv("DAVO_B200_HOST_CHUNK"))              // experiment knob
-    cs = std::max(1, std::min(atoi(e), std::max(1, ctx->mb / ups)));
-  if (ctx->s_img[0] && ctx->s_chunk != cs) return fail(ctx, DAVO_ERR_STATE, "davo_forward_host: chunk size changed");
-  if (!ctx->s_img[0]) {
-    ctx->s_chunk = cs;
-    for (int i = 0; i < davo_ctx::kStage; ++i) {
-      CU_OK(cudaMalloc((void**)&ctx->s_img[i], n_img * cs));
-      CU_OK(cudaMalloc((void**)&ctx->s_flow[i], n_flow * 4 * cs));
-      CU_OK(cudaMalloc((void**)&ctx->s_seg[i], n_seg * 4 * cs));
-      CU_OK(cudaMemset(ctx->s_flow[i], 0, n_flow * 4 * cs));
-      CU_OK(cudaMemset(ctx->s_seg[i], 0, n_seg * 4 * cs));
-      if (c.att_src == 5 || c.depth_split) CU_OK(cudaMalloc((void**)&ctx->s_depth[i], n_seg * 4 * cs));
-      if (c.att_src != 0) {
-        CU_OK(cudaMalloc((void**)&ctx->s_seg8[i], n_seg * cs));
-        if (ctx->host_seg8) CU_OK(cudaHostAlloc((void**)&ctx->h_seg8[i], n_seg * cs, cudaHostAllocDefault));
-      }
-      if (uses_flow) {
-        CU_OK(cudaMalloc((void**)&ctx->s_flow16[i], n_flow / 2 * sizeof(uint16_t) * cs));
-        if (ctx->host_flow16) CU_OK(cudaHostAlloc((void**)&ctx->h_flow16[i], n_flow / 2 * sizeof(uint16_t) * cs, cudaHostAllocDefault));
-      }
-      CU_OK(cudaEventCreateWithFlags(&ctx->ev_seg8[i], cudaEventDisableTiming));
-      CU_OK(cudaEventCreateWithFlags(&ctx->ev_copied[i], cudaEventDisableTiming));
-      CU_OK(cudaEventCreateWithFlags(&ctx->ev_consumed[i], cudaEventDisableTiming));
-    }
-    CU_OK(cudaMalloc((void**)&ctx->s_pose, (size_t)12 * 4 * c.max_batch));
-    if ((ctx->host_seg8 && c.att_src != 0) || (ctx->host_flow16 && uses_flow)) {
-      // conversion threads: the host's hardware threads shared among the ranks of the box (torchrun sets
-      // LOCAL_WORLD_SIZE), at most 16: one thread streams ~9 GB/s and a chunk is ~30 MB of traffic
-      int ranks_here = 1;
-      if (const char* e = getenv("LOCAL_WORLD_SIZE")) ranks_here = std::max(1, atoi(e));
-      int nthreads = std::max(2, std::min(16, (int)std::thread::hardware_concurrency() / ranks_here));
-      if (const char* e = getenv("DAVO_B200_HOST_THREADS")) nthreads = std::max(1, std::min(atoi(e), 32));
-      // Narrowing the flow only pays when this process has the host's cores and memory system to
-      // itself: with 16 threads it is +10 % on one GPU; with the 4 threads per rank of an 8-GPU box
-      // (32 host threads) it costs 35 % (profiles/r1_e2e_n8_flow_transport.log), and ranks that share
-      // a host share its memory bandwidth too, which the conversion doubles.  So: a single rank with
-      // >= 16 threads, unless an explicit fraction says otherwise.
-      if ((nthreads < 16 || ranks_here > 1) && !getenv("DAVO_B200_HOST_FLOW16_FRAC")) ctx->flow16_frac = 0.0f;
-      ctx->pool = new HostPool(nthreads - 1);
-    }
-    CU_OK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    CU_OK(cudaEventCreateWithFlags(&ctx->ev_start, cudaEventDisableTiming));
-  }
+  const int cs = host_setup(ctx, "davo_forward_host");
+  if (cs < 0) return cs;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   cudaStream_t cp = ctx->copy_stream;
-  // the copy stream must not run ahead of work already queued on the caller's stream
-  // (staging buffers are protected by their own events below, so consecutive calls may overlap: the copies of call
-  // k+1 run under the compute of call k.  Only the first use of the copy stream is ordered behind the caller's stream.)
-  if (ctx->host_calls++ == 0) {
-    CU_OK(cudaEventRecord(ctx->ev_start, st));
-    CU_OK(cudaStreamWaitEvent(cp, ctx->ev_start, 0));
-  }
+  if (int rc = host_order_first_call(ctx, st)) return rc;
   const bool need_flow = uses_flow;
   const bool need_seg = c.att_src != 0;
   const bool seg_tgt = need_seg && !c.att_tgt_ones;
@@ -1933,6 +2075,7 @@ static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img
   // pairs) are nearly balanced, so equal chunks are best: tapering the last ones (tried) only adds
   // passes that are too small to fill the GPU.
   int ns = 0, last_ns = 0;
+  InputView in{};
   for (int s0 = 0; s0 < B; s0 += ns, ++chunk) {
     ns = std::min(cs, B - s0);
     last_ns = ns;
@@ -1954,52 +2097,32 @@ static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img
     const bool conv_flow = n16 > 0;
     const int planes[3] = {0, 2, 1};
     const int npl = seg_tgt ? 3 : 2;
-    std::atomic<int> flow_bad{0};
+    bool flow_ok = true;
     if (conv_seg || conv_flow) {
       CU_OK(cudaEventSynchronize(ctx->ev_seg8[buf]));              // the pinned staging of this slot has been copied out (no-op before its first use)
-      const float* lsrc = conv_seg ? seg + n_seg * s0 : nullptr;
-      uint8_t* ldst = ctx->h_seg8[buf];
-      const float* fsrc = conv_flow ? flow + n_flow * s0 : nullptr;
-      uint16_t* fdst = ctx->h_flow16[buf];
-      const size_t ljobs = conv_seg ? (size_t)ns * npl : 0, fjobs = conv_flow ? (size_t)n16 * 2 : 0;
-      const size_t fl = hw * 2;                                  // floats per flow plane
-      ctx->pool->run([&](int part, int parts) {
-        // Work units are pieces of a plane: `sub` pieces per plane so that every thread gets a few
-        // long contiguous streams (a label plane costs half a flow plane: 4 bytes read per pixel vs 8).
-        const size_t sub = (fjobs + ljobs) >= (size_t)4 * parts ? 1 : (size_t)parts;
-        const size_t units = (fjobs + ljobs) * sub;
-        for (size_t u = part; u < units; u += parts) {
-          const size_t j = u / sub, piece = u % sub;
-          if (j < fjobs) {
-            const size_t beg = (fl * piece / sub) & ~(size_t)15, end = piece + 1 == sub ? fl : ((fl * (piece + 1) / sub) & ~(size_t)15);
-            if (!davo_host::flows_to_half(fsrc + (j / 2) * n_flow + (j % 2) * fl + beg, fdst + j * fl + beg, end - beg))
-              flow_bad.store(1, std::memory_order_relaxed);
-          } else {
-            const size_t jl = j - fjobs;
-            const size_t off = ((jl / npl) * 3 + planes[jl % npl]) * hw;
-            const size_t beg = (hw * piece / sub) & ~(size_t)15, end = piece + 1 == sub ? hw : ((hw * (piece + 1) / sub) & ~(size_t)15);
-            davo_host::labels_to_bytes(lsrc + off + beg, ldst + off + beg, end - beg);
-          }
-        }
-      });
+      std::vector<NarrowJob> jobs;
+      const size_t fl = hw * 2;                                    // floats per flow plane
+      for (int j = 0; conv_flow && j < 2 * n16; ++j)
+        jobs.push_back({flow + n_flow * s0 + (j / 2) * n_flow + (j % 2) * fl, ctx->h_flow16[buf] + j * fl, fl, true});
+      for (int jl = 0; conv_seg && jl < ns * npl; ++jl) {
+        const size_t off = ((size_t)(jl / npl) * 3 + planes[jl % npl]) * hw;
+        jobs.push_back({seg + n_seg * s0 + off, ctx->h_seg8[buf] + off, hw, false});
+      }
+      flow_ok = host_narrow(ctx, jobs);
     }
-    ctx->cur_flow16 = nullptr;
-    ctx->cur_n16 = 0;
-    if (conv_flow && flow_bad.load()) n16 = 0;                  // a value with no finite half: the whole chunk as float32
+    if (conv_flow && !flow_ok) n16 = 0;                            // a value with no finite half: the whole chunk as float32
     if (flow16_in && need_flow) n16 = ns;                         // the caller's binary16 planes, as they are
     if (n16 > 0) {
       CU_OK(cudaMemcpyAsync(ctx->s_flow16[buf], flow16_in ? flow16_in + hw * 4 * (size_t)s0 : ctx->h_flow16[buf],
                             hw * 4 * sizeof(uint16_t) * n16, cudaMemcpyHostToDevice, cp));
       h2d += hw * 4 * sizeof(uint16_t) * n16;
-      ctx->cur_flow16 = ctx->s_flow16[buf];
-      ctx->cur_n16 = n16;
     }
     if (need_flow && n16 < ns) {
       CU_OK(cudaMemcpy2DAsync(ctx->s_flow[buf] + n_flow * n16, n_flow * 4, flow + n_flow * (s0 + n16), n_flow * 4, n_flow * 2,
                               ns - n16, cudaMemcpyHostToDevice, cp));
       h2d += n_flow * 2 * (ns - n16);
     }
-    ctx->cur_seg8 = nullptr;
+    const uint8_t* seg8_dev = nullptr;
     if (conv_seg || (seg8_in && need_seg)) {
       const uint8_t* dst = seg8_in ? seg8_in + n_seg * (size_t)s0 : ctx->h_seg8[buf];
       if (seg_tgt) {
@@ -2010,7 +2133,7 @@ static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img
           CU_OK(cudaMemcpy2DAsync(ctx->s_seg8[buf] + hw * pl, n_seg, dst + hw * pl, n_seg, hw, ns, cudaMemcpyHostToDevice, cp));
         h2d += hw * 2 * ns;
       }
-      ctx->cur_seg8 = ctx->s_seg8[buf];
+      seg8_dev = ctx->s_seg8[buf];
     } else if (need_seg) {
       if (seg_tgt) {
         CU_OK(cudaMemcpyAsync(ctx->s_seg[buf], seg + n_seg * s0, n_seg * 4 * ns, cudaMemcpyHostToDevice, cp));
@@ -2026,43 +2149,178 @@ static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img
       CU_OK(cudaMemcpyAsync(ctx->s_depth[buf], depth + n_seg * s0, n_seg * 4 * ns, cudaMemcpyHostToDevice, cp));
       h2d += n_seg * 4 * ns;
     }
-    ctx->cur_depth = ctx->s_depth[buf];
     if (conv_seg || conv_flow) CU_OK(cudaEventRecord(ctx->ev_seg8[buf], cp));   // pinned staging of this slot has been read
     CU_OK(cudaEventRecord(ctx->ev_copied[buf], cp));
     CU_OK(cudaStreamWaitEvent(st, ctx->ev_copied[buf], 0));
+    in = triplet_view(c.H, c.W, ctx->s_img[buf], ctx->s_flow[buf], seg8_dev ? nullptr : ctx->s_seg[buf], seg8_dev,
+                      ctx->s_depth[buf], n16 > 0 ? ctx->s_flow16[buf] : nullptr, n16);
     // a chunk is a batch of its own: only the first one may hold the first sample's tgt->src0
     const int chunk_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && s0 > 0) ? DAVO_PAIRS_TRAJECTORY : pairs;
-    const int np_chunk = pairs_selected(chunk_pairs, ns);
-    const bool copy_only = getenv("DAVO_B200_HOST_COPY_ONLY") != nullptr;   // measurement: the copies alone (bench.py e2e.copy_only)
-    for (int q0 = 0; q0 < np_chunk && !copy_only; q0 += ctx->mb)
-      if (int rc = run_microbatch(ctx, chunk_pairs, q0, std::min(ctx->mb, np_chunk - q0), ctx->s_img[buf],
-                                  ctx->s_flow[buf], ctx->cur_seg8 ? nullptr : ctx->s_seg[buf],
-                                  ctx->s_pose + (size_t)12 * s0, st, &launches))
-        return rc;
+    if (int rc = host_run_chunk(ctx, chunk_pairs, s0, ns, in, st, &launches, &last_n)) return rc;
     CU_OK(cudaEventRecord(ctx->ev_consumed[buf], st));
-    last_n = np_chunk;
   }
-  CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
-  if (ticket) {
-    const long long t = ++ctx->host_tickets;
-    cudaEvent_t& ev = ctx->ev_host_done[t % davo_ctx::kTickets];
-    if (!ev) CU_OK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    CU_OK(cudaEventRecord(ev, st));
-    *ticket = t;
-  } else {
-    CU_OK(cudaStreamSynchronize(st));
-  }
+  if (int rc = host_finish(ctx, B, pose_out, st, ticket)) return rc;
   ctx->last_launches = launches;
   ctx->last_npairs_mb = last_n;
   ctx->last_h2d = (long long)h2d;
-  ctx->last_d2h = (long long)12 * 4 * B;
-  const int lastbuf = (chunk - 1) % davo_ctx::kStage;
-  ctx->last_img = ctx->s_img[lastbuf]; ctx->last_flow = ctx->s_flow[lastbuf];
-  ctx->last_flow16 = ctx->cur_flow16; ctx->last_n16 = ctx->cur_n16;
-  ctx->last_seg = ctx->cur_seg8 ? nullptr : ctx->s_seg[lastbuf]; ctx->last_seg8 = ctx->cur_seg8;
+  ctx->last_in = in;
   ctx->last_pose = ctx->s_pose; ctx->last_B = last_ns;
   ctx->last_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && chunk > 1) ? DAVO_PAIRS_TRAJECTORY : pairs;
   return 0;
+}
+
+// Host-buffer sequence entry point (include/davo_b200.h: davo_forward_sequence_host).  The samples are cut into the
+// chunks of the triplet entry point.  Flow entries belong to one sample each and go through the chunk slots like the
+// triplet flow planes.  Frames (images, labels, depth) are shared by up to three samples, so they are staged at their
+// final place in one of two per-call frame sets: a chunk copies the frames that the call reads and that no earlier
+// chunk copied, and the chunk's passes read the set through a sequence view.  Every copied frame or flow crosses PCIe
+// once; those that no computed pair reads are not copied.
+static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, const uint8_t* img, const float* flow_fwd,
+                                      const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                                      void* stream, long long* ticket) {
+  const char* who = ticket ? "davo_forward_sequence_host_async" : "davo_forward_sequence_host";
+  if (int rc = check_sequence(ctx, who, n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
+  if (ctx->cfg.batch_norm)
+    return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm needs the whole batch in one pass; the chunked host entry point does not take it (copy the frames to the device and call davo_forward_sequence)", who);
+  const davo_config& c = ctx->cfg;
+  CU_OK(cudaSetDevice(ctx->device));
+  const SeqReads r = seq_reads(ctx, pairs);
+  pairs = r.pairs;
+  const int B = n_frames - 2;
+  const size_t hw = (size_t)c.H * c.W, fl = hw * 2;               // pixels per frame, floats per flow entry
+  const int cs = host_setup(ctx, who);
+  if (cs < 0) return cs;
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  cudaStream_t cp = ctx->copy_stream;
+  if (int rc = host_order_first_call(ctx, st)) return rc;
+  const bool seg8 = r.labels && ctx->host_seg8;
+  const int set = (int)(ctx->q_calls++ & 1);
+  if (!ctx->q_img[set]) {
+    const size_t nf = (size_t)c.max_batch + 2;
+    CU_OK(cudaMalloc((void**)&ctx->q_img[set], nf * hw * 3));
+    if (c.att_src != 0 && ctx->host_seg8) CU_OK(cudaMalloc((void**)&ctx->q_seg8[set], nf * hw));
+    if (c.att_src != 0 && !ctx->host_seg8) CU_OK(cudaMalloc((void**)&ctx->q_seg[set], nf * hw * 4));
+    if (r.depth) CU_OK(cudaMalloc((void**)&ctx->q_depth[set], nf * hw * 4));
+    CU_OK(cudaEventCreateWithFlags(&ctx->ev_q_done[set], cudaEventDisableTiming));
+  } else {
+    CU_OK(cudaStreamWaitEvent(cp, ctx->ev_q_done[set], 0));         // the call before the previous one has read this set
+  }
+  size_t h2d = 0;
+  int launches = 0, last_n = 0, chunk = 0, ns = 0, last_ns = 0;
+  int staged = 0;                                                  // frames [0, staged) are on the device (or never read)
+  if (pairs == DAVO_PAIRS_TRAJECTORY || pairs == DAVO_PAIRS_TRAJECTORY_FIRST)
+    CU_OK(cudaMemsetAsync(ctx->s_pose, 0, (size_t)B * 12 * sizeof(float), st));
+  // copies runs of consecutive frames in [f0, f1) that `read` selects: copy(first frame, frame count)
+  auto runs = [](int f0, int f1, auto read, auto copy) -> int {
+    for (int f = f0; f < f1;) {
+      if (!read(f)) { ++f; continue; }
+      int e = f;
+      while (e < f1 && read(e)) ++e;
+      if (int rc = copy(f, e - f)) return rc;
+      f = e;
+    }
+    return 0;
+  };
+  InputView in{};
+  for (int s0 = 0; s0 < B; s0 += ns, ++chunk) {
+    ns = std::min(cs, B - s0);
+    last_ns = ns;
+    const int buf = chunk % davo_ctx::kStage;
+    const int f0 = staged, f1 = s0 + ns + 2;                       // frames this chunk stages
+    CU_OK(cudaStreamWaitEvent(cp, ctx->ev_consumed[buf], 0));       // whoever read this staging slot last is done
+    auto img_rd = [&](int f) { return r.img(f, n_frames); };
+    auto lab_rd = [&](int f) { return r.lab(f, n_frames); };
+    auto dep_rd = [&](int f) { return r.depth && r.img(f, n_frames); };
+    if (int rc = runs(f0, f1, img_rd, [&](int f, int n) -> int {
+          CU_OK(cudaMemcpyAsync(ctx->q_img[set] + hw * 3 * f, img + hw * 3 * f, hw * 3 * n, cudaMemcpyHostToDevice, cp));
+          h2d += hw * 3 * n;
+          return 0;
+        })) return rc;
+    if (int rc = runs(f0, f1, dep_rd, [&](int f, int n) -> int {
+          CU_OK(cudaMemcpyAsync(ctx->q_depth[set] + hw * f, depth + hw * f, hw * 4 * n, cudaMemcpyHostToDevice, cp));
+          h2d += hw * 4 * n;
+          return 0;
+        })) return rc;
+    // flow entries of the chunk: flow_fwd[s0 + i] at slot entry i, flow_bwd[s0 + 1 + i] at slot entry cs + i
+    const int nfwd = r.fwd(s0) ? (r.k0(s0 + ns - 1) ? ns : 1) : 0;    // fwd entries read: all, the first one (FIRST), none
+    const bool need_bwd = r.flow;
+    int n16 = (r.flow && ctx->host_flow16) ? std::min(ns, (int)std::lround(ctx->flow16_frac * ns)) : 0;
+    const bool conv_flow = n16 > 0;
+    bool flow_ok = true;
+    if (seg8 || conv_flow) {
+      CU_OK(cudaEventSynchronize(ctx->ev_seg8[buf]));              // the pinned staging of this slot has been copied out
+      std::vector<NarrowJob> jobs;
+      uint16_t* h16 = ctx->h_flow16[buf];
+      for (int i = 0; conv_flow && i < n16; ++i) {
+        if (i < nfwd) jobs.push_back({flow_fwd + fl * (s0 + i), h16 + fl * i, fl, true});
+        jobs.push_back({flow_bwd + fl * (s0 + 1 + i), h16 + fl * (cs + i), fl, true});
+      }
+      for (int f = f0; seg8 && f < f1; ++f)                         // pinned label staging: frame f at f - f0
+        if (lab_rd(f)) jobs.push_back({seg + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw, false});
+      flow_ok = host_narrow(ctx, jobs);
+    }
+    if (conv_flow && !flow_ok) n16 = 0;                            // a value with no finite half: the whole chunk as float32
+    const int n16_fwd = std::min(n16, nfwd);
+    if (n16 > 0) {
+      uint16_t* d16 = ctx->s_flow16[buf];
+      const uint16_t* h16 = ctx->h_flow16[buf];
+      if (n16_fwd > 0) CU_OK(cudaMemcpyAsync(d16, h16, fl * 2 * n16_fwd, cudaMemcpyHostToDevice, cp));
+      CU_OK(cudaMemcpyAsync(d16 + fl * cs, h16 + fl * cs, fl * 2 * n16, cudaMemcpyHostToDevice, cp));
+      h2d += fl * 2 * (n16_fwd + n16);
+    }
+    float* dflow = ctx->s_flow[buf];
+    if (nfwd > n16_fwd) {
+      CU_OK(cudaMemcpyAsync(dflow + fl * n16_fwd, flow_fwd + fl * (s0 + n16_fwd), fl * 4 * (nfwd - n16_fwd), cudaMemcpyHostToDevice, cp));
+      h2d += fl * 4 * (nfwd - n16_fwd);
+    }
+    if (need_bwd && ns > n16) {
+      CU_OK(cudaMemcpyAsync(dflow + fl * (cs + n16), flow_bwd + fl * (s0 + 1 + n16), fl * 4 * (ns - n16), cudaMemcpyHostToDevice, cp));
+      h2d += fl * 4 * (ns - n16);
+    }
+    if (seg8) {
+      if (int rc = runs(f0, f1, lab_rd, [&](int f, int n) -> int {
+            CU_OK(cudaMemcpyAsync(ctx->q_seg8[set] + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw * n, cudaMemcpyHostToDevice, cp));
+            h2d += hw * n;
+            return 0;
+          })) return rc;
+    } else if (r.labels) {
+      if (int rc = runs(f0, f1, lab_rd, [&](int f, int n) -> int {
+            CU_OK(cudaMemcpyAsync(ctx->q_seg[set] + hw * f, seg + hw * f, hw * 4 * n, cudaMemcpyHostToDevice, cp));
+            h2d += hw * 4 * n;
+            return 0;
+          })) return rc;
+    }
+    staged = f1;
+    if (seg8 || conv_flow) CU_OK(cudaEventRecord(ctx->ev_seg8[buf], cp));   // pinned staging of this slot has been read
+    CU_OK(cudaEventRecord(ctx->ev_copied[buf], cp));
+    CU_OK(cudaStreamWaitEvent(st, ctx->ev_copied[buf], 0));
+    // the chunk's view: sample 0 is sequence sample s0; a flow_fwd the chunk does not read stands in as its flow_bwd
+    // (davo_profile_layers re-runs every pair of the last chunk)
+    in = sequence_view(c.H, c.W, ctx->q_img[set] + hw * 3 * s0, nfwd ? dflow : dflow + fl * cs, dflow + fl * cs,
+                       seg8 ? nullptr : (ctx->q_seg[set] ? ctx->q_seg[set] + hw * s0 : nullptr),
+                       seg8 ? ctx->q_seg8[set] + hw * s0 : nullptr, ctx->q_depth[set] ? ctx->q_depth[set] + hw * s0 : nullptr,
+                       n16 > 0 ? (n16_fwd > 0 ? ctx->s_flow16[buf] : ctx->s_flow16[buf] + fl * cs) : nullptr,
+                       n16 > 0 ? ctx->s_flow16[buf] + fl * cs : nullptr, n16);
+    const int chunk_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && s0 > 0) ? DAVO_PAIRS_TRAJECTORY : pairs;
+    if (int rc = host_run_chunk(ctx, chunk_pairs, s0, ns, in, st, &launches, &last_n)) return rc;
+    CU_OK(cudaEventRecord(ctx->ev_consumed[buf], st));
+  }
+  CU_OK(cudaEventRecord(ctx->ev_q_done[set], st));
+  if (int rc = host_finish(ctx, B, pose_out, st, ticket)) return rc;
+  ctx->last_launches = launches;
+  ctx->last_npairs_mb = last_n;
+  ctx->last_h2d = (long long)h2d;
+  ctx->last_in = in;
+  ctx->last_pose = ctx->s_pose; ctx->last_B = last_ns;
+  ctx->last_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && chunk > 1) ? DAVO_PAIRS_TRAJECTORY : pairs;
+  return 0;
+}
+
+extern "C" int davo_forward_sequence_host(davo_ctx* ctx, int n_frames, int pairs, const uint8_t* img, const float* flow_fwd,
+                                          const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                                          void* stream, long long* ticket) {
+  if (!ctx) return DAVO_ERR_ARG;
+  return forward_sequence_host_impl(ctx, n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out, stream, ticket);
 }
 
 extern "C" int davo_last_host_copy_bytes(const davo_ctx* ctx, long long* h2d, long long* d2h) {
@@ -2138,8 +2396,6 @@ extern "C" int davo_debug_layer_timing(davo_ctx* ctx, int layer, long long* out,
   if (!ctx || layer < 0 || layer > 6 || !out) return DAVO_ERR_ARG;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int npairs = std::min(ctx->last_B * (ctx->unit_sample ? 1 : 2), ctx->mb);
-  ctx->cur_seg8 = ctx->last_seg8;
-  ctx->cur_flow16 = ctx->last_flow16; ctx->cur_n16 = ctx->last_n16;
   Layer& L = pick_layer(ctx, (size_t)layer, npairs);     // the plan a forward of this size runs (latency twin included)
   if (int rc = launch_conv(ctx, L, npairs, st)) return rc;
   if (int rc = launch_conv(ctx, L, npairs, st)) return rc;
@@ -2162,8 +2418,6 @@ extern "C" int davo_profile_layers(davo_ctx* ctx, int iters, float* ms_out, int*
   CU_OK(cudaSetDevice(ctx->device));
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int npairs = std::min(ctx->last_B * (ctx->unit_sample ? 1 : 2), ctx->mb);
-  ctx->cur_seg8 = ctx->last_seg8;
-  ctx->cur_flow16 = ctx->last_flow16; ctx->cur_n16 = ctx->last_n16;
   if (npairs_out) *npairs_out = npairs;
   cudaEvent_t e0, e1;
   CU_OK(cudaEventCreate(&e0));
@@ -2181,7 +2435,7 @@ extern "C" int davo_profile_layers(davo_ctx* ctx, int iters, float* ms_out, int*
     *ms_dst = ms / iters;
     return 0;
   };
-  if (int rc = timed([&] { return launch_front(ctx, ctx->unit_sample ? kUnitsAreSamples : 0, 0, npairs, ctx->last_img, ctx->last_flow, ctx->last_seg, st, &dummy); }, &ms_out[0])) return rc;
+  if (int rc = timed([&] { return launch_front(ctx, ctx->unit_sample ? kUnitsAreSamples : 0, 0, npairs, ctx->last_in, st, &dummy); }, &ms_out[0])) return rc;
   for (int i = 0; i < 7; ++i) {
     const Layer& L = pick_layer(ctx, i, npairs);
     if (i == 5 && ctx->cfg.posenn_se == 3) { ms_out[1 + i] = 0.f; continue; }      // -se_replace has no cnv6 convolution
@@ -2309,8 +2563,8 @@ extern "C" int davo_forward_features(davo_ctx* ctx, int B, const uint8_t* img, c
   // what frame_attention reads: the variant's flags and the flow / depth planes of this batch
   fp.fp.H = c.H; fp.fp.W = c.W; fp.fp.att_src = c.att_src; fp.fp.pixel_map = c.pixel_map; fp.fp.depth_norm = c.depth_norm;
   fp.fp.depth_split = c.depth_split; fp.fp.depth_thres = ctx->depth_thres; fp.fp.flow_abs = c.flow_abs; fp.fp.flow_norm = c.flow_norm;
-  fp.fp.flow = flow; fp.fp.depth = depth; fp.fp.flow_f16 = c.flow_f16;
-  fp.img = img; fp.flow = flow; fp.seg = seg; fp.att_w = ctx->d_attw; fp.static_w = ctx->d_staticw;
+  fp.fp.in = triplet_view(c.H, c.W, img, flow, seg, nullptr, depth, nullptr, 0); fp.fp.flow_f16 = c.flow_f16;
+  fp.att_w = ctx->d_attw; fp.static_w = ctx->d_staticw;
   fp.wheel = ctx->d_wheel; fp.maxrad = ctx->d_maxrad;
   fp.image = out->image; fp.attention = out->attention; fp.masked_image = out->masked_image;
   fp.seg_19 = out->seg_19; fp.seg_color = out->seg_color; fp.flow_color = out->flow_color;

@@ -18,12 +18,9 @@
 namespace davo {
 
 struct FeatureParams {
-  FrontParams fp;         // the variant's flags and the flow / depth inputs, as the pack kernels see them (frame_attention)
+  FrontParams fp;         // the variant's flags and the inputs (fp.in), as the pack kernels see them (frame_attention)
   int B, H, W;
   int unit_sample, att_src, att_tgt_ones, mask_rgb;
-  const uint8_t* img;     // [B][H][3W][3]
-  const float* flow;      // [B][4][H][W][2]
-  const float* seg;       // [B][3][H][W][1]
   const float* att_w;     // [units][kAttFrames][kAttStride] of the pass that just ran (pair mode 'all')
   const float* static_w;  // [19]
   const float* wheel;     // [55][3] Middlebury colour wheel / 255 (double division, then fp32), built by the host
@@ -75,12 +72,13 @@ __global__ void __launch_bounds__(256) feature_frames_kernel(const FeatureParams
   const bool need_flow = p.fp.pixel_map && (p.att_src == 6 || p.fp.pixel_map == 2);
   const bool ones = s_ones != 0;
   const int plane = f == 0 ? 1 : f == 1 ? 0 : 2;        // position in the inputs: [src0, tgt, src1]
-  const uint8_t* img_b = p.img + (size_t)b * p.H * 3 * p.W * 3;
-  const float* seg_p = p.seg ? p.seg + ((size_t)b * 3 + plane) * hw : nullptr;
+  const InputView& in = p.fp.in;
+  const uint8_t* img_f = frame_img(in, b, plane);
+  const float* seg_p = in.seg ? in.seg + frame_plane(in, b, plane, hw) : nullptr;
   const size_t fb = (size_t)f * p.B + b;
   for (int gi = blockIdx.x * blockDim.x + threadIdx.x; gi < groups; gi += gridDim.x * blockDim.x) {
     const int p0 = gi * 4, h = p0 / p.W, w = p0 - h * p.W;
-    const uint32_t* px = reinterpret_cast<const uint32_t*>(img_b + ((size_t)h * 3 * p.W + plane * p.W + w) * 3);
+    const uint32_t* px = reinterpret_cast<const uint32_t*>(img_f + (size_t)h * in.img_row + w * 3);
     float r[4], g[4], bl[4];
     unpack_rgb4(__ldg(px), __ldg(px + 1), __ldg(px + 2), r, g, bl);
     int lab[4] = {-1, -1, -1, -1};
@@ -94,8 +92,8 @@ __global__ void __launch_bounds__(256) feature_frames_kernel(const FeatureParams
       if (ones) { a[i] = 1.0f; continue; }
       float ds = 0.f, dt = 0.f, sfx = se_in_x(0.f, p.fp), sfy = se_in_y(0.f, p.fp);   // the target's flow is zeros
       if (need_depth) {
-        ds = __ldg(p.fp.depth + ((size_t)b * 3 + plane) * hw + p0 + i);
-        dt = __ldg(p.fp.depth + ((size_t)b * 3 + 1) * hw + p0 + i);
+        ds = __ldg(in.depth + frame_plane(in, b, plane, hw) + p0 + i);
+        dt = __ldg(in.depth + frame_plane(in, b, 1, hw) + p0 + i);
       }
       if (need_flow && f != 0) {
         const float2 v = flow1_at(p.fp, b, f - 1, p0 + i, hw);
@@ -168,7 +166,7 @@ __global__ void __launch_bounds__(256) flow_maxrad_kernel(const FeatureParams p)
   float m = 0.f;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const size_t b = i / hw, px = i - b * hw;
-    const float2 f = __ldg(reinterpret_cast<const float2*>(p.flow + (((size_t)b * 4 + k) * hw + px) * 2));
+    const float2 f = __ldg(reinterpret_cast<const float2*>(flow_plane(p.fp.in, b, k) + (size_t)px * 2));
     const float u = fabsf(f.x) > kUnknownFlow ? 0.f : f.x, v = fabsf(f.y) > kUnknownFlow ? 0.f : f.y;
     m = fmaxf(m, flow_rad(u, v));
   }
@@ -184,7 +182,7 @@ __global__ void __launch_bounds__(256) flow_color_kernel(const FeatureParams p) 
   const float denom = __fadd_rn(__uint_as_float(p.maxrad[k]), 1e-5f);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const size_t b = i / hw, px = i - b * hw;
-    const float2 f = __ldg(reinterpret_cast<const float2*>(p.flow + (((size_t)b * 4 + k) * hw + px) * 2));
+    const float2 f = __ldg(reinterpret_cast<const float2*>(flow_plane(p.fp.in, b, k) + (size_t)px * 2));
     float u = fabsf(f.x) > kUnknownFlow ? 0.f : f.x, v = fabsf(f.y) > kUnknownFlow ? 0.f : f.y;
     u = __fdiv_rn(u, denom);
     v = __fdiv_rn(v, denom);

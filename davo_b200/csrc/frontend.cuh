@@ -11,6 +11,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "input_view.cuh"
 #include "ptx.cuh"
 
 namespace davo {
@@ -74,15 +75,10 @@ struct FrontParams {
   int se_act;            // 0 relu, 1 tanh, 2 lrelu
   int flow_abs;          // 0 none, 1 both, 2 h, 3 v
   int flow_norm;
-  const uint8_t* img;    // [B][H][3W][3]
-  const float* flow;     // [B][4][H][W][2]
-  const __half* flow16;  // the two planes the graph reads, already binary16: [B][2][H][W][2] (host entry point) ...
-  int n_flow16;          // ... for samples b < n_flow16 of this batch; the others are read from `flow`
+  InputView in;          // images, labels, depth and flow of the batch, triplet or sequence layout (input_view.cuh);
+                         // the host entry points convert float labels to bytes on the CPU (in.seg8) so that a quarter
+                         // of their bytes crosses PCIe
   int flow_f16;          // davo_config.flow_f16: 1 = float32 flow values are rounded to binary16 when read (flow_q)
-  const float* seg;      // [B][3][H][W][1]
-  const uint8_t* seg8;   // the same labels as bytes (255 = outside 0..18), or NULL: the host entry point
-                         // converts the float labels on the CPU so that a quarter of their bytes crosses PCIe
-  const float* depth;    // [B][3][H][W][1] ([src0, tgt, src1]); se_depth sources only
   const float* se_w;     // W1[in][hid] b1[hid] W2[hid][19] b2[19]
   const float* static_w; // sigmoid(seg_channel_weight)[19]
   float* pool_part;      // [mb][kAttFrames][kPoolSplits][kPoolDim]
@@ -97,16 +93,16 @@ struct FrontParams {
 // would give 0, i.e. class "road")
 __device__ __forceinline__ int label_of(float v) { return v == v ? (int)v : -1; }
 __device__ __forceinline__ int label_at(const FrontParams& p, size_t plane_off, int pix) {
-  if (p.seg8) return p.seg8[plane_off + pix];
-  return label_of(__ldg(p.seg + plane_off + pix));
+  if (p.in.seg8) return p.in.seg8[plane_off + pix];
+  return label_of(__ldg(p.in.seg + plane_off + pix));
 }
 // four consecutive labels (pix % 4 == 0)
 __device__ __forceinline__ void labels4_at(const FrontParams& p, size_t plane_off, int pix, int (&lab)[4]) {
-  if (p.seg8) {
-    const uint32_t w = __ldg(reinterpret_cast<const uint32_t*>(p.seg8 + plane_off + pix));
+  if (p.in.seg8) {
+    const uint32_t w = __ldg(reinterpret_cast<const uint32_t*>(p.in.seg8 + plane_off + pix));
     lab[0] = w & 255u; lab[1] = (w >> 8) & 255u; lab[2] = (w >> 16) & 255u; lab[3] = w >> 24;
   } else {
-    const float4 v = __ldg(reinterpret_cast<const float4*>(p.seg + plane_off + pix));
+    const float4 v = __ldg(reinterpret_cast<const float4*>(p.in.seg + plane_off + pix));
     lab[0] = label_of(v.x); lab[1] = label_of(v.y); lab[2] = label_of(v.z); lab[3] = label_of(v.w);
   }
 }
@@ -127,22 +123,22 @@ __device__ __forceinline__ float2 flow_q2(float x, float y) {
 }
 // pixel `pix` (x, y) of flow plane k (0: src0 -> tgt, 1: src1 -> tgt; davo.py:978-982) of sample b
 __device__ __forceinline__ float2 flow1_at(const FrontParams& p, int b, int k, int pix, int hw) {
-  if (b < p.n_flow16) {
-    const __half2 h = *reinterpret_cast<const __half2*>(p.flow16 + (((size_t)b * 2 + k) * hw + pix) * 2);
+  if (b < p.in.n_flow16) {
+    const __half2 h = *reinterpret_cast<const __half2*>(flow16_plane(p.in, b, k) + (size_t)pix * 2);
     return __half22float2(h);
   }
-  const float2 v = __ldg(reinterpret_cast<const float2*>(p.flow + (((size_t)b * 4 + k) * hw + pix) * 2));
+  const float2 v = __ldg(reinterpret_cast<const float2*>(flow_plane(p.in, b, k) + (size_t)pix * 2));
   return p.flow_f16 ? flow_q2(v.x, v.y) : v;
 }
 // pixels pix, pix + 1 (pix even): (x0, y0, x1, y1)
 __device__ __forceinline__ float4 flow2_at(const FrontParams& p, int b, int k, int pix, int hw) {
-  if (b < p.n_flow16) {
-    const uint2 raw = __ldg(reinterpret_cast<const uint2*>(p.flow16 + (((size_t)b * 2 + k) * hw + pix) * 2));
+  if (b < p.in.n_flow16) {
+    const uint2 raw = __ldg(reinterpret_cast<const uint2*>(flow16_plane(p.in, b, k) + (size_t)pix * 2));
     const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&raw.x));
     const float2 c = __half22float2(*reinterpret_cast<const __half2*>(&raw.y));
     return make_float4(a.x, a.y, c.x, c.y);
   }
-  const float4 v = __ldg(reinterpret_cast<const float4*>(p.flow + (((size_t)b * 4 + k) * hw + pix) * 2));
+  const float4 v = __ldg(reinterpret_cast<const float4*>(flow_plane(p.in, b, k) + (size_t)pix * 2));
   if (!p.flow_f16) return v;
   const float2 lo = flow_q2(v.x, v.y), hi = flow_q2(v.z, v.w);
   return make_float4(lo.x, lo.y, hi.x, hi.y);
@@ -227,7 +223,7 @@ __device__ __forceinline__ bool se_pool_body(const FrontParams& p, const int bx,
   if (p.att_src == 3 || p.att_src == 6) {
     if (threadIdx.x < kNumClasses) s_hist[threadIdx.x] = 0;
     __syncthreads();
-    const size_t seg_off = ((size_t)b * 3 + f) * hw;
+    const size_t seg_off = frame_plane(p.in, b, f, hw);
     const int per = (hw + kPoolSplits - 1) / kPoolSplits;
     const int beg = bx * per, end = min(beg + per, hw);
     for (int i = beg + threadIdx.x; i < end; i += 256) {
@@ -264,8 +260,8 @@ __device__ __forceinline__ bool se_pool_body(const FrontParams& p, const int bx,
   } else {
     float s0 = 0.f, s1 = 0.f, s2 = 0.f;
     if (p.att_src == 5) {
-      const float4* df = reinterpret_cast<const float4*>(p.depth + ((size_t)b * 3 + f) * hw);
-      const float4* dt = reinterpret_cast<const float4*>(p.depth + ((size_t)b * 3 + 1) * hw);
+      const float4* df = reinterpret_cast<const float4*>(p.in.depth + frame_plane(p.in, b, f, hw));
+      const float4* dt = reinterpret_cast<const float4*>(p.in.depth + frame_plane(p.in, b, 1, hw));
       const int n4 = hw / 4;
       const int per = (n4 + kPoolSplits - 1) / kPoolSplits;
       const int beg = bx * per, end = min(beg + per, n4);
@@ -328,14 +324,13 @@ __device__ __forceinline__ bool se_pool_body(const FrontParams& p, const int bx,
       }
     } else {
       // byte sums are exact; the affine map to [-1, 1] (davo.py:1519-1522) is applied to the mean
-      const uint8_t* img_b = p.img + (size_t)b * p.H * 3 * p.W * 3;
-      const int col0 = f * p.W;
+      const uint8_t* img_f = frame_img(p.in, b, f);
       const int per = (hw + kPoolSplits - 1) / kPoolSplits;
       const int beg = bx * per, end = min(beg + per, hw);
       unsigned int u0 = 0, u1 = 0, u2 = 0;
       for (int i = beg + threadIdx.x; i < end; i += 256) {
         const int h = i / p.W, w = i - h * p.W;
-        const uint8_t* px = img_b + ((size_t)h * 3 * p.W + col0 + w) * 3;
+        const uint8_t* px = img_f + (size_t)h * p.in.img_row + w * 3;
         u0 += px[0]; u1 += px[1]; u2 += px[2];
       }
       s0 = (float)u0; s1 = (float)u1; s2 = (float)u2;
@@ -462,7 +457,7 @@ __global__ void __launch_bounds__(256) se_segcells_kernel(const FrontParams p) {
   pair_of_slot(p.pair_mode, p.pair0 + pl, &b, &k);
   const int hw = p.H * p.W;
   const int f = unit_frame(p.unit_sample, k, fr);
-  const size_t seg_off = ((size_t)b * 3 + f) * hw;
+  const size_t seg_off = frame_plane(p.in, b, f, hw);
   __shared__ float s_pool[kSegCellsMaxDim];
   __shared__ int s_hist[8][kNumClasses];
   __shared__ float s_fc1[kPoolDim];
@@ -586,17 +581,17 @@ __global__ void __launch_bounds__(256) pack_kernel(const FrontParams p) {
   __syncthreads();
   const int lane = threadIdx.x & 31, j = lane & 3;
   const float inv_w = 1.0f / (float)p.W;
-  const uint8_t* img_b = p.img + (size_t)b * p.H * 3 * p.W * 3;
-  const size_t seg_src = ((size_t)b * 3 + (k == 0 ? 0 : 2)) * hw, seg_tgt = ((size_t)b * 3 + 1) * hw;
+  const uint8_t* img_t = frame_img(p.in, b, 1);                // tgt = centre frame
+  const uint8_t* img_s = frame_img(p.in, b, k == 0 ? 0 : 2);
+  const size_t seg_src = frame_plane(p.in, b, k == 0 ? 0 : 2, hw), seg_tgt = frame_plane(p.in, b, 1, hw);
   float4* out = reinterpret_cast<float4*>(p.packed + (size_t)pl * hw * kPackedC);
-  const int src_col0 = (k == 0) ? 0 : 2 * p.W;
   for (int base = blockIdx.x * 256; base < hw; base += kPackBlocksPerPair * 256) {
     const int pix_raw = base + threadIdx.x;
     const int pix = min(pix_raw, hw - 1);                       // keep every lane in the shuffles
     const int h = (int)(((float)pix + 0.5f) * inv_w);           // exact for these sizes
-    const int row_off = pix + 2 * p.W * h;                      // h * 3W + w
-    const uint8_t* pt = img_b + (size_t)(row_off + p.W) * 3;    // tgt = centre frame
-    const uint8_t* ps = img_b + (size_t)(row_off + src_col0) * 3;
+    const size_t px_off = (size_t)h * p.in.img_row + (pix - h * p.W) * 3;
+    const uint8_t* pt = img_t + px_off;
+    const uint8_t* ps = img_s + px_off;
     const float tr0 = img_norm(pt[0]), tg0 = img_norm(pt[1]), tb0 = img_norm(pt[2]);
     const float sr0 = img_norm(ps[0]), sg0 = img_norm(ps[1]), sb0 = img_norm(ps[2]);
     float2 fl = make_float2(0.f, 0.f);
@@ -607,8 +602,8 @@ __global__ void __launch_bounds__(256) pack_kernel(const FrontParams p) {
       const bool need_depth = p.depth_split || (p.pixel_map && p.att_src == 5);
       float ds = 0.f, dt = 0.f;
       if (need_depth) {
-        dt = __ldg(p.depth + ((size_t)b * 3 + 1) * hw + pix);
-        ds = __ldg(p.depth + ((size_t)b * 3 + (k == 0 ? 0 : 2)) * hw + pix);
+        dt = __ldg(p.in.depth + seg_tgt + pix);                // depth planes are placed as label planes
+        ds = __ldg(p.in.depth + seg_src + pix);
       }
       const int ls = need_lab ? label_at(p, seg_src, pix) : -1;          // tf.cast truncates toward zero
       a_src = frame_attention(p, s_w, s_wt, ls, sr0, sg0, sb0, ds, dt, se_in_x(fl.x, p), se_in_y(fl.y, p));
@@ -726,19 +721,19 @@ __device__ __forceinline__ void pack8_body(const FrontParams& p, const int bx, c
   }
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint8_t* img_b = p.img + (size_t)b * p.H * 3 * p.W * 3;
-  const size_t seg_src = ((size_t)b * 3 + (k == 0 ? 0 : 2)) * hw, seg_tgt = ((size_t)b * 3 + 1) * hw;
+  const uint8_t* img_t = frame_img(p.in, b, 1);
+  const long long img_ds = k == 0 ? -p.in.img_frame : p.in.img_frame;   // the source frame, relative to the target
+  const size_t seg_src = frame_plane(p.in, b, k == 0 ? 0 : 2, hw), seg_tgt = frame_plane(p.in, b, 1, hw);
   float4* out = reinterpret_cast<float4*>(p.packed + (size_t)pl * hw * 8);
-  const int src_col0 = (k == 0) ? 0 : 2 * p.W;
   float4* st = s_stage[warp];
   for (int base = bx * 256; base < groups; base += nbx * 256) {
     const int gi = base + threadIdx.x;
     float4 q[8];
     if (gi < groups) {
       const int p0 = gi * 4, h = p0 / p.W, w = p0 - h * p.W;
-      const size_t row = (size_t)h * 3 * p.W;
-      const uint32_t* pt = reinterpret_cast<const uint32_t*>(img_b + (row + p.W + w) * 3);
-      const uint32_t* ps = reinterpret_cast<const uint32_t*>(img_b + (row + src_col0 + w) * 3);
+      const size_t px_off = (size_t)h * p.in.img_row + w * 3;
+      const uint32_t* pt = reinterpret_cast<const uint32_t*>(img_t + px_off);
+      const uint32_t* ps = reinterpret_cast<const uint32_t*>(img_t + img_ds + px_off);
       int lsv[4] = {-1, -1, -1, -1}, ltv[4] = {-1, -1, -1, -1};
       if (p.att_src != 0) {
         labels4_at(p, seg_src, p0, lsv);                            // tf.cast truncates toward zero
@@ -861,26 +856,24 @@ __global__ void __launch_bounds__(256) pack_sample_kernel(const FrontParams p) {
   const bool need_lab = !p.pixel_map || p.att_src == 6;
   const bool need_depth = p.depth_split || (p.pixel_map && p.att_src == 5);
   const bool need_seflow = (p.pixel_map && p.att_src == 6) || p.pixel_map == 2;
-  const uint8_t* img_b = p.img + (size_t)b * p.H * 3 * p.W * 3;
-  const size_t seg_b = (size_t)b * 3 * hw;
   float4* out = reinterpret_cast<float4*>(p.packed + (size_t)pl * hw * 16);
   for (int pix = blockIdx.x * 256 + threadIdx.x; pix < hw; pix += kPackBlocksPerPair * 256) {
     const int h = pix / p.W, w = pix - h * p.W;
-    const uint8_t* row = img_b + ((size_t)h * 3 * p.W + w) * 3;
+    const size_t px_off = (size_t)h * p.in.img_row + w * 3;
     float a[3] = {1.f, 1.f, 1.f};                            // A_src0, A_src1, A_tgt
     if (p.att_src != 0) {
-      const float dt = need_depth ? __ldg(p.depth + ((size_t)b * 3 + 1) * hw + pix) : 0.f;
+      const float dt = need_depth ? __ldg(p.in.depth + frame_plane(p.in, b, 1, hw) + pix) : 0.f;
 #pragma unroll
       for (int fr = 0; fr < 3; ++fr) {
         if (fr == 2 && p.att_tgt_ones) continue;
         const int plane = unit_frame(1, 0, fr);              // 0 = src0, 2 = src1, 1 = tgt: label / depth plane, image column block
-        const int lab = need_lab ? label_at(p, seg_b + (size_t)plane * hw, pix) : -1;   // tf.cast truncates
+        const int lab = need_lab ? label_at(p, frame_plane(p.in, b, plane, hw), pix) : -1;   // tf.cast truncates
         float r = 0.f, g = 0.f, bl = 0.f, ds = 0.f, sfx = se_in_x(0.f, p), sfy = se_in_y(0.f, p);   // the target's flow is zeros (davo.py:979)
         if (p.pixel_map && p.att_src == 4) {
-          const uint8_t* pf = row + (size_t)plane * p.W * 3;
+          const uint8_t* pf = frame_img(p.in, b, plane) + px_off;
           r = img_norm(pf[0]); g = img_norm(pf[1]); bl = img_norm(pf[2]);
         }
-        if (need_depth) ds = __ldg(p.depth + ((size_t)b * 3 + plane) * hw + pix);
+        if (need_depth) ds = __ldg(p.in.depth + frame_plane(p.in, b, plane, hw) + pix);
         if (need_seflow && fr != 2) {
           const float2 f = flow1_at(p, b, fr, pix, hw);      // slot 0 = src0 -> flow[:, 0], slot 1 = src1 -> flow[:, 1]
           sfx = se_in_x(f.x, p); sfy = se_in_y(f.y, p);
@@ -894,13 +887,13 @@ __global__ void __launch_bounds__(256) pack_sample_kernel(const FrontParams p) {
 #pragma unroll
     for (int i = 0; i < 16; ++i) v[i] = 0.f;
     const float mt = p.mask_rgb ? a[2] : 1.0f;
-    const uint8_t* pt = row + (size_t)p.W * 3;
+    const uint8_t* pt = frame_img(p.in, b, 1) + px_off;
 #pragma unroll
     for (int c = 0; c < 3; ++c) v[c] = img_norm(pt[c]) * mt;
 #pragma unroll
     for (int sidx = 0; sidx < 2; ++sidx) {
       const float ms = p.mask_rgb ? a[sidx] : 1.0f, mf = p.mask_flow ? a[sidx] : 1.0f;
-      const uint8_t* ps = row + (size_t)(sidx == 0 ? 0 : 2 * p.W) * 3;
+      const uint8_t* ps = frame_img(p.in, b, sidx == 0 ? 0 : 2) + px_off;
 #pragma unroll
       for (int c = 0; c < 3; ++c) v[3 + 5 * sidx + c] = img_norm(ps[c]) * ms;
       if (p.in_mode == 1) {

@@ -349,6 +349,83 @@ class DAVO(object):
                     "davo_forward_host_async")
         return DAVO._Pending(self, ticket.value, out, (img, flow, seg, depth))
 
+    # ------------------------------------------------------------ frame-sequence inputs
+    def _sequence_args(self, img, flow_fwd, flow_bwd, seg, depth, pairs, who):
+        if pairs not in _capi.PAIRS:
+            raise ValueError("DAVO.%s: pairs must be one of %s" % (who, sorted(_capi.PAIRS)))
+        if not self._weights_loaded:
+            raise RuntimeError("DAVO.%s: weights not loaded" % who)
+        if self.config.att_src != V.ATT_SE_DEPTH_SEG and not self.config.depth_split:
+            depth = None                                  # only the depth sources read it
+        elif depth is None:
+            raise ValueError("DAVO.%s: version %r reads depth [N,H,W,1]" % (who, self.version))
+        N, H, W = int(img.shape[0]), self.img_height, self.img_width
+        want = {"img": (N, H, W, 3), "flow_fwd": (N - 1, H, W, 2), "flow_bwd": (N - 1, H, W, 2), "seg": (N, H, W, 1),
+                "depth": (N, H, W, 1)}
+        for name, t in (("img", img), ("flow_fwd", flow_fwd), ("flow_bwd", flow_bwd), ("seg", seg), ("depth", depth)):
+            if t is not None and tuple(t.shape) != want[name]:
+                raise ValueError("DAVO.%s: %s has shape %s, expected %s" % (who, name, tuple(t.shape), want[name]))
+        return N, _capi.PAIRS[pairs], depth
+
+    def inference_sequence(self, img, flow_fwd, flow_bwd, seg, depth=None, pairs='all', as_torch=False):
+        """Poses of a frame sequence -> ``{'pose': [N-2,2,6]}`` (include/davo_b200.h: davo_forward_sequence).
+
+        ``img`` uint8 [N,H,W,3]; ``flow_fwd`` / ``flow_bwd`` float32 [N-1,H,W,2], entry i the flow from frame i to i+1 /
+        from i+1 to i; ``seg`` float32 [N,H,W,1]; ``depth`` float32 [N,H,W,1] (depth sources only).  Sample s is frames
+        (s, s+1, s+2); the poses equal ``inference`` on ``sequence_to_triplets`` of the same frames, bit for bit.
+        ``flow_fwd`` may be None under ``pairs='trajectory'`` for the shared nets.  numpy arrays take the host path
+        (each frame crosses PCIe once), CUDA tensors the device path; ``-batch_norm`` uploads and takes the device
+        path.  A long sequence continues with a call that starts two frames before the previous one ended."""
+        N, sel, depth = self._sequence_args(img, flow_fwd, flow_bwd, seg, depth, pairs, "inference_sequence")
+        if not _is_torch(img) and not self.config.batch_norm:
+            return self.inference_sequence_async(img, flow_fwd, flow_bwd, seg, depth, pairs, _block=True).result()
+        import torch
+        dev = "cuda:%d" % self.device
+        up = lambda t, dt: None if t is None else (t if _is_torch(t) else torch.as_tensor(np.ascontiguousarray(t))).to(
+            device=dev, dtype=dt)
+        img, flow_fwd, flow_bwd = up(img, torch.uint8), up(flow_fwd, torch.float32), up(flow_bwd, torch.float32)
+        seg, depth = up(seg, torch.float32), up(depth, torch.float32)
+        for name, t in (("img", img), ("flow_fwd", flow_fwd), ("flow_bwd", flow_bwd), ("seg", seg), ("depth", depth)):
+            if t is not None and not (t.device.index == self.device and t.is_contiguous()):
+                raise ValueError("DAVO.inference_sequence: %s must be a contiguous tensor on %s" % (name, dev))
+        out = torch.empty((N - 2, 2, 6), dtype=torch.float32, device=dev)
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        self._check(self._lib.davo_forward_sequence(self._h, N, sel, ptr(img), ptr(flow_fwd), ptr(flow_bwd), ptr(seg),
+                                                    ptr(depth), ptr(out), C.c_void_p(stream)), "davo_forward_sequence")
+        return {'pose': out if as_torch else out.cpu().numpy()}
+
+    def inference_sequence_async(self, img, flow_fwd, flow_bwd, seg, depth=None, pairs='all', _block=False):
+        """``inference_sequence`` on host arrays without waiting (davo_forward_sequence_host with a ticket): returns
+        the handle of ``inference_async``, whose ``.result()`` gives ``{'pose': [N-2,2,6]}``.  The arrays must not be
+        modified before ``.result()``; up to 8 calls may be in flight."""
+        N, sel, depth = self._sequence_args(img, flow_fwd, flow_bwd, seg, depth, pairs, "inference_sequence_async")
+        if self.config.batch_norm:
+            raise NotImplementedError("DAVO.inference_sequence_async: -batch_norm takes the device path (one pass per batch)")
+        arr = lambda a, dt: None if a is None else np.ascontiguousarray(a, dtype=dt)
+        img, flow_fwd, flow_bwd = arr(img, np.uint8), arr(flow_fwd, np.float32), arr(flow_bwd, np.float32)
+        seg, depth = arr(seg, np.float32), arr(depth, np.float32)
+        ptr = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None else None
+        if _block:
+            out = np.empty((N - 2, 2, 6), np.float32)
+            self._check(self._lib.davo_forward_sequence_host(self._h, N, sel, ptr(img), ptr(flow_fwd), ptr(flow_bwd),
+                                                             ptr(seg), ptr(depth), ptr(out), None, None),
+                        "davo_forward_sequence_host")
+            return DAVO._Pending(self, None, out, None)
+        import torch
+        ring = getattr(self, "_async_out", None)
+        if ring is None or ring[0].shape[0] < N - 2:
+            ring = self._async_out = [torch.empty((max(N - 2, self.batch_size), 2, 6), dtype=torch.float32).pin_memory()
+                                      for _ in range(8)]
+            self._async_n = 0
+        out = ring[self._async_n % 8][:N - 2].numpy()
+        self._async_n += 1
+        ticket = C.c_longlong(0)
+        self._check(self._lib.davo_forward_sequence_host(self._h, N, sel, ptr(img), ptr(flow_fwd), ptr(flow_bwd), ptr(seg),
+                                                         ptr(depth), ptr(out), None, C.byref(ticket)),
+                    "davo_forward_sequence_host")
+        return DAVO._Pending(self, ticket.value, out, (img, flow_fwd, flow_bwd, seg, depth))
+
     def bind_host_numa(self):
         """Bind this thread (and threads created after it) to the CPUs next to this handle's GPU
         (``davo_bind_host_numa``); call it before allocating pinned inputs.  Returns the NUMA node or -1."""

@@ -68,6 +68,26 @@ def make_depth(batch: int, height: int = 128, width: int = 416, seed: int = 4321
     return d.astype(np.float32)[..., None].copy()
 
 
+def make_sequence(n_frames: int, height: int = 128, width: int = 416, seed: int = 1234, seg_block: int = 16):
+    """A seeded frame sequence in the layout of ``DAVO.inference_sequence``: ``(img [N,H,W,3] uint8,
+    flow_fwd [N-1,H,W,2] float32, flow_bwd [N-1,H,W,2] float32, seg [N,H,W,1] float32, depth [N,H,W,1] float32)``.
+    ``flow_fwd[i]`` stands for the flow from frame i to i+1 and ``flow_bwd[i]`` for the flow from i+1 to i; labels
+    are integer-valued over ``seg_block`` x ``seg_block`` blocks, depth (1..80 m) over 8 x 8 blocks, as in
+    ``make_inputs`` / ``make_depth``."""
+    if n_frames < 3:
+        raise ValueError("make_sequence: a sequence has at least 3 frames")
+    rng = np.random.default_rng(seed)
+    img = rng.integers(0, 256, size=(n_frames, height, width, 3), dtype=np.uint8)
+    flow_fwd = rng.normal(FLOW_MEAN, FLOW_STD, size=(n_frames - 1, height, width, 2)).astype(np.float32)
+    flow_bwd = rng.normal(FLOW_MEAN, FLOW_STD, size=(n_frames - 1, height, width, 2)).astype(np.float32)
+    hb, wb = -(-height // seg_block), -(-width // seg_block)
+    blocks = rng.integers(0, NUM_CLASSES, size=(n_frames, hb, wb), dtype=np.int64)
+    seg = np.repeat(np.repeat(blocks, seg_block, axis=1), seg_block, axis=2)[:, :height, :width].astype(np.float32)
+    dblocks = rng.uniform(1.0, 80.0, size=(n_frames, -(-height // 8), -(-width // 8)))
+    depth = np.repeat(np.repeat(dblocks, 8, axis=1), 8, axis=2)[:, :height, :width].astype(np.float32)
+    return img, flow_fwd, flow_bwd, seg[..., None].copy(), depth[..., None].copy()
+
+
 def _xavier_uniform(rng, shape):
     kh, kw, cin, cout = shape
     lim = math.sqrt(6.0 / (kh * kw * cin + kh * kw * cout))

@@ -195,6 +195,36 @@ int davo_forward_host_compact_async(davo_ctx*, int B, int pairs, const uint8_t* 
                                     long long* ticket);
 int davo_host_wait(davo_ctx*, long long ticket);
 
+/* --- frame-sequence inputs ---
+ * A camera stream or a video as it comes: N >= 3 frames and the flow between neighbours, each frame sent once
+ * instead of once per sample that holds it.  Sample s (0 <= s < N-2) is frames (s, s+1, s+2) in the roles
+ * (src0, tgt, src1); poses land in pose_out [N-2,2,6] with the rows, columns and pair selections (`pairs`) of
+ * davo_forward_pairs.  Every buffer is contiguous and 16-byte aligned:
+ *   img       uint8 [N,H,W,3]
+ *   flow_fwd  float [N-1,H,W,2]  entry i: flow from frame i to frame i+1   (sample s: flow[:,0] = flow_fwd[s])
+ *   flow_bwd  float [N-1,H,W,2]  entry i: flow from frame i+1 to frame i   (sample s: flow[:,1] = flow_bwd[s+1])
+ *   seg       float [N,H,W,1]    labels as in davo_forward; NULL for variants without attention source
+ *   depth     float [N,H,W,1]    the depth sources only, otherwise NULL
+ * flow_fwd may be NULL for the shared nets under DAVO_PAIRS_TRAJECTORY (only flow_fwd[0] is read under
+ * DAVO_PAIRS_TRAJECTORY_FIRST); both may be NULL for variants that read no flow.  The poses are bit-identical to
+ * davo_forward_pairs on the triplet batch built from the same frames (davo_b200.sequence_to_triplets).  A long
+ * sequence continues with a call that starts two frames before the previous one ended: only those two frames are
+ * sent again, no flow is.  Argument errors (N < 3, N-2 > max_batch, a NULL input the variant and selection read, a
+ * misaligned buffer) return DAVO_ERR_ARG with a message naming the input.
+ *
+ * davo_forward_sequence: device buffers, as davo_forward_pairs (-batch_norm included: one pass, DAVO_PAIRS_ALL).
+ * davo_forward_sequence_host: host buffers, as davo_forward_host_pairs: chunked, copies overlapping compute, labels
+ *   (and with flow_f16 = 1 the flow) narrowed on the CPU.  Each frame plane and flow entry crosses PCIe at most once
+ *   per call, and those that no computed pair reads are not copied (davo_last_host_copy_bytes counts them).
+ *   ticket == NULL: blocks until the poses are in pose_out; otherwise the asynchronous form of
+ *   davo_forward_host_pairs_async, waited for with davo_host_wait. */
+int davo_forward_sequence(davo_ctx*, int n_frames, int pairs, const uint8_t* img_u8, const float* flow_fwd,
+                          const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                          void* cuda_stream);
+int davo_forward_sequence_host(davo_ctx*, int n_frames, int pairs, const uint8_t* img_u8, const float* flow_fwd,
+                               const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                               void* cuda_stream, long long* ticket);
+
 /* Binds the calling thread (and the threads it creates afterwards: the handle's conversion pool, the caller's
  * loader threads) to the CPUs of the NUMA node the handle's GPU hangs off (/sys/bus/pci/devices/<id>/numa_node,
  * local_cpulist), so that pinned staging allocated afterwards is first-touched next to the GPU and the conversion
@@ -211,7 +241,8 @@ int davo_bind_host_numa(davo_ctx*);
 int davo_get_intermediate(davo_ctx*, const char* name, int pair, float* out,
                           int64_t cap, int64_t* n);
 
-/* Bytes the last davo_forward_host moved host->device and device->host. */
+/* Bytes the last host entry point (davo_forward_host*, davo_forward_sequence_host) moved host->device and
+ * device->host. */
 int davo_last_host_copy_bytes(const davo_ctx*, long long* h2d, long long* d2h);
 
 /* Number of kernel launches the last davo_forward issued. */
