@@ -24,8 +24,9 @@ SYMBOLS = (
     "davo_forward_host_pairs_async", "davo_forward_host_compact_async", "davo_host_wait",
     "davo_comm_unique_id", "davo_comm_create", "davo_comm_world", "davo_allgather_poses",
     "davo_forward_sequence", "davo_forward_sequence_host",
+    "davo_odometry_create", "davo_odometry_push", "davo_odometry_reset", "davo_odometry_frames",
     "davo_last_error",
-    "davo_destroy", "davo_build_info", "davo_config_bytes",
+    "davo_destroy", "davo_build_info", "davo_config_bytes", "davo_odometry_destroy",
 )
 
 
@@ -83,6 +84,13 @@ def load() -> C.CDLL:
     lib.davo_host_wait.argtypes = [vp, C.c_longlong]
     lib.davo_forward_sequence.argtypes = [vp, ip, ip, vp, vp, vp, vp, vp, vp, vp]
     lib.davo_forward_sequence_host.argtypes = [vp, ip, ip, vp, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_longlong)]
+    lib.davo_odometry_create.argtypes = [vp, ip, ip, ip, C.POINTER(vp)]
+    lib.davo_odometry_push.argtypes = [vp, ip, vp, vp, vp, vp, vp, vp, vp, C.POINTER(ip), C.POINTER(ip), vp,
+                                       C.POINTER(C.c_longlong)]
+    lib.davo_odometry_reset.argtypes = [vp]
+    lib.davo_odometry_frames.argtypes = [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
+    lib.davo_odometry_destroy.argtypes = [vp]
+    lib.davo_odometry_destroy.restype = None
     lib.davo_get_intermediate.argtypes = [vp, C.c_char_p, ip, vp, C.c_int64, C.POINTER(C.c_int64)]
     lib.davo_last_launch_count.argtypes = [vp]
     lib.davo_last_host_copy_bytes.argtypes = [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]

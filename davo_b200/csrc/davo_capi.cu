@@ -21,7 +21,9 @@
 
 #include <condition_variable>
 #include <functional>
+#include <climits>
 #include <map>
+#include <set>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -1342,8 +1344,11 @@ extern "C" int davo_create(const davo_config* cfg, int device, davo_ctx** out) {
   return 0;
 }
 
+static void destroy_sessions_of(davo_ctx* ctx);
+
 extern "C" void davo_destroy(davo_ctx* ctx) {
   if (!ctx) return;
+  destroy_sessions_of(ctx);
   cudaSetDevice(ctx->device);
   for (void* p : ctx->allocs) cudaFree(p);
   if (ctx->d_traj_scratch) cudaFree(ctx->d_traj_scratch);
@@ -2010,9 +2015,12 @@ bool host_narrow(davo_ctx* ctx, const std::vector<NarrowJob>& jobs) {
   return flow_bad.load() == 0;
 }
 
-// Poses of a host call back to the caller's memory; blocking, or the asynchronous form's ticket.
-int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket) {
-  CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
+// Poses of a host call back to the caller's memory, and an odometry push's n_traj absolute poses from traj_dev;
+// blocking, or the asynchronous form's ticket.
+int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket, const double* traj_dev = nullptr,
+                double* traj_out = nullptr, int n_traj = 0) {
+  if (B > 0) CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
+  if (n_traj > 0) CU_OK(cudaMemcpyAsync(traj_out, traj_dev, (size_t)16 * 8 * n_traj, cudaMemcpyDeviceToHost, st));
   if (ticket) {
     const long long t = ++ctx->host_tickets;
     cudaEvent_t& ev = ctx->ev_host_done[t % davo_ctx::kTickets];
@@ -2022,7 +2030,7 @@ int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long lon
   } else {
     CU_OK(cudaStreamSynchronize(st));
   }
-  ctx->last_d2h = (long long)12 * 4 * B;
+  ctx->last_d2h = (long long)12 * 4 * B + (long long)16 * 8 * n_traj;
   return 0;
 }
 
@@ -2169,24 +2177,70 @@ static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img
   return 0;
 }
 
+// An online odometry session (include/davo_b200.h: davo_odometry_*).  A push of k frames runs as a sequence call over
+// a virtual sequence: the session's last `head` (<= 2) frames, then the k new ones.  Virtual frame v is global frame
+// g0 + v, and every sample of that call is new.  The carried state lives in the session's own buffers, because other
+// calls on the handle reuse the handle's frame sets and staging slots.
+struct davo_odometry {
+  davo_ctx* ctx = nullptr;
+  int max_push = 0, pairs = DAVO_PAIRS_TRAJECTORY;
+  bool host = true;
+  long long pushed = 0, posed = 0;               // frames pushed; frames whose absolute pose has been written
+  // frame sets of max_push + 2 frames, in the form the passes read (labels as bytes on the host path with byte labels);
+  // two, so that a host push's copies can run under the previous push
+  uint8_t* q_img[2] = {}; uint8_t* q_seg8[2] = {}; float *q_seg[2] = {}, *q_depth[2] = {};
+  cudaEvent_t ev_q_done[2] = {};
+  long long q_calls = 0;
+  // carried state: the last two frames (same forms as a set), the last flow_fwd entry when a later sample reads it, the
+  // last absolute pose
+  uint8_t* c_img = nullptr; uint8_t* c_seg8 = nullptr; float *c_seg = nullptr, *c_depth = nullptr, *c_fwd = nullptr;
+  double* d_P = nullptr;
+  Mat4 *d_rel = nullptr, *d_traj = nullptr;      // this push's relative motions; a host push's absolute poses
+  float* d_fwd = nullptr;                        // device pushes: the carried flow_fwd entry followed by the pushed ones
+  int head() const { return (int)std::min<long long>(pushed, 2); }
+};
+
+namespace {
+
+std::mutex g_odo_mutex;
+std::set<davo_odometry*> g_odo_live;             // sessions not yet destroyed (a push on any other pointer is refused)
+
+// One push as a sequence call: n_frames virtual frames of which frames [0, head) are carried, flow entries e >= fe of
+// the caller's arrays are virtual entries e (fe = 1: virtual flow_fwd entry 0 is the carried one).
+struct OdoPush {
+  davo_odometry* o;
+  int head, fe;
+  long long g0;
+  double* traj_out;
+  int n_traj;
+};
+
+}  // namespace
+
 // Host-buffer sequence entry point (include/davo_b200.h: davo_forward_sequence_host).  The samples are cut into the
 // chunks of the triplet entry point.  Flow entries belong to one sample each and go through the chunk slots like the
 // triplet flow planes.  Frames (images, labels, depth) are shared by up to three samples, so they are staged at their
 // final place in one of two per-call frame sets: a chunk copies the frames that the call reads and that no earlier
 // chunk copied, and the chunk's passes read the set through a sequence view.  Every copied frame or flow crosses PCIe
 // once; those that no computed pair reads are not copied.
+// An odometry push (`op`) is the same call over its virtual sequence, on the session's frame sets: the carried frames
+// are copied device to device to the head of the set, frames [0, head) count as staged, and the carried flow_fwd entry
+// stands in for the first chunk's first fwd slot.  A frame or flow entry is copied when any sample of the whole stream
+// reads it, now or in a later push, which then finds it in the carried state.
 static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, const uint8_t* img, const float* flow_fwd,
                                       const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
-                                      void* stream, long long* ticket) {
-  const char* who = ticket ? "davo_forward_sequence_host_async" : "davo_forward_sequence_host";
-  if (int rc = check_sequence(ctx, who, n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
-  if (ctx->cfg.batch_norm)
-    return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm needs the whole batch in one pass; the chunked host entry point does not take it (copy the frames to the device and call davo_forward_sequence)", who);
+                                      void* stream, long long* ticket, const OdoPush* op = nullptr) {
+  const char* who = op ? "davo_odometry_push" : ticket ? "davo_forward_sequence_host_async" : "davo_forward_sequence_host";
+  if (!op) {
+    if (int rc = check_sequence(ctx, who, n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
+    if (ctx->cfg.batch_norm)
+      return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm needs the whole batch in one pass; the chunked host entry point does not take it (copy the frames to the device and call davo_forward_sequence)", who);
+  }
   const davo_config& c = ctx->cfg;
   CU_OK(cudaSetDevice(ctx->device));
   const SeqReads r = seq_reads(ctx, pairs);
   pairs = r.pairs;
-  const int B = n_frames - 2;
+  const int B = std::max(0, n_frames - 2);
   const size_t hw = (size_t)c.H * c.W, fl = hw * 2;               // pixels per frame, floats per flow entry
   const int cs = host_setup(ctx, who);
   if (cs < 0) return cs;
@@ -2194,20 +2248,38 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
   cudaStream_t cp = ctx->copy_stream;
   if (int rc = host_order_first_call(ctx, st)) return rc;
   const bool seg8 = r.labels && ctx->host_seg8;
-  const int set = (int)(ctx->q_calls++ & 1);
-  if (!ctx->q_img[set]) {
-    const size_t nf = (size_t)c.max_batch + 2;
-    CU_OK(cudaMalloc((void**)&ctx->q_img[set], nf * hw * 3));
-    if (c.att_src != 0 && ctx->host_seg8) CU_OK(cudaMalloc((void**)&ctx->q_seg8[set], nf * hw));
-    if (c.att_src != 0 && !ctx->host_seg8) CU_OK(cudaMalloc((void**)&ctx->q_seg[set], nf * hw * 4));
-    if (r.depth) CU_OK(cudaMalloc((void**)&ctx->q_depth[set], nf * hw * 4));
-    CU_OK(cudaEventCreateWithFlags(&ctx->ev_q_done[set], cudaEventDisableTiming));
+  davo_odometry* o = op ? op->o : nullptr;
+  const int set = (int)((o ? o->q_calls : ctx->q_calls)++ & 1);
+  uint8_t*& q_img = o ? o->q_img[set] : ctx->q_img[set];
+  uint8_t*& q_seg8 = o ? o->q_seg8[set] : ctx->q_seg8[set];
+  float*& q_seg = o ? o->q_seg[set] : ctx->q_seg[set];
+  float*& q_depth = o ? o->q_depth[set] : ctx->q_depth[set];
+  cudaEvent_t& ev_q_done = o ? o->ev_q_done[set] : ctx->ev_q_done[set];
+  if (!q_img) {
+    const size_t nf = (size_t)(o ? o->max_push : c.max_batch) + 2;
+    CU_OK(cudaMalloc((void**)&q_img, nf * hw * 3));
+    if (c.att_src != 0 && ctx->host_seg8) CU_OK(cudaMalloc((void**)&q_seg8, nf * hw));
+    if (c.att_src != 0 && !ctx->host_seg8) CU_OK(cudaMalloc((void**)&q_seg, nf * hw * 4));
+    if (r.depth) CU_OK(cudaMalloc((void**)&q_depth, nf * hw * 4));
+    CU_OK(cudaEventCreateWithFlags(&ev_q_done, cudaEventDisableTiming));
   } else {
-    CU_OK(cudaStreamWaitEvent(cp, ctx->ev_q_done[set], 0));         // the call before the previous one has read this set
+    CU_OK(cudaStreamWaitEvent(cp, ev_q_done, 0));                   // the call before the previous one has read this set
+  }
+  const int head = op ? op->head : 0, fe = op ? op->fe : 0;
+  // which frames and flow_fwd entries some pair reads: this call's, or for a push the whole stream's (global index
+  // g0 + f; every read predicate is true from frame 2 on, hence the clamp)
+  const SeqReads rg = o ? seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST) : r;
+  const int n_rd = o ? INT_MAX : n_frames;
+  auto glob = [&](int f) { return o ? (int)std::min<long long>(op->g0 + f, 2) : f; };
+  if (head > 0) {                                                  // the carried frames to the head of the set
+    CU_OK(cudaMemcpyAsync(q_img, o->c_img, hw * 3 * head, cudaMemcpyDeviceToDevice, cp));
+    if (seg8) CU_OK(cudaMemcpyAsync(q_seg8, o->c_seg8, hw * head, cudaMemcpyDeviceToDevice, cp));
+    else if (r.labels) CU_OK(cudaMemcpyAsync(q_seg, o->c_seg, hw * 4 * head, cudaMemcpyDeviceToDevice, cp));
+    if (r.depth) CU_OK(cudaMemcpyAsync(q_depth, o->c_depth, hw * 4 * head, cudaMemcpyDeviceToDevice, cp));
   }
   size_t h2d = 0;
   int launches = 0, last_n = 0, chunk = 0, ns = 0, last_ns = 0;
-  int staged = 0;                                                  // frames [0, staged) are on the device (or never read)
+  int staged = head;                                               // frames [0, staged) are on the device (or never read)
   if (pairs == DAVO_PAIRS_TRAJECTORY || pairs == DAVO_PAIRS_TRAJECTORY_FIRST)
     CU_OK(cudaMemsetAsync(ctx->s_pose, 0, (size_t)B * 12 * sizeof(float), st));
   // copies runs of consecutive frames in [f0, f1) that `read` selects: copy(first frame, frame count)
@@ -2222,29 +2294,31 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
     return 0;
   };
   InputView in{};
-  for (int s0 = 0; s0 < B; s0 += ns, ++chunk) {
+  // a push too short to hold a sample still stages its frames: one chunk of no samples
+  for (int s0 = 0; s0 < B || (o && chunk == 0); s0 += ns, ++chunk) {
     ns = std::min(cs, B - s0);
     last_ns = ns;
     const int buf = chunk % davo_ctx::kStage;
-    const int f0 = staged, f1 = s0 + ns + 2;                       // frames this chunk stages
+    const int f0 = staged, f1 = s0 + ns < B ? s0 + ns + 2 : n_frames;   // frames this chunk stages
     CU_OK(cudaStreamWaitEvent(cp, ctx->ev_consumed[buf], 0));       // whoever read this staging slot last is done
-    auto img_rd = [&](int f) { return r.img(f, n_frames); };
-    auto lab_rd = [&](int f) { return r.lab(f, n_frames); };
-    auto dep_rd = [&](int f) { return r.depth && r.img(f, n_frames); };
+    auto img_rd = [&](int f) { return rg.img(glob(f), n_rd); };
+    auto lab_rd = [&](int f) { return rg.lab(glob(f), n_rd); };
+    auto dep_rd = [&](int f) { return r.depth && img_rd(f); };
     if (int rc = runs(f0, f1, img_rd, [&](int f, int n) -> int {
-          CU_OK(cudaMemcpyAsync(ctx->q_img[set] + hw * 3 * f, img + hw * 3 * f, hw * 3 * n, cudaMemcpyHostToDevice, cp));
+          CU_OK(cudaMemcpyAsync(q_img + hw * 3 * f, img + hw * 3 * (f - head), hw * 3 * n, cudaMemcpyHostToDevice, cp));
           h2d += hw * 3 * n;
           return 0;
         })) return rc;
     if (int rc = runs(f0, f1, dep_rd, [&](int f, int n) -> int {
-          CU_OK(cudaMemcpyAsync(ctx->q_depth[set] + hw * f, depth + hw * f, hw * 4 * n, cudaMemcpyHostToDevice, cp));
+          CU_OK(cudaMemcpyAsync(q_depth + hw * f, depth + hw * (f - head), hw * 4 * n, cudaMemcpyHostToDevice, cp));
           h2d += hw * 4 * n;
           return 0;
         })) return rc;
     // flow entries of the chunk: flow_fwd[s0 + i] at slot entry i, flow_bwd[s0 + 1 + i] at slot entry cs + i
-    const int nfwd = r.fwd(s0) ? (r.k0(s0 + ns - 1) ? ns : 1) : 0;    // fwd entries read: all, the first one (FIRST), none
+    const int nfwd = ns > 0 && r.fwd(s0) ? (r.k0(s0 + ns - 1) ? ns : 1) : 0;   // fwd entries read: all, the first one (FIRST), none
     const bool need_bwd = r.flow;
-    int n16 = (r.flow && ctx->host_flow16) ? std::min(ns, (int)std::lround(ctx->flow16_frac * ns)) : 0;
+    const int carried = s0 < fe && nfwd > 0 ? 1 : 0;              // the session's flow_fwd entry takes slot entry 0
+    int n16 = (r.flow && ctx->host_flow16 && !carried) ? std::min(ns, (int)std::lround(ctx->flow16_frac * ns)) : 0;
     const bool conv_flow = n16 > 0;
     bool flow_ok = true;
     if (seg8 || conv_flow) {
@@ -2252,11 +2326,11 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
       std::vector<NarrowJob> jobs;
       uint16_t* h16 = ctx->h_flow16[buf];
       for (int i = 0; conv_flow && i < n16; ++i) {
-        if (i < nfwd) jobs.push_back({flow_fwd + fl * (s0 + i), h16 + fl * i, fl, true});
-        jobs.push_back({flow_bwd + fl * (s0 + 1 + i), h16 + fl * (cs + i), fl, true});
+        if (i < nfwd) jobs.push_back({flow_fwd + fl * (s0 + i - fe), h16 + fl * i, fl, true});
+        jobs.push_back({flow_bwd + fl * (s0 + 1 + i - fe), h16 + fl * (cs + i), fl, true});
       }
       for (int f = f0; seg8 && f < f1; ++f)                         // pinned label staging: frame f at f - f0
-        if (lab_rd(f)) jobs.push_back({seg + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw, false});
+        if (lab_rd(f)) jobs.push_back({seg + hw * (f - head), ctx->h_seg8[buf] + hw * (f - f0), hw, false});
       flow_ok = host_narrow(ctx, jobs);
     }
     if (conv_flow && !flow_ok) n16 = 0;                            // a value with no finite half: the whole chunk as float32
@@ -2269,23 +2343,25 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
       h2d += fl * 2 * (n16_fwd + n16);
     }
     float* dflow = ctx->s_flow[buf];
-    if (nfwd > n16_fwd) {
-      CU_OK(cudaMemcpyAsync(dflow + fl * n16_fwd, flow_fwd + fl * (s0 + n16_fwd), fl * 4 * (nfwd - n16_fwd), cudaMemcpyHostToDevice, cp));
-      h2d += fl * 4 * (nfwd - n16_fwd);
+    if (carried) CU_OK(cudaMemcpyAsync(dflow, o->c_fwd, fl * 4, cudaMemcpyDeviceToDevice, cp));
+    const int fwd0 = std::max(n16_fwd, carried);                   // first fwd slot entry copied as float32
+    if (nfwd > fwd0) {
+      CU_OK(cudaMemcpyAsync(dflow + fl * fwd0, flow_fwd + fl * (s0 + fwd0 - fe), fl * 4 * (nfwd - fwd0), cudaMemcpyHostToDevice, cp));
+      h2d += fl * 4 * (nfwd - fwd0);
     }
     if (need_bwd && ns > n16) {
-      CU_OK(cudaMemcpyAsync(dflow + fl * (cs + n16), flow_bwd + fl * (s0 + 1 + n16), fl * 4 * (ns - n16), cudaMemcpyHostToDevice, cp));
+      CU_OK(cudaMemcpyAsync(dflow + fl * (cs + n16), flow_bwd + fl * (s0 + 1 + n16 - fe), fl * 4 * (ns - n16), cudaMemcpyHostToDevice, cp));
       h2d += fl * 4 * (ns - n16);
     }
     if (seg8) {
       if (int rc = runs(f0, f1, lab_rd, [&](int f, int n) -> int {
-            CU_OK(cudaMemcpyAsync(ctx->q_seg8[set] + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw * n, cudaMemcpyHostToDevice, cp));
+            CU_OK(cudaMemcpyAsync(q_seg8 + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw * n, cudaMemcpyHostToDevice, cp));
             h2d += hw * n;
             return 0;
           })) return rc;
     } else if (r.labels) {
       if (int rc = runs(f0, f1, lab_rd, [&](int f, int n) -> int {
-            CU_OK(cudaMemcpyAsync(ctx->q_seg[set] + hw * f, seg + hw * f, hw * 4 * n, cudaMemcpyHostToDevice, cp));
+            CU_OK(cudaMemcpyAsync(q_seg + hw * f, seg + hw * (f - head), hw * 4 * n, cudaMemcpyHostToDevice, cp));
             h2d += hw * 4 * n;
             return 0;
           })) return rc;
@@ -2296,23 +2372,48 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
     CU_OK(cudaStreamWaitEvent(st, ctx->ev_copied[buf], 0));
     // the chunk's view: sample 0 is sequence sample s0; a flow_fwd the chunk does not read stands in as its flow_bwd
     // (davo_profile_layers re-runs every pair of the last chunk)
-    in = sequence_view(c.H, c.W, ctx->q_img[set] + hw * 3 * s0, nfwd ? dflow : dflow + fl * cs, dflow + fl * cs,
-                       seg8 ? nullptr : (ctx->q_seg[set] ? ctx->q_seg[set] + hw * s0 : nullptr),
-                       seg8 ? ctx->q_seg8[set] + hw * s0 : nullptr, ctx->q_depth[set] ? ctx->q_depth[set] + hw * s0 : nullptr,
+    in = sequence_view(c.H, c.W, q_img + hw * 3 * s0, nfwd ? dflow : dflow + fl * cs, dflow + fl * cs,
+                       seg8 ? nullptr : (q_seg ? q_seg + hw * s0 : nullptr),
+                       seg8 ? q_seg8 + hw * s0 : nullptr, q_depth ? q_depth + hw * s0 : nullptr,
                        n16 > 0 ? (n16_fwd > 0 ? ctx->s_flow16[buf] : ctx->s_flow16[buf] + fl * cs) : nullptr,
                        n16 > 0 ? ctx->s_flow16[buf] + fl * cs : nullptr, n16);
     const int chunk_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && s0 > 0) ? DAVO_PAIRS_TRAJECTORY : pairs;
-    if (int rc = host_run_chunk(ctx, chunk_pairs, s0, ns, in, st, &launches, &last_n)) return rc;
+    if (ns > 0)
+      if (int rc = host_run_chunk(ctx, chunk_pairs, s0, ns, in, st, &launches, &last_n)) return rc;
     CU_OK(cudaEventRecord(ctx->ev_consumed[buf], st));
   }
-  CU_OK(cudaEventRecord(ctx->ev_q_done[set], st));
-  if (int rc = host_finish(ctx, B, pose_out, st, ticket)) return rc;
-  ctx->last_launches = launches;
-  ctx->last_npairs_mb = last_n;
+  if (o) {
+    // carried state for the next push: the last two frames from the set, and the last flow_fwd entry (virtual entry
+    // n_frames - 2, which no sample of this push reads) when the sample that reads it is computed later
+    const int nc = std::min(n_frames, 2), fc = n_frames - nc;
+    CU_OK(cudaMemcpyAsync(o->c_img, q_img + hw * 3 * fc, hw * 3 * nc, cudaMemcpyDeviceToDevice, cp));
+    if (seg8) CU_OK(cudaMemcpyAsync(o->c_seg8, q_seg8 + hw * fc, hw * nc, cudaMemcpyDeviceToDevice, cp));
+    else if (r.labels) CU_OK(cudaMemcpyAsync(o->c_seg, q_seg + hw * fc, hw * 4 * nc, cudaMemcpyDeviceToDevice, cp));
+    if (r.depth) CU_OK(cudaMemcpyAsync(o->c_depth, q_depth + hw * fc, hw * 4 * nc, cudaMemcpyDeviceToDevice, cp));
+    const int e = n_frames - 2;
+    if (e >= fe && rg.fwd(glob(e))) {
+      CU_OK(cudaMemcpyAsync(o->c_fwd, flow_fwd + fl * (e - fe), fl * 4, cudaMemcpyHostToDevice, cp));
+      h2d += fl * 4;
+    }
+  }
+  CU_OK(cudaEventRecord(ev_q_done, st));
+  if (o && B > 0) {                                                // this push's absolute poses, after the last pass
+    const int first = op->g0 == 0, m = B + first;
+    pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(ctx->s_pose, B, first, o->d_rel);
+    CU_OK(cudaGetLastError());
+    traj_extend_kernel<<<1, 32, 0, st>>>(o->d_rel, m, first, o->d_P, o->d_traj);
+    CU_OK(cudaGetLastError());
+  }
+  if (int rc = host_finish(ctx, B, pose_out, st, ticket, o ? reinterpret_cast<double*>(o->d_traj) : nullptr,
+                           op ? op->traj_out : nullptr, op ? op->n_traj : 0)) return rc;
   ctx->last_h2d = (long long)h2d;
-  ctx->last_in = in;
-  ctx->last_pose = ctx->s_pose; ctx->last_B = last_ns;
-  ctx->last_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && chunk > 1) ? DAVO_PAIRS_TRAJECTORY : pairs;
+  if (B > 0) {                                                     // a push without samples ran no forward
+    ctx->last_launches = launches;
+    ctx->last_npairs_mb = last_n;
+    ctx->last_in = in;
+    ctx->last_pose = ctx->s_pose; ctx->last_B = last_ns;
+    ctx->last_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && chunk > 1) ? DAVO_PAIRS_TRAJECTORY : pairs;
+  }
   return 0;
 }
 
@@ -2321,6 +2422,187 @@ extern "C" int davo_forward_sequence_host(davo_ctx* ctx, int n_frames, int pairs
                                           void* stream, long long* ticket) {
   if (!ctx) return DAVO_ERR_ARG;
   return forward_sequence_host_impl(ctx, n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out, stream, ticket);
+}
+
+// ---- online odometry sessions (include/davo_b200.h: davo_odometry_*) ----
+static void odometry_free(davo_odometry* o) {
+  cudaSetDevice(o->ctx->device);
+  for (int i = 0; i < 2; ++i) {
+    cudaFree(o->q_img[i]); cudaFree(o->q_seg8[i]); cudaFree(o->q_seg[i]); cudaFree(o->q_depth[i]);
+    if (o->ev_q_done[i]) cudaEventDestroy(o->ev_q_done[i]);
+  }
+  cudaFree(o->c_img); cudaFree(o->c_seg8); cudaFree(o->c_seg); cudaFree(o->c_depth); cudaFree(o->c_fwd);
+  cudaFree(o->d_P); cudaFree(o->d_rel); cudaFree(o->d_traj); cudaFree(o->d_fwd);
+  delete o;
+}
+
+extern "C" int davo_odometry_create(davo_ctx* ctx, int max_push, int pairs, int host_inputs, davo_odometry** out) {
+  if (!ctx) return DAVO_ERR_ARG;
+  const char* who = "davo_odometry_create";
+  if (!out) return fail(ctx, DAVO_ERR_ARG, "%s: out is NULL", who);
+  *out = nullptr;
+  if (!ctx->finalized) return fail(ctx, DAVO_ERR_STATE, "%s: weights not finalized", who);
+  if (ctx->cfg.batch_norm)
+    return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm normalises with the statistics of the samples that share a call, so its poses depend on how the stream is cut into pushes; a session does not take it", who);
+  if (pairs != DAVO_PAIRS_TRAJECTORY && pairs != DAVO_PAIRS_ALL)
+    return fail(ctx, DAVO_ERR_ARG, "%s: pairs %d: a session takes DAVO_PAIRS_TRAJECTORY or DAVO_PAIRS_ALL", who, pairs);
+  if (max_push < 1 || max_push > ctx->cfg.max_batch)
+    return fail(ctx, DAVO_ERR_ARG, "%s: max_push=%d outside 1..max_batch %d", who, max_push, ctx->cfg.max_batch);
+  CU_OK(cudaSetDevice(ctx->device));
+  davo_odometry* o = new davo_odometry;
+  o->ctx = ctx; o->max_push = max_push; o->pairs = pairs; o->host = host_inputs != 0;
+  const davo_config& c = ctx->cfg;
+  const SeqReads r = seq_reads(ctx, pairs);
+  const size_t hw = (size_t)c.H * c.W, nf = (size_t)max_push + 2;
+  const bool seg8 = o->host && ctx->host_seg8;                     // the form the passes read the labels in
+  auto alloc = [&](void** p, size_t bytes) -> int {
+    CU_OK(cudaMalloc(p, bytes));
+    return 0;
+  };
+  int rc = alloc((void**)&o->c_img, hw * 3 * 2);
+  if (!rc && c.att_src != 0) rc = seg8 ? alloc((void**)&o->c_seg8, hw * 2) : alloc((void**)&o->c_seg, hw * 4 * 2);
+  if (!rc && r.depth) rc = alloc((void**)&o->c_depth, hw * 4 * 2);
+  if (!rc && r.flow) rc = alloc((void**)&o->c_fwd, hw * 2 * 4);
+  if (!rc) rc = alloc((void**)&o->d_P, 16 * sizeof(double));
+  if (!rc) rc = alloc((void**)&o->d_rel, (size_t)(max_push + 1) * sizeof(Mat4));
+  if (!rc && o->host) rc = alloc((void**)&o->d_traj, (size_t)(max_push + 2) * sizeof(Mat4));
+  if (!rc && !o->host) {                                           // one frame set, filled on the caller's stream
+    rc = alloc((void**)&o->q_img[0], nf * hw * 3);
+    if (!rc && c.att_src != 0) rc = alloc((void**)&o->q_seg[0], nf * hw * 4);
+    if (!rc && r.depth) rc = alloc((void**)&o->q_depth[0], nf * hw * 4);
+    if (!rc && r.flow) rc = alloc((void**)&o->d_fwd, (size_t)(max_push + 1) * hw * 2 * 4);
+  }
+  if (rc) { odometry_free(o); return rc; }
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    g_odo_live.insert(o);
+  }
+  *out = o;
+  return 0;
+}
+
+extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
+                                  const float* seg, const float* depth, float* pose_out, double* traj_out, int* n_samples,
+                                  int* n_traj, void* stream, long long* ticket) {
+  const char* who = "davo_odometry_push";
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    if (!o || !g_odo_live.count(o)) return fail(nullptr, DAVO_ERR_ARG, "%s: the session is NULL or was destroyed", who);
+  }
+  davo_ctx* ctx = o->ctx;
+  const davo_config& c = ctx->cfg;
+  if (k < 1 || k > o->max_push) return fail(ctx, DAVO_ERR_ARG, "%s: k=%d new frames outside 1..max_push %d", who, k, o->max_push);
+  if (ticket && !o->host) return fail(ctx, DAVO_ERR_ARG, "%s: ticket: a device session runs on the caller's stream; only host sessions take a ticket", who);
+  const long long f0 = o->pushed;
+  const int head = o->head(), fe = head == 2 ? 1 : 0, n = head + k, ns = std::max(0, n - 2);
+  const long long g0 = f0 - head;
+  const int first = g0 == 0 && ns > 0, nt = ns + 2 * first;
+  const int vpairs = o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : first ? DAVO_PAIRS_TRAJECTORY_FIRST : DAVO_PAIRS_TRAJECTORY;
+  // what the stream reads of this push's flow entries: flow_fwd global entry e is read by sample e (as its plane 0)
+  // now or later, flow_bwd entry e by sample e - 1 (plane 1), which is computed now when it exists
+  const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
+  const long long e0 = std::max(f0 - 1, 0LL), e1 = f0 + k - 1;    // global flow entries [e0, e1) arrive with this push
+  const bool fwd_read = rg.flow && e1 > e0 && rg.k0((int)std::min(e0, 2LL));
+  const bool bwd_read = rg.flow && ns > 0;
+  struct { const void* p; bool needed; const char* name; } in[] = {
+      {img, true, "img"}, {pose_out, ns > 0, "pose_out"}, {traj_out, nt > 0, "traj_out"}, {seg, c.att_src != 0, "seg"},
+      {depth, rg.depth, "depth"}, {flow_bwd, bwd_read, "flow_bwd"}, {flow_fwd, fwd_read, "flow_fwd"}};
+  for (const auto& x : in) {
+    if (x.needed && !x.p) return fail(ctx, DAVO_ERR_ARG, "%s: %s is NULL; this variant and pair selection read it", who, x.name);
+    if (x.p && (reinterpret_cast<uintptr_t>(x.p) & 15)) return fail(ctx, DAVO_ERR_ARG, "%s: %s is not 16-byte aligned", who, x.name);
+  }
+  CU_OK(cudaSetDevice(ctx->device));
+  if (o->host) {
+    OdoPush op{o, head, fe, g0, traj_out, nt};
+    if (int rc = forward_sequence_host_impl(ctx, n, vpairs, img, flow_fwd, flow_bwd, seg, depth, pose_out, stream, ticket, &op))
+      return rc;
+  } else {
+    // the carried frames and the pushed ones into the session's set, the carried flow_fwd entry in front of the pushed
+    // ones, all on the caller's stream (which orders the caller's buffers); then the passes of davo_forward_sequence
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    const SeqReads r = seq_reads(ctx, vpairs);
+    const size_t hw = (size_t)c.H * c.W, fl = hw * 2;
+    auto d2d = [&](void* dst, const void* src, size_t bytes) -> int {
+      if (bytes) CU_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st));
+      return 0;
+    };
+    const bool labels = c.att_src != 0;
+    int rc = d2d(o->q_img[0], o->c_img, hw * 3 * head);
+    if (!rc) rc = d2d(o->q_img[0] + hw * 3 * head, img, hw * 3 * k);
+    if (!rc && labels) rc = d2d(o->q_seg[0], o->c_seg, hw * 4 * head);
+    if (!rc && labels) rc = d2d(o->q_seg[0] + hw * head, seg, hw * 4 * k);
+    if (!rc && r.depth) rc = d2d(o->q_depth[0], o->c_depth, hw * 4 * head);
+    if (!rc && r.depth) rc = d2d(o->q_depth[0] + hw * head, depth, hw * 4 * k);
+    // virtual flow entry v is the caller's entry v - fe; plane 1 of sample s is virtual flow_bwd entry s + 1
+    const float* fwd = flow_fwd;
+    if (!rc && fe && ns > 0 && r.fwd(0)) {
+      const int nfwd = r.k0(ns - 1) ? ns : 1;
+      rc = d2d(o->d_fwd, o->c_fwd, fl * 4);
+      if (!rc) rc = d2d(o->d_fwd + fl, flow_fwd, fl * 4 * (nfwd - 1));
+      fwd = o->d_fwd;
+    }
+    const float* bwd1 = flow_bwd ? flow_bwd + fl * (1 - fe) : nullptr;
+    if (!rc && ns > 0) {
+      const InputView v = sequence_view(c.H, c.W, o->q_img[0], fwd ? fwd : bwd1, bwd1, labels ? o->q_seg[0] : nullptr, nullptr,
+                                        o->q_depth[0], nullptr, nullptr, 0);
+      rc = forward_device(ctx, who, ns, vpairs, v, pose_out, st);
+    }
+    const int nc = std::min(n, 2), fc = n - nc;
+    if (!rc) rc = d2d(o->c_img, o->q_img[0] + hw * 3 * fc, hw * 3 * nc);
+    if (!rc && labels) rc = d2d(o->c_seg, o->q_seg[0] + hw * fc, hw * 4 * nc);
+    if (!rc && r.depth) rc = d2d(o->c_depth, o->q_depth[0] + hw * fc, hw * 4 * nc);
+    const int e = n - 2;                                           // the last flow_fwd entry, read by a later sample
+    if (!rc && e >= fe && rg.fwd((int)std::min(g0 + e, 2LL))) rc = d2d(o->c_fwd, flow_fwd + fl * (e - fe), fl * 4);
+    if (rc) return rc;
+    if (ns > 0) {
+      const int m = ns + first;
+      pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(pose_out, ns, first, o->d_rel);
+      CU_OK(cudaGetLastError());
+      traj_extend_kernel<<<1, 32, 0, st>>>(o->d_rel, m, first, o->d_P, reinterpret_cast<Mat4*>(traj_out));
+      CU_OK(cudaGetLastError());
+    }
+  }
+  o->pushed += k;
+  o->posed += nt;
+  if (n_samples) *n_samples = ns;
+  if (n_traj) *n_traj = nt;
+  return 0;
+}
+
+extern "C" int davo_odometry_reset(davo_odometry* o) {
+  std::lock_guard<std::mutex> lk(g_odo_mutex);
+  if (!o || !g_odo_live.count(o)) return fail(nullptr, DAVO_ERR_ARG, "davo_odometry_reset: the session is NULL or was destroyed");
+  o->pushed = 0; o->posed = 0;
+  return 0;
+}
+
+extern "C" int davo_odometry_frames(const davo_odometry* o, long long* pushed, long long* posed) {
+  std::lock_guard<std::mutex> lk(g_odo_mutex);
+  if (!o || !g_odo_live.count(const_cast<davo_odometry*>(o)))
+    return fail(nullptr, DAVO_ERR_ARG, "davo_odometry_frames: the session is NULL or was destroyed");
+  if (pushed) *pushed = o->pushed;
+  if (posed) *posed = o->posed;
+  return 0;
+}
+
+extern "C" void davo_odometry_destroy(davo_odometry* o) {
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    if (!o || !g_odo_live.erase(o)) return;
+  }
+  cudaSetDevice(o->ctx->device);
+  cudaDeviceSynchronize();                                         // work still queued may read the session's buffers
+  odometry_free(o);
+}
+
+// davo_destroy: the handle's sessions go with it
+static void destroy_sessions_of(davo_ctx* ctx) {
+  std::vector<davo_odometry*> mine;
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    for (davo_odometry* o : g_odo_live) if (o->ctx == ctx) mine.push_back(o);
+  }
+  for (davo_odometry* o : mine) davo_odometry_destroy(o);
 }
 
 extern "C" int davo_last_host_copy_bytes(const davo_ctx* ctx, long long* h2d, long long* d2h) {
@@ -2628,7 +2910,7 @@ extern "C" int davo_compose_trajectory(davo_ctx* ctx, const float* poses, int n,
   const int m = n + 1;                                   // relative motions
   if (int rc = traj_scratch(ctx, (size_t)m * sizeof(Mat4))) return rc;
   Mat4* rel = reinterpret_cast<Mat4*>(ctx->d_traj_scratch);
-  pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(poses, n, rel);
+  pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(poses, n, 1, rel);
   CU_OK(cudaGetLastError());
   const int threads = 256, chunk = (m + threads - 1) / threads;
   traj_scan_kernel<<<1, threads, threads * 16 * sizeof(double), st>>>(rel, m, chunk, reinterpret_cast<Mat4*>(traj));

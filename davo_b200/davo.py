@@ -426,6 +426,13 @@ class DAVO(object):
                     "davo_forward_sequence_host")
         return DAVO._Pending(self, ticket.value, out, (img, flow_fwd, flow_bwd, seg, depth))
 
+    def odometry(self, pairs='trajectory', max_push=None, host=True):
+        """An online odometry session on this handle (include/davo_b200.h: davo_odometry_*): push frames as they
+        arrive, get every frame's absolute pose.  ``pairs``: ``'trajectory'`` (what the trajectory reads) or ``'all'``;
+        ``max_push``: most frames per push (default: the handle's batch size); ``host``: pushes take numpy arrays and
+        return numpy arrays, else CUDA tensors in and out."""
+        return Odometry(self, pairs, self.batch_size if max_push is None else max_push, host)
+
     def bind_host_numa(self):
         """Bind this thread (and threads created after it) to the CPUs next to this handle's GPU
         (``davo_bind_host_numa``); call it before allocating pinned inputs.  Returns the NUMA node or -1."""
@@ -514,6 +521,141 @@ class DAVO(object):
         if self._h is not None and self._lib is not None:
             self._lib.davo_destroy(self._h)
             self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Odometry(object):
+    """An online odometry session (``DAVO.odometry``).  ``push(img, flow_fwd, flow_bwd, seg, depth=None)`` takes the next
+    k frames of the sequence: ``img`` uint8 [k,H,W,3], ``seg`` / ``depth`` float32 [k,H,W,1], ``flow_fwd`` / ``flow_bwd``
+    float32 [k',H,W,2] with k' = k, or k-1 on the first push (entry j: the flow between the frame before frame j of the
+    push and frame j; on the first push between frames j and j+1).  It returns ``{'pose': [n_s,2,6], 'trajectory':
+    [n_t,4,4] float64, 'frames': range of the frame indices of the trajectory rows}``: the poses of the samples whose
+    last frame is new and the absolute poses that became known.  ``push_async`` queues a host push and returns a handle
+    whose ``.result()`` gives that dict (the inputs must stay unmodified until then; up to 8 in flight)."""
+
+    def __init__(self, system, pairs, max_push, host):
+        if pairs not in ('trajectory', 'all'):
+            raise ValueError("DAVO.odometry: pairs must be 'trajectory' or 'all'")
+        if not system._weights_loaded:
+            raise RuntimeError("DAVO.odometry: weights not loaded")
+        self._system, self._host, self._pushed, self._posed = system, bool(host), 0, 0
+        self._ring, self._ring_n = None, 0
+        h = C.c_void_p()
+        system._check(system._lib.davo_odometry_create(system._h, int(max_push), _capi.PAIRS[pairs], int(self._host),
+                                                       C.byref(h)), "davo_odometry_create")
+        self._o, self.max_push = h, int(max_push)
+
+    def _counts(self, k):
+        f0 = self._pushed
+        ns = max(0, f0 + k - 2) - max(0, f0 - 2)
+        return ns, ns + 2 if (f0 <= 2 and ns > 0) else ns
+
+    def _args(self, img, flow_fwd, flow_bwd, seg, depth):
+        s = self._system
+        if self._o is None:
+            raise RuntimeError("Odometry.push: the session is closed")
+        if s.config.att_src != V.ATT_SE_DEPTH_SEG and not s.config.depth_split:
+            depth = None
+        elif depth is None:
+            raise ValueError("Odometry.push: version %r reads depth [k,H,W,1]" % (s.version,))
+        k, H, W = int(img.shape[0]), s.img_height, s.img_width
+        kf = k if self._pushed > 0 else k - 1
+        want = {"img": (k, H, W, 3), "flow_fwd": (kf, H, W, 2), "flow_bwd": (kf, H, W, 2), "seg": (k, H, W, 1),
+                "depth": (k, H, W, 1)}
+        for name, t in (("img", img), ("flow_fwd", flow_fwd), ("flow_bwd", flow_bwd), ("seg", seg), ("depth", depth)):
+            if t is not None and tuple(t.shape) != want[name]:
+                raise ValueError("Odometry.push: %s has shape %s, expected %s" % (name, tuple(t.shape), want[name]))
+        return k, depth
+
+    def _call(self, k, ins, pose, traj, stream, ticket):
+        s = self._system
+        ns, nt = C.c_int(0), C.c_int(0)
+        s._check(s._lib.davo_odometry_push(self._o, k, *ins, pose, traj, C.byref(ns), C.byref(nt), stream, ticket),
+                 "davo_odometry_push")
+        frames = range(self._posed, self._posed + nt.value)
+        self._pushed += k
+        self._posed += nt.value
+        return frames
+
+    def push_async(self, img, flow_fwd, flow_bwd, seg=None, depth=None, _block=False):
+        k, depth = self._args(img, flow_fwd, flow_bwd, seg, depth)
+        n_s, n_t = self._counts(k)
+        if not self._host:
+            import torch
+            dev = "cuda:%d" % self._system.device
+            for name, t, dt in (("img", img, torch.uint8), ("flow_fwd", flow_fwd, torch.float32),
+                                ("flow_bwd", flow_bwd, torch.float32), ("seg", seg, torch.float32),
+                                ("depth", depth, torch.float32)):
+                if t is not None and not (_is_torch(t) and t.is_cuda and t.device.index == self._system.device
+                                          and t.dtype == dt and t.is_contiguous()):
+                    raise ValueError("Odometry.push: %s must be a contiguous %s tensor on %s" % (name, dt, dev))
+            pose = torch.zeros((n_s, 2, 6), dtype=torch.float32, device=dev)
+            traj = torch.empty((n_t, 4, 4), dtype=torch.float64, device=dev)
+            ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None and t.numel() else None
+            stream = torch.cuda.current_stream(self._system.device).cuda_stream
+            frames = self._call(k, [ptr(t) for t in (img, flow_fwd, flow_bwd, seg, depth)], ptr(pose), ptr(traj),
+                                C.c_void_p(stream), None)
+            return Odometry._Pending(None, {'pose': pose, 'trajectory': traj, 'frames': frames}, None)
+        arr = lambda a, dt: None if a is None else np.ascontiguousarray(a, dtype=dt)
+        ins = (arr(img, np.uint8), arr(flow_fwd, np.float32), arr(flow_bwd, np.float32), arr(seg, np.float32),
+               arr(depth, np.float32))
+        hp = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None and a.size else None
+        if _block:
+            pose, traj = np.zeros((n_s, 2, 6), np.float32), np.empty((n_t, 4, 4), np.float64)
+            frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, None)
+            return Odometry._Pending(None, {'pose': pose, 'trajectory': traj, 'frames': frames}, None)
+        import torch
+        if self._ring is None:                      # page-locked results, one slot per call that can be in flight
+            self._ring = [(torch.empty((self.max_push, 2, 6), dtype=torch.float32).pin_memory(),
+                           torch.empty((self.max_push + 2, 4, 4), dtype=torch.float64).pin_memory()) for _ in range(8)]
+        slot = self._ring[self._ring_n % 8]
+        self._ring_n += 1
+        pose, traj = slot[0][:n_s].numpy(), slot[1][:n_t].numpy()
+        ticket = C.c_longlong(0)
+        frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, C.byref(ticket))
+        return Odometry._Pending(self._system, {'pose': pose, 'trajectory': traj, 'frames': frames}, ticket.value, ins)
+
+    def push(self, img, flow_fwd, flow_bwd, seg=None, depth=None):
+        return self.push_async(img, flow_fwd, flow_bwd, seg, depth, _block=True).result()
+
+    class _Pending(object):
+        def __init__(self, system, out, ticket=None, keep=None):
+            self._system, self._out, self._ticket, self._keep = system, out, ticket, keep
+
+        def result(self):
+            if self._ticket is not None:
+                s = self._system
+                s._check(s._lib.davo_host_wait(s._h, self._ticket), "davo_host_wait")
+                self._ticket, self._keep = None, None
+                self._out = {'pose': np.array(self._out['pose']), 'trajectory': np.array(self._out['trajectory']),
+                             'frames': self._out['frames']}           # own copies: the pinned ring slot is reused
+            return self._out
+
+    def frames(self):
+        """(frames pushed, frames whose absolute pose has been returned)."""
+        return self._pushed, self._posed
+
+    def reset(self):
+        """The next push is frame 0 of a new sequence."""
+        if self._o is not None:
+            self._system._check(self._system._lib.davo_odometry_reset(self._o), "davo_odometry_reset")
+        self._pushed, self._posed = 0, 0
+
+    def close(self):
+        if self._o is not None and self._system._h is not None:
+            self._system._lib.davo_odometry_destroy(self._o)
+        self._o = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
 
     def __del__(self):
         try:

@@ -225,6 +225,49 @@ int davo_forward_sequence_host(davo_ctx*, int n_frames, int pairs, const uint8_t
                                const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
                                void* cuda_stream, long long* ticket);
 
+/* --- online odometry sessions ---
+ * A camera loop: push frames as they arrive, get each frame's absolute pose, composed on the device.  A session
+ * belongs to one handle and takes one sequence in order, k >= 1 new frames per push.  With f0 frames pushed so far, a
+ * push carries frames f0 .. f0+k-1 in the layouts of davo_forward_sequence:
+ *   img       uint8 [k,H,W,3];  seg float [k,H,W,1] (NULL for variants without attention source);  depth float
+ *             [k,H,W,1] (depth sources only)
+ *   flow_fwd, flow_bwd  float [k',H,W,2], k' = k (k-1 on the first push): entry j is the sequence's flow entry
+ *             f0-1+j (j on the first push), i.e. a push is img[a:b], flow[a-1:b-1] of a whole-sequence call
+ *             (flow[0:b-1] for the first).  A flow no computed pair reads may be NULL, as in davo_forward_sequence.
+ * It computes every sample whose last frame is new (s+2 in [f0, f0+k): none for a first push of 1 or 2 frames):
+ *   pose_out  float [n_samples,2,6]  rows and columns of davo_forward_pairs; under DAVO_PAIRS_TRAJECTORY only
+ *             pose[s][1], plus pose[0][0] for sample 0 (the trajectory reads it)
+ *   traj_out  double [n_traj,4,4]    absolute poses of the frames whose pose became known: frames 0, 1, 2 with
+ *             sample 0 (P_0 = I, P_1 = T(pose[0][0])), then frame s+2 for sample s, P_{s+2} = P_{s+1} . inv(T(pose[s][1]))
+ *             -- the loop of reference test_kitti_pose.py:136-149 with T = pose_vec2mat in fp32, chained in fp64 in
+ *             frame order, so the bits do not depend on how the stream is cut into pushes
+ * The poses equal davo_forward_sequence over the whole sequence (DAVO_PAIRS_TRAJECTORY_FIRST or DAVO_PAIRS_ALL) bit
+ * for bit for every cut; each frame, label plane, depth plane and flow entry a computed pair reads is sent once over
+ * the whole stream (davo_last_host_copy_bytes counts a host push's bytes).  The session keeps the last two frames, the
+ * last flow_fwd entry when a later sample reads it and the last absolute pose in buffers of its own: sessions on one
+ * handle are independent, and other calls on the handle may run between pushes.
+ *
+ * davo_odometry_create: max_push = most frames per push (1..max_batch); pairs = DAVO_PAIRS_TRAJECTORY or
+ *   DAVO_PAIRS_ALL; host_inputs = 1: pushes pass host buffers and get host results (chunked, copies under compute,
+ *   CPU narrowing, as davo_forward_sequence_host); 0: device buffers in, device results out, asynchronous on
+ *   cuda_stream.  -batch_norm is refused (its poses depend on which samples share a call).
+ * davo_odometry_push: *n_samples / *n_traj (either may be NULL) receive the counts.  Host sessions: ticket == NULL
+ *   blocks until the results are in pose_out / traj_out; otherwise they must be page-locked, the call returns once
+ *   queued, and davo_host_wait(ctx, *ticket) waits for it.  Argument errors (k outside 1..max_push, a NULL input the
+ *   variant and selection read, a misaligned buffer, a ticket on a device session, a destroyed session) return
+ *   DAVO_ERR_ARG with a message naming the input (davo_last_error(NULL) for a destroyed session).
+ * davo_odometry_reset: the next push is frame 0 of a new sequence (P_0 = I).
+ * davo_odometry_frames: frames pushed, and frames whose absolute pose has been written.
+ * davo_odometry_destroy: waits for the device and frees the session; davo_destroy destroys the handle's sessions. */
+typedef struct davo_odometry davo_odometry;
+int davo_odometry_create(davo_ctx*, int max_push, int pairs, int host_inputs, davo_odometry** out);
+int davo_odometry_push(davo_odometry*, int k, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
+                       const float* seg, const float* depth, float* pose_out, double* traj_out, int* n_samples,
+                       int* n_traj, void* cuda_stream, long long* ticket);
+int davo_odometry_reset(davo_odometry*);
+int davo_odometry_frames(const davo_odometry*, long long* pushed, long long* posed);
+void davo_odometry_destroy(davo_odometry*);
+
 /* Binds the calling thread (and the threads it creates afterwards: the handle's conversion pool, the caller's
  * loader threads) to the CPUs of the NUMA node the handle's GPU hangs off (/sys/bus/pci/devices/<id>/numa_node,
  * local_cpulist), so that pinned staging allocated afterwards is first-touched next to the GPU and the conversion
