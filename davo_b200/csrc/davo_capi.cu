@@ -2625,20 +2625,37 @@ extern "C" int davo_get_intermediate(davo_ctx* ctx, const char* name, int pair, 
   const float* src = nullptr;
   int64_t n = 0;
   std::string s(name);
+  // A caller whose buffer is too small learns the size it needs from *n_out.
+  auto too_small = [&](int64_t need) {
+    *n_out = need;
+    return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: buffer too small (%lld < %lld)", (long long)cap, (long long)need);
+  };
+  // the fused cnv1 never writes the packed input: pack8_kernel, the same arithmetic (frontend.cuh: pack8_quad), on the last pass's inputs
+  auto materialise_packed = [&]() -> int {
+    if (ctx->fuse_front && ctx->conv_impl == 0 && ctx->layers[0].fused_front) {
+      if (int rc = launch_k(ctx, pack8_kernel, dim3(pack8_blocks(ctx->fp_cur.npairs), ctx->fp_cur.npairs), dim3(256), 0, (cudaStream_t)0, false, ctx->fp_cur)) return rc;
+      CU_OK(cudaDeviceSynchronize());
+    }
+    return 0;
+  };
+  const size_t colon = s.find(':');
+  const std::string lname = s.substr(0, colon), part = colon == std::string::npos ? "" : s.substr(colon + 1);
+  int li = -1;
+  for (int i = 0; i < (int)ctx->layers.size(); ++i) if (lname == ctx->layers[i].name) li = i;
   if (s == "att_weights") {
     n = kNumClasses;
-    if (cap < n) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: buffer too small");
+    if (cap < n) return too_small(n);
     if (c.att_src == 1 || c.att_src >= 3) src = ctx->d_attw + (size_t)pair * kAttFrames * kAttStride;
     else if (c.att_src == 2) src = ctx->d_staticw;
     else { for (int i = 0; i < n; ++i) out[i] = 1.0f; *n_out = n; return 0; }
   }
   else if (s == "packed") {
     n = (int64_t)c.H * c.W * ctx->packed_c; src = ctx->d_packed + (size_t)pair * n;
-    if (ctx->fuse_front && ctx->conv_impl == 0 && ctx->layers[0].fused_front) {
-      // the fused cnv1 never wrote it: pack8_kernel, the same arithmetic (frontend.cuh: pack8_quad), on the last pass's inputs
-      if (int rc = launch_k(ctx, pack8_kernel, dim3(pack8_blocks(ctx->fp_cur.npairs), ctx->fp_cur.npairs), dim3(256), 0, (cudaStream_t)0, false, ctx->fp_cur)) return rc;
-      CU_OK(cudaDeviceSynchronize());
-    }
+    if (int rc = materialise_packed()) return rc;
+  }
+  else if (s == "se5_scale") {
+    if (!ctx->d_se5scale) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: se5_scale: this variant has no SE block on cnv5 / cnv6");
+    n = (int64_t)ctx->nbr * 256; src = ctx->d_se5scale + (size_t)pair * n;
   }
   else if (s == "cnv7_sum") {
     // reduce the deterministic partials on the host
@@ -2646,7 +2663,7 @@ extern "C" int davo_get_intermediate(davo_ctx* ctx, const char* name, int pair, 
     const int nbr = ctx->nbr;
     std::vector<float> tmp((size_t)nbr * np * 256);
     CU_OK(cudaMemcpy(tmp.data(), ctx->d_sum7 + (size_t)pair * nbr * np * 256, tmp.size() * 4, cudaMemcpyDeviceToHost));
-    if (cap < nbr * 256) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: buffer too small");
+    if (cap < nbr * 256) return too_small(nbr * 256);
     for (int br = 0; br < nbr; ++br)
       for (int ch = 0; ch < 256; ++ch) {
         float a = 0.f;
@@ -2655,18 +2672,66 @@ extern "C" int davo_get_intermediate(davo_ctx* ctx, const char* name, int pair, 
       }
     *n_out = nbr * 256;
     return 0;
-  } else {
-    for (int i = 0; i < 6; ++i)
-      if (s == ctx->layers[i].name) {
-        const Layer& L = ctx->layers[i];
-        if (L.pitched_out()) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s is stored with a padded pitch", L.name);
-        if (!L.d_out) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s is not computed by this variant", L.name);
+  } else if (li >= 0) {
+    const Layer& L = ctx->layers[li];
+    const bool rep6 = li == 5 && c.posenn_se == 3;          // -se_replace: no cnv6 convolution
+    if (part.empty() || part == "pitched") {
+      // the map [Hout][Wout][C] with the pad row / column of an odd map removed, or the whole [Hout_p][Wout_p][C] buffer
+      if (!L.d_out) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s is not stored by this variant", L.name);
+      const int64_t per = (int64_t)L.Hout_p * L.Wout_p * L.out_stride;
+      if (part == "pitched" || !L.pitched_out()) { n = per; src = L.d_out + (size_t)pair * per; }
+      else {
         n = (int64_t)L.Hout * L.Wout * L.out_stride;
-        src = L.d_out + (size_t)pair * n;
+        if (cap < n) return too_small(n);
+        const size_t row = (size_t)L.Wout * L.out_stride * 4;
+        CU_OK(cudaMemcpy2D(out, row, L.d_out + (size_t)pair * per, (size_t)L.Wout_p * L.out_stride * 4, row, L.Hout, cudaMemcpyDeviceToHost));
+        *n_out = n;
+        return 0;
       }
+    } else if (part == "in") {
+      // what the layer's kernel reads: [Hin_p][Win_p][Cin_total] (cnv1: the packed input; d_se5out under the SE variants)
+      if (rep6) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s is not computed by this variant", L.name);
+      n = (int64_t)L.Hin_p * L.Win_p * L.Cin_total; src = L.d_in + (size_t)pair * n;
+      if (li == 0)
+        if (int rc = materialise_packed()) return rc;
+    } else if (part == "b") {
+      // the bias the weight pack was built with (-batch_norm: beta; the conv itself adds nothing)
+      if (rep6) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s is not computed by this variant", L.name);
+      n = (int64_t)L.groups * L.BN; src = c.batch_norm ? L.d_beta : L.d_bias;
+    } else if (part.size() >= 2 && part[0] == 'w' && part.find_first_not_of("0123456789", 1) == std::string::npos) {
+      // TF32 weights of group g as the pack was built from them (round_weights_tf32), HWIO over the input tensor's
+      // channels of that group: [k][k][Cin_g][BN], zero for an input channel no weight reads (cnv1's packed layout)
+      const int g = atoi(part.c_str() + 1);
+      if (rep6) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s is not computed by this variant", L.name);
+      if (g >= L.groups) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s has %d group(s)", L.name, L.groups);
+      const int T = L.k * L.k;
+      n = (int64_t)T * L.Cin_g * L.BN;
+      if (cap < n) return too_small(n);
+      std::vector<float> hw((size_t)T * L.Cin_w * L.BN);
+      CU_OK(cudaMemcpy(hw.data(), L.d_whwio[g], hw.size() * 4, cudaMemcpyDeviceToHost));
+      for (int t = 0; t < T; ++t)
+        for (int j = 0; j < L.Cin_g; ++j) {
+          const int ci = li == 0 ? L.pc2w[j] : j;
+          for (int o = 0; o < L.BN; ++o) out[((size_t)t * L.Cin_g + j) * L.BN + o] = ci >= 0 ? hw[((size_t)t * L.Cin_w + ci) * L.BN + o] : 0.f;
+        }
+      *n_out = n;
+      return 0;
+    } else if (part == "plan") {
+      // the plan the last pass ran for this layer (its latency twin included)
+      if (rep6) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s is not computed by this variant", L.name);
+      const Layer& P = pick_layer(ctx, (size_t)li, ctx->last_npairs_mb);
+      const float v[] = {(float)P.orient, (float)P.npix, (float)P.wide_G, (float)P.wide_tw, (float)P.cm_staged,
+                         (float)P.cm_cluster, (float)P.strips, (float)P.m_blocks, (float)P.groups, (float)(c.batch_norm ? 1 : 0),
+                         (float)P.epi, (float)P.BN, (float)P.b_resident, (float)P.fused_front};
+      n = (int64_t)(sizeof v / sizeof v[0]);
+      if (cap < n) return too_small(n);
+      for (int i = 0; i < n; ++i) out[i] = v[i];
+      *n_out = n;
+      return 0;
+    }
   }
   if (!src) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: unknown name '%s'", name);
-  if (cap < n) return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: buffer too small (%lld < %lld)", (long long)cap, (long long)n);
+  if (cap < n) return too_small(n);
   CU_OK(cudaMemcpy(out, src, (size_t)n * 4, cudaMemcpyDeviceToHost));
   *n_out = n;
   return 0;

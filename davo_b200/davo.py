@@ -440,11 +440,16 @@ class DAVO(object):
 
     # ------------------------------------------------------ test / debug taps
     def get_intermediate(self, name: str, pair: int) -> np.ndarray:
+        """What the last forward left for ``pair`` under ``name`` (include/davo_b200.h: davo_get_intermediate), flat."""
         buf = np.empty((self.img_height * self.img_width * 16,), np.float32)
         n = C.c_int64(0)
-        self._check(self._lib.davo_get_intermediate(self._h, name.encode(), pair,
-                                                    buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(n)),
-                    "davo_get_intermediate(%s)" % name)
+        rc = self._lib.davo_get_intermediate(self._h, name.encode(), pair, buf.ctypes.data_as(C.c_void_p), buf.size,
+                                             C.byref(n))
+        if rc != 0 and n.value > buf.size:                   # the library names the size it needs
+            buf = np.empty((n.value,), np.float32)
+            rc = self._lib.davo_get_intermediate(self._h, name.encode(), pair, buf.ctypes.data_as(C.c_void_p), buf.size,
+                                                 C.byref(n))
+        self._check(rc, "davo_get_intermediate(%s)" % name)
         return buf[:n.value].copy()
 
     def last_host_copy_bytes(self):

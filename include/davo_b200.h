@@ -278,9 +278,25 @@ int davo_bind_host_numa(davo_ctx*);
 /* Test / mode='feature' access to what the last davo_forward left in the
  * workspace for frame pair `pair` (= 2*sample + source index) of the LAST
  * micro-batch: "att_weights" [19], "packed" [H,W,16], "cnv1".."cnv5",
- * "cnv6" [h,w,2*cnv6_out] (rotation | translation), "cnv7_sum" [2,256].
+ * "cnv6" [h,w,2*cnv6_out] (rotation | translation), "cnv7_sum" [2,256],
+ * "cnv7" where it is stored (-batch_norm: the plain conv sums), "se5_scale"
+ * [branches,256] (the excitation of -se_insert / -se_skipadd / -se_replace).
+ * Per conv layer "<layer>" also takes a suffix:
+ *   "<layer>"          the map [h,w,C]; an odd map stored with an even pitch
+ *                      comes back without its zero pad row / column;
+ *   "<layer>:pitched"  the whole stored buffer [h_p,w_p,C];
+ *   "<layer>:in"       the input the layer's kernel reads [h_in_p,w_in_p,C_in];
+ *   "<layer>:w<g>"     the TF32 weights of group g the kernel's weight pack was
+ *                      built from, HWIO over the group's input channels
+ *                      [k,k,C_in_g,C_out_g] (zero where no weight is read);
+ *   "<layer>:b"        the bias [groups*C_out_g] (-batch_norm: beta);
+ *   "<layer>:plan"     the plan the last pass ran: orient (0 pixels-on-M,
+ *                      1 channels-on-M), pixels per tile, widened G, widened
+ *                      runs per tile row, cm staged, cm cluster, strips,
+ *                      m-blocks, groups, raw (-batch_norm), epilogue (0 store,
+ *                      1 sum), C_out_g, weights resident, fused front end.
  * Copies to HOST memory `out` (capacity `cap` floats); writes the element
- * count to *n.  Synchronises. */
+ * count to *n, or the count needed when `cap` is too small.  Synchronises. */
 int davo_get_intermediate(davo_ctx*, const char* name, int pair, float* out,
                           int64_t cap, int64_t* n);
 
