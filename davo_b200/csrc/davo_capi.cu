@@ -2649,6 +2649,21 @@ extern "C" int davo_get_intermediate(davo_ctx* ctx, const char* name, int pair, 
     else if (c.att_src == 2) src = ctx->d_staticw;
     else { for (int i = 0; i < n; ++i) out[i] = 1.0f; *n_out = n; return 0; }
   }
+  else if (lname == "att_weights") {
+    // slot <k> of the unit's attention weights, laid out as unit_frame / pack_sample_kernel read them (frontend.cuh):
+    // the slots the SE kernels write, or the static table for every frame that has a map; anything else is refused
+    const int slot = (part.size() == 1 && part[0] >= '0' && part[0] <= '9') ? part[0] - '0' : -1;
+    const int src_frames = ctx->unit_sample ? 2 : 1;
+    const int nslots = c.att_src == 0 ? 0 : c.depth_split ? 2 * src_frames : src_frames + (c.att_tgt_ones ? 0 : 1);
+    if (slot < 0 || slot >= nslots)
+      return fail(ctx, DAVO_ERR_ARG, "davo_get_intermediate: %s: this variant computes %d attention-weight slot(s) per unit (%s)",
+                  name, nslots, ctx->unit_sample ? "0 src0, 1 src1, 2 target; depth split: 0/1 src0 near/far, 2/3 src1 near/far"
+                                                 : "0 source, 1 target or, under the depth split, the far table");
+    // width: 19 class weights, or the excitation of a per-pixel source (its SE input channels)
+    n = !c.pixel_map ? kNumClasses : c.pixel_map == 2 ? 3 : c.att_src == 4 ? 3 : c.att_src == 5 ? 1 : kNumClasses + 2;
+    if (cap < n) return too_small(n);
+    src = c.att_src == 2 ? ctx->d_staticw : ctx->d_attw + ((size_t)pair * kAttFrames + slot) * kAttStride;
+  }
   else if (s == "packed") {
     n = (int64_t)c.H * c.W * ctx->packed_c; src = ctx->d_packed + (size_t)pair * n;
     if (int rc = materialise_packed()) return rc;

@@ -84,7 +84,7 @@ struct FrontParams {
   float* pool_part;      // [mb][kAttFrames][kPoolSplits][kPoolDim]
   unsigned int* pool_count;  // [mb][kAttFrames], zero between launches
   float* att_w;          // [mb][kAttFrames][kAttStride], slots as in unit_frame
-  float* packed;         // [mb][H][W][16]
+  float* packed;         // [mb][H][W][packed_c]
 };
 
 // Label of pixel `pix` of plane `plane` (element offset of the plane = plane index * H*W) as the
@@ -580,7 +580,6 @@ __global__ void __launch_bounds__(256) pack_kernel(const FrontParams p) {
   }
   __syncthreads();
   const int lane = threadIdx.x & 31, j = lane & 3;
-  const float inv_w = 1.0f / (float)p.W;
   const uint8_t* img_t = frame_img(p.in, b, 1);                // tgt = centre frame
   const uint8_t* img_s = frame_img(p.in, b, k == 0 ? 0 : 2);
   const size_t seg_src = frame_plane(p.in, b, k == 0 ? 0 : 2, hw), seg_tgt = frame_plane(p.in, b, 1, hw);
@@ -588,7 +587,7 @@ __global__ void __launch_bounds__(256) pack_kernel(const FrontParams p) {
   for (int base = blockIdx.x * 256; base < hw; base += kPackBlocksPerPair * 256) {
     const int pix_raw = base + threadIdx.x;
     const int pix = min(pix_raw, hw - 1);                       // keep every lane in the shuffles
-    const int h = (int)(((float)pix + 0.5f) * inv_w);           // exact for these sizes
+    const int h = pix / p.W;                                    // (a float reciprocal picks the wrong row at some widths)
     const size_t px_off = (size_t)h * p.in.img_row + (pix - h * p.W) * 3;
     const uint8_t* pt = img_t + px_off;
     const uint8_t* ps = img_s + px_off;

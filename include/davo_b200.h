@@ -277,10 +277,23 @@ int davo_bind_host_numa(davo_ctx*);
 
 /* Test / mode='feature' access to what the last davo_forward left in the
  * workspace for frame pair `pair` (= 2*sample + source index) of the LAST
- * micro-batch: "att_weights" [19], "packed" [H,W,16], "cnv1".."cnv5",
- * "cnv6" [h,w,2*cnv6_out] (rotation | translation), "cnv7_sum" [2,256],
- * "cnv7" where it is stored (-batch_norm: the plain conv sums), "se5_scale"
- * [branches,256] (the excitation of -se_insert / -se_skipadd / -se_replace).
+ * micro-batch: "att_weights" [19] (slot 0 below; the static table; ones
+ * without an attention source), "packed" [H,W,packed_c] (the cnv1 input:
+ * packed_c = 8 for the 8-channel layout, 16 for the 16-channel and the
+ * whole-sample layouts), "cnv1".."cnv5", "cnv6" [h,w,2*cnv6_out]
+ * (rotation | translation), "cnv7_sum" [2,256] (the head's partial sums
+ * added in the head's order), "cnv7" where it is stored (-batch_norm: the
+ * plain conv sums), "se5_scale" [branches,256] (the excitation of -se_insert
+ * / -se_skipadd / -se_replace).
+ * "att_weights:<k>" is slot k of the unit's attention weights: 19 class
+ * weights, or the excitation of a per-pixel source (its SE input's channels:
+ * 3 rgb, 1 depth term, 3 depth term + SE flow, 21 one-hot + SE flow).  Slots:
+ *   frame-pair units (shared nets): 0 the source frame, 1 the target (or,
+ *     under -se_flow_on_depthseg_seplayers, the "far" table of the source);
+ *   sample units (non-shared nets): 0 src0, 1 src1, 2 the target; with the
+ *     depth split (0, 1) src0 near / far and (2, 3) src1 near / far.
+ * Static variants give the static table for every frame that has a map.  A
+ * slot the variant does not compute is refused (DAVO_ERR_ARG).
  * Per conv layer "<layer>" also takes a suffix:
  *   "<layer>"          the map [h,w,C]; an odd map stored with an even pitch
  *                      comes back without its zero pad row / column;
