@@ -25,6 +25,7 @@ SYMBOLS = (
     "davo_comm_unique_id", "davo_comm_create", "davo_comm_world", "davo_allgather_poses",
     "davo_forward_sequence", "davo_forward_sequence_host",
     "davo_odometry_create", "davo_odometry_push", "davo_odometry_reset", "davo_odometry_frames",
+    "davo_odometry_push_many",
     "davo_last_error",
     "davo_destroy", "davo_build_info", "davo_config_bytes", "davo_odometry_destroy",
 )
@@ -87,6 +88,8 @@ def load() -> C.CDLL:
     lib.davo_odometry_create.argtypes = [vp, ip, ip, ip, C.POINTER(vp)]
     lib.davo_odometry_push.argtypes = [vp, ip, vp, vp, vp, vp, vp, vp, vp, C.POINTER(ip), C.POINTER(ip), vp,
                                        C.POINTER(C.c_longlong)]
+    lib.davo_odometry_push_many.argtypes = [ip, C.POINTER(vp), C.POINTER(ip)] + [C.POINTER(vp)] * 7 + [
+        C.POINTER(ip), C.POINTER(ip), vp]
     lib.davo_odometry_reset.argtypes = [vp]
     lib.davo_odometry_frames.argtypes = [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     lib.davo_odometry_destroy.argtypes = [vp]

@@ -35,6 +35,7 @@
 #include "features.cuh"
 #include "comm.cuh"
 #include "trajectory.cuh"
+#include "odometry_many.cuh"
 #include "bn.cuh"
 #include "jpeg.cuh"
 #include "host_convert.h"
@@ -261,8 +262,16 @@ struct davo_ctx {
   uint8_t* q_img[2] = {}; uint8_t* q_seg8[2] = {}; float *q_seg[2] = {}, *q_depth[2] = {};
   cudaEvent_t ev_q_done[2] = {};    // the call that last used set i has finished reading it
   long long q_calls = 0;
-  // Function attributes are per device: what this context has already raised, by kernel.
-  std::map<const void*, int> smem_attr;
+  // davo_odometry_push_many: one stacked-triplet staging batch of max_batch samples (input_view.cuh: stacked_view) and
+  // its poses, allocated by the first batched push; the per-call session and sample descriptors go from a pinned ring
+  // slot to its device twin in one copy, and a slot is refilled once the call that used it has finished
+  uint8_t *m_img = nullptr, *m_lab = nullptr;
+  float *m_depth = nullptr, *m_flow = nullptr, *m_pose = nullptr;
+  static constexpr int kManyRing = 4;
+  void *m_hdesc[kManyRing] = {}, *m_ddesc[kManyRing] = {};
+  size_t m_desc_cap[kManyRing] = {};
+  cudaEvent_t m_ev[kManyRing] = {};
+  long long m_calls = 0;
   std::map<std::pair<const void*, int>, int> max_clusters;   // by (kernel, dynamic shared memory)
   float depth_thres = 0.f;          // -se_flow_on_depthseg_seplayers: the variable se_flow/depth_threshold
   // mode='feature' (features.cuh)
@@ -335,10 +344,15 @@ int launch_k(davo_ctx* ctx, void (*kern)(KArgs...), dim3 grid, dim3 block, size_
   return 0;
 }
 
-// Opt the kernel in to `bytes` of dynamic shared memory on this context's device (once per size).
+// Opt the kernel in to `bytes` of dynamic shared memory on this context's device (once per size).  The attribute
+// belongs to the kernel on the device, not to a handle, so what has been raised is kept per (device, kernel) for the
+// whole process and only ever raised: two handles on one device must not lower it under each other's launches.
+std::mutex g_smem_mutex;
+std::map<std::pair<int, const void*>, int> g_smem_attr;
 template <class K>
 int ensure_smem(davo_ctx* ctx, K kern, int bytes) {
-  int& have = ctx->smem_attr[reinterpret_cast<const void*>(kern)];
+  std::lock_guard<std::mutex> lk(g_smem_mutex);
+  int& have = g_smem_attr[std::make_pair(ctx->device, reinterpret_cast<const void*>(kern))];
   if (have < bytes) {
     CU_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     have = bytes;
@@ -1366,6 +1380,12 @@ extern "C" void davo_destroy(davo_ctx* ctx) {
     if (ctx->ev_seg8[i]) cudaEventDestroy(ctx->ev_seg8[i]);
     if (ctx->ev_copied[i]) cudaEventDestroy(ctx->ev_copied[i]);
     if (ctx->ev_consumed[i]) cudaEventDestroy(ctx->ev_consumed[i]);
+  }
+  cudaFree(ctx->m_img); cudaFree(ctx->m_lab); cudaFree(ctx->m_depth); cudaFree(ctx->m_flow); cudaFree(ctx->m_pose);
+  for (int i = 0; i < davo_ctx::kManyRing; ++i) {
+    if (ctx->m_hdesc[i]) cudaFreeHost(ctx->m_hdesc[i]);
+    if (ctx->m_ddesc[i]) cudaFree(ctx->m_ddesc[i]);
+    if (ctx->m_ev[i]) cudaEventDestroy(ctx->m_ev[i]);
   }
   for (int i = 0; i < 2; ++i) {
     if (ctx->q_img[i]) cudaFree(ctx->q_img[i]);
@@ -2566,6 +2586,148 @@ extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, c
   o->posed += nt;
   if (n_samples) *n_samples = ns;
   if (n_traj) *n_traj = nt;
+  return 0;
+}
+
+// A batched push (include/davo_b200.h: davo_odometry_push_many): entry i is davo_odometry_push(sessions[i], k[i], ...)
+// on a device session, and all of them share one forward.  The samples are staged as stacked triplets, those that
+// compute both pairs (all-mode sessions, sample 0 of a trajectory session that opens its sequence, every sample of the
+// non-shared nets) first, so that the forward is at most one DAVO_PAIRS_ALL and one DAVO_PAIRS_TRAJECTORY call.  A
+// pair's result does not depend on which pairs share its pass, so every pose is the bits of the single push; the
+// trajectory is chained by the single push's code (traj_chain).  Launches: stage, carry, the forward's, compose --
+// none per session.
+extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
+                                       const float* const* flow_fwd, const float* const* flow_bwd,
+                                       const float* const* seg, const float* const* depth, float* const* pose_out,
+                                       double* const* traj_out, int* n_samples, int* n_traj, void* stream) {
+  const char* who = "davo_odometry_push_many";
+  if (n < 1) return fail(nullptr, DAVO_ERR_ARG, "%s: n=%d: at least one session", who, n);
+  if (!sessions) return fail(nullptr, DAVO_ERR_ARG, "%s: sessions is NULL", who);
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    for (int i = 0; i < n; ++i)
+      if (!sessions[i] || !g_odo_live.count(sessions[i]))
+        return fail(nullptr, DAVO_ERR_ARG, "%s: sessions[%d] is NULL or was destroyed", who, i);
+  }
+  davo_ctx* ctx = sessions[0]->ctx;
+  const davo_config& c = ctx->cfg;
+  if (n > 65535) return fail(ctx, DAVO_ERR_ARG, "%s: n=%d sessions, more than 65535", who, n);
+  if (!k) return fail(ctx, DAVO_ERR_ARG, "%s: k is NULL", who);
+  if (!img) return fail(ctx, DAVO_ERR_ARG, "%s: img is NULL", who);
+  std::set<const davo_odometry*> seen;
+  for (int i = 0; i < n; ++i) {
+    const davo_odometry* o = sessions[i];
+    if (!seen.insert(o).second) return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] is given twice", who, i);
+    if (o->ctx != ctx) return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] belongs to another handle than sessions[0]", who, i);
+    if (o->host) return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] is a host session; a batched push takes device sessions", who, i);
+  }
+  const SeqReads rv = seq_reads(ctx, DAVO_PAIRS_ALL);                      // what the variant reads at all
+  const size_t hw = (size_t)c.H * c.W;
+  std::vector<OdoManySession> ds(n);
+  int B = 0, nA = 0;
+  for (int i = 0; i < n; ++i) {                                           // the checks and counts of davo_odometry_push
+    davo_odometry* o = sessions[i];
+    if (k[i] < 1 || k[i] > o->max_push)
+      return fail(ctx, DAVO_ERR_ARG, "%s: k[%d]=%d new frames outside 1..max_push %d", who, i, k[i], o->max_push);
+    const long long f0 = o->pushed;
+    const int head = o->head(), fe = head == 2 ? 1 : 0, nn = head + k[i], ns = std::max(0, nn - 2);
+    const long long g0 = f0 - head;
+    const int first = g0 == 0 && ns > 0;
+    const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
+    const long long e0 = std::max(f0 - 1, 0LL), e1 = f0 + k[i] - 1;
+    const bool fwd_read = rg.flow && e1 > e0 && rg.k0((int)std::min(e0, 2LL));
+    const bool bwd_read = rg.flow && ns > 0;
+    auto at = [&](auto* const* a) { return a ? a[i] : nullptr; };
+    OdoManySession& d = ds[i];
+    d.img = img[i]; d.seg = at(seg); d.depth = at(depth); d.fwd = at(flow_fwd); d.bwd = at(flow_bwd);
+    d.pose_out = at(pose_out); d.traj_out = reinterpret_cast<Mat4*>(at(traj_out));
+    struct { const void* p; bool needed; const char* name; } in[] = {
+        {d.img, true, "img"}, {d.pose_out, ns > 0, "pose_out"}, {d.traj_out, ns + 2 * first > 0, "traj_out"},
+        {d.seg, c.att_src != 0, "seg"}, {d.depth, rg.depth, "depth"}, {d.bwd, bwd_read, "flow_bwd"},
+        {d.fwd, fwd_read, "flow_fwd"}};
+    for (const auto& x : in) {
+      if (x.needed && !x.p) return fail(ctx, DAVO_ERR_ARG, "%s: %s[%d] is NULL; this variant and pair selection read it", who, x.name, i);
+      if (x.p && (reinterpret_cast<uintptr_t>(x.p) & 15)) return fail(ctx, DAVO_ERR_ARG, "%s: %s[%d] is not 16-byte aligned", who, x.name, i);
+    }
+    d.c_img = o->c_img; d.c_seg = o->c_seg; d.c_depth = rv.depth ? o->c_depth : nullptr; d.c_fwd = o->c_fwd;
+    d.P = o->d_P; d.rel = o->d_rel;
+    d.head = head; d.fe = fe; d.k = k[i]; d.ns = ns; d.first = first;
+    d.na = (ctx->unit_sample || o->pairs == DAVO_PAIRS_ALL) ? ns : first;
+    const int e = nn - 2;                                                 // the last flow_fwd entry, read by a later sample
+    d.carry_fwd = e >= fe && rg.fwd((int)std::min(g0 + e, 2LL)) ? e - fe : -1;
+    B += ns;
+    nA += d.na;
+  }
+  if (B > c.max_batch) return fail(ctx, DAVO_ERR_ARG, "%s: %d samples in all, more than max_batch %d", who, B, c.max_batch);
+  std::vector<int2> smp(B);                                               // staging order: both-pair samples first
+  for (int i = 0, a = 0, t = nA; i < n; ++i) {
+    OdoManySession& d = ds[i];
+    d.ba = a; d.bt = t;
+    for (int s = 0; s < d.ns; ++s) smp[s < d.na ? a++ : t++] = make_int2(i, s);
+  }
+  CU_OK(cudaSetDevice(ctx->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (!ctx->m_img) {                                                      // the staging batch, once per handle
+    const size_t mb = (size_t)c.max_batch;
+    CU_OK(cudaMalloc((void**)&ctx->m_img, mb * hw * 9));
+    if (rv.labels) CU_OK(cudaMalloc((void**)&ctx->m_lab, mb * hw * 3));
+    if (rv.depth) CU_OK(cudaMalloc((void**)&ctx->m_depth, mb * hw * 3 * 4));
+    if (rv.flow) CU_OK(cudaMalloc((void**)&ctx->m_flow, mb * hw * 4 * 4));
+    CU_OK(cudaMalloc((void**)&ctx->m_pose, mb * 12 * 4));
+  }
+  // the descriptors: one copy from a pinned ring slot, refilled only after the call that last used it has finished
+  const int slot = (int)(ctx->m_calls++ % davo_ctx::kManyRing);
+  const size_t sess_bytes = sizeof(OdoManySession) * n, bytes = sess_bytes + sizeof(int2) * B;
+  if (ctx->m_ev[slot]) CU_OK(cudaEventSynchronize(ctx->m_ev[slot]));
+  else CU_OK(cudaEventCreateWithFlags(&ctx->m_ev[slot], cudaEventDisableTiming));
+  if (ctx->m_desc_cap[slot] < bytes) {
+    const size_t cap = std::max<size_t>(bytes, 2 * ctx->m_desc_cap[slot]);
+    if (ctx->m_hdesc[slot]) { CU_OK(cudaFreeHost(ctx->m_hdesc[slot])); ctx->m_hdesc[slot] = nullptr; }
+    if (ctx->m_ddesc[slot]) { CU_OK(cudaFree(ctx->m_ddesc[slot])); ctx->m_ddesc[slot] = nullptr; }
+    ctx->m_desc_cap[slot] = 0;
+    CU_OK(cudaHostAlloc(&ctx->m_hdesc[slot], cap, cudaHostAllocDefault));
+    CU_OK(cudaMalloc(&ctx->m_ddesc[slot], cap));
+    ctx->m_desc_cap[slot] = cap;
+  }
+  uint8_t* h = static_cast<uint8_t*>(ctx->m_hdesc[slot]);
+  memcpy(h, ds.data(), sess_bytes);
+  if (B) memcpy(h + sess_bytes, smp.data(), sizeof(int2) * B);
+  CU_OK(cudaMemcpyAsync(ctx->m_ddesc[slot], h, bytes, cudaMemcpyHostToDevice, st));
+  const OdoManySession* dsess = static_cast<const OdoManySession*>(ctx->m_ddesc[slot]);
+  constexpr int kCopyBlocks = 4 * 148;                                     // blocks of a copy launch, over its rows
+  if (B > 0) {
+    OdoStageParams sp;
+    sp.sess = dsess;
+    sp.smp = reinterpret_cast<const int2*>(static_cast<const uint8_t*>(ctx->m_ddesc[slot]) + sess_bytes);
+    sp.hw = (long long)hw; sp.na = nA;
+    sp.flow = rv.flow; sp.labels = rv.labels; sp.tgt_labels = rv.tgt_labels; sp.depth = rv.depth;
+    sp.img = ctx->m_img; sp.lab = ctx->m_lab; sp.dep = ctx->m_depth; sp.fl = ctx->m_flow;
+    odo_stage_kernel<<<dim3(std::min(32, std::max(1, kCopyBlocks / B)), B), 256, 0, st>>>(sp);
+    CU_OK(cudaGetLastError());
+  }
+  // a separate launch: the stage kernel reads the carried frames this one overwrites
+  odo_carry_kernel<<<dim3(std::min(16, std::max(1, kCopyBlocks / n)), n), 256, 0, st>>>(dsess, (long long)hw, rv.depth);
+  CU_OK(cudaGetLastError());
+  if (B > 0) {
+    auto view = [&](int b0) {
+      return stacked_view(c.H, c.W, ctx->m_img + hw * 9 * b0, ctx->m_flow ? ctx->m_flow + hw * 4 * b0 : nullptr,
+                          ctx->m_lab ? ctx->m_lab + hw * 3 * b0 : nullptr, ctx->m_depth ? ctx->m_depth + hw * 3 * b0 : nullptr);
+    };
+    if (nA > 0)
+      if (int rc = forward_device(ctx, who, nA, DAVO_PAIRS_ALL, view(0), ctx->m_pose, st)) return rc;
+    if (B > nA)
+      if (int rc = forward_device(ctx, who, B - nA, DAVO_PAIRS_TRAJECTORY, view(nA), ctx->m_pose + 12 * nA, st)) return rc;
+    odo_compose_many_kernel<<<(n + 3) / 4, 128, 0, st>>>(dsess, n, ctx->m_pose);
+    CU_OK(cudaGetLastError());
+  }
+  CU_OK(cudaEventRecord(ctx->m_ev[slot], st));
+  for (int i = 0; i < n; ++i) {                                           // host bookkeeping, once all is enqueued
+    const int nt = ds[i].ns + 2 * ds[i].first;
+    sessions[i]->pushed += k[i];
+    sessions[i]->posed += nt;
+    if (n_samples) n_samples[i] = ds[i].ns;
+    if (n_traj) n_traj[i] = nt;
+  }
   return 0;
 }
 

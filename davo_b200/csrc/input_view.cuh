@@ -8,7 +8,7 @@
 // Sequence layout (davo_forward_sequence): sample b is frames (b, b+1, b+2) of an N-frame sequence,
 //   img [N][H][W][3], seg / depth [N][H][W], flow_fwd / flow_bwd [N-1][H][W][2];
 //   plane 0 of sample b is flow_fwd[b] (frame b -> b+1), plane 1 is flow_bwd[b+1] (frame b+2 -> b+1).
-// Only addresses differ between the two: the same kernels compute the same values.
+// Only addresses differ between the layouts: the same kernels compute the same values.
 #pragma once
 #include <cuda_fp16.h>
 #include <stdint.h>
@@ -56,6 +56,18 @@ inline InputView sequence_view(int H, int W, const uint8_t* img, const float* fw
   v.flow0 = fwd; v.flow1 = bwd; v.flow_sample = 2 * hw;
   v.flow16_0 = static_cast<const __half*>(fwd16); v.flow16_1 = static_cast<const __half*>(bwd16);
   v.flow16_sample = 2 * hw; v.n_flow16 = (fwd16 || bwd16) ? n16 : 0;
+  return v;
+}
+
+// Stacked-triplet layout (davo_odometry_push_many's staging batch): the frames of a sample one after another,
+//   img [B][3][H][W][3], labels as bytes (seg8) / depth [B][3][H][W], flow [B][2][H][W][2].
+inline InputView stacked_view(int H, int W, const uint8_t* img, const float* flow, const uint8_t* seg8, const float* depth) {
+  const long long hw = (long long)H * W;
+  InputView v;
+  v.img = img; v.img_sample = hw * 9; v.img_frame = hw * 3; v.img_row = W * 3;
+  v.seg = nullptr; v.seg8 = seg8; v.depth = depth; v.plane_sample = 3 * hw;
+  v.flow0 = flow; v.flow1 = flow ? flow + 2 * hw : nullptr; v.flow_sample = 4 * hw;
+  v.flow16_0 = nullptr; v.flow16_1 = nullptr; v.flow16_sample = 0; v.n_flow16 = 0;
   return v;
 }
 

@@ -114,12 +114,13 @@ __global__ void __launch_bounds__(128) pose_rel_kernel(const float* __restrict__
 
 // The online form of the chain (davo_odometry_push): P <- P . rel[i] for i < m in frame order, traj[first + i] = P; with
 // `first` the chain starts from P_0 = I (also written to traj[0]) instead of the carried *P, which receives the last P.
-// One warp: lane l < 16 owns element l of P and sums its row-by-column product in k = 0..3 order, as mat4_mul does, so
-// that the result does not depend on how the frames were cut into pushes; P[r][k] comes from its owner by shuffle.
-__global__ void __launch_bounds__(32) traj_extend_kernel(const Mat4* __restrict__ rel, int m, int first, double* __restrict__ P,
-                                                         Mat4* __restrict__ traj) {
-  const int l = threadIdx.x & 15, r = l >> 2, c = l & 3;
-  const bool owner = threadIdx.x < 16;
+// One whole warp: lane l < 16 owns element l of P and sums its row-by-column product in k = 0..3 order, as mat4_mul
+// does, so that the result does not depend on how the frames were cut into pushes; P[r][k] comes from its owner by
+// shuffle.  A single push (traj_extend_kernel) and a batched one (odo_compose_many_kernel) both run this code, so a
+// session's trajectory is the same bits whichever way it was pushed.
+__device__ __forceinline__ void traj_chain(const Mat4* rel, int m, int first, double* P, Mat4* traj) {
+  const int lane = threadIdx.x & 31, l = lane & 15, r = l >> 2, c = l & 3;
+  const bool owner = lane < 16;
   double p = first ? (l % 5 == 0 ? 1.0 : 0.0) : P[l];
   if (first && owner) traj[0].m[l] = p;
   for (int i = 0; i < m; ++i) {
@@ -130,6 +131,11 @@ __global__ void __launch_bounds__(32) traj_extend_kernel(const Mat4* __restrict_
     if (owner) traj[first + i].m[l] = p;
   }
   if (owner) P[l] = p;
+}
+
+__global__ void __launch_bounds__(32) traj_extend_kernel(const Mat4* __restrict__ rel, int m, int first, double* __restrict__ P,
+                                                         Mat4* __restrict__ traj) {
+  traj_chain(rel, m, first, P, traj);
 }
 
 // traj[0] = I, traj[i + 1] = traj[i] . rel[i], i < m.  One block; thread t owns elements [t*chunk, (t+1)*chunk).

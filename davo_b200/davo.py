@@ -433,6 +433,58 @@ class DAVO(object):
         return numpy arrays, else CUDA tensors in and out."""
         return Odometry(self, pairs, self.batch_size if max_push is None else max_push, host)
 
+    def odometry_push_many(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None):
+        """One push on each of several device sessions of this handle, in one forward pass (include/davo_b200.h:
+        davo_odometry_push_many).  ``img``, ``flow_fwd``, ``flow_bwd``, ``seg`` and ``depth`` are lists aligned with
+        ``sessions``, entry i holding the CUDA tensors ``sessions[i].push`` takes (None, or a list of None, where no
+        entry has one).  Returns the list of the dicts ``push`` returns; the results are the bits of pushing each
+        session alone, in list order.  Enqueued on the current stream."""
+        sessions = list(sessions)
+        n = len(sessions)
+        per = lambda x: [None] * n if x is None else list(x)
+        lists = {"img": per(img), "flow_fwd": per(flow_fwd), "flow_bwd": per(flow_bwd), "seg": per(seg), "depth": per(depth)}
+        for name, x in lists.items():
+            if len(x) != n:
+                raise ValueError("DAVO.odometry_push_many: %s has %d entries for %d sessions" % (name, len(x), n))
+        if n == 0:
+            raise ValueError("DAVO.odometry_push_many: no session")
+        for i, od in enumerate(sessions):
+            if not isinstance(od, Odometry) or od._system is not self:
+                raise ValueError("DAVO.odometry_push_many: session %d is not a session of this handle" % i)
+            if od._host:
+                raise ValueError("DAVO.odometry_push_many: session %d is a host session; a batched push takes device "
+                                 "sessions (DAVO.odometry(host=False))" % i)
+            if any(od is o for o in sessions[:i]):
+                raise ValueError("DAVO.odometry_push_many: session %d is given twice" % i)
+        ins, counts = [], []
+        for i, od in enumerate(sessions):                    # shapes of every entry, then where the tensors live
+            x = [lists[name][i] for name in ("img", "flow_fwd", "flow_bwd", "seg", "depth")]
+            k, x[4] = od._args(*x, who="DAVO.odometry_push_many: session %d" % i)
+            ins.append(x)
+            counts.append((k,) + od._counts(k))
+        for i, (od, x) in enumerate(zip(sessions, ins)):
+            od._check_device(*x, who="DAVO.odometry_push_many: session %d" % i)
+        import torch
+        dev = "cuda:%d" % self.device
+        outs = [(torch.zeros((ns, 2, 6), dtype=torch.float32, device=dev),
+                 torch.empty((nt, 4, 4), dtype=torch.float64, device=dev)) for _, ns, nt in counts]
+        vp = C.c_void_p
+        ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None
+        arr = lambda vals: (vp * n)(*vals)
+        cols = [arr([ptr(x[j]) for x in ins]) for j in range(5)]
+        ns, nt = (C.c_int * n)(), (C.c_int * n)()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        self._check(self._lib.davo_odometry_push_many(
+            n, arr([od._o.value for od in sessions]), (C.c_int * n)(*[c[0] for c in counts]), *cols,
+            arr([ptr(o[0]) for o in outs]), arr([ptr(o[1]) for o in outs]), ns, nt, vp(stream)),
+            "davo_odometry_push_many")
+        res = []
+        for od, (k, _, _), (pose, traj), m in zip(sessions, counts, outs, nt):
+            res.append({'pose': pose, 'trajectory': traj, 'frames': range(od._posed, od._posed + m)})
+            od._pushed += k
+            od._posed += m
+        return res
+
     def bind_host_numa(self):
         """Bind this thread (and threads created after it) to the CPUs next to this handle's GPU
         (``davo_bind_host_numa``); call it before allocating pinned inputs.  Returns the NUMA node or -1."""
@@ -560,22 +612,32 @@ class Odometry(object):
         ns = max(0, f0 + k - 2) - max(0, f0 - 2)
         return ns, ns + 2 if (f0 <= 2 and ns > 0) else ns
 
-    def _args(self, img, flow_fwd, flow_bwd, seg, depth):
+    def _args(self, img, flow_fwd, flow_bwd, seg, depth, who="Odometry.push"):
         s = self._system
         if self._o is None:
-            raise RuntimeError("Odometry.push: the session is closed")
+            raise RuntimeError("%s: the session is closed" % who)
         if s.config.att_src != V.ATT_SE_DEPTH_SEG and not s.config.depth_split:
             depth = None
         elif depth is None:
-            raise ValueError("Odometry.push: version %r reads depth [k,H,W,1]" % (s.version,))
+            raise ValueError("%s: version %r reads depth [k,H,W,1]" % (who, s.version))
         k, H, W = int(img.shape[0]), s.img_height, s.img_width
         kf = k if self._pushed > 0 else k - 1
         want = {"img": (k, H, W, 3), "flow_fwd": (kf, H, W, 2), "flow_bwd": (kf, H, W, 2), "seg": (k, H, W, 1),
                 "depth": (k, H, W, 1)}
         for name, t in (("img", img), ("flow_fwd", flow_fwd), ("flow_bwd", flow_bwd), ("seg", seg), ("depth", depth)):
             if t is not None and tuple(t.shape) != want[name]:
-                raise ValueError("Odometry.push: %s has shape %s, expected %s" % (name, tuple(t.shape), want[name]))
+                raise ValueError("%s: %s has shape %s, expected %s" % (who, name, tuple(t.shape), want[name]))
         return k, depth
+
+    def _check_device(self, img, flow_fwd, flow_bwd, seg, depth, who="Odometry.push"):
+        import torch
+        dev = "cuda:%d" % self._system.device
+        for name, t, dt in (("img", img, torch.uint8), ("flow_fwd", flow_fwd, torch.float32),
+                            ("flow_bwd", flow_bwd, torch.float32), ("seg", seg, torch.float32),
+                            ("depth", depth, torch.float32)):
+            if t is not None and not (_is_torch(t) and t.is_cuda and t.device.index == self._system.device
+                                      and t.dtype == dt and t.is_contiguous()):
+                raise ValueError("%s: %s must be a contiguous %s tensor on %s" % (who, name, dt, dev))
 
     def _call(self, k, ins, pose, traj, stream, ticket):
         s = self._system
@@ -593,12 +655,7 @@ class Odometry(object):
         if not self._host:
             import torch
             dev = "cuda:%d" % self._system.device
-            for name, t, dt in (("img", img, torch.uint8), ("flow_fwd", flow_fwd, torch.float32),
-                                ("flow_bwd", flow_bwd, torch.float32), ("seg", seg, torch.float32),
-                                ("depth", depth, torch.float32)):
-                if t is not None and not (_is_torch(t) and t.is_cuda and t.device.index == self._system.device
-                                          and t.dtype == dt and t.is_contiguous()):
-                    raise ValueError("Odometry.push: %s must be a contiguous %s tensor on %s" % (name, dt, dev))
+            self._check_device(img, flow_fwd, flow_bwd, seg, depth)
             pose = torch.zeros((n_s, 2, 6), dtype=torch.float32, device=dev)
             traj = torch.empty((n_t, 4, 4), dtype=torch.float64, device=dev)
             ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None and t.numel() else None

@@ -264,6 +264,26 @@ int davo_odometry_create(davo_ctx*, int max_push, int pairs, int host_inputs, da
 int davo_odometry_push(davo_odometry*, int k, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
                        const float* seg, const float* depth, float* pose_out, double* traj_out, int* n_samples,
                        int* n_traj, void* cuda_stream, long long* ticket);
+/* davo_odometry_push_many: one push on each of n device sessions (host_inputs = 0) of one handle, in one forward pass
+ *   -- many cameras, a few frames each, at the same time.  Every array has n entries and lives in host memory; the
+ *   pointers it holds are device buffers.  Entry i is what davo_odometry_push(sessions[i], k[i], img[i], flow_fwd[i],
+ *   flow_bwd[i], seg[i], depth[i], pose_out[i], traj_out[i], &n_samples[i], &n_traj[i], cuda_stream, NULL) takes:
+ *   the same shapes, NULL rules, 16-byte alignment and output rows.  flow_fwd, flow_bwd, seg, depth, n_samples and
+ *   n_traj may be NULL as whole arrays when no entry needs them.
+ *   The results are bit-identical to pushing each session alone with davo_odometry_push, in array order: pose_out
+ *   (with the zero rows of trajectory mode), traj_out, the counts and every later push on those sessions, single or
+ *   batched.  Sessions may be in any state (first push, mid-stream, just reset), and trajectory and all-mode sessions
+ *   may be mixed; the handle's other sessions are untouched.  Asynchronous on cuda_stream, no synchronisation; the
+ *   number of kernel launches does not depend on n.  The first batched push on a handle allocates a staging batch of
+ *   max_batch samples, freed with the handle.
+ *   Argument errors return DAVO_ERR_ARG with a message naming the input and the session index: n < 1; a NULL or
+ *   destroyed session (davo_last_error(NULL)); a session given twice; a host session; sessions of two handles; k[i]
+ *   outside 1..max_push; more than max_batch samples in all; a NULL or misaligned buffer entry i reads.  A refused
+ *   call enqueues nothing and changes no session. */
+int davo_odometry_push_many(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
+                            const float* const* flow_fwd, const float* const* flow_bwd, const float* const* seg,
+                            const float* const* depth, float* const* pose_out, double* const* traj_out,
+                            int* n_samples, int* n_traj, void* cuda_stream);
 int davo_odometry_reset(davo_odometry*);
 int davo_odometry_frames(const davo_odometry*, long long* pushed, long long* posed);
 void davo_odometry_destroy(davo_odometry*);
