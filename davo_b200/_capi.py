@@ -25,7 +25,7 @@ SYMBOLS = (
     "davo_comm_unique_id", "davo_comm_create", "davo_comm_world", "davo_allgather_poses",
     "davo_forward_sequence", "davo_forward_sequence_host",
     "davo_odometry_create", "davo_odometry_push", "davo_odometry_reset", "davo_odometry_frames",
-    "davo_odometry_push_many",
+    "davo_odometry_push_many", "davo_odometry_push_many_host",
     "davo_last_error",
     "davo_destroy", "davo_build_info", "davo_config_bytes", "davo_odometry_destroy",
 )
@@ -90,6 +90,8 @@ def load() -> C.CDLL:
                                        C.POINTER(C.c_longlong)]
     lib.davo_odometry_push_many.argtypes = [ip, C.POINTER(vp), C.POINTER(ip)] + [C.POINTER(vp)] * 7 + [
         C.POINTER(ip), C.POINTER(ip), vp]
+    lib.davo_odometry_push_many_host.argtypes = [ip, C.POINTER(vp), C.POINTER(ip)] + [C.POINTER(vp)] * 7 + [
+        C.POINTER(ip), C.POINTER(ip), vp, C.POINTER(C.c_longlong)]
     lib.davo_odometry_reset.argtypes = [vp]
     lib.davo_odometry_frames.argtypes = [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     lib.davo_odometry_destroy.argtypes = [vp]

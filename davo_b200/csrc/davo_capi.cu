@@ -272,6 +272,14 @@ struct davo_ctx {
   size_t m_desc_cap[kManyRing] = {};
   cudaEvent_t m_ev[kManyRing] = {};
   long long m_calls = 0;
+  // davo_odometry_push_many_host: two arrivals sets (device; pinned byte labels), the caller's frames and flow entries
+  // of a call at the indices the stage kernel reads them; set i is refilled once the stage and carry kernels of the call
+  // that last used it have finished (a_done[i]), so that the copies of call t+1 run under the forward of call t
+  uint8_t* a_dev[2] = {}; uint8_t* a_hlab[2] = {};
+  size_t a_dev_cap[2] = {}, a_hlab_cap[2] = {};
+  cudaEvent_t a_copied[2] = {}, a_done[2] = {};
+  long long a_calls = 0;
+  float* m_hpose = nullptr;           // the pose rows of each session's push, [max_batch,2,6], copied to the host from here
   std::map<std::pair<const void*, int>, int> max_clusters;   // by (kernel, dynamic shared memory)
   float depth_thres = 0.f;          // -se_flow_on_depthseg_seplayers: the variable se_flow/depth_threshold
   // mode='feature' (features.cuh)
@@ -1393,7 +1401,12 @@ extern "C" void davo_destroy(davo_ctx* ctx) {
     if (ctx->q_seg[i]) cudaFree(ctx->q_seg[i]);
     if (ctx->q_depth[i]) cudaFree(ctx->q_depth[i]);
     if (ctx->ev_q_done[i]) cudaEventDestroy(ctx->ev_q_done[i]);
+    if (ctx->a_dev[i]) cudaFree(ctx->a_dev[i]);
+    if (ctx->a_hlab[i]) cudaFreeHost(ctx->a_hlab[i]);
+    if (ctx->a_copied[i]) cudaEventDestroy(ctx->a_copied[i]);
+    if (ctx->a_done[i]) cudaEventDestroy(ctx->a_done[i]);
   }
+  cudaFree(ctx->m_hpose);
   delete ctx->pool;
   if (ctx->comm) davo_comm::api().CommDestroy(ctx->comm);
   if (ctx->s_pose) cudaFree(ctx->s_pose);
@@ -2035,12 +2048,8 @@ bool host_narrow(davo_ctx* ctx, const std::vector<NarrowJob>& jobs) {
   return flow_bad.load() == 0;
 }
 
-// Poses of a host call back to the caller's memory, and an odometry push's n_traj absolute poses from traj_dev;
-// blocking, or the asynchronous form's ticket.
-int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket, const double* traj_dev = nullptr,
-                double* traj_out = nullptr, int n_traj = 0) {
-  if (B > 0) CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
-  if (n_traj > 0) CU_OK(cudaMemcpyAsync(traj_out, traj_dev, (size_t)16 * 8 * n_traj, cudaMemcpyDeviceToHost, st));
+// The end of a host call whose copies back are queued on st: blocking, or the asynchronous form's ticket.
+int host_done(davo_ctx* ctx, cudaStream_t st, long long* ticket) {
   if (ticket) {
     const long long t = ++ctx->host_tickets;
     cudaEvent_t& ev = ctx->ev_host_done[t % davo_ctx::kTickets];
@@ -2050,6 +2059,16 @@ int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long lon
   } else {
     CU_OK(cudaStreamSynchronize(st));
   }
+  return 0;
+}
+
+// Poses of a host call back to the caller's memory, and an odometry push's n_traj absolute poses from traj_dev;
+// blocking, or the asynchronous form's ticket.
+int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket, const double* traj_dev = nullptr,
+                double* traj_out = nullptr, int n_traj = 0) {
+  if (B > 0) CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
+  if (n_traj > 0) CU_OK(cudaMemcpyAsync(traj_out, traj_dev, (size_t)16 * 8 * n_traj, cudaMemcpyDeviceToHost, st));
+  if (int rc = host_done(ctx, st, ticket)) return rc;
   ctx->last_d2h = (long long)12 * 4 * B + (long long)16 * 8 * n_traj;
   return 0;
 }
@@ -2589,18 +2608,161 @@ extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, c
   return 0;
 }
 
-// A batched push (include/davo_b200.h: davo_odometry_push_many): entry i is davo_odometry_push(sessions[i], k[i], ...)
-// on a device session, and all of them share one forward.  The samples are staged as stacked triplets, those that
-// compute both pairs (all-mode sessions, sample 0 of a trajectory session that opens its sequence, every sample of the
-// non-shared nets) first, so that the forward is at most one DAVO_PAIRS_ALL and one DAVO_PAIRS_TRAJECTORY call.  A
-// pair's result does not depend on which pairs share its pass, so every pose is the bits of the single push; the
-// trajectory is chained by the single push's code (traj_chain).  Launches: stage, carry, the forward's, compose --
-// none per session.
-extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
-                                       const float* const* flow_fwd, const float* const* flow_bwd,
-                                       const float* const* seg, const float* const* depth, float* const* pose_out,
-                                       double* const* traj_out, int* n_samples, int* n_traj, void* stream) {
-  const char* who = "davo_odometry_push_many";
+namespace {
+
+// davo_odometry_push_many_host: each session's new frames, label planes, depth planes and flow entries that some
+// computed pair of its stream reads, now or in a later push (the rule of a single host push:
+// forward_sequence_host_impl's img_rd / lab_rd / dep_rd and its carried flow_fwd entry), copied on the copy stream into
+// one of the two arrivals sets.  Session i's part of the set holds its caller frame u and caller flow entry u at index
+// u, so that the stage and carry kernels read it as they read a device session's buffers; ds[i]'s caller pointers are
+// replaced by pointers into the set.  Labels are narrowed to bytes on the CPU for all sessions in one pool pass into the
+// set's pinned area (float labels with DAVO_B200_HOST_SEG8=0); the label planes of consecutive sessions sit back to back
+// there and on the device, so one copy sends them all, except where a plane no pair reads (global frame 1 in trajectory
+// mode when the target's labels are not read) breaks the run.  The flow goes as float32: with flow_f16 = 1 the front
+// end rounds it when read (frontend.cuh: flow_q), so the bits are those of a single push either way.
+int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, OdoManySession* ds,
+                       cudaStream_t st, int set, size_t* h2d_out) {
+  const davo_config& c = ctx->cfg;
+  const SeqReads rv = seq_reads(ctx, DAVO_PAIRS_ALL);
+  const size_t hw = (size_t)c.H * c.W, fl = hw * 2;
+  const bool seg8 = rv.labels && ctx->host_seg8;
+  cudaStream_t cp = ctx->copy_stream;
+  // the set's regions: session i's k[i] frames (or flow entries) at its running offset in each
+  size_t kt = 0;
+  for (int i = 0; i < n; ++i) kt += (size_t)ds[i].k;
+  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const size_t b_img = up(kt * hw * 3), b_lab = seg8 ? up(kt * hw) : 0, b_seg = rv.labels && !seg8 ? up(kt * hw * 4) : 0;
+  const size_t b_dep = rv.depth ? up(kt * hw * 4) : 0, b_fl = rv.flow ? up(kt * fl * 4) : 0;
+  const size_t total = b_img + b_lab + b_seg + b_dep + 2 * b_fl;
+  cudaEvent_t& done = ctx->a_done[set];
+  if (!done) {
+    CU_OK(cudaEventCreateWithFlags(&done, cudaEventDisableTiming));
+    CU_OK(cudaEventCreateWithFlags(&ctx->a_copied[set], cudaEventDisableTiming));
+  }
+  if (ctx->a_dev_cap[set] < total || (seg8 && ctx->a_hlab_cap[set] < kt * hw)) {
+    CU_OK(cudaEventSynchronize(done));                             // the call that last used the set has read it
+    if (ctx->a_dev_cap[set] < total) {
+      const size_t cap = std::max(total, 2 * ctx->a_dev_cap[set]);
+      if (ctx->a_dev[set]) { CU_OK(cudaFree(ctx->a_dev[set])); ctx->a_dev[set] = nullptr; }
+      ctx->a_dev_cap[set] = 0;
+      CU_OK(cudaMalloc((void**)&ctx->a_dev[set], cap));
+      ctx->a_dev_cap[set] = cap;
+    }
+    if (seg8 && ctx->a_hlab_cap[set] < kt * hw) {
+      const size_t cap = std::max(kt * hw, 2 * ctx->a_hlab_cap[set]);
+      if (ctx->a_hlab[set]) { CU_OK(cudaFreeHost(ctx->a_hlab[set])); ctx->a_hlab[set] = nullptr; }
+      ctx->a_hlab_cap[set] = 0;
+      CU_OK(cudaHostAlloc((void**)&ctx->a_hlab[set], cap, cudaHostAllocDefault));
+      ctx->a_hlab_cap[set] = cap;
+    }
+  }
+  uint8_t* a_img = ctx->a_dev[set];
+  uint8_t* a_lab = a_img + b_img;
+  float* a_seg = reinterpret_cast<float*>(a_lab + b_lab);
+  float* a_dep = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(a_seg) + b_seg);
+  float* a_fwd = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(a_dep) + b_dep);
+  float* a_bwd = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(a_fwd) + b_fl);
+  CU_OK(cudaStreamWaitEvent(cp, done, 0));                         // the device part of the set is free
+  size_t h2d = 0;
+  auto h2d_copy = [&](void* dst, const void* src, size_t bytes) -> int {
+    CU_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, cp));
+    h2d += bytes;
+    return 0;
+  };
+  // copies runs of consecutive indices in [0, m) that `read` selects: copy(first index, count)
+  auto runs = [](int m, auto read, auto copy) -> int {
+    for (int u = 0; u < m;) {
+      if (!read(u)) { ++u; continue; }
+      int e = u;
+      while (e < m && read(e)) ++e;
+      if (int rc = copy(u, e - u)) return rc;
+      u = e;
+    }
+    return 0;
+  };
+  std::vector<NarrowJob> jobs;
+  std::vector<std::pair<size_t, size_t>> lab_runs;                  // byte label planes read: [begin, end) in the area
+  size_t off = 0;
+  for (int i = 0; i < n; off += (size_t)ds[i].k, ++i) {
+    OdoManySession& d = ds[i];
+    const davo_odometry* o = sessions[i];
+    const int head = d.head, k = d.k;
+    const long long g0 = o->pushed - head;
+    const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
+    auto glob = [&](int u) { return (int)std::min<long long>(g0 + head + u, 2); };   // caller frame u: virtual head + u
+    auto img_rd = [&](int u) { return rg.img(glob(u), INT_MAX); };
+    auto lab_rd = [&](int u) { return rg.lab(glob(u), INT_MAX); };
+    const uint8_t* img = d.img;
+    const float *seg = d.seg, *depth = d.depth, *fwd = d.fwd, *bwd = d.bwd;
+    uint8_t* ai = a_img + off * hw * 3;
+    d.img = ai;
+    if (int rc = runs(k, img_rd, [&](int u, int m) { return h2d_copy(ai + u * hw * 3, img + u * hw * 3, hw * 3 * m); }))
+      return rc;
+    if (rv.depth) {
+      float* ad = a_dep + off * hw;
+      d.depth = ad;
+      if (int rc = runs(k, img_rd, [&](int u, int m) { return h2d_copy(ad + u * hw, depth + u * hw, hw * 4 * m); })) return rc;
+    }
+    d.seg = nullptr;
+    d.c_seg = nullptr;
+    if (seg8) {
+      d.seg8 = a_lab + off * hw;
+      d.c_seg8 = o->c_seg8;
+      for (int u = 0; u < k; ++u) {
+        if (!lab_rd(u)) continue;
+        const size_t b = (off + u) * hw;
+        jobs.push_back({seg + u * hw, ctx->a_hlab[set] + b, hw, false});
+        if (!lab_runs.empty() && lab_runs.back().second == b) lab_runs.back().second = b + hw;
+        else lab_runs.push_back({b, b + hw});
+      }
+    } else if (rv.labels) {
+      float* as = a_seg + off * hw;
+      d.seg = as;
+      d.c_seg = o->c_seg;
+      if (int rc = runs(k, lab_rd, [&](int u, int m) { return h2d_copy(as + u * hw, seg + u * hw, hw * 4 * m); })) return rc;
+    }
+    if (rv.flow) {
+      // flow_fwd entry u is read as plane 0 of sample u + fe when that sample computes both pairs, or carried; flow_bwd
+      // entry u as plane 1 of sample u + fe - 1, for every sample
+      float *af = a_fwd + off * fl, *ab = a_bwd + off * fl;
+      d.fwd = af;
+      d.bwd = ab;
+      auto fwd_rd = [&](int u) { return u + d.fe < d.na || u == d.carry_fwd; };
+      if (int rc = runs(k, fwd_rd, [&](int u, int m) { return h2d_copy(af + u * fl, fwd + u * fl, fl * 4 * m); })) return rc;
+      if (d.ns > 0)
+        if (int rc = h2d_copy(ab + (1 - d.fe) * fl, bwd + (1 - d.fe) * fl, fl * 4 * d.ns)) return rc;
+    }
+  }
+  if (!jobs.empty()) {
+    CU_OK(cudaEventSynchronize(done));                             // the pinned area has been copied out by that call
+    host_narrow(ctx, jobs);
+    for (const auto& r : lab_runs)
+      if (int rc = h2d_copy(a_lab + r.first, ctx->a_hlab[set] + r.first, r.second - r.first)) return rc;
+  }
+  // The stage kernel reads the carried state, which a single host push writes on the copy stream (the carried frames
+  // at the tail of forward_sequence_host_impl, the c_fwd upload).  Recorded after this call's copies, the event also
+  // follows that earlier work, so the wait orders the stage kernel behind it.
+  CU_OK(cudaEventRecord(ctx->a_copied[set], cp));
+  CU_OK(cudaStreamWaitEvent(st, ctx->a_copied[set], 0));
+  *h2d_out = h2d;
+  return 0;
+}
+
+}  // namespace
+
+// A batched push (include/davo_b200.h: davo_odometry_push_many, davo_odometry_push_many_host): entry i is
+// davo_odometry_push(sessions[i], k[i], ...), and all of them share one forward.  The samples are staged as stacked
+// triplets, those that compute both pairs (all-mode sessions, sample 0 of a trajectory session that opens its sequence,
+// every sample of the non-shared nets) first, so that the forward is at most one DAVO_PAIRS_ALL and one
+// DAVO_PAIRS_TRAJECTORY call.  A pair's result does not depend on which pairs share its pass, so every pose is the bits
+// of the single push; the trajectory is chained by the single push's code (traj_chain).  Launches: stage, carry, the
+// forward's, compose -- none per session.  Host sessions (`host`) first copy what the call reads into an arrivals set
+// (many_host_arrivals); their pose rows and absolute poses go back to the caller's host buffers at the end.
+static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
+                                   const float* const* flow_fwd, const float* const* flow_bwd,
+                                   const float* const* seg, const float* const* depth, float* const* pose_out,
+                                   double* const* traj_out, int* n_samples, int* n_traj, void* stream, long long* ticket) {
+  const char* who = host ? "davo_odometry_push_many_host" : "davo_odometry_push_many";
   if (n < 1) return fail(nullptr, DAVO_ERR_ARG, "%s: n=%d: at least one session", who, n);
   if (!sessions) return fail(nullptr, DAVO_ERR_ARG, "%s: sessions is NULL", who);
   {
@@ -2619,7 +2781,9 @@ extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, co
     const davo_odometry* o = sessions[i];
     if (!seen.insert(o).second) return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] is given twice", who, i);
     if (o->ctx != ctx) return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] belongs to another handle than sessions[0]", who, i);
-    if (o->host) return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] is a host session; a batched push takes device sessions", who, i);
+    if (o->host && !host) return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] is a host session; a batched push takes device sessions", who, i);
+    if (!o->host && host)
+      return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] is a device session; davo_odometry_push_many takes it", who, i);
   }
   const SeqReads rv = seq_reads(ctx, DAVO_PAIRS_ALL);                      // what the variant reads at all
   const size_t hw = (size_t)c.H * c.W;
@@ -2675,6 +2839,19 @@ extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, co
     if (rv.flow) CU_OK(cudaMalloc((void**)&ctx->m_flow, mb * hw * 4 * 4));
     CU_OK(cudaMalloc((void**)&ctx->m_pose, mb * 12 * 4));
   }
+  size_t h2d = 0;
+  int set = 0;
+  if (host) {
+    if (int rc = host_setup(ctx, who); rc < 0) return rc;
+    if (int rc = host_order_first_call(ctx, st)) return rc;
+    if (!ctx->m_hpose) CU_OK(cudaMalloc((void**)&ctx->m_hpose, (size_t)c.max_batch * 12 * 4));
+    for (int i = 0, s = 0; i < n; s += ds[i].ns, ++i) {                   // device results, copied back at the end
+      ds[i].pose_out = ctx->m_hpose + (size_t)12 * s;
+      ds[i].traj_out = sessions[i]->d_traj;
+    }
+    set = (int)(ctx->a_calls++ & 1);
+    if (int rc = many_host_arrivals(ctx, n, sessions, ds.data(), st, set, &h2d)) return rc;
+  }
   // the descriptors: one copy from a pinned ring slot, refilled only after the call that last used it has finished
   const int slot = (int)(ctx->m_calls++ % davo_ctx::kManyRing);
   const size_t sess_bytes = sizeof(OdoManySession) * n, bytes = sess_bytes + sizeof(int2) * B;
@@ -2701,6 +2878,7 @@ extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, co
     sp.smp = reinterpret_cast<const int2*>(static_cast<const uint8_t*>(ctx->m_ddesc[slot]) + sess_bytes);
     sp.hw = (long long)hw; sp.na = nA;
     sp.flow = rv.flow; sp.labels = rv.labels; sp.tgt_labels = rv.tgt_labels; sp.depth = rv.depth;
+    sp.lab8 = host && ctx->host_seg8;
     sp.img = ctx->m_img; sp.lab = ctx->m_lab; sp.dep = ctx->m_depth; sp.fl = ctx->m_flow;
     odo_stage_kernel<<<dim3(std::min(32, std::max(1, kCopyBlocks / B)), B), 256, 0, st>>>(sp);
     CU_OK(cudaGetLastError());
@@ -2708,6 +2886,12 @@ extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, co
   // a separate launch: the stage kernel reads the carried frames this one overwrites
   odo_carry_kernel<<<dim3(std::min(16, std::max(1, kCopyBlocks / n)), n), 256, 0, st>>>(dsess, (long long)hw, rv.depth);
   CU_OK(cudaGetLastError());
+  if (host) {
+    // the arrivals set is free again, and a single host push, which reads and writes the carried state on the copy
+    // stream, must not start before the carry kernel has written it
+    CU_OK(cudaEventRecord(ctx->a_done[set], st));
+    CU_OK(cudaStreamWaitEvent(ctx->copy_stream, ctx->a_done[set], 0));
+  }
   if (B > 0) {
     auto view = [&](int b0) {
       return stacked_view(c.H, c.W, ctx->m_img + hw * 9 * b0, ctx->m_flow ? ctx->m_flow + hw * 4 * b0 : nullptr,
@@ -2721,6 +2905,18 @@ extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, co
     CU_OK(cudaGetLastError());
   }
   CU_OK(cudaEventRecord(ctx->m_ev[slot], st));
+  if (host) {                                                             // each session's results to its host buffers
+    long long d2h = 0;
+    for (int i = 0; i < n; ++i) {
+      const size_t np = (size_t)12 * 4 * ds[i].ns, nt = (size_t)16 * 8 * (ds[i].ns + 2 * ds[i].first);
+      if (np) CU_OK(cudaMemcpyAsync(pose_out[i], ds[i].pose_out, np, cudaMemcpyDeviceToHost, st));
+      if (nt) CU_OK(cudaMemcpyAsync(traj_out[i], ds[i].traj_out, nt, cudaMemcpyDeviceToHost, st));
+      d2h += (long long)(np + nt);
+    }
+    if (int rc = host_done(ctx, st, ticket)) return rc;
+    ctx->last_h2d = (long long)h2d;
+    ctx->last_d2h = d2h;
+  }
   for (int i = 0; i < n; ++i) {                                           // host bookkeeping, once all is enqueued
     const int nt = ds[i].ns + 2 * ds[i].first;
     sessions[i]->pushed += k[i];
@@ -2729,6 +2925,23 @@ extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, co
     if (n_traj) n_traj[i] = nt;
   }
   return 0;
+}
+
+extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
+                                       const float* const* flow_fwd, const float* const* flow_bwd,
+                                       const float* const* seg, const float* const* depth, float* const* pose_out,
+                                       double* const* traj_out, int* n_samples, int* n_traj, void* stream) {
+  return odometry_push_many_impl(false, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, n_samples,
+                                 n_traj, stream, nullptr);
+}
+
+extern "C" int davo_odometry_push_many_host(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
+                                            const float* const* flow_fwd, const float* const* flow_bwd,
+                                            const float* const* seg, const float* const* depth, float* const* pose_out,
+                                            double* const* traj_out, int* n_samples, int* n_traj, void* stream,
+                                            long long* ticket) {
+  return odometry_push_many_impl(true, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, n_samples,
+                                 n_traj, stream, ticket);
 }
 
 extern "C" int davo_odometry_reset(davo_odometry* o) {

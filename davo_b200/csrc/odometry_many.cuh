@@ -2,14 +2,17 @@
 //
 //   odo_stage_kernel        : every sample of the call into one stacked-triplet staging batch (input_view.cuh:
 //                             stacked_view), each frame slot from the session's carried state or the caller's buffer,
-//                             only the planes the sample's pair selection reads; labels become bytes on the way
+//                             only the planes the sample's pair selection reads; float labels become bytes on the
+//                             way, byte labels (host sessions: davo_odometry_push_many_host) are copied
 //   odo_carry_kernel        : each session's new carried state (last two frames, the flow_fwd entry a later sample
 //                             reads) from its old carried state and the caller's buffers
 //   odo_compose_many_kernel : one warp per session: its pose rows out of the staging poses, its relative motions and
 //                             its absolute poses, chained with the code of a single push (trajectory.cuh: traj_chain)
 // A push of session i is the virtual sequence of davo_odometry_push: its last `head` carried frames, then its k new
 // ones; virtual frame v < head is carried frame v, else the caller's frame v - head; virtual flow entry v < fe is the
-// carried flow_fwd entry, else the caller's entry v - fe.  Sample s is virtual frames (s, s+1, s+2).
+// carried flow_fwd entry, else the caller's entry v - fe.  Sample s is virtual frames (s, s+1, s+2).  For host sessions
+// "the caller's buffers" are the call's arrivals set on the device, which holds the caller's frames and entries at
+// the same indices (davo_capi.cu: many_host_arrivals).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -22,8 +25,10 @@ namespace davo {
 struct OdoManySession {
   const uint8_t* img;                       // the caller's buffers of this push
   const float *seg, *depth, *fwd, *bwd;
-  uint8_t* c_img;                           // carried state (davo_odometry: c_img, c_seg, c_depth, c_fwd, d_P)
+  const uint8_t* seg8;                      // the labels as bytes (host sessions with byte labels), else NULL
+  uint8_t* c_img;                           // carried state (davo_odometry: c_img, c_seg or c_seg8, c_depth, c_fwd, d_P)
   float *c_seg, *c_depth, *c_fwd;
+  uint8_t* c_seg8;
   double* P;
   float* pose_out;                          // [ns,2,6]
   Mat4 *traj_out, *rel;                     // [ns + 2 first]; the session's relative-motion scratch
@@ -39,6 +44,7 @@ struct OdoStageParams {
   long long hw;
   int na;                                   // staging samples [0, na) compute both pairs, the rest tgt -> src1 only
   int flow, labels, tgt_labels, depth;      // what the variant reads (davo_capi.cu: SeqReads)
+  int lab8;                                 // the sessions hold their labels as bytes (seg8, c_seg8), else as floats
   uint8_t* img;                             // staging batch, stacked triplets
   uint8_t* lab;
   float *dep, *fl;
@@ -101,8 +107,10 @@ __global__ void __launch_bounds__(256) odo_stage_kernel(const OdoStageParams p) 
     const size_t f = carried ? (size_t)v : (size_t)(v - head);
     const size_t slot = (size_t)b * 3 + j;
     odo_copy(p.img + slot * hw * 3, (carried ? d.c_img : d.img) + f * hw * 3, hw * 3, t, stride);
-    if (p.labels && (j == 2 || j == 0 || p.tgt_labels))
-      odo_labels(p.lab + slot * hw, (carried ? d.c_seg : d.seg) + f * hw, hw, t, stride);
+    if (p.labels && (j == 2 || j == 0 || p.tgt_labels)) {
+      if (p.lab8) odo_copy(p.lab + slot * hw, (carried ? d.c_seg8 : d.seg8) + f * hw, hw, t, stride);
+      else odo_labels(p.lab + slot * hw, (carried ? d.c_seg : d.seg) + f * hw, hw, t, stride);
+    }
     if (p.depth)
       odo_copy(reinterpret_cast<uint8_t*>(p.dep + slot * hw),
                reinterpret_cast<const uint8_t*>((carried ? d.c_depth : d.depth) + f * hw), hw * 4, t, stride);
@@ -161,6 +169,7 @@ __global__ void __launch_bounds__(256) odo_carry_kernel(const OdoManySession* __
   if (d.c_seg)
     odo_carry_frames(reinterpret_cast<uint8_t*>(d.c_seg), reinterpret_cast<const uint8_t*>(d.c_seg),
                      reinterpret_cast<const uint8_t*>(d.seg), d.head, n, hw * 4, t, stride);
+  if (d.c_seg8) odo_carry_frames(d.c_seg8, d.c_seg8, d.seg8, d.head, n, hw, t, stride);   // byte labels
   if (depth)
     odo_carry_frames(reinterpret_cast<uint8_t*>(d.c_depth), reinterpret_cast<const uint8_t*>(d.c_depth),
                      reinterpret_cast<const uint8_t*>(d.depth), d.head, n, hw * 4, t, stride);

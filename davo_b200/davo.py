@@ -433,36 +433,45 @@ class DAVO(object):
         return numpy arrays, else CUDA tensors in and out."""
         return Odometry(self, pairs, self.batch_size if max_push is None else max_push, host)
 
-    def odometry_push_many(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None):
-        """One push on each of several device sessions of this handle, in one forward pass (include/davo_b200.h:
-        davo_odometry_push_many).  ``img``, ``flow_fwd``, ``flow_bwd``, ``seg`` and ``depth`` are lists aligned with
-        ``sessions``, entry i holding the CUDA tensors ``sessions[i].push`` takes (None, or a list of None, where no
-        entry has one).  Returns the list of the dicts ``push`` returns; the results are the bits of pushing each
-        session alone, in list order.  Enqueued on the current stream."""
+    def _many_args(self, sessions, img, flow_fwd, flow_bwd, seg, depth, host, who):
+        """The list and session checks of the batched pushes; returns the sessions, each entry's inputs and its
+        (k, n_samples, n_traj)."""
         sessions = list(sessions)
         n = len(sessions)
         per = lambda x: [None] * n if x is None else list(x)
         lists = {"img": per(img), "flow_fwd": per(flow_fwd), "flow_bwd": per(flow_bwd), "seg": per(seg), "depth": per(depth)}
         for name, x in lists.items():
             if len(x) != n:
-                raise ValueError("DAVO.odometry_push_many: %s has %d entries for %d sessions" % (name, len(x), n))
+                raise ValueError("DAVO.%s: %s has %d entries for %d sessions" % (who, name, len(x), n))
         if n == 0:
-            raise ValueError("DAVO.odometry_push_many: no session")
+            raise ValueError("DAVO.%s: no session" % who)
         for i, od in enumerate(sessions):
             if not isinstance(od, Odometry) or od._system is not self:
-                raise ValueError("DAVO.odometry_push_many: session %d is not a session of this handle" % i)
-            if od._host:
-                raise ValueError("DAVO.odometry_push_many: session %d is a host session; a batched push takes device "
-                                 "sessions (DAVO.odometry(host=False))" % i)
+                raise ValueError("DAVO.%s: session %d is not a session of this handle" % (who, i))
+            if od._host and not host:
+                raise ValueError("DAVO.%s: session %d is a host session; a batched push takes device sessions "
+                                 "(DAVO.odometry(host=False)); DAVO.odometry_push_many_host takes host sessions" % (who, i))
+            if host and not od._host:
+                raise ValueError("DAVO.%s: session %d is a device session; DAVO.odometry_push_many takes it" % (who, i))
             if any(od is o for o in sessions[:i]):
-                raise ValueError("DAVO.odometry_push_many: session %d is given twice" % i)
+                raise ValueError("DAVO.%s: session %d is given twice" % (who, i))
         ins, counts = [], []
-        for i, od in enumerate(sessions):                    # shapes of every entry, then where the tensors live
+        for i, od in enumerate(sessions):                    # shapes of every entry
             x = [lists[name][i] for name in ("img", "flow_fwd", "flow_bwd", "seg", "depth")]
-            k, x[4] = od._args(*x, who="DAVO.odometry_push_many: session %d" % i)
+            k, x[4] = od._args(*x, who="DAVO.%s: session %d" % (who, i))
             ins.append(x)
             counts.append((k,) + od._counts(k))
-        for i, (od, x) in enumerate(zip(sessions, ins)):
+        return sessions, ins, counts
+
+    def odometry_push_many(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None):
+        """One push on each of several device sessions of this handle, in one forward pass (include/davo_b200.h:
+        davo_odometry_push_many).  ``img``, ``flow_fwd``, ``flow_bwd``, ``seg`` and ``depth`` are lists aligned with
+        ``sessions``, entry i holding the CUDA tensors ``sessions[i].push`` takes (None, or a list of None, where no
+        entry has one).  Returns the list of the dicts ``push`` returns; the results are the bits of pushing each
+        session alone, in list order.  Enqueued on the current stream."""
+        sessions, ins, counts = self._many_args(sessions, img, flow_fwd, flow_bwd, seg, depth, False, "odometry_push_many")
+        n = len(sessions)
+        for i, (od, x) in enumerate(zip(sessions, ins)):     # where the tensors live
             od._check_device(*x, who="DAVO.odometry_push_many: session %d" % i)
         import torch
         dev = "cuda:%d" % self.device
@@ -484,6 +493,60 @@ class DAVO(object):
             od._pushed += k
             od._posed += m
         return res
+
+    def odometry_push_many_host(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None):
+        """One push on each of several host sessions of this handle, in one forward pass (include/davo_b200.h:
+        davo_odometry_push_many_host): many cameras whose frames arrive in host memory.  The lists are those of
+        ``odometry_push_many``, holding the numpy arrays ``sessions[i].push`` takes.  Returns the list of the dicts
+        ``push`` returns; the results are the bits of pushing each session alone, in list order."""
+        return self.odometry_push_many_host_async(sessions, img, flow_fwd, flow_bwd, seg, depth, _block=True).result()
+
+    def odometry_push_many_host_async(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None, _block=False):
+        """``odometry_push_many_host`` without waiting: returns a handle whose ``.result()`` gives the list of dicts.
+        The results land in each session's page-locked ring slot (as ``Odometry.push_async``); the inputs must stay
+        unmodified until ``.result()``.  Up to 8 calls may be in flight."""
+        who = "odometry_push_many_host"
+        sessions, ins, counts = self._many_args(sessions, img, flow_fwd, flow_bwd, seg, depth, True, who)
+        n = len(sessions)
+        conv = lambda a, dt: None if a is None else np.ascontiguousarray(a, dtype=dt)
+        dts = (np.uint8, np.float32, np.float32, np.float32, np.float32)
+        ins = [tuple(conv(a, dt) for a, dt in zip(x, dts)) for x in ins]
+        if _block:
+            outs = [(np.zeros((ns, 2, 6), np.float32), np.empty((nt, 4, 4), np.float64)) for _, ns, nt in counts]
+        else:
+            outs = [od._ring_slot(ns, nt) for od, (_, ns, nt) in zip(sessions, counts)]
+        vp = C.c_void_p
+        hp = lambda a: a.ctypes.data if a is not None and a.size else None
+        arr = lambda vals: (vp * n)(*vals)
+        cols = [arr([hp(x[j]) for x in ins]) for j in range(5)]
+        ns, nt = (C.c_int * n)(), (C.c_int * n)()
+        ticket = C.c_longlong(0)
+        self._check(self._lib.davo_odometry_push_many_host(
+            n, arr([od._o.value for od in sessions]), (C.c_int * n)(*[c[0] for c in counts]), *cols,
+            arr([hp(o[0]) for o in outs]), arr([hp(o[1]) for o in outs]), ns, nt, None,
+            None if _block else C.byref(ticket)), "davo_odometry_push_many_host")
+        res = []
+        for od, (k, _, _), (pose, traj), m in zip(sessions, counts, outs, nt):
+            res.append(Odometry._Pending(None, {'pose': pose, 'trajectory': traj, 'frames': range(od._posed, od._posed + m)}))
+            od._pushed += k
+            od._posed += m
+        return DAVO._PendingMany(self, None if _block else ticket.value, res, None if _block else ins)
+
+    class _PendingMany(object):
+        """A queued batched host push; ``result()`` waits for it and returns the list of the dicts ``push`` returns."""
+
+        def __init__(self, system, ticket, pending, keep):
+            self._system, self._ticket, self._pending, self._keep = system, ticket, pending, keep
+
+        def result(self):
+            if self._ticket is not None:
+                s = self._system
+                s._check(s._lib.davo_host_wait(s._h, self._ticket), "davo_host_wait")
+                self._ticket, self._keep = None, None
+                for p in self._pending:                      # own copies: the pinned ring slots are reused
+                    p._out = {'pose': np.array(p._out['pose']), 'trajectory': np.array(p._out['trajectory']),
+                              'frames': p._out['frames']}
+            return [p.result() for p in self._pending]
 
     def bind_host_numa(self):
         """Bind this thread (and threads created after it) to the CPUs next to this handle's GPU
@@ -671,16 +734,20 @@ class Odometry(object):
             pose, traj = np.zeros((n_s, 2, 6), np.float32), np.empty((n_t, 4, 4), np.float64)
             frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, None)
             return Odometry._Pending(None, {'pose': pose, 'trajectory': traj, 'frames': frames}, None)
+        pose, traj = self._ring_slot(n_s, n_t)
+        ticket = C.c_longlong(0)
+        frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, C.byref(ticket))
+        return Odometry._Pending(self._system, {'pose': pose, 'trajectory': traj, 'frames': frames}, ticket.value, ins)
+
+    def _ring_slot(self, n_s, n_t):
+        """The next page-locked (pose, trajectory) output pair of an asynchronous host push, single or batched."""
         import torch
         if self._ring is None:                      # page-locked results, one slot per call that can be in flight
             self._ring = [(torch.empty((self.max_push, 2, 6), dtype=torch.float32).pin_memory(),
                            torch.empty((self.max_push + 2, 4, 4), dtype=torch.float64).pin_memory()) for _ in range(8)]
         slot = self._ring[self._ring_n % 8]
         self._ring_n += 1
-        pose, traj = slot[0][:n_s].numpy(), slot[1][:n_t].numpy()
-        ticket = C.c_longlong(0)
-        frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, C.byref(ticket))
-        return Odometry._Pending(self._system, {'pose': pose, 'trajectory': traj, 'frames': frames}, ticket.value, ins)
+        return slot[0][:n_s].numpy(), slot[1][:n_t].numpy()
 
     def push(self, img, flow_fwd, flow_bwd, seg=None, depth=None):
         return self.push_async(img, flow_fwd, flow_bwd, seg, depth, _block=True).result()

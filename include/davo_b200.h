@@ -284,6 +284,27 @@ int davo_odometry_push_many(int n, davo_odometry* const* sessions, const int* k,
                             const float* const* flow_fwd, const float* const* flow_bwd, const float* const* seg,
                             const float* const* depth, float* const* pose_out, double* const* traj_out,
                             int* n_samples, int* n_traj, void* cuda_stream);
+/* davo_odometry_push_many_host: one push on each of n host sessions (host_inputs = 1) of one handle, in one forward
+ *   pass -- many cameras whose frames arrive in host memory.  Entry i is what davo_odometry_push(sessions[i], k[i],
+ *   img[i], ..., cuda_stream, ticket) takes on a host session: the same host buffers, shapes, NULL rules, 16-byte
+ *   alignment and output rows; whole arrays may be NULL as for davo_odometry_push_many.  The results are bit-identical
+ *   to pushing each session alone with davo_odometry_push, in array order (pose_out, traj_out, the counts and every
+ *   later push, single or batched); sessions may be in any state and either pair mode, and single and batched host
+ *   pushes mix freely on the same sessions.  ticket == NULL: blocks until every session's results are in host memory;
+ *   otherwise the outputs must be page-locked, the call returns once everything is queued, davo_host_wait(ctx, *ticket)
+ *   waits for it, and the inputs must not be written before then.  Each new frame, label plane, depth plane and flow
+ *   entry that some computed pair of its stream reads is copied once, as by the single push (labels narrowed to bytes
+ *   on the CPU unless DAVO_B200_HOST_SEG8=0; the flow as float32); davo_last_host_copy_bytes reports the call's data
+ *   bytes, with the default configuration the sum of what the same pushes made one by one report.  The kernel launches
+ *   do not depend on n; the copies are per session.  The first call allocates two arrivals sets that grow on demand,
+ *   freed with the handle.
+ *   Argument errors return DAVO_ERR_ARG with a message naming the input and the session index, as for
+ *   davo_odometry_push_many; a device session is refused (davo_odometry_push_many takes it).  A refused call enqueues
+ *   nothing and changes no session. */
+int davo_odometry_push_many_host(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
+                                 const float* const* flow_fwd, const float* const* flow_bwd, const float* const* seg,
+                                 const float* const* depth, float* const* pose_out, double* const* traj_out,
+                                 int* n_samples, int* n_traj, void* cuda_stream, long long* ticket);
 int davo_odometry_reset(davo_odometry*);
 int davo_odometry_frames(const davo_odometry*, long long* pushed, long long* posed);
 void davo_odometry_destroy(davo_odometry*);
