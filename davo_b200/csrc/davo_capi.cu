@@ -197,6 +197,7 @@ struct davo_ctx {
   std::string err;
   std::map<std::string, HostTensor> weights;
   bool finalized = false;
+  uint64_t weights_digest = 0;      // of the values davo_finalize_weights was given (weights_digest_of)
   int mb = 0;                       // frame pairs per micro-batch
   int packed_c = 16;                // channels per pixel of the packed PoseNN input (8 or 16)
   int conv_impl = 0;                // 0 tcgen05 (product), 1 direct fp32 (debug cross-check)
@@ -378,6 +379,26 @@ int dev_alloc(davo_ctx* ctx, void** p, size_t bytes) {
 const HostTensor* find_w(davo_ctx* ctx, const std::string& name) {
   auto it = ctx->weights.find(name);
   return it == ctx->weights.end() ? nullptr : &it->second;
+}
+
+// 64-bit digest of every variable in name order: its name, shape and float32 bits (davo_odometry_move compares two
+// handles' weights with it).  Each step, h = f(h ^ word) with f a bijection, so a single differing word changes it.
+uint64_t weights_digest_of(const std::map<std::string, HostTensor>& weights) {
+  uint64_t h = 0xcbf29ce484222325ull;
+  auto mix = [&h](uint64_t x) { h ^= x; h *= 0x100000001b3ull; h ^= h >> 32; };
+  for (const auto& kv : weights) {
+    mix(kv.first.size());
+    for (unsigned char ch : kv.first) mix(ch);
+    mix(kv.second.shape.size());
+    for (int64_t d : kv.second.shape) mix((uint64_t)d);
+    const std::vector<float>& v = kv.second.data;
+    for (size_t i = 0; i < v.size(); ++i) {
+      uint32_t u;
+      memcpy(&u, &v[i], 4);
+      mix(u);
+    }
+  }
+  return h;
 }
 
 bool shape_is(const HostTensor* t, std::initializer_list<int64_t> s) {
@@ -1774,6 +1795,7 @@ extern "C" int davo_finalize_weights(davo_ctx* ctx) {
     CU_OK(cudaMemcpy(ctx->d_staticw, s.data(), 19 * 4, cudaMemcpyHostToDevice));
   }
   CU_OK(cudaDeviceSynchronize());
+  ctx->weights_digest = weights_digest_of(ctx->weights);
   ctx->finalized = true;
   return 0;
 }
@@ -2475,6 +2497,35 @@ static void odometry_free(davo_odometry* o) {
   delete o;
 }
 
+// A session's buffers on its handle's device (o->ctx): the carried state, the relative motions, a host session's
+// absolute poses, a device session's frame set.  A host session's frame sets come with its first push.
+static int odometry_alloc(davo_odometry* o) {
+  davo_ctx* ctx = o->ctx;
+  CU_OK(cudaSetDevice(ctx->device));
+  const davo_config& c = ctx->cfg;
+  const SeqReads r = seq_reads(ctx, o->pairs);
+  const size_t hw = (size_t)c.H * c.W, nf = (size_t)o->max_push + 2;
+  const bool seg8 = o->host && ctx->host_seg8;                     // the form the passes read the labels in
+  auto alloc = [&](void** p, size_t bytes) -> int {
+    CU_OK(cudaMalloc(p, bytes));
+    return 0;
+  };
+  int rc = alloc((void**)&o->c_img, hw * 3 * 2);
+  if (!rc && c.att_src != 0) rc = seg8 ? alloc((void**)&o->c_seg8, hw * 2) : alloc((void**)&o->c_seg, hw * 4 * 2);
+  if (!rc && r.depth) rc = alloc((void**)&o->c_depth, hw * 4 * 2);
+  if (!rc && r.flow) rc = alloc((void**)&o->c_fwd, hw * 2 * 4);
+  if (!rc) rc = alloc((void**)&o->d_P, 16 * sizeof(double));
+  if (!rc) rc = alloc((void**)&o->d_rel, (size_t)(o->max_push + 1) * sizeof(Mat4));
+  if (!rc && o->host) rc = alloc((void**)&o->d_traj, (size_t)(o->max_push + 2) * sizeof(Mat4));
+  if (!rc && !o->host) {                                           // one frame set, filled on the caller's stream
+    rc = alloc((void**)&o->q_img[0], nf * hw * 3);
+    if (!rc && c.att_src != 0) rc = alloc((void**)&o->q_seg[0], nf * hw * 4);
+    if (!rc && r.depth) rc = alloc((void**)&o->q_depth[0], nf * hw * 4);
+    if (!rc && r.flow) rc = alloc((void**)&o->d_fwd, (size_t)(o->max_push + 1) * hw * 2 * 4);
+  }
+  return rc;
+}
+
 extern "C" int davo_odometry_create(davo_ctx* ctx, int max_push, int pairs, int host_inputs, davo_odometry** out) {
   if (!ctx) return DAVO_ERR_ARG;
   const char* who = "davo_odometry_create";
@@ -2487,31 +2538,9 @@ extern "C" int davo_odometry_create(davo_ctx* ctx, int max_push, int pairs, int 
     return fail(ctx, DAVO_ERR_ARG, "%s: pairs %d: a session takes DAVO_PAIRS_TRAJECTORY or DAVO_PAIRS_ALL", who, pairs);
   if (max_push < 1 || max_push > ctx->cfg.max_batch)
     return fail(ctx, DAVO_ERR_ARG, "%s: max_push=%d outside 1..max_batch %d", who, max_push, ctx->cfg.max_batch);
-  CU_OK(cudaSetDevice(ctx->device));
   davo_odometry* o = new davo_odometry;
   o->ctx = ctx; o->max_push = max_push; o->pairs = pairs; o->host = host_inputs != 0;
-  const davo_config& c = ctx->cfg;
-  const SeqReads r = seq_reads(ctx, pairs);
-  const size_t hw = (size_t)c.H * c.W, nf = (size_t)max_push + 2;
-  const bool seg8 = o->host && ctx->host_seg8;                     // the form the passes read the labels in
-  auto alloc = [&](void** p, size_t bytes) -> int {
-    CU_OK(cudaMalloc(p, bytes));
-    return 0;
-  };
-  int rc = alloc((void**)&o->c_img, hw * 3 * 2);
-  if (!rc && c.att_src != 0) rc = seg8 ? alloc((void**)&o->c_seg8, hw * 2) : alloc((void**)&o->c_seg, hw * 4 * 2);
-  if (!rc && r.depth) rc = alloc((void**)&o->c_depth, hw * 4 * 2);
-  if (!rc && r.flow) rc = alloc((void**)&o->c_fwd, hw * 2 * 4);
-  if (!rc) rc = alloc((void**)&o->d_P, 16 * sizeof(double));
-  if (!rc) rc = alloc((void**)&o->d_rel, (size_t)(max_push + 1) * sizeof(Mat4));
-  if (!rc && o->host) rc = alloc((void**)&o->d_traj, (size_t)(max_push + 2) * sizeof(Mat4));
-  if (!rc && !o->host) {                                           // one frame set, filled on the caller's stream
-    rc = alloc((void**)&o->q_img[0], nf * hw * 3);
-    if (!rc && c.att_src != 0) rc = alloc((void**)&o->q_seg[0], nf * hw * 4);
-    if (!rc && r.depth) rc = alloc((void**)&o->q_depth[0], nf * hw * 4);
-    if (!rc && r.flow) rc = alloc((void**)&o->d_fwd, (size_t)(max_push + 1) * hw * 2 * 4);
-  }
-  if (rc) { odometry_free(o); return rc; }
+  if (int rc = odometry_alloc(o)) { odometry_free(o); return rc; }
   {
     std::lock_guard<std::mutex> lk(g_odo_mutex);
     g_odo_live.insert(o);
@@ -2968,6 +2997,89 @@ extern "C" void davo_odometry_destroy(davo_odometry* o) {
   cudaSetDevice(o->ctx->device);
   cudaDeviceSynchronize();                                         // work still queued may read the session's buffers
   odometry_free(o);
+}
+
+// Re-homes a session (include/davo_b200.h: davo_odometry_move).  A push reads of the session only the counts and the
+// carried state, and a pose does not depend on the handle that computes it (same configuration and weights: a
+// pair's result does not depend on which pairs share its pass, so not on max_batch either); so the carried state,
+// copied as it is onto buffers allocated as davo_odometry_create allocates them on dst, continues the stream with the
+// same bits.  The new buffers are allocated first, so a failure leaves the session where it was.
+extern "C" int davo_odometry_move(davo_odometry* o, davo_ctx* dst) {
+  const char* who = "davo_odometry_move";
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    if (!o || !g_odo_live.count(o)) return fail(nullptr, DAVO_ERR_ARG, "%s: the session is NULL or was destroyed", who);
+  }
+  davo_ctx* ctx = o->ctx;
+  if (!dst) return fail(ctx, DAVO_ERR_ARG, "%s: dst is NULL", who);
+  if (dst == ctx) return 0;
+  const davo_config &a = ctx->cfg, &b = dst->cfg;
+  static const struct { const char* name; int32_t davo_config::*f; } fields[] = {
+      {"H", &davo_config::H}, {"W", &davo_config::W}, {"posenn", &davo_config::posenn},
+      {"cnv6_out", &davo_config::cnv6_out}, {"in_mode", &davo_config::in_mode}, {"att_src", &davo_config::att_src},
+      {"att_tgt_ones", &davo_config::att_tgt_ones}, {"mask_mode", &davo_config::mask_mode},
+      {"se_act", &davo_config::se_act}, {"flow_abs", &davo_config::flow_abs}, {"flow_norm", &davo_config::flow_norm},
+      {"posenn_se", &davo_config::posenn_se}, {"micro_batch", &davo_config::micro_batch},
+      {"depth_norm", &davo_config::depth_norm}, {"se_pool", &davo_config::se_pool},
+      {"se_hidden", &davo_config::se_hidden}, {"pixel_map", &davo_config::pixel_map},
+      {"depth_split", &davo_config::depth_split}, {"flow_f16", &davo_config::flow_f16},
+      {"batch_norm", &davo_config::batch_norm}};                     // every field but max_batch
+  static_assert(sizeof fields / sizeof fields[0] + 1 == sizeof(davo_config) / sizeof(int32_t), "a davo_config field is missing");
+  for (const auto& x : fields)
+    if (a.*x.f != b.*x.f)
+      return fail(ctx, DAVO_ERR_ARG, "%s: dst's davo_config differs in %s (%d here, %d on dst); only max_batch may differ",
+                  who, x.name, a.*x.f, b.*x.f);
+  if (o->max_push > b.max_batch)
+    return fail(ctx, DAVO_ERR_ARG, "%s: the session's max_push %d is more than dst's max_batch %d", who, o->max_push, b.max_batch);
+  if (!ctx->finalized || !dst->finalized)
+    return fail(ctx, DAVO_ERR_ARG, "%s: weights not finalized on the %s handle", who, ctx->finalized ? "dst" : "session's");
+  if (ctx->weights_digest != dst->weights_digest)
+    return fail(ctx, DAVO_ERR_ARG, "%s: the two handles hold different weights", who);
+  // settings fixed at davo_create from the environment that change what a push computes or how a session holds it
+  if (ctx->compensated_rounding != dst->compensated_rounding || ctx->conv_impl != dst->conv_impl)
+    return fail(ctx, DAVO_ERR_ARG, "%s: the two handles round the weights (DAVO_B200_WEIGHT_ROUNDING) or run the convolutions differently", who);
+  if (o->host && a.att_src != 0 && ctx->host_seg8 != dst->host_seg8)
+    return fail(ctx, DAVO_ERR_ARG, "%s: the two handles hold a host session's labels in different forms (DAVO_B200_HOST_SEG8)", who);
+  davo_odometry* t = new davo_odometry;
+  t->ctx = dst; t->max_push = o->max_push; t->pairs = o->pairs; t->host = o->host;
+  if (int rc = odometry_alloc(t)) {
+    ctx->err = dst->err;
+    odometry_free(t);
+    return rc;
+  }
+  const davo_config& c = ctx->cfg;
+  const size_t hw = (size_t)c.H * c.W;
+  const int head = o->head();
+  // the carried flow_fwd entry (global entry pushed - 2) is there when the push that ended at frame `pushed` kept it
+  const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
+  const bool fwd = o->c_fwd && o->pushed >= 2 && rg.fwd((int)std::min(o->pushed - 2, 2LL));
+  struct { void* d; const void* s; size_t bytes; } cp[] = {
+      {t->c_img, o->c_img, hw * 3 * head},
+      {t->c_seg8, o->c_seg8, o->c_seg8 ? hw * head : 0},
+      {t->c_seg, o->c_seg, o->c_seg ? hw * 4 * head : 0},
+      {t->c_depth, o->c_depth, o->c_depth ? hw * 4 * head : 0},
+      {t->c_fwd, o->c_fwd, fwd ? hw * 2 * 4 : 0},
+      {t->d_P, o->d_P, o->posed > 0 ? 16 * sizeof(double) : 0}};
+  auto copy = [&]() -> int {
+    // as davo_odometry_destroy: work still queued on the source device may read or write the carried state
+    CU_OK(cudaSetDevice(ctx->device));
+    CU_OK(cudaDeviceSynchronize());
+    for (const auto& x : cp)                                       // peer access is not needed, and is not enabled
+      if (x.bytes) CU_OK(cudaMemcpyPeerAsync(x.d, dst->device, x.s, ctx->device, x.bytes, 0));
+    CU_OK(cudaStreamSynchronize(0));
+    return 0;
+  };
+  if (int rc = copy()) {
+    odometry_free(t);
+    return rc;
+  }
+  t->pushed = o->pushed; t->posed = o->posed;
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    std::swap(*o, *t);                                             // t: the old buffers, on the source handle
+  }
+  odometry_free(t);
+  return 0;
 }
 
 // davo_destroy: the handle's sessions go with it

@@ -765,6 +765,34 @@ class Odometry(object):
                              'frames': self._out['frames']}           # own copies: the pinned ring slot is reused
             return self._out
 
+    def move_to(self, system):
+        """Re-home this session onto the handle ``system``, which may be on another GPU (include/davo_b200.h:
+        davo_odometry_move): every later push gives the bits it would have given without the move, and the session now
+        belongs to ``system`` (its ``close`` destroys the session; a batched push on ``system`` takes it).  The target
+        is checked before any device work: set up, weights loaded, the same version and frame size.  Waits for the
+        session's device and returns once the carried state has been copied.  Returns ``self``."""
+        s = self._system
+        if self._o is None:
+            raise RuntimeError("Odometry.move_to: the session is closed")
+        if s._h is None:
+            raise RuntimeError("Odometry.move_to: the session was destroyed with its handle")
+        if system is s:
+            return self
+        if not isinstance(system, DAVO) or getattr(system, "_h", None) is None:
+            raise ValueError("Odometry.move_to: the target is not set up (DAVO.setup_inference(mode='davo'))")
+        if not system._weights_loaded:
+            raise ValueError("Odometry.move_to: the target has no weights loaded")
+        if system.version != s.version:
+            raise ValueError("Odometry.move_to: the target runs version %r, the session %r" % (system.version, s.version))
+        if (system.img_height, system.img_width) != (s.img_height, s.img_width):
+            raise ValueError("Odometry.move_to: the target's frames are %dx%d, the session's %dx%d"
+                             % (system.img_height, system.img_width, s.img_height, s.img_width))
+        import torch
+        with torch.cuda.device(s.device):                 # the call switches devices; torch's current one is restored
+            s._check(s._lib.davo_odometry_move(self._o, system._h), "davo_odometry_move")
+        self._system = system
+        return self
+
     def frames(self):
         """(frames pushed, frames whose absolute pose has been returned)."""
         return self._pushed, self._posed

@@ -308,6 +308,24 @@ int davo_odometry_push_many_host(int n, davo_odometry* const* sessions, const in
 int davo_odometry_reset(davo_odometry*);
 int davo_odometry_frames(const davo_odometry*, long long* pushed, long long* posed);
 void davo_odometry_destroy(davo_odometry*);
+/* davo_odometry_move: re-homes a live session onto handle `dst`, which may be on another device -- to rebalance
+ *   cameras over the GPUs of a box, or to drain a handle without restarting its cameras' trajectories.  The session
+ *   pointer stays valid; afterwards it belongs to dst (davo_destroy(dst) destroys it, davo_destroy of the old handle no
+ *   longer does) and takes pushes, single or batched with dst's other sessions, of dst.  Every later push gives the
+ *   bits it would have given without the move: pose_out, traj_out, the counts, davo_odometry_frames, and the host to
+ *   device bytes of a host push.  The counts and the carried state (last two frames with their labels and depth, the
+ *   last flow_fwd entry when a later sample reads it, the last absolute pose) are copied with cudaMemcpyPeerAsync, which
+ *   needs no peer access (none is enabled); the frame sets and per-push buffers are allocated again on dst at the
+ *   session's max_push, and the old buffers are freed.
+ *   Synchronises: first waits for all work on the session's device (as davo_odometry_destroy), then returns once the
+ *   copies are complete.  Tickets issued on the old handle before the move stay valid there.
+ *   A move to the session's own handle returns 0 and does nothing.  Refused with DAVO_ERR_ARG, changing nothing, and a
+ *   message on the session's handle (davo_last_error(NULL) for a NULL or destroyed session) naming the reason: a NULL
+ *   or destroyed session; dst NULL; a davo_config field other than max_batch that differs (named); the session's
+ *   max_push above dst's max_batch; weights not finalized on either handle; different weights (a digest of the values
+ *   davo_finalize_weights was given); a different DAVO_B200_WEIGHT_ROUNDING or conv implementation; for a host session
+ *   with labels, a different DAVO_B200_HOST_SEG8. */
+int davo_odometry_move(davo_odometry*, davo_ctx* dst);
 
 /* Binds the calling thread (and the threads it creates afterwards: the handle's conversion pool, the caller's
  * loader threads) to the CPUs of the NUMA node the handle's GPU hangs off (/sys/bus/pci/devices/<id>/numa_node,
