@@ -26,6 +26,8 @@ SYMBOLS = (
     "davo_forward_sequence", "davo_forward_sequence_host",
     "davo_odometry_create", "davo_odometry_push", "davo_odometry_reset", "davo_odometry_frames",
     "davo_odometry_push_many", "davo_odometry_push_many_host", "davo_odometry_move",
+    "davo_odometry_state_bytes", "davo_odometry_save", "davo_odometry_load", "davo_odometry_save_many",
+    "davo_odometry_load_many",
     "davo_last_error",
     "davo_destroy", "davo_build_info", "davo_config_bytes", "davo_odometry_destroy",
 )
@@ -93,6 +95,12 @@ def load() -> C.CDLL:
     lib.davo_odometry_push_many_host.argtypes = [ip, C.POINTER(vp), C.POINTER(ip)] + [C.POINTER(vp)] * 7 + [
         C.POINTER(ip), C.POINTER(ip), vp, C.POINTER(C.c_longlong)]
     lib.davo_odometry_move.argtypes = [vp, vp]
+    i64, i64p = C.c_int64, C.POINTER(C.c_int64)
+    lib.davo_odometry_state_bytes.argtypes = [vp, i64p]
+    lib.davo_odometry_save.argtypes = [vp, vp, i64, i64p]
+    lib.davo_odometry_load.argtypes = [vp, vp, i64, C.POINTER(vp)]
+    lib.davo_odometry_save_many.argtypes = [ip, C.POINTER(vp), vp, i64, i64p]
+    lib.davo_odometry_load_many.argtypes = [vp, ip, vp, i64p, C.POINTER(vp)]
     lib.davo_odometry_reset.argtypes = [vp]
     lib.davo_odometry_frames.argtypes = [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     lib.davo_odometry_destroy.argtypes = [vp]

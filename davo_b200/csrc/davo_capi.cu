@@ -36,6 +36,7 @@
 #include "comm.cuh"
 #include "trajectory.cuh"
 #include "odometry_many.cuh"
+#include "odometry_state.cuh"
 #include "bn.cuh"
 #include "jpeg.cuh"
 #include "host_convert.h"
@@ -281,6 +282,13 @@ struct davo_ctx {
   cudaEvent_t a_copied[2] = {}, a_done[2] = {};
   long long a_calls = 0;
   float* m_hpose = nullptr;           // the pose rows of each session's push, [max_batch,2,6], copied to the host from here
+  // davo_odometry_save_many / load_many: a staging area laid out as the caller's blobs (a chunk of them at a time), and
+  // the call's blob descriptors, headers and checksum accumulators in one pinned area and its device twin; grown on
+  // demand, used by one synchronous call at a time
+  uint8_t* b_stage = nullptr;
+  size_t b_stage_cap = 0;
+  void *b_hdesc = nullptr, *b_ddesc = nullptr;
+  size_t b_desc_cap = 0;
   std::map<std::pair<const void*, int>, int> max_clusters;   // by (kernel, dynamic shared memory)
   float depth_thres = 0.f;          // -se_flow_on_depthseg_seplayers: the variable se_flow/depth_threshold
   // mode='feature' (features.cuh)
@@ -1428,6 +1436,8 @@ extern "C" void davo_destroy(davo_ctx* ctx) {
     if (ctx->a_done[i]) cudaEventDestroy(ctx->a_done[i]);
   }
   cudaFree(ctx->m_hpose);
+  cudaFree(ctx->b_stage); cudaFree(ctx->b_ddesc);
+  if (ctx->b_hdesc) cudaFreeHost(ctx->b_hdesc);
   delete ctx->pool;
   if (ctx->comm) davo_comm::api().CommDestroy(ctx->comm);
   if (ctx->s_pose) cudaFree(ctx->s_pose);
@@ -2999,6 +3009,158 @@ extern "C" void davo_odometry_destroy(davo_odometry* o) {
   odometry_free(o);
 }
 
+namespace {
+
+// Every davo_config field but max_batch, in the order of davo_config: what two handles must agree on for one to
+// continue the other's sessions (davo_odometry_move, davo_odometry_load).  A saved blob's header stores them so.
+const struct { const char* name; int32_t davo_config::*f; } kSessionConfig[] = {
+    {"H", &davo_config::H}, {"W", &davo_config::W}, {"posenn", &davo_config::posenn},
+    {"cnv6_out", &davo_config::cnv6_out}, {"in_mode", &davo_config::in_mode}, {"att_src", &davo_config::att_src},
+    {"att_tgt_ones", &davo_config::att_tgt_ones}, {"mask_mode", &davo_config::mask_mode},
+    {"se_act", &davo_config::se_act}, {"flow_abs", &davo_config::flow_abs}, {"flow_norm", &davo_config::flow_norm},
+    {"posenn_se", &davo_config::posenn_se}, {"micro_batch", &davo_config::micro_batch},
+    {"depth_norm", &davo_config::depth_norm}, {"se_pool", &davo_config::se_pool},
+    {"se_hidden", &davo_config::se_hidden}, {"pixel_map", &davo_config::pixel_map},
+    {"depth_split", &davo_config::depth_split}, {"flow_f16", &davo_config::flow_f16},
+    {"batch_norm", &davo_config::batch_norm}};
+constexpr int kSessionConfigFields = sizeof kSessionConfig / sizeof kSessionConfig[0];
+static_assert(kSessionConfigFields + 1 == sizeof(davo_config) / sizeof(int32_t), "a davo_config field is missing");
+
+// the form a session of this kind holds its labels in on this handle: 0 none, 1 bytes, 2 float32
+int label_form(const davo_ctx* ctx, bool host) { return ctx->cfg.att_src == 0 ? 0 : host && ctx->host_seg8 ? 1 : 2; }
+
+// What a session carries from one push to the next, decided here alone: davo_odometry_move, _save and _load copy
+// exactly these sections.  They are the last min(pushed, 2) frames' images, labels (in the form the session holds
+// them) and depth planes, the flow_fwd entry a later sample reads (global entry pushed - 2, there when the push that
+// ended at frame `pushed` kept it) and the last absolute pose.  The sizes follow from the handle's configuration, the
+// session's kind and its counts, so they hold for a session whose buffers are not allocated yet; p[] are its buffers.
+// Frame sets, events, per-push buffers and q_calls are not state: a push writes them before it reads them.
+enum { kSecImg, kSecSeg8, kSecSeg, kSecDepth, kSecFwd, kSecPose };
+struct Carried {
+  void* p[kOdoSections];
+  size_t bytes[kOdoSections];
+};
+
+Carried carried_state(const davo_odometry* o) {
+  const davo_ctx* ctx = o->ctx;
+  const size_t hw = (size_t)ctx->cfg.H * ctx->cfg.W, head = (size_t)o->head();
+  const SeqReads r = seq_reads(ctx, o->pairs);                       // what odometry_alloc allocates
+  const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
+  const int lf = label_form(ctx, o->host);
+  const bool fwd = r.flow && o->pushed >= 2 && rg.fwd((int)std::min(o->pushed - 2, 2LL));
+  return {{o->c_img, o->c_seg8, o->c_seg, o->c_depth, o->c_fwd, o->d_P},
+          {hw * 3 * head, lf == 1 ? hw * head : 0, lf == 2 ? hw * 4 * head : 0, r.depth ? hw * 4 * head : 0,
+           fwd ? hw * 2 * 4 : 0, o->posed > 0 ? 16 * sizeof(double) : 0}};
+}
+
+// The header of a saved session (include/davo_b200.h: davo_odometry_save), format version 1, little-endian, no padding.
+struct OdoBlobHeader {
+  char magic[8];                                 // "DAVOSESS"
+  uint32_t version, header_bytes;
+  uint64_t total_bytes;
+  int32_t config[kSessionConfigFields];          // kSessionConfig
+  uint64_t weights_digest;                       // weights_digest_of
+  int32_t weight_rounding, conv_impl;            // 1 compensated, 0 nearest (DAVO_B200_WEIGHT_ROUNDING); davo_ctx::conv_impl
+  int32_t host, label_form;
+  int32_t pairs, max_push;
+  int64_t pushed, posed;
+  int32_t carried_frames, carried_fwd, carried_pose, reserved;
+  uint64_t section_off[kOdoSections], section_bytes[kOdoSections];
+  uint64_t checksum;                             // odometry_state.cuh, over the blob with this field zero
+};
+static_assert(sizeof(OdoBlobHeader) == 272 && offsetof(OdoBlobHeader, checksum) == 264, "the documented header layout");
+constexpr uint32_t kOdoBlobVersion = 1;
+
+// the header of session o's blob, checksum zero; sections back to back after it, each 16-byte aligned
+OdoBlobHeader blob_header(const davo_odometry* o, const Carried& cs) {
+  const davo_ctx* ctx = o->ctx;
+  OdoBlobHeader h;
+  memset(&h, 0, sizeof h);
+  memcpy(h.magic, "DAVOSESS", 8);
+  h.version = kOdoBlobVersion;
+  h.header_bytes = sizeof h;
+  for (int i = 0; i < kSessionConfigFields; ++i) h.config[i] = ctx->cfg.*kSessionConfig[i].f;
+  h.weights_digest = ctx->weights_digest;
+  h.weight_rounding = ctx->compensated_rounding;
+  h.conv_impl = ctx->conv_impl;
+  h.host = o->host;
+  h.label_form = label_form(ctx, o->host);
+  h.pairs = o->pairs;
+  h.max_push = o->max_push;
+  h.pushed = o->pushed;
+  h.posed = o->posed;
+  h.carried_frames = o->head();
+  h.carried_fwd = cs.bytes[kSecFwd] != 0;
+  h.carried_pose = cs.bytes[kSecPose] != 0;
+  uint64_t at = sizeof h;
+  for (int j = 0; j < kOdoSections; ++j) {
+    h.section_off[j] = at;
+    h.section_bytes[j] = cs.bytes[j];
+    at += (cs.bytes[j] + 15) & ~(uint64_t)15;
+  }
+  h.total_bytes = at;
+  return h;
+}
+
+// The descriptor area of a save or load call: n OdoBlob, n headers (save), n checksum accumulators, n block counters.
+struct BlobArea {
+  size_t headers, sums, done, bytes;
+};
+BlobArea blob_area(int n) {
+  auto up = [](size_t b) { return (b + 15) & ~(size_t)15; };
+  BlobArea a;
+  a.headers = up(sizeof(OdoBlob) * n);
+  a.sums = a.headers + sizeof(OdoBlobHeader) * n;
+  a.done = a.sums + 8 * (size_t)n;
+  a.bytes = up(a.done + 4 * (size_t)n);
+  return a;
+}
+
+// Consecutive blobs [first, end) staged together: at most kBlobChunk bytes (a larger blob alone) and one grid's rows.
+// *stage: the staging bytes the largest chunk needs.
+constexpr size_t kBlobChunk = (size_t)256 << 20;
+std::vector<std::pair<int, int>> blob_chunks(int n, const int64_t* offsets, size_t* stage) {
+  std::vector<std::pair<int, int>> ch;
+  *stage = 0;
+  for (int i = 0; i < n;) {
+    int e = i + 1;
+    while (e < n && e - i < 65535 && (size_t)(offsets[e + 1] - offsets[i]) <= kBlobChunk) ++e;
+    ch.push_back({i, e});
+    *stage = std::max(*stage, (size_t)(offsets[e] - offsets[i]));
+    i = e;
+  }
+  return ch;
+}
+
+// the handle's staging and descriptor areas at least this large (the calls using them are synchronous)
+int blob_buffers(davo_ctx* ctx, size_t stage, size_t desc) {
+  if (ctx->b_stage_cap < stage) {
+    if (ctx->b_stage) { CU_OK(cudaFree(ctx->b_stage)); ctx->b_stage = nullptr; }
+    ctx->b_stage_cap = 0;
+    CU_OK(cudaMalloc((void**)&ctx->b_stage, stage));
+    ctx->b_stage_cap = stage;
+  }
+  if (ctx->b_desc_cap < desc) {
+    const size_t cap = std::max(desc, 2 * ctx->b_desc_cap);
+    if (ctx->b_hdesc) { CU_OK(cudaFreeHost(ctx->b_hdesc)); ctx->b_hdesc = nullptr; }
+    if (ctx->b_ddesc) { CU_OK(cudaFree(ctx->b_ddesc)); ctx->b_ddesc = nullptr; }
+    ctx->b_desc_cap = 0;
+    CU_OK(cudaHostAlloc(&ctx->b_hdesc, cap, cudaHostAllocDefault));
+    CU_OK(cudaMalloc(&ctx->b_ddesc, cap));
+    ctx->b_desc_cap = cap;
+  }
+  return 0;
+}
+
+dim3 blob_grid(int rows) { return dim3(std::min(32, std::max(1, 4 * 148 / rows)), rows); }
+
+// "sessions[i]: " / "blob i: " for the _many forms, nothing for the single ones
+std::string at_index(bool many, const char* what, int i) {
+  return many ? std::string(what) + "[" + std::to_string(i) + "]: " : std::string();
+}
+
+}  // namespace
+
 // Re-homes a session (include/davo_b200.h: davo_odometry_move).  A push reads of the session only the counts and the
 // carried state, and a pose does not depend on the handle that computes it (same configuration and weights: a
 // pair's result does not depend on which pairs share its pass, so not on max_batch either); so the carried state,
@@ -3014,18 +3176,7 @@ extern "C" int davo_odometry_move(davo_odometry* o, davo_ctx* dst) {
   if (!dst) return fail(ctx, DAVO_ERR_ARG, "%s: dst is NULL", who);
   if (dst == ctx) return 0;
   const davo_config &a = ctx->cfg, &b = dst->cfg;
-  static const struct { const char* name; int32_t davo_config::*f; } fields[] = {
-      {"H", &davo_config::H}, {"W", &davo_config::W}, {"posenn", &davo_config::posenn},
-      {"cnv6_out", &davo_config::cnv6_out}, {"in_mode", &davo_config::in_mode}, {"att_src", &davo_config::att_src},
-      {"att_tgt_ones", &davo_config::att_tgt_ones}, {"mask_mode", &davo_config::mask_mode},
-      {"se_act", &davo_config::se_act}, {"flow_abs", &davo_config::flow_abs}, {"flow_norm", &davo_config::flow_norm},
-      {"posenn_se", &davo_config::posenn_se}, {"micro_batch", &davo_config::micro_batch},
-      {"depth_norm", &davo_config::depth_norm}, {"se_pool", &davo_config::se_pool},
-      {"se_hidden", &davo_config::se_hidden}, {"pixel_map", &davo_config::pixel_map},
-      {"depth_split", &davo_config::depth_split}, {"flow_f16", &davo_config::flow_f16},
-      {"batch_norm", &davo_config::batch_norm}};                     // every field but max_batch
-  static_assert(sizeof fields / sizeof fields[0] + 1 == sizeof(davo_config) / sizeof(int32_t), "a davo_config field is missing");
-  for (const auto& x : fields)
+  for (const auto& x : kSessionConfig)
     if (a.*x.f != b.*x.f)
       return fail(ctx, DAVO_ERR_ARG, "%s: dst's davo_config differs in %s (%d here, %d on dst); only max_batch may differ",
                   who, x.name, a.*x.f, b.*x.f);
@@ -3038,7 +3189,7 @@ extern "C" int davo_odometry_move(davo_odometry* o, davo_ctx* dst) {
   // settings fixed at davo_create from the environment that change what a push computes or how a session holds it
   if (ctx->compensated_rounding != dst->compensated_rounding || ctx->conv_impl != dst->conv_impl)
     return fail(ctx, DAVO_ERR_ARG, "%s: the two handles round the weights (DAVO_B200_WEIGHT_ROUNDING) or run the convolutions differently", who);
-  if (o->host && a.att_src != 0 && ctx->host_seg8 != dst->host_seg8)
+  if (label_form(ctx, o->host) != label_form(dst, o->host))
     return fail(ctx, DAVO_ERR_ARG, "%s: the two handles hold a host session's labels in different forms (DAVO_B200_HOST_SEG8)", who);
   davo_odometry* t = new davo_odometry;
   t->ctx = dst; t->max_push = o->max_push; t->pairs = o->pairs; t->host = o->host;
@@ -3047,25 +3198,13 @@ extern "C" int davo_odometry_move(davo_odometry* o, davo_ctx* dst) {
     odometry_free(t);
     return rc;
   }
-  const davo_config& c = ctx->cfg;
-  const size_t hw = (size_t)c.H * c.W;
-  const int head = o->head();
-  // the carried flow_fwd entry (global entry pushed - 2) is there when the push that ended at frame `pushed` kept it
-  const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
-  const bool fwd = o->c_fwd && o->pushed >= 2 && rg.fwd((int)std::min(o->pushed - 2, 2LL));
-  struct { void* d; const void* s; size_t bytes; } cp[] = {
-      {t->c_img, o->c_img, hw * 3 * head},
-      {t->c_seg8, o->c_seg8, o->c_seg8 ? hw * head : 0},
-      {t->c_seg, o->c_seg, o->c_seg ? hw * 4 * head : 0},
-      {t->c_depth, o->c_depth, o->c_depth ? hw * 4 * head : 0},
-      {t->c_fwd, o->c_fwd, fwd ? hw * 2 * 4 : 0},
-      {t->d_P, o->d_P, o->posed > 0 ? 16 * sizeof(double) : 0}};
+  const Carried from = carried_state(o), to = carried_state(t);
   auto copy = [&]() -> int {
     // as davo_odometry_destroy: work still queued on the source device may read or write the carried state
     CU_OK(cudaSetDevice(ctx->device));
     CU_OK(cudaDeviceSynchronize());
-    for (const auto& x : cp)                                       // peer access is not needed, and is not enabled
-      if (x.bytes) CU_OK(cudaMemcpyPeerAsync(x.d, dst->device, x.s, ctx->device, x.bytes, 0));
+    for (int j = 0; j < kOdoSections; ++j)                        // peer access is not needed, and is not enabled
+      if (from.bytes[j]) CU_OK(cudaMemcpyPeerAsync(to.p[j], dst->device, from.p[j], ctx->device, from.bytes[j], 0));
     CU_OK(cudaStreamSynchronize(0));
     return 0;
   };
@@ -3080,6 +3219,232 @@ extern "C" int davo_odometry_move(davo_odometry* o, davo_ctx* dst) {
   }
   odometry_free(t);
   return 0;
+}
+
+// Saves sessions (include/davo_b200.h: davo_odometry_save_many): after the device has finished the work queued on it,
+// odo_save_kernel stages every blob as the caller's buffer lays them out, chunk by chunk, and each chunk goes to the
+// caller's buffer in one copy.  The sessions are only read.
+static int odometry_save_impl(const char* who, bool many, int n, davo_odometry* const* sessions, void* buf,
+                              int64_t capacity, int64_t* offsets) {
+  if (n < 1) return fail(nullptr, DAVO_ERR_ARG, "%s: n=%d: at least one session", who, n);
+  if (!sessions) return fail(nullptr, DAVO_ERR_ARG, "%s: sessions is NULL", who);
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    for (int i = 0; i < n; ++i)
+      if (!sessions[i] || !g_odo_live.count(sessions[i]))
+        return fail(nullptr, DAVO_ERR_ARG, "%s: %sthe session is NULL or was destroyed", who, at_index(many, "sessions", i).c_str());
+  }
+  davo_ctx* ctx = sessions[0]->ctx;
+  if (!offsets) return fail(ctx, DAVO_ERR_ARG, "%s: %s is NULL", who, many ? "offsets" : "bytes");
+  for (int i = 1; i < n; ++i)
+    if (sessions[i]->ctx != ctx)
+      return fail(ctx, DAVO_ERR_ARG, "%s: sessions[%d] belongs to another handle than sessions[0]", who, i);
+  std::vector<Carried> cs(n);
+  std::vector<OdoBlobHeader> hd(n);
+  offsets[0] = 0;
+  for (int i = 0; i < n; ++i) {
+    cs[i] = carried_state(sessions[i]);
+    hd[i] = blob_header(sessions[i], cs[i]);
+    offsets[i + 1] = offsets[i] + (int64_t)hd[i].total_bytes;
+  }
+  if (!buf || capacity < offsets[n])
+    return fail(ctx, DAVO_ERR_ARG, "%s: capacity %lld bytes%s; the blobs take %lld (%s)", who, (long long)capacity,
+                buf ? "" : " (buf is NULL)", (long long)offsets[n], many ? "offsets[n]" : "*bytes");
+  CU_OK(cudaSetDevice(ctx->device));
+  CU_OK(cudaDeviceSynchronize());          // as davo_odometry_move: queued pushes and host tickets write the carried state
+  size_t stage = 0;
+  const auto chunks = blob_chunks(n, offsets, &stage);
+  const BlobArea A = blob_area(n);
+  if (int rc = blob_buffers(ctx, stage, A.bytes)) return rc;
+  uint8_t* h = static_cast<uint8_t*>(ctx->b_hdesc);
+  uint8_t* dd = static_cast<uint8_t*>(ctx->b_ddesc);
+  memset(h, 0, A.bytes);
+  OdoBlob* hb = reinterpret_cast<OdoBlob*>(h);
+  for (const auto& ch : chunks)
+    for (int i = ch.first; i < ch.second; ++i) {
+      OdoBlob& b = hb[i];
+      b.blob = ctx->b_stage + (offsets[i] - offsets[ch.first]);
+      memcpy(h + A.headers + sizeof(OdoBlobHeader) * i, &hd[i], sizeof(OdoBlobHeader));
+      b.header = dd + A.headers + sizeof(OdoBlobHeader) * i;
+      for (int j = 0; j < kOdoSections; ++j) {
+        b.sec[j] = static_cast<uint8_t*>(cs[i].p[j]);
+        b.off[j] = hd[i].section_off[j];
+        b.bytes[j] = cs[i].bytes[j];
+      }
+      b.sum = reinterpret_cast<unsigned long long*>(dd + A.sums) + i;
+      b.done = reinterpret_cast<unsigned int*>(dd + A.done) + i;
+    }
+  cudaStream_t st = 0;
+  CU_OK(cudaMemcpyAsync(dd, h, A.bytes, cudaMemcpyHostToDevice, st));
+  int launches = 0;
+  for (const auto& ch : chunks) {
+    odo_save_kernel<<<blob_grid(ch.second - ch.first), 256, 0, st>>>(reinterpret_cast<const OdoBlob*>(dd) + ch.first,
+                                                                     (unsigned)sizeof(OdoBlobHeader));
+    CU_OK(cudaGetLastError());
+    ++launches;
+    CU_OK(cudaMemcpyAsync(static_cast<uint8_t*>(buf) + offsets[ch.first], ctx->b_stage,
+                          (size_t)(offsets[ch.second] - offsets[ch.first]), cudaMemcpyDeviceToHost, st));
+  }
+  CU_OK(cudaStreamSynchronize(st));
+  ctx->last_launches = launches;
+  ctx->last_h2d = (long long)A.bytes;
+  ctx->last_d2h = (long long)offsets[n];
+  return 0;
+}
+
+// Loads sessions (include/davo_b200.h: davo_odometry_load_many): every header is checked on the host first, against a
+// session of its kind and counts on dst (blob_header), so a blob whose fields disagree with each other or with dst is
+// refused before anything is allocated.  Then the sessions are allocated, each chunk of blobs goes to the staging area
+// in one copy, odo_load_kernel scatters the sections and sums the blobs, and the sessions are handed out only when
+// every sum equals its stored checksum.
+static int odometry_load_impl(const char* who, bool many, davo_ctx* dst, int n, const void* buf, const int64_t* offsets,
+                              davo_odometry** out) {
+  if (!dst) return fail(nullptr, DAVO_ERR_ARG, "%s: dst is NULL", who);
+  davo_ctx* ctx = dst;                                             // CU_OK reports on it
+  if (n < 1) return fail(dst, DAVO_ERR_ARG, "%s: n=%d: at least one blob", who, n);
+  if (!buf) return fail(dst, DAVO_ERR_ARG, "%s: buf is NULL", who);
+  if (!offsets) return fail(dst, DAVO_ERR_ARG, "%s: %s is NULL", who, many ? "offsets" : "bytes");
+  if (!out) return fail(dst, DAVO_ERR_ARG, "%s: out is NULL", who);
+  if (!dst->finalized) return fail(dst, DAVO_ERR_ARG, "%s: weights not finalized on dst", who);
+  if (dst->cfg.batch_norm) return fail(dst, DAVO_ERR_ARG, "%s: -batch_norm: a session does not take it (davo_odometry_create)", who);
+  const uint8_t* base = static_cast<const uint8_t*>(buf);
+  std::vector<OdoBlobHeader> hd(n);
+  for (int i = 0; i < n; ++i) {
+    const std::string at = at_index(many, "blob", i);
+    const char* p = at.c_str();
+    const int64_t size = offsets[i + 1] - offsets[i];
+    if (offsets[i] < 0 || size < (int64_t)sizeof(OdoBlobHeader))
+      return fail(dst, DAVO_ERR_ARG, "%s: %s%lld bytes at offset %lld: shorter than the %d-byte header (truncated?)", who, p,
+                  (long long)size, (long long)offsets[i], (int)sizeof(OdoBlobHeader));
+    OdoBlobHeader& h = hd[i];
+    memcpy(&h, base + offsets[i], sizeof h);
+    if (memcmp(h.magic, "DAVOSESS", 8) != 0)
+      return fail(dst, DAVO_ERR_ARG, "%s: %snot a saved odometry session (bad magic)", who, p);
+    if (h.version != kOdoBlobVersion || h.header_bytes != sizeof h)
+      return fail(dst, DAVO_ERR_ARG, "%s: %sformat version %u with a %u-byte header; this library reads version %u (%d bytes)",
+                  who, p, h.version, h.header_bytes, kOdoBlobVersion, (int)sizeof h);
+    if (h.total_bytes != (uint64_t)size)
+      return fail(dst, DAVO_ERR_ARG, "%s: %sthe blob is %lld bytes, its header says %llu (truncated or cut wrongly)", who, p,
+                  (long long)size, (unsigned long long)h.total_bytes);
+    for (int f = 0; f < kSessionConfigFields; ++f)
+      if (h.config[f] != dst->cfg.*kSessionConfig[f].f)
+        return fail(dst, DAVO_ERR_ARG, "%s: %sdst's davo_config differs in %s (%d in the blob, %d on dst); only max_batch may differ",
+                    who, p, kSessionConfig[f].name, h.config[f], dst->cfg.*kSessionConfig[f].f);
+    if (h.weights_digest != dst->weights_digest)
+      return fail(dst, DAVO_ERR_ARG, "%s: %sthe blob was saved from different weights than dst holds", who, p);
+    if (h.weight_rounding != (int32_t)dst->compensated_rounding || h.conv_impl != dst->conv_impl)
+      return fail(dst, DAVO_ERR_ARG, "%s: %sthe blob's handle rounded the weights (DAVO_B200_WEIGHT_ROUNDING) or ran the convolutions differently than dst", who, p);
+    if ((h.host != 0 && h.host != 1) || (h.pairs != DAVO_PAIRS_TRAJECTORY && h.pairs != DAVO_PAIRS_ALL) || h.max_push < 1 ||
+        h.pushed < 0 || h.posed < 0)
+      return fail(dst, DAVO_ERR_ARG, "%s: %sthe header's session kind or counts are out of range", who, p);
+    if (h.label_form != label_form(dst, h.host))
+      return fail(dst, DAVO_ERR_ARG, "%s: %sthe blob holds a host session's labels in another form (%d) than dst does (%d) (DAVO_B200_HOST_SEG8)",
+                  who, p, h.label_form, label_form(dst, h.host));
+    if (h.max_push > dst->cfg.max_batch)
+      return fail(dst, DAVO_ERR_ARG, "%s: %sthe session's max_push %d is more than dst's max_batch %d", who, p, h.max_push,
+                  dst->cfg.max_batch);
+    davo_odometry s;                                               // its kind and counts on dst, no buffers
+    s.ctx = dst; s.max_push = h.max_push; s.pairs = h.pairs; s.host = h.host; s.pushed = h.pushed; s.posed = h.posed;
+    OdoBlobHeader want = blob_header(&s, carried_state(&s));
+    want.checksum = h.checksum;
+    if (memcmp(&want, &h, sizeof h) != 0)
+      return fail(dst, DAVO_ERR_ARG, "%s: %sthe header's carried sections disagree with its counts", who, p);
+  }
+  CU_OK(cudaSetDevice(dst->device));
+  std::vector<davo_odometry*> made;
+  auto drop = [&]() {
+    for (davo_odometry* o : made) odometry_free(o);
+  };
+  std::vector<Carried> cs(n);
+  for (int i = 0; i < n; ++i) {
+    davo_odometry* t = new davo_odometry;
+    t->ctx = dst; t->max_push = hd[i].max_push; t->pairs = hd[i].pairs; t->host = hd[i].host;
+    made.push_back(t);
+    if (int rc = odometry_alloc(t)) { drop(); return rc; }
+    t->pushed = hd[i].pushed; t->posed = hd[i].posed;
+    cs[i] = carried_state(t);
+  }
+  size_t stage = 0;
+  const auto chunks = blob_chunks(n, offsets, &stage);
+  const BlobArea A = blob_area(n);
+  cudaStream_t st = 0;
+  int launches = 0;
+  auto run = [&]() -> int {
+    if (int rc = blob_buffers(dst, stage, A.bytes)) return rc;
+    uint8_t* h = static_cast<uint8_t*>(dst->b_hdesc);
+    uint8_t* dd = static_cast<uint8_t*>(dst->b_ddesc);
+    memset(h, 0, A.bytes);
+    OdoBlob* hb = reinterpret_cast<OdoBlob*>(h);
+    for (const auto& ch : chunks)
+      for (int i = ch.first; i < ch.second; ++i) {
+        OdoBlob& b = hb[i];
+        b.blob = dst->b_stage + (offsets[i] - offsets[ch.first]);
+        for (int j = 0; j < kOdoSections; ++j) {
+          b.sec[j] = static_cast<uint8_t*>(cs[i].p[j]);
+          b.off[j] = hd[i].section_off[j];
+          b.bytes[j] = cs[i].bytes[j];
+        }
+        b.sum = reinterpret_cast<unsigned long long*>(dd + A.sums) + i;
+      }
+    CU_OK(cudaMemcpyAsync(dd, h, A.bytes, cudaMemcpyHostToDevice, st));
+    for (const auto& ch : chunks) {
+      CU_OK(cudaMemcpyAsync(dst->b_stage, base + offsets[ch.first], (size_t)(offsets[ch.second] - offsets[ch.first]),
+                            cudaMemcpyHostToDevice, st));
+      odo_load_kernel<<<blob_grid(ch.second - ch.first), 256, 0, st>>>(reinterpret_cast<const OdoBlob*>(dd) + ch.first,
+                                                                       (unsigned)sizeof(OdoBlobHeader));
+      CU_OK(cudaGetLastError());
+      ++launches;
+    }
+    CU_OK(cudaMemcpyAsync(h + A.sums, dd + A.sums, 8 * (size_t)n, cudaMemcpyDeviceToHost, st));
+    CU_OK(cudaStreamSynchronize(st));
+    const unsigned long long* sum = reinterpret_cast<const unsigned long long*>(h + A.sums);
+    for (int i = 0; i < n; ++i)
+      if (sum[i] != hd[i].checksum)
+        return fail(dst, DAVO_ERR_ARG, "%s: %schecksum mismatch: the blob is corrupt", who, at_index(many, "blob", i).c_str());
+    return 0;
+  };
+  if (int rc = run()) {
+    drop();
+    return rc;
+  }
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    for (davo_odometry* o : made) g_odo_live.insert(o);
+  }
+  for (int i = 0; i < n; ++i) out[i] = made[i];
+  dst->last_launches = launches;
+  dst->last_h2d = (long long)(A.bytes + (offsets[n] - offsets[0]));
+  dst->last_d2h = 8LL * n;
+  return 0;
+}
+
+extern "C" int davo_odometry_state_bytes(const davo_odometry* o, int64_t* bytes) {
+  std::lock_guard<std::mutex> lk(g_odo_mutex);
+  if (!o || !g_odo_live.count(const_cast<davo_odometry*>(o)))
+    return fail(nullptr, DAVO_ERR_ARG, "davo_odometry_state_bytes: the session is NULL or was destroyed");
+  if (!bytes) return fail(o->ctx, DAVO_ERR_ARG, "davo_odometry_state_bytes: bytes is NULL");
+  *bytes = (int64_t)blob_header(o, carried_state(o)).total_bytes;
+  return 0;
+}
+
+extern "C" int davo_odometry_save(davo_odometry* o, void* buf, int64_t capacity, int64_t* bytes) {
+  int64_t off[2] = {0, 0};
+  const int rc = odometry_save_impl("davo_odometry_save", false, 1, &o, buf, capacity, bytes ? off : nullptr);
+  if (bytes) *bytes = off[1];
+  return rc;
+}
+
+extern "C" int davo_odometry_save_many(int n, davo_odometry* const* sessions, void* buf, int64_t capacity, int64_t* offsets) {
+  return odometry_save_impl("davo_odometry_save_many", true, n, sessions, buf, capacity, offsets);
+}
+
+extern "C" int davo_odometry_load(davo_ctx* dst, const void* buf, int64_t bytes, davo_odometry** out) {
+  const int64_t off[2] = {0, bytes};
+  return odometry_load_impl("davo_odometry_load", false, dst, 1, buf, off, out);
+}
+
+extern "C" int davo_odometry_load_many(davo_ctx* dst, int n, const void* buf, const int64_t* offsets, davo_odometry** out) {
+  return odometry_load_impl("davo_odometry_load_many", true, dst, n, buf, offsets, out);
 }
 
 // davo_destroy: the handle's sessions go with it

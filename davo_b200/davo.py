@@ -20,6 +20,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import struct
 
 import numpy as np
 
@@ -30,6 +31,31 @@ from . import version as V
 
 def _is_torch(x) -> bool:
     return type(x).__module__.startswith("torch")
+
+
+# include/davo_b200.h: the header of a saved odometry session, format version 1
+_BLOB_HEADER = struct.Struct("<8sIIQ20iQ6i2q4i6Q6QQ")
+_BLOB_CONFIG = [n for n, _ in _capi.DavoConfigC._fields_ if n != "max_batch"]
+
+
+def odometry_blob_header(blob):
+    """The header of a saved odometry session (include/davo_b200.h: davo_odometry_save) of any buffer-protocol object,
+    as a dict.  Raises ValueError for what is not a version-1 blob: too short, a bad magic, another version."""
+    mv = memoryview(blob).cast("B")
+    if mv.nbytes < _BLOB_HEADER.size:
+        raise ValueError("a saved odometry session is at least %d bytes; this is %d (truncated?)" % (_BLOB_HEADER.size, mv.nbytes))
+    f = _BLOB_HEADER.unpack_from(mv, 0)
+    if f[0] != b"DAVOSESS":
+        raise ValueError("not a saved odometry session (bad magic)")
+    if f[1] != 1 or f[2] != _BLOB_HEADER.size:
+        raise ValueError("saved odometry session of format version %d; this library reads version 1" % f[1])
+    cfg, rest = f[4:24], f[24:]
+    return {"bytes": mv.nbytes, "total_bytes": f[3], "config": dict(zip(_BLOB_CONFIG, cfg)), "weights_digest": rest[0],
+            "weight_rounding": rest[1], "conv_impl": rest[2], "host": bool(rest[3]), "label_form": rest[4],
+            "pairs": {v: k for k, v in _capi.PAIRS.items()}.get(rest[5], rest[5]), "max_push": rest[6],
+            "pushed": rest[7], "posed": rest[8], "carried_frames": rest[9], "carried_fwd": bool(rest[10]),
+            "carried_pose": bool(rest[11]), "section_off": list(rest[13:19]), "section_bytes": list(rest[19:25]),
+            "checksum": rest[25]}
 
 
 class DAVO(object):
@@ -82,6 +108,7 @@ class DAVO(object):
             depth_split=self.config.depth_split, batch_norm=self.config.batch_norm,
             flow_f16=int(os.environ.get("DAVO_B200_FLOW16", "0") == "1") if flow_f16 is None else int(bool(flow_f16)))
         self.flow_f16 = bool(cfg.flow_f16)
+        self._cfg = cfg
         h = C.c_void_p()
         rc = self._lib.davo_create(C.byref(cfg), self.device, C.byref(h))
         if rc != 0:
@@ -433,6 +460,90 @@ class DAVO(object):
         return numpy arrays, else CUDA tensors in and out."""
         return Odometry(self, pairs, self.batch_size if max_push is None else max_push, host)
 
+    def _blob_header(self, blob, who):
+        """The header of a blob this handle is to load, checked before any device work: the handle set up with weights
+        loaded, a version-1 blob, saved by a handle of the same version, frame size and configuration."""
+        if getattr(self, "_h", None) is None:
+            raise ValueError("DAVO.%s: the handle is not set up (DAVO.setup_inference(mode='davo'))" % who)
+        if not self._weights_loaded:
+            raise ValueError("DAVO.%s: the handle has no weights loaded" % who)
+        try:
+            hdr = odometry_blob_header(blob)
+        except ValueError as e:
+            raise ValueError("DAVO.%s: %s" % (who, e))
+        cfg = hdr["config"]
+        if (cfg["H"], cfg["W"]) != (self.img_height, self.img_width):
+            raise ValueError("DAVO.%s: the session's frames are %dx%d, this handle's %dx%d"
+                             % (who, cfg["H"], cfg["W"], self.img_height, self.img_width))
+        for name in _BLOB_CONFIG:
+            if cfg[name] != getattr(self._cfg, name):
+                raise ValueError("DAVO.%s: the session was saved by a handle of another version or configuration "
+                                 "(davo_config.%s: %d in the blob, %d here)" % (who, name, cfg[name], getattr(self._cfg, name)))
+        return hdr
+
+    def odometry_load(self, blob):
+        """A session saved by ``Odometry.save`` -- on this handle or another, in this process or another -- as a new
+        session of this handle (include/davo_b200.h: davo_odometry_load).  Every later push gives the bits the saved
+        session would have given; loading a blob twice forks the stream.  ``blob``: a buffer-protocol object."""
+        hdr = self._blob_header(blob, "odometry_load")
+        a = np.frombuffer(blob, np.uint8)
+        out = C.c_void_p()
+        import torch
+        with torch.cuda.device(self.device):             # the call switches devices; torch's current one is restored
+            self._check(self._lib.davo_odometry_load(self._h, C.c_void_p(a.ctypes.data), a.size, C.byref(out)),
+                        "davo_odometry_load")
+        return Odometry._adopt(self, out, hdr)
+
+    def odometry_save_many(self, sessions):
+        """The blobs of several sessions of this handle (include/davo_b200.h: davo_odometry_save_many), each what
+        ``Odometry.save`` gives, as slices of one page-locked buffer (buffer-protocol objects), in list order.  The
+        launches do not depend on the number of sessions; the sessions do not change."""
+        sessions = list(sessions)
+        if not sessions:
+            raise ValueError("DAVO.odometry_save_many: no session")
+        for i, od in enumerate(sessions):
+            if not isinstance(od, Odometry) or od._system is not self:
+                raise ValueError("DAVO.odometry_save_many: session %d is not a session of this handle" % i)
+            if od._o is None:
+                raise RuntimeError("DAVO.odometry_save_many: session %d is closed" % i)
+        n = len(sessions)
+        size = C.c_int64(0)
+        total = 0
+        for od in sessions:
+            self._check(self._lib.davo_odometry_state_bytes(od._o, C.byref(size)), "davo_odometry_state_bytes")
+            total += size.value
+        import torch
+        buf = torch.empty((total,), dtype=torch.uint8).pin_memory().numpy()
+        offsets = (C.c_int64 * (n + 1))()
+        with torch.cuda.device(self.device):
+            self._check(self._lib.davo_odometry_save_many(n, (C.c_void_p * n)(*[od._o.value for od in sessions]),
+                                                          C.c_void_p(buf.ctypes.data), total, offsets),
+                        "davo_odometry_save_many")
+        mv = memoryview(buf)
+        return [mv[offsets[i]:offsets[i + 1]] for i in range(n)]
+
+    def odometry_load_many(self, blobs):
+        """New sessions of this handle from several blobs (include/davo_b200.h: davo_odometry_load_many), each as
+        ``odometry_load`` would load it, in list order; all are checked before any is loaded, and a refused call loads
+        none.  The blobs are gathered into one page-locked buffer, sent in one copy."""
+        blobs = list(blobs)
+        if not blobs:
+            raise ValueError("DAVO.odometry_load_many: no blob")
+        hdrs = [self._blob_header(b, "odometry_load_many: blob %d" % i) for i, b in enumerate(blobs)]
+        n = len(blobs)
+        offsets = (C.c_int64 * (n + 1))()
+        for i, h in enumerate(hdrs):
+            offsets[i + 1] = offsets[i] + h["bytes"]
+        import torch
+        buf = torch.empty((offsets[n],), dtype=torch.uint8).pin_memory().numpy()
+        for i, b in enumerate(blobs):
+            buf[offsets[i]:offsets[i + 1]] = np.frombuffer(b, np.uint8)
+        out = (C.c_void_p * n)()
+        with torch.cuda.device(self.device):
+            self._check(self._lib.davo_odometry_load_many(self._h, n, C.c_void_p(buf.ctypes.data), offsets, out),
+                        "davo_odometry_load_many")
+        return [Odometry._adopt(self, C.c_void_p(out[i]), h) for i, h in enumerate(hdrs)]
+
     def _many_args(self, sessions, img, flow_fwd, flow_bwd, seg, depth, host, who):
         """The list and session checks of the batched pushes; returns the sessions, each entry's inputs and its
         (k, n_samples, n_traj)."""
@@ -665,6 +776,7 @@ class Odometry(object):
             raise RuntimeError("DAVO.odometry: weights not loaded")
         self._system, self._host, self._pushed, self._posed = system, bool(host), 0, 0
         self._ring, self._ring_n = None, 0
+        self.pairs = pairs
         h = C.c_void_p()
         system._check(system._lib.davo_odometry_create(system._h, int(max_push), _capi.PAIRS[pairs], int(self._host),
                                                        C.byref(h)), "davo_odometry_create")
@@ -792,6 +904,37 @@ class Odometry(object):
             s._check(s._lib.davo_odometry_move(self._o, system._h), "davo_odometry_move")
         self._system = system
         return self
+
+    @classmethod
+    def _adopt(cls, system, h, hdr):
+        """The Python side of a session the library loaded onto ``system`` (DAVO.odometry_load): its kind from the
+        blob's header, its counts from the library."""
+        od = cls.__new__(cls)
+        od._system, od._host, od._o, od.max_push, od.pairs = system, hdr["host"], h, hdr["max_push"], hdr["pairs"]
+        od._ring, od._ring_n = None, 0
+        pushed, posed = C.c_longlong(0), C.c_longlong(0)
+        system._check(system._lib.davo_odometry_frames(h, C.byref(pushed), C.byref(posed)), "davo_odometry_frames")
+        od._pushed, od._posed = int(pushed.value), int(posed.value)
+        return od
+
+    def save(self):
+        """This session's carried state as bytes (include/davo_b200.h: davo_odometry_save): ``DAVO.odometry_load`` on a
+        handle of the same version, frame size and weights -- in this process or another -- continues the stream with
+        the bits this session would give.  Does not change the session; waits for the work queued on its device,
+        host pushes in flight included."""
+        s = self._system
+        if self._o is None:
+            raise RuntimeError("Odometry.save: the session is closed")
+        if s._h is None:
+            raise RuntimeError("Odometry.save: the session was destroyed with its handle")
+        size = C.c_int64(0)
+        s._check(s._lib.davo_odometry_state_bytes(self._o, C.byref(size)), "davo_odometry_state_bytes")
+        buf = np.empty((size.value,), np.uint8)
+        import torch
+        with torch.cuda.device(s.device):
+            s._check(s._lib.davo_odometry_save(self._o, C.c_void_p(buf.ctypes.data), buf.size, C.byref(size)),
+                     "davo_odometry_save")
+        return buf.tobytes()
 
     def frames(self):
         """(frames pushed, frames whose absolute pose has been returned)."""

@@ -1,9 +1,10 @@
 """Many cameras over several ``DAVO`` handles, usually one per GPU of a box (include/davo_b200.h: davo_odometry_*).
 
 Each camera is an odometry session on one handle.  ``push`` advances any set of cameras by one batched push per handle
-(``DAVO.odometry_push_many_host`` / ``odometry_push_many``), and ``rebalance`` evens out the handles with
-``Odometry.move_to``.  The pool holds no numerics of its own: every result is that of the batched push on one handle,
-and a camera's results do not depend on which handle it is on or on whether it moved.
+(``DAVO.odometry_push_many_host`` / ``odometry_push_many``), ``rebalance`` evens out the handles with
+``Odometry.move_to``, and ``save`` / ``load`` carry every camera across a restart of the process.  The pool holds no
+numerics of its own: every result is that of the batched push on one handle, and a camera's results do not depend on
+which handle it is on, on whether it moved, or on whether it was saved and loaded.
 """
 from __future__ import annotations
 
@@ -106,6 +107,52 @@ class OdometryPool(object):
             for j, r in zip(pos, p.result()):
                 out[j] = r
         return out
+
+    def save(self):
+        """``{camera id: blob}`` of every camera (``Odometry.save``'s bytes, as buffer-protocol objects): one
+        ``DAVO.odometry_save_many`` per handle.  The cameras do not change."""
+        out = {}
+        for s in self._systems:
+            cams = sorted(c for c, od in self._cams.items() if od._system is s)
+            if cams:
+                out.update(zip(cams, s.odometry_save_many([self._cams[c] for c in cams])))
+        return out
+
+    def load(self, blobs):
+        """Restores the cameras of ``blobs`` (``{camera id: blob}`` from ``save``, of this pool or another, in this
+        process or another) under the same ids: each goes to the handle with the fewest sessions, in id order, and
+        each handle takes its cameras in one ``DAVO.odometry_load_many``.  Every blob is checked before any is loaded;
+        ids that ``open`` gives afterwards are above the restored ones.  Returns the restored ids."""
+        items = sorted(dict(blobs).items())
+        n = self.counts()
+        groups = {}                                      # handle index -> [(camera, blob)]
+        for cam, blob in items:
+            if cam in self._cams:
+                raise ValueError("OdometryPool.load: camera %r is open" % (cam,))
+            i = n.index(min(n))
+            hdr = self._systems[i]._blob_header(blob, "odometry_load_many: camera %r" % (cam,))
+            if (hdr["host"], hdr["pairs"], hdr["max_push"]) != (self._host, self._pairs, self._max_push):
+                raise ValueError("OdometryPool.load: camera %r was saved as a %s session, pairs=%r, max_push=%d; this pool "
+                                 "holds %s sessions, pairs=%r, max_push=%d" % (
+                                     cam, "host" if hdr["host"] else "device", hdr["pairs"], hdr["max_push"],
+                                     "host" if self._host else "device", self._pairs, self._max_push))
+            n[i] += 1
+            groups.setdefault(i, []).append((cam, blob))
+        import torch
+        loaded = []
+        try:
+            for i, group in sorted(groups.items()):
+                s = self._systems[i]
+                with torch.cuda.device(s.device):
+                    loaded += zip([c for c, _ in group], s.odometry_load_many([b for _, b in group]))
+        except Exception:
+            for _, od in loaded:                         # all or nothing
+                od.close()
+            raise
+        self._cams.update(loaded)
+        if items:
+            self._next = max(self._next, max(c for c, _ in items) + 1)
+        return [c for c, _ in items]
 
     def rebalance(self):
         """Moves sessions from the fullest handle to the emptiest (``Odometry.move_to``, the most recently opened

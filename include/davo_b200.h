@@ -326,6 +326,52 @@ void davo_odometry_destroy(davo_odometry*);
  *   davo_finalize_weights was given); a different DAVO_B200_WEIGHT_ROUNDING or conv implementation; for a host session
  *   with labels, a different DAVO_B200_HOST_SEG8. */
 int davo_odometry_move(davo_odometry*, davo_ctx* dst);
+/* Saved sessions: a live session's carried state as a byte blob that a handle of the same configuration and weights,
+ *   in this process or another one, loads as a new session -- to survive a restart of the serving process, to hand a
+ *   camera to another process, or to checkpoint a long replay.  Every push on the loaded session gives the bits the
+ *   original would have given: pose_out, traj_out, the counts, davo_odometry_frames, a host push's host to device bytes.
+ * davo_odometry_state_bytes: the exact size a save of the session writes now (it changes with the counts).
+ * davo_odometry_save: writes the blob into buf[0, *bytes).  Does not change the session.  Waits for all work on the
+ *   session's device (as davo_odometry_move), so queued device pushes and host tickets in flight are included, and
+ *   returns once the blob is in buf; tickets issued before the save stay valid.
+ * davo_odometry_load: a new session on dst (max_push, pair mode, host or device kind and counts of the saved one),
+ *   owned by dst as if davo_odometry_create had made it.  Loading a blob twice, or while the original keeps running,
+ *   forks the stream: each copy continues with the same bits.  Synchronous.
+ * davo_odometry_save_many / davo_odometry_load_many: the same for n sessions of one handle, blobs back to back in one
+ *   buffer: blob i is buf[offsets[i], offsets[i+1]) (save writes offsets[0] = 0 and offsets[1..n]), and each slice is a
+ *   blob davo_odometry_load takes on its own.  The kernel launches do not depend on n (a call larger than the staging
+ *   bound of 256 MB is cut into chunks), and a save's device to host bytes are the blobs' (davo_last_launch_count,
+ *   davo_last_host_copy_bytes).  The single forms are the n = 1 case.
+ * The blob, format version 1, little-endian, a multiple of 16 bytes:
+ *   header, 272 bytes:
+ *     0 char[8] magic "DAVOSESS"; 8 u32 version (1); 12 u32 header bytes (272); 16 u64 total bytes;
+ *     24 i32[20] every davo_config field but max_batch, in declaration order;
+ *     104 u64 weight digest (of the values davo_finalize_weights was given); 112 i32 weight rounding (1 compensated,
+ *     0 nearest: DAVO_B200_WEIGHT_ROUNDING); 116 i32 conv implementation (0 tcgen05); 120 i32 host session;
+ *     124 i32 label form (0 none, 1 bytes: host sessions under DAVO_B200_HOST_SEG8, 2 float32); 128 i32 pairs;
+ *     132 i32 max_push; 136 i64 frames pushed; 144 i64 frames posed; 152 i32 carried frames (min(pushed, 2));
+ *     156 i32 a flow_fwd entry is carried; 160 i32 a pose is carried; 164 i32 zero;
+ *     168 u64[6] section offsets; 216 u64[6] section bytes; 264 u64 checksum.
+ *   sections, in this order, each at a 16-byte aligned offset and zero-padded to 16 bytes, empty when not carried:
+ *     the carried frames' images (uint8 [f,H,W,3]); their labels as bytes ([f,H,W]) or as float32 ([f,H,W]); their
+ *     depth (float32 [f,H,W], depth sources); the carried flow_fwd entry (float32 [H,W,2]); the last absolute pose
+ *     (float64 [4,4]) -- the state davo_odometry_move copies.
+ *   checksum: sum over the blob's 8-byte words w_i (i = 0, 1, ...; the checksum word taken as 0) of
+ *     splitmix64_mix(w_i + (i + 1) * 0x9E3779B97F4A7C15) mod 2^64, where splitmix64_mix(z): z = (z ^ z >> 30) *
+ *     0xBF58476D1CE4E5B9; z = (z ^ z >> 27) * 0x94D049BB133111EB; return z ^ z >> 31.
+ * Refusals return DAVO_ERR_ARG with a message naming the reason (and the index, as "sessions[i]" or "blob[i]", for the
+ *   _many forms).  A save: a NULL or destroyed session (davo_last_error(NULL)); sessions of two handles; bytes /
+ *   offsets NULL; buf NULL or capacity below the size, which is still written to *bytes / offsets[n].  A load, which
+ *   then allocates nothing that outlives the call and leaves *out untouched: dst, buf, offsets / bytes or out NULL;
+ *   weights not finalized on dst; a blob shorter than the header or of another size than its header says; a bad magic
+ *   or another format version; a davo_config field other than max_batch that differs (named); different weights; a
+ *   different DAVO_B200_WEIGHT_ROUNDING or conv implementation; a host session's label form that differs on dst; the
+ *   session's max_push above dst's max_batch; header fields that disagree with each other; a checksum mismatch. */
+int davo_odometry_state_bytes(const davo_odometry*, int64_t* bytes);
+int davo_odometry_save(davo_odometry*, void* buf, int64_t capacity, int64_t* bytes);
+int davo_odometry_load(davo_ctx* dst, const void* buf, int64_t bytes, davo_odometry** out);
+int davo_odometry_save_many(int n, davo_odometry* const* sessions, void* buf, int64_t capacity, int64_t* offsets);
+int davo_odometry_load_many(davo_ctx* dst, int n, const void* buf, const int64_t* offsets, davo_odometry** out);
 
 /* Binds the calling thread (and the threads it creates afterwards: the handle's conversion pool, the caller's
  * loader threads) to the CPUs of the NUMA node the handle's GPU hangs off (/sys/bus/pci/devices/<id>/numa_node,
