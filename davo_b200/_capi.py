@@ -27,7 +27,8 @@ SYMBOLS = (
     "davo_odometry_create", "davo_odometry_push", "davo_odometry_reset", "davo_odometry_frames",
     "davo_odometry_push_many", "davo_odometry_push_many_host", "davo_odometry_move",
     "davo_odometry_state_bytes", "davo_odometry_save", "davo_odometry_load", "davo_odometry_save_many",
-    "davo_odometry_load_many",
+    "davo_odometry_load_many", "davo_forward_sequence_features", "davo_odometry_push_attention",
+    "davo_odometry_push_many_attention", "davo_odometry_push_many_host_attention",
     "davo_last_error",
     "davo_destroy", "davo_build_info", "davo_config_bytes", "davo_odometry_destroy",
 )
@@ -44,6 +45,11 @@ class DavoFeaturesC(C.Structure):
     """include/davo_b200.h: davo_features (device pointers, NULL skips the output)."""
     _fields_ = [(n, C.c_void_p) for n in (
         "image", "attention", "masked_image", "seg_19", "seg_color", "flow_color", "cnv6_rot", "cnv6_trans")]
+
+
+class DavoOdometryAttentionC(C.Structure):
+    """include/davo_b200.h: davo_odometry_attention (NULL skips the output)."""
+    _fields_ = [(n, C.c_void_p) for n in ("map", "weights")]
 
 
 def lib_path() -> str:
@@ -94,6 +100,13 @@ def load() -> C.CDLL:
         C.POINTER(ip), C.POINTER(ip), vp]
     lib.davo_odometry_push_many_host.argtypes = [ip, C.POINTER(vp), C.POINTER(ip)] + [C.POINTER(vp)] * 7 + [
         C.POINTER(ip), C.POINTER(ip), vp, C.POINTER(C.c_longlong)]
+    att = C.POINTER(DavoOdometryAttentionC)
+    lib.davo_odometry_push_attention.argtypes = [vp, ip, vp, vp, vp, vp, vp, vp, vp, att, C.POINTER(ip), C.POINTER(ip),
+                                                 vp, C.POINTER(C.c_longlong)]
+    lib.davo_odometry_push_many_attention.argtypes = [ip, C.POINTER(vp), C.POINTER(ip)] + [C.POINTER(vp)] * 7 + [
+        att, C.POINTER(ip), C.POINTER(ip), vp]
+    lib.davo_odometry_push_many_host_attention.argtypes = [ip, C.POINTER(vp), C.POINTER(ip)] + [C.POINTER(vp)] * 7 + [
+        att, C.POINTER(ip), C.POINTER(ip), vp, C.POINTER(C.c_longlong)]
     lib.davo_odometry_move.argtypes = [vp, vp]
     i64, i64p = C.c_int64, C.POINTER(C.c_int64)
     lib.davo_odometry_state_bytes.argtypes = [vp, i64p]
@@ -111,6 +124,7 @@ def load() -> C.CDLL:
     lib.davo_profile_layers.argtypes = [vp, ip, fp, C.POINTER(ip), vp]
     lib.davo_debug_set_conv_impl.argtypes = [vp, ip]
     lib.davo_forward_features.argtypes = [vp, ip, vp, vp, vp, vp, vp, C.POINTER(DavoFeaturesC), vp]
+    lib.davo_forward_sequence_features.argtypes = [vp, ip, vp, vp, vp, vp, vp, vp, C.POINTER(DavoFeaturesC), vp]
     lib.davo_debug_flows_to_half.argtypes = [vp, vp, C.c_longlong, ip]
     lib.davo_debug_labels_to_bytes.argtypes = [vp, vp, C.c_longlong, ip]
     lib.davo_comm_unique_id.argtypes = [vp]

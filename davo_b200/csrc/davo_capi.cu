@@ -294,6 +294,19 @@ struct davo_ctx {
   // mode='feature' (features.cuh)
   float* d_wheel = nullptr;         // Middlebury colour wheel / 255
   unsigned int* d_maxrad = nullptr; // largest flow magnitude per source frame
+  // attention outputs of odometry pushes (features.cuh: attention_out_kernel).  While a push that asked for them runs
+  // its forward, att_units / att_rows are the device unit table of the forward (or of the host chunk) being launched
+  // and its destination rows; NULL otherwise.  The tables go from a pinned ring slot to its device twin in one copy, a
+  // slot refilled once the call that used it has finished.  Host sessions' maps and weights are written to att_stage
+  // and copied back on the caller's stream, like s_pose.
+  const int4* att_units = nullptr;
+  const AttRow* att_rows = nullptr;
+  void *att_hdesc[kManyRing] = {}, *att_ddesc[kManyRing] = {};
+  size_t att_desc_cap[kManyRing] = {};
+  cudaEvent_t att_ev[kManyRing] = {};
+  long long att_calls = 0;
+  float* att_stage = nullptr;
+  size_t att_stage_cap = 0;
   // pose all-gather (comm.cuh): the handle's own communicator, if davo_comm_create made one
   davo_comm::Comm comm = nullptr;
   int comm_rank = 0, comm_world = 1;
@@ -1168,6 +1181,7 @@ int launch_front(davo_ctx* ctx, int pair_mode, int pair0, int npairs, const Inpu
       const int grid = std::min(work, ctx->num_sms * 4);
       if (int rc = launch_k(ctx, front_pipeline_kernel, dim3(grid), dim3(256), 0, st, false, fp, q)) return rc;
       ++*launches;
+      ctx->fp_cur = fp;
       return 0;
     }
     if (c.se_pool >= 2) {                         // mode='spp': out_pool_size [2,1] / [2] / [8,6,4]
@@ -1220,9 +1234,23 @@ Layer& pick_layer(davo_ctx* ctx, size_t li, int npairs) {
   return B;
 }
 
+// Width of a weight row of the attention outputs: what davo_get_intermediate("att_weights:<k>") returns (19 class
+// weights, or the excitation of a per-pixel source: 3 rgb, 1 depth term, 3 depth term and SE flow, 21 labels and SE flow)
+int att_width(const davo_config& c) {
+  return !c.pixel_map ? kNumClasses : c.pixel_map == 2 ? 3 : c.att_src == 4 ? 3 : c.att_src == 5 ? 1 : kNumClasses + 2;
+}
+
 int run_microbatch(davo_ctx* ctx, int pair_mode, int pair0, int npairs, const InputView& in, float* pose_out,
                    cudaStream_t st, int* launches) {
   if (int rc = launch_front(ctx, pair_mode, pair0, npairs, in, st, launches)) return rc;
+  if (ctx->att_units) {          // an odometry push asked for each posed frame's attention: att_w holds this pass's tables
+    AttentionOutParams ap;
+    ap.fp = ctx->fp_cur; ap.units = ctx->att_units; ap.rows = ctx->att_rows; ap.width = att_width(ctx->cfg);
+    const int groups = ctx->cfg.H * ctx->cfg.W / 4;
+    attention_out_kernel<<<dim3((groups + 255) / 256, npairs), 256, 0, st>>>(ap);
+    CU_OK(cudaGetLastError());
+    ++*launches;
+  }
   for (size_t li = 0; li < ctx->layers.size(); ++li) {
     Layer& L = pick_layer(ctx, li, npairs);
     const int pse = ctx->cfg.posenn_se;
@@ -1436,6 +1464,12 @@ extern "C" void davo_destroy(davo_ctx* ctx) {
     if (ctx->a_done[i]) cudaEventDestroy(ctx->a_done[i]);
   }
   cudaFree(ctx->m_hpose);
+  for (int i = 0; i < davo_ctx::kManyRing; ++i) {
+    if (ctx->att_hdesc[i]) cudaFreeHost(ctx->att_hdesc[i]);
+    if (ctx->att_ddesc[i]) cudaFree(ctx->att_ddesc[i]);
+    if (ctx->att_ev[i]) cudaEventDestroy(ctx->att_ev[i]);
+  }
+  cudaFree(ctx->att_stage);
   cudaFree(ctx->b_stage); cudaFree(ctx->b_ddesc);
   if (ctx->b_hdesc) cudaFreeHost(ctx->b_hdesc);
   delete ctx->pool;
@@ -1906,17 +1940,24 @@ int check_sequence(davo_ctx* ctx, const char* who, int n_frames, int pairs, cons
 
 }  // namespace
 
+namespace {
+// The view of a device-buffer sequence call.  Plane 1 of sample s is flow_bwd[s + 1]; a flow_fwd nobody reads stands in
+// as flow_bwd, so that a front end re-run over every pair (davo_profile_layers) still reads mapped memory.
+InputView sequence_device_view(const davo_ctx* ctx, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
+                               const float* seg, const float* depth) {
+  const davo_config& c = ctx->cfg;
+  const size_t hw = (size_t)c.H * c.W;
+  const float* bwd1 = flow_bwd ? flow_bwd + 2 * hw : nullptr;
+  return sequence_view(c.H, c.W, img, flow_fwd ? flow_fwd : flow_bwd, bwd1, seg, nullptr, depth, nullptr, nullptr, 0);
+}
+}  // namespace
+
 extern "C" int davo_forward_sequence(davo_ctx* ctx, int n_frames, int pairs, const uint8_t* img, const float* flow_fwd,
                                      const float* flow_bwd, const float* seg, const float* depth, float* pose_out, void* stream) {
   if (!ctx) return DAVO_ERR_ARG;
   if (int rc = check_sequence(ctx, "davo_forward_sequence", n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
-  const davo_config& c = ctx->cfg;
-  const size_t hw = (size_t)c.H * c.W;
-  // plane 1 of sample s is flow_bwd[s + 1]; a flow_fwd nobody reads stands in as flow_bwd, so that a front end re-run
-  // over every pair (davo_profile_layers) still reads mapped memory
-  const float* bwd1 = flow_bwd ? flow_bwd + 2 * hw : nullptr;
-  const InputView in = sequence_view(c.H, c.W, img, flow_fwd ? flow_fwd : flow_bwd, bwd1, seg, nullptr, depth, nullptr, nullptr, 0);
-  return forward_device(ctx, "davo_forward_sequence", n_frames - 2, pairs, in, pose_out, stream);
+  return forward_device(ctx, "davo_forward_sequence", n_frames - 2, pairs,
+                        sequence_device_view(ctx, img, flow_fwd, flow_bwd, seg, depth), pose_out, stream);
 }
 
 // Host-buffer entry point: the batch is cut into micro-batch chunks; chunk i+1 is copied
@@ -2096,12 +2137,21 @@ int host_done(davo_ctx* ctx, cudaStream_t st, long long* ticket) {
 
 // Poses of a host call back to the caller's memory, and an odometry push's n_traj absolute poses from traj_dev;
 // blocking, or the asynchronous form's ticket.
+// `att`: a push's maps and weights rows from the device staging (att_maps, att_weights) to the caller's host buffers.
 int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket, const double* traj_dev = nullptr,
-                double* traj_out = nullptr, int n_traj = 0) {
+                double* traj_out = nullptr, int n_traj = 0, const davo_odometry_attention* att = nullptr,
+                const float* att_maps = nullptr, const float* att_weights = nullptr) {
   if (B > 0) CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
   if (n_traj > 0) CU_OK(cudaMemcpyAsync(traj_out, traj_dev, (size_t)16 * 8 * n_traj, cudaMemcpyDeviceToHost, st));
+  long long att_bytes = 0;
+  if (att && n_traj > 0) {
+    const size_t mb = (size_t)ctx->cfg.H * ctx->cfg.W * 4 * n_traj, wb = (size_t)2 * 24 * 4 * n_traj;
+    if (att->map) CU_OK(cudaMemcpyAsync(att->map, att_maps, mb, cudaMemcpyDeviceToHost, st));
+    if (att->weights) CU_OK(cudaMemcpyAsync(att->weights, att_weights, wb, cudaMemcpyDeviceToHost, st));
+    att_bytes = (att->map ? (long long)mb : 0) + (att->weights ? (long long)wb : 0);
+  }
   if (int rc = host_done(ctx, st, ticket)) return rc;
-  ctx->last_d2h = (long long)12 * 4 * B + (long long)16 * 8 * n_traj;
+  ctx->last_d2h = (long long)12 * 4 * B + (long long)16 * 8 * n_traj + att_bytes;
   return 0;
 }
 
@@ -2284,7 +2334,118 @@ struct OdoPush {
   long long g0;
   double* traj_out;
   int n_traj;
+  const davo_odometry_attention* att;   // each posed frame's map and weights, or NULL
 };
+
+// ---- each posed frame's attention (include/davo_b200.h: davo_odometry_attention) ----
+// Row r of a push's outputs is the frame of traj_out[r]: with sample 0 of the stream, frame 0 (src0 of sample 0) and
+// frame 1 (its target), then frame s+2, src1 of sample s.  attention_out_kernel writes the rows through a unit table:
+// the only code that knows how a single push, the chunks of a host push and the staging of a batched push order their
+// units.
+
+// Where view sample b's frames go: the row of its src1 frame, and whether it opens its stream (its src0 and target then
+// take the two rows before), or row -1 when no frame of it has a row.
+struct AttSample { int row; bool opens; };
+
+// The unit table of a forward over `nsel` selection slots of pair mode `mode` (pair_of_slot; kUnitsAreSamples for the
+// non-shared nets): unit -> (row of its target, src0, src1 frame or -1, view sample).  A pair unit tgt -> src1 places
+// src1; the unit tgt -> src0 of a sample that opens its stream places src0 and the target, whose maps it masks; a
+// sample unit places all three.
+template <class F>
+void att_unit_table(std::vector<int4>& out, int mode, int nsel, F sample_of) {
+  for (int q = 0; q < nsel; ++q) {
+    int b = 0, k = 0;
+    pair_of_slot(mode, q, &b, &k);
+    const AttSample a = sample_of(b);
+    int4 e = make_int4(-1, -1, -1, b);
+    if (a.row >= 0) {
+      const bool sample_unit = mode == kUnitsAreSamples;
+      if (sample_unit || k == 1) e.z = a.row;
+      if (a.opens && (sample_unit || k == 0)) { e.y = a.row - 2; e.x = a.row - 1; }
+    }
+    out.push_back(e);
+  }
+}
+
+// The tables of a call to the device: one copy from a pinned ring slot (refilled once the call that last used it has
+// finished), recorded as done after the call's last use on st by att_tables_done.  Returns the slot.
+int att_tables_upload(davo_ctx* ctx, const std::vector<int4>& units, const std::vector<AttRow>& rows, cudaStream_t st,
+                      const int4** d_units, const AttRow** d_rows, int* slot_out) {
+  const int slot = (int)(ctx->att_calls++ % davo_ctx::kManyRing);
+  const size_t ub = sizeof(int4) * units.size(), bytes = ub + sizeof(AttRow) * rows.size();
+  if (ctx->att_ev[slot]) CU_OK(cudaEventSynchronize(ctx->att_ev[slot]));
+  else CU_OK(cudaEventCreateWithFlags(&ctx->att_ev[slot], cudaEventDisableTiming));
+  if (ctx->att_desc_cap[slot] < bytes) {
+    const size_t cap = std::max<size_t>(bytes, 2 * ctx->att_desc_cap[slot]);
+    if (ctx->att_hdesc[slot]) { CU_OK(cudaFreeHost(ctx->att_hdesc[slot])); ctx->att_hdesc[slot] = nullptr; }
+    if (ctx->att_ddesc[slot]) { CU_OK(cudaFree(ctx->att_ddesc[slot])); ctx->att_ddesc[slot] = nullptr; }
+    ctx->att_desc_cap[slot] = 0;
+    CU_OK(cudaHostAlloc(&ctx->att_hdesc[slot], cap, cudaHostAllocDefault));
+    CU_OK(cudaMalloc(&ctx->att_ddesc[slot], cap));
+    ctx->att_desc_cap[slot] = cap;
+  }
+  uint8_t* h = static_cast<uint8_t*>(ctx->att_hdesc[slot]);
+  if (ub) memcpy(h, units.data(), ub);
+  if (!rows.empty()) memcpy(h + ub, rows.data(), bytes - ub);
+  if (bytes) CU_OK(cudaMemcpyAsync(ctx->att_ddesc[slot], h, bytes, cudaMemcpyHostToDevice, st));
+  *d_units = static_cast<const int4*>(ctx->att_ddesc[slot]);
+  *d_rows = reinterpret_cast<const AttRow*>(static_cast<const uint8_t*>(ctx->att_ddesc[slot]) + ub);
+  *slot_out = slot;
+  return 0;
+}
+int att_tables_done(davo_ctx* ctx, int slot, cudaStream_t st) {
+  CU_OK(cudaEventRecord(ctx->att_ev[slot], st));
+  return 0;
+}
+
+// The unit table in use while a forward is launched; cleared on every way out.
+struct AttScope {
+  davo_ctx* ctx;
+  AttScope(davo_ctx* c, const int4* units, const AttRow* rows) : ctx(c) { ctx->att_units = units; ctx->att_rows = rows; }
+  ~AttScope() { ctx->att_units = nullptr; ctx->att_rows = nullptr; }
+};
+
+constexpr size_t kAttWeightFloats = 2 * kAttStride;      // a frame's weight rows
+
+// Device staging of host sessions' maps and weights for `n_rows` rows: maps [n_rows][H][W], then weights
+// [n_rows][2][kAttStride].  Grown on demand, after the work that may still write or read it.
+int att_stage(davo_ctx* ctx, size_t n_rows, float** maps, float** weights) {
+  const size_t hw = (size_t)ctx->cfg.H * ctx->cfg.W, need = n_rows * (hw + kAttWeightFloats);
+  if (ctx->att_stage_cap < need) {
+    if (ctx->att_stage) {
+      CU_OK(cudaDeviceSynchronize());
+      CU_OK(cudaFree(ctx->att_stage));
+      ctx->att_stage = nullptr;
+    }
+    const size_t cap = std::max(need, 2 * ctx->att_stage_cap);
+    ctx->att_stage_cap = 0;
+    CU_OK(cudaMalloc((void**)&ctx->att_stage, cap * sizeof(float)));
+    ctx->att_stage_cap = cap;
+  }
+  *maps = ctx->att_stage;
+  *weights = ctx->att_stage + n_rows * hw;
+  return 0;
+}
+
+// A session's attention entry where `n_rows` rows are due: map / weights each NULL (not written) or 16-byte aligned,
+// not both NULL.  `idx` >= 0 names the entry of a batched push.
+int att_check(davo_ctx* ctx, const char* who, const davo_odometry_attention& a, int n_rows, int idx) {
+  char name[32];
+  if (idx >= 0) snprintf(name, sizeof name, "att[%d]", idx);
+  else snprintf(name, sizeof name, "att");
+  if (n_rows > 0 && !a.map && !a.weights)
+    return fail(ctx, DAVO_ERR_ARG, "%s: %s has neither map nor weights; %d row(s) are due", who, name, n_rows);
+  if ((reinterpret_cast<uintptr_t>(a.map) | reinterpret_cast<uintptr_t>(a.weights)) & 15)
+    return fail(ctx, DAVO_ERR_ARG, "%s: %s.%s is not 16-byte aligned", who, name,
+                (reinterpret_cast<uintptr_t>(a.map) & 15) ? "map" : "weights");
+  return 0;
+}
+
+// Row pointers of `n` rows from the start of a session's (or the staging's) map and weight buffers
+void att_rows_of(std::vector<AttRow>& rows, float* map, float* weights, int n, size_t hw) {
+  for (int r = 0; r < n; ++r)
+    rows.push_back({map ? map + hw * r : nullptr, weights ? weights + kAttWeightFloats * r : nullptr});
+}
 
 }  // namespace
 
@@ -2365,6 +2526,28 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
     return 0;
   };
   InputView in{};
+  // a push's attention outputs: rows staged on the device, one unit table per chunk (the chunks' own pair modes)
+  const davo_odometry_attention* att = op && op->att && B > 0 ? op->att : nullptr;
+  float *att_maps = nullptr, *att_wts = nullptr;
+  const int4* att_units = nullptr;
+  const AttRow* att_rows = nullptr;
+  std::vector<int> att_off;
+  int att_slot = -1;
+  if (att) {
+    if (int rc = att_stage(ctx, (size_t)op->n_traj, &att_maps, &att_wts)) return rc;
+    std::vector<int4> units;
+    std::vector<AttRow> rows;
+    const bool opens = op->g0 == 0;
+    for (int a0 = 0; a0 < B; a0 += cs) {
+      const int an = std::min(cs, B - a0);
+      const int cp_ = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && a0 > 0) ? DAVO_PAIRS_TRAJECTORY : pairs;
+      att_off.push_back((int)units.size());
+      att_unit_table(units, cp_, pairs_selected(cp_, an),
+                     [&](int b) { const int sm = a0 + b; return AttSample{sm + 2 * opens, opens && sm == 0}; });
+    }
+    att_rows_of(rows, att->map ? att_maps : nullptr, att->weights ? att_wts : nullptr, op->n_traj, hw);
+    if (int rc = att_tables_upload(ctx, units, rows, st, &att_units, &att_rows, &att_slot)) return rc;
+  }
   // a push too short to hold a sample still stages its frames: one chunk of no samples
   for (int s0 = 0; s0 < B || (o && chunk == 0); s0 += ns, ++chunk) {
     ns = std::min(cs, B - s0);
@@ -2449,8 +2632,10 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
                        n16 > 0 ? (n16_fwd > 0 ? ctx->s_flow16[buf] : ctx->s_flow16[buf] + fl * cs) : nullptr,
                        n16 > 0 ? ctx->s_flow16[buf] + fl * cs : nullptr, n16);
     const int chunk_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && s0 > 0) ? DAVO_PAIRS_TRAJECTORY : pairs;
-    if (ns > 0)
+    if (ns > 0) {
+      AttScope scope(ctx, att ? att_units + att_off[chunk] : nullptr, att_rows);
       if (int rc = host_run_chunk(ctx, chunk_pairs, s0, ns, in, st, &launches, &last_n)) return rc;
+    }
     CU_OK(cudaEventRecord(ctx->ev_consumed[buf], st));
   }
   if (o) {
@@ -2475,8 +2660,10 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
     traj_extend_kernel<<<1, 32, 0, st>>>(o->d_rel, m, first, o->d_P, o->d_traj);
     CU_OK(cudaGetLastError());
   }
+  if (att)
+    if (int rc = att_tables_done(ctx, att_slot, st)) return rc;
   if (int rc = host_finish(ctx, B, pose_out, st, ticket, o ? reinterpret_cast<double*>(o->d_traj) : nullptr,
-                           op ? op->traj_out : nullptr, op ? op->n_traj : 0)) return rc;
+                           op ? op->traj_out : nullptr, op ? op->n_traj : 0, att, att_maps, att_wts)) return rc;
   ctx->last_h2d = (long long)h2d;
   if (B > 0) {                                                     // a push without samples ran no forward
     ctx->last_launches = launches;
@@ -2559,10 +2746,10 @@ extern "C" int davo_odometry_create(davo_ctx* ctx, int max_push, int pairs, int 
   return 0;
 }
 
-extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
-                                  const float* seg, const float* depth, float* pose_out, double* traj_out, int* n_samples,
-                                  int* n_traj, void* stream, long long* ticket) {
-  const char* who = "davo_odometry_push";
+static int odometry_push_impl(const char* who, davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd,
+                              const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                              double* traj_out, const davo_odometry_attention* att, int* n_samples, int* n_traj,
+                              void* stream, long long* ticket) {
   {
     std::lock_guard<std::mutex> lk(g_odo_mutex);
     if (!o || !g_odo_live.count(o)) return fail(nullptr, DAVO_ERR_ARG, "%s: the session is NULL or was destroyed", who);
@@ -2589,9 +2776,11 @@ extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, c
     if (x.needed && !x.p) return fail(ctx, DAVO_ERR_ARG, "%s: %s is NULL; this variant and pair selection read it", who, x.name);
     if (x.p && (reinterpret_cast<uintptr_t>(x.p) & 15)) return fail(ctx, DAVO_ERR_ARG, "%s: %s is not 16-byte aligned", who, x.name);
   }
+  if (att)
+    if (int rc = att_check(ctx, who, *att, nt, -1)) return rc;
   CU_OK(cudaSetDevice(ctx->device));
   if (o->host) {
-    OdoPush op{o, head, fe, g0, traj_out, nt};
+    OdoPush op{o, head, fe, g0, traj_out, nt, att};
     if (int rc = forward_sequence_host_impl(ctx, n, vpairs, img, flow_fwd, flow_bwd, seg, depth, pose_out, stream, ticket, &op))
       return rc;
   } else {
@@ -2623,7 +2812,24 @@ extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, c
     if (!rc && ns > 0) {
       const InputView v = sequence_view(c.H, c.W, o->q_img[0], fwd ? fwd : bwd1, bwd1, labels ? o->q_seg[0] : nullptr, nullptr,
                                         o->q_depth[0], nullptr, nullptr, 0);
-      rc = forward_device(ctx, who, ns, vpairs, v, pose_out, st);
+      if (att) {                                                   // the frames' maps and weights: one unit table
+        const int mode = ctx->unit_sample ? kUnitsAreSamples : vpairs;
+        std::vector<int4> units;
+        std::vector<AttRow> rows;
+        att_unit_table(units, mode, pairs_selected(mode, ns), [&](int b) { return AttSample{b + 2 * first, first && b == 0}; });
+        att_rows_of(rows, att->map, att->weights, nt, hw);
+        const int4* du = nullptr;
+        const AttRow* dr = nullptr;
+        int slot = -1;
+        rc = att_tables_upload(ctx, units, rows, st, &du, &dr, &slot);
+        if (!rc) {
+          AttScope scope(ctx, du, dr);
+          rc = forward_device(ctx, who, ns, vpairs, v, pose_out, st);
+        }
+        if (!rc) rc = att_tables_done(ctx, slot, st);
+      } else {
+        rc = forward_device(ctx, who, ns, vpairs, v, pose_out, st);
+      }
     }
     const int nc = std::min(n, 2), fc = n - nc;
     if (!rc) rc = d2d(o->c_img, o->q_img[0] + hw * 3 * fc, hw * 3 * nc);
@@ -2645,6 +2851,21 @@ extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, c
   if (n_samples) *n_samples = ns;
   if (n_traj) *n_traj = nt;
   return 0;
+}
+
+extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
+                                  const float* seg, const float* depth, float* pose_out, double* traj_out, int* n_samples,
+                                  int* n_traj, void* stream, long long* ticket) {
+  return odometry_push_impl("davo_odometry_push", o, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, nullptr,
+                            n_samples, n_traj, stream, ticket);
+}
+
+extern "C" int davo_odometry_push_attention(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd,
+                                            const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                                            double* traj_out, const davo_odometry_attention* att, int* n_samples,
+                                            int* n_traj, void* stream, long long* ticket) {
+  return odometry_push_impl("davo_odometry_push_attention", o, k, img, flow_fwd, flow_bwd, seg, depth, pose_out,
+                            traj_out, att, n_samples, n_traj, stream, ticket);
 }
 
 namespace {
@@ -2800,8 +3021,8 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
 static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
                                    const float* const* flow_fwd, const float* const* flow_bwd,
                                    const float* const* seg, const float* const* depth, float* const* pose_out,
-                                   double* const* traj_out, int* n_samples, int* n_traj, void* stream, long long* ticket) {
-  const char* who = host ? "davo_odometry_push_many_host" : "davo_odometry_push_many";
+                                   double* const* traj_out, const davo_odometry_attention* att, int* n_samples,
+                                   int* n_traj, void* stream, long long* ticket, const char* who) {
   if (n < 1) return fail(nullptr, DAVO_ERR_ARG, "%s: n=%d: at least one session", who, n);
   if (!sessions) return fail(nullptr, DAVO_ERR_ARG, "%s: sessions is NULL", who);
   {
@@ -2858,6 +3079,8 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
     d.na = (ctx->unit_sample || o->pairs == DAVO_PAIRS_ALL) ? ns : first;
     const int e = nn - 2;                                                 // the last flow_fwd entry, read by a later sample
     d.carry_fwd = e >= fe && rg.fwd((int)std::min(g0 + e, 2LL)) ? e - fe : -1;
+    if (att)
+      if (int rc = att_check(ctx, who, att[i], ns + 2 * first, i)) return rc;
     B += ns;
     nA += d.na;
   }
@@ -2910,6 +3133,37 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
   if (B) memcpy(h + sess_bytes, smp.data(), sizeof(int2) * B);
   CU_OK(cudaMemcpyAsync(ctx->m_ddesc[slot], h, bytes, cudaMemcpyHostToDevice, st));
   const OdoManySession* dsess = static_cast<const OdoManySession*>(ctx->m_ddesc[slot]);
+  // each posed frame's attention: session i's rows from rb[i] on, one unit table per forward (staging order: the
+  // both-pair samples, then the trajectory samples); host sessions' rows are staged on the device
+  std::vector<int> rb(n + 1, 0);
+  for (int i = 0; i < n; ++i) rb[i + 1] = rb[i] + ds[i].ns + 2 * ds[i].first;
+  const bool want_att = att && B > 0;
+  float *att_maps = nullptr, *att_wts = nullptr;
+  const int4* att_units = nullptr;
+  const AttRow* att_rows = nullptr;
+  int att_slot = -1, nsel_a = 0;
+  if (want_att) {
+    if (host)
+      if (int rc = att_stage(ctx, (size_t)rb[n], &att_maps, &att_wts)) return rc;
+    std::vector<AttRow> rows;
+    for (int i = 0; i < n; ++i) {
+      const int nt = rb[i + 1] - rb[i];
+      if (host) att_rows_of(rows, att[i].map ? att_maps + hw * rb[i] : nullptr,
+                            att[i].weights ? att_wts + kAttWeightFloats * rb[i] : nullptr, nt, hw);
+      else att_rows_of(rows, att[i].map, att[i].weights, nt, hw);
+    }
+    auto sample_at = [&](int b) {
+      const int2 m = smp[b];
+      const OdoManySession& d = ds[m.x];
+      return AttSample{rb[m.x] + m.y + 2 * d.first, d.first && m.y == 0};
+    };
+    std::vector<int4> units;
+    const int mode_a = ctx->unit_sample ? kUnitsAreSamples : DAVO_PAIRS_ALL;
+    nsel_a = pairs_selected(mode_a, nA);
+    att_unit_table(units, mode_a, nsel_a, sample_at);
+    att_unit_table(units, DAVO_PAIRS_TRAJECTORY, B - nA, [&](int b) { return sample_at(nA + b); });
+    if (int rc = att_tables_upload(ctx, units, rows, st, &att_units, &att_rows, &att_slot)) return rc;
+  }
   constexpr int kCopyBlocks = 4 * 148;                                     // blocks of a copy launch, over its rows
   if (B > 0) {
     OdoStageParams sp;
@@ -2936,10 +3190,16 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
       return stacked_view(c.H, c.W, ctx->m_img + hw * 9 * b0, ctx->m_flow ? ctx->m_flow + hw * 4 * b0 : nullptr,
                           ctx->m_lab ? ctx->m_lab + hw * 3 * b0 : nullptr, ctx->m_depth ? ctx->m_depth + hw * 3 * b0 : nullptr);
     };
-    if (nA > 0)
+    if (nA > 0) {
+      AttScope scope(ctx, want_att ? att_units : nullptr, att_rows);
       if (int rc = forward_device(ctx, who, nA, DAVO_PAIRS_ALL, view(0), ctx->m_pose, st)) return rc;
-    if (B > nA)
+    }
+    if (B > nA) {
+      AttScope scope(ctx, want_att ? att_units + nsel_a : nullptr, att_rows);
       if (int rc = forward_device(ctx, who, B - nA, DAVO_PAIRS_TRAJECTORY, view(nA), ctx->m_pose + 12 * nA, st)) return rc;
+    }
+    if (want_att)
+      if (int rc = att_tables_done(ctx, att_slot, st)) return rc;
     odo_compose_many_kernel<<<(n + 3) / 4, 128, 0, st>>>(dsess, n, ctx->m_pose);
     CU_OK(cudaGetLastError());
   }
@@ -2951,6 +3211,13 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
       if (np) CU_OK(cudaMemcpyAsync(pose_out[i], ds[i].pose_out, np, cudaMemcpyDeviceToHost, st));
       if (nt) CU_OK(cudaMemcpyAsync(traj_out[i], ds[i].traj_out, nt, cudaMemcpyDeviceToHost, st));
       d2h += (long long)(np + nt);
+      const int na = rb[i + 1] - rb[i];
+      if (want_att && na > 0) {
+        const size_t mb = hw * 4 * na, wb = kAttWeightFloats * 4 * na;
+        if (att[i].map) CU_OK(cudaMemcpyAsync(att[i].map, att_maps + hw * rb[i], mb, cudaMemcpyDeviceToHost, st));
+        if (att[i].weights) CU_OK(cudaMemcpyAsync(att[i].weights, att_wts + kAttWeightFloats * rb[i], wb, cudaMemcpyDeviceToHost, st));
+        d2h += (att[i].map ? (long long)mb : 0) + (att[i].weights ? (long long)wb : 0);
+      }
     }
     if (int rc = host_done(ctx, st, ticket)) return rc;
     ctx->last_h2d = (long long)h2d;
@@ -2970,8 +3237,8 @@ extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, co
                                        const float* const* flow_fwd, const float* const* flow_bwd,
                                        const float* const* seg, const float* const* depth, float* const* pose_out,
                                        double* const* traj_out, int* n_samples, int* n_traj, void* stream) {
-  return odometry_push_many_impl(false, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, n_samples,
-                                 n_traj, stream, nullptr);
+  return odometry_push_many_impl(false, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, nullptr,
+                                 n_samples, n_traj, stream, nullptr, "davo_odometry_push_many");
 }
 
 extern "C" int davo_odometry_push_many_host(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
@@ -2979,8 +3246,28 @@ extern "C" int davo_odometry_push_many_host(int n, davo_odometry* const* session
                                             const float* const* seg, const float* const* depth, float* const* pose_out,
                                             double* const* traj_out, int* n_samples, int* n_traj, void* stream,
                                             long long* ticket) {
-  return odometry_push_many_impl(true, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, n_samples,
-                                 n_traj, stream, ticket);
+  return odometry_push_many_impl(true, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, nullptr,
+                                 n_samples, n_traj, stream, ticket, "davo_odometry_push_many_host");
+}
+
+extern "C" int davo_odometry_push_many_attention(int n, davo_odometry* const* sessions, const int* k,
+                                                 const uint8_t* const* img, const float* const* flow_fwd,
+                                                 const float* const* flow_bwd, const float* const* seg,
+                                                 const float* const* depth, float* const* pose_out,
+                                                 double* const* traj_out, const davo_odometry_attention* att,
+                                                 int* n_samples, int* n_traj, void* stream) {
+  return odometry_push_many_impl(false, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, att,
+                                 n_samples, n_traj, stream, nullptr, "davo_odometry_push_many_attention");
+}
+
+extern "C" int davo_odometry_push_many_host_attention(int n, davo_odometry* const* sessions, const int* k,
+                                                      const uint8_t* const* img, const float* const* flow_fwd,
+                                                      const float* const* flow_bwd, const float* const* seg,
+                                                      const float* const* depth, float* const* pose_out,
+                                                      double* const* traj_out, const davo_odometry_attention* att,
+                                                      int* n_samples, int* n_traj, void* stream, long long* ticket) {
+  return odometry_push_many_impl(true, n, sessions, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, att,
+                                 n_samples, n_traj, stream, ticket, "davo_odometry_push_many_host_attention");
 }
 
 extern "C" int davo_odometry_reset(davo_odometry* o) {
@@ -3746,17 +4033,20 @@ void middlebury_wheel(float (*wheel)[3]) {
 }
 }  // namespace
 
-extern "C" int davo_forward_features(davo_ctx* ctx, int B, const uint8_t* img, const float* flow,
-                                     const float* seg, const float* depth, float* pose_out,
-                                     const davo_features* out, void* stream) {
-  if (!ctx) return DAVO_ERR_ARG;
-  if (!out) return fail(ctx, DAVO_ERR_ARG, "davo_forward_features: null output table");
+namespace {
+// The output table's checks of mode='feature' on B samples (davo_forward_features, davo_forward_sequence_features).
+int features_check(davo_ctx* ctx, const char* who, const char* samples, int B, const davo_features* out, bool flow, bool seg) {
+  if (!out) return fail(ctx, DAVO_ERR_ARG, "%s: null output table", who);
   const int units = ctx->unit_sample ? B : 2 * B;
   if (ctx->finalized && units > ctx->mb)
-    return fail(ctx, DAVO_ERR_ARG, "davo_forward_features: B=%d needs %d units, one pass holds %d", B, units, ctx->mb);
-  if ((out->flow_color) && !flow) return fail(ctx, DAVO_ERR_ARG, "davo_forward_features: flow colouring needs input_flow");
-  if ((out->seg_19 || out->seg_color) && !seg) return fail(ctx, DAVO_ERR_ARG, "davo_forward_features: label outputs need input_seglabel");
-  if (int rc = davo_forward_pairs(ctx, B, DAVO_PAIRS_ALL, img, flow, seg, depth, pose_out, stream)) return rc;
+    return fail(ctx, DAVO_ERR_ARG, "%s: %s needs %d units, one pass holds %d", who, samples, units, ctx->mb);
+  if ((out->flow_color) && !flow) return fail(ctx, DAVO_ERR_ARG, "%s: flow colouring needs input_flow", who);
+  if ((out->seg_19 || out->seg_color) && !seg) return fail(ctx, DAVO_ERR_ARG, "%s: label outputs need input_seglabel", who);
+  return 0;
+}
+
+// The feature outputs of the one pass that just ran over the B samples of `in` (either layout).
+int features_outputs(davo_ctx* ctx, int B, const InputView& in, const davo_features* out, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const davo_config& c = ctx->cfg;
   if (!ctx->d_wheel) {
@@ -3777,7 +4067,7 @@ extern "C" int davo_forward_features(davo_ctx* ctx, int B, const uint8_t* img, c
   // what frame_attention reads: the variant's flags and the flow / depth planes of this batch
   fp.fp.H = c.H; fp.fp.W = c.W; fp.fp.att_src = c.att_src; fp.fp.pixel_map = c.pixel_map; fp.fp.depth_norm = c.depth_norm;
   fp.fp.depth_split = c.depth_split; fp.fp.depth_thres = ctx->depth_thres; fp.fp.flow_abs = c.flow_abs; fp.fp.flow_norm = c.flow_norm;
-  fp.fp.in = triplet_view(c.H, c.W, img, flow, seg, nullptr, depth, nullptr, 0); fp.fp.flow_f16 = c.flow_f16;
+  fp.fp.in = in; fp.fp.flow_f16 = c.flow_f16;
   fp.att_w = ctx->d_attw; fp.static_w = ctx->d_staticw;
   fp.wheel = ctx->d_wheel; fp.maxrad = ctx->d_maxrad;
   fp.image = out->image; fp.attention = out->attention; fp.masked_image = out->masked_image;
@@ -3821,6 +4111,33 @@ extern "C" int davo_forward_features(davo_ctx* ctx, int B, const uint8_t* img, c
   }
   ctx->last_launches = launches;
   return 0;
+}
+}  // namespace
+
+extern "C" int davo_forward_features(davo_ctx* ctx, int B, const uint8_t* img, const float* flow,
+                                     const float* seg, const float* depth, float* pose_out,
+                                     const davo_features* out, void* stream) {
+  if (!ctx) return DAVO_ERR_ARG;
+  char samples[32];
+  snprintf(samples, sizeof samples, "B=%d", B);
+  if (int rc = features_check(ctx, "davo_forward_features", samples, B, out, flow != nullptr, seg != nullptr)) return rc;
+  if (int rc = davo_forward_pairs(ctx, B, DAVO_PAIRS_ALL, img, flow, seg, depth, pose_out, stream)) return rc;
+  return features_outputs(ctx, B, triplet_view(ctx->cfg.H, ctx->cfg.W, img, flow, seg, nullptr, depth, nullptr, 0), out, stream);
+}
+
+extern "C" int davo_forward_sequence_features(davo_ctx* ctx, int n_frames, const uint8_t* img, const float* flow_fwd,
+                                              const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                                              const davo_features* out, void* stream) {
+  if (!ctx) return DAVO_ERR_ARG;
+  const char* who = "davo_forward_sequence_features";
+  if (int rc = check_sequence(ctx, who, n_frames, DAVO_PAIRS_ALL, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
+  const int B = n_frames - 2;
+  char samples[64];
+  snprintf(samples, sizeof samples, "n_frames=%d (B=%d samples)", n_frames, B);
+  if (int rc = features_check(ctx, who, samples, B, out, flow_fwd && flow_bwd, seg != nullptr)) return rc;
+  const InputView in = sequence_device_view(ctx, img, flow_fwd, flow_bwd, seg, depth);
+  if (int rc = forward_device(ctx, who, B, DAVO_PAIRS_ALL, in, pose_out, stream)) return rc;
+  return features_outputs(ctx, B, in, out, stream);
 }
 
 // Test hook (no GPU needed): the CPU float32 -> binary16 conversion of the host entry point.

@@ -41,17 +41,53 @@ __constant__ uint8_t c_cityscapes[kNumClasses][3] = {
     {250, 170, 30}, {220, 220, 0}, {107, 142, 35}, {152, 251, 152}, {70, 130, 180}, {220, 20, 60},
     {255, 0, 0}, {0, 0, 142}, {0, 0, 70}, {0, 60, 100}, {0, 80, 100}, {0, 0, 230}, {119, 11, 32}};
 
-// Class weights of frame f of sample b, or NULL when the map is all ones (tf.ones_like: davo.py
-// 1385-1389 for -no_segmask, 1408-1412 / 1218 / 1283 / 1310 / 1393 for the forced target map).
+// Class weights of frame f (0 tgt, 1 src0, 2 src1) out of the attention-weight slots of `unit`, or NULL when the map is
+// all ones (tf.ones_like: davo.py 1385-1389 for -no_segmask, 1408-1412 / 1218 / 1283 / 1310 / 1393 for the forced target
+// map).  A frame-pair unit holds its source frame (slot 0) and the target (slot 1); a sample unit holds all three
+// (frontend.cuh: unit_frame).  The one place that picks a frame's table: the feature outputs and the sessions'
+// attention outputs both read it.
+__device__ __forceinline__ const float* unit_frame_weights(int att_src, int tgt_ones, int unit_sample, int depth_split,
+                                                           const float* att_w, const float* static_w, int unit, int f) {
+  if (att_src == 0) return nullptr;
+  if (f == 0 && tgt_ones) return nullptr;
+  if (att_src == 2) return static_w;
+  const int slot = unit_sample && depth_split ? 2 * (f - 1)           // (near, far) of src f-1
+                 : unit_sample ? (f == 0 ? 2 : f - 1)
+                 : f == 0 ? 1 : 0;
+  return att_w + ((size_t)unit * kAttFrames + slot) * kAttStride;
+}
+
+// Frame f of sample b of a DAVO_PAIRS_ALL pass: the sample's unit, or the pair tgt -> src0 (target, src0) / tgt -> src1
 __device__ __forceinline__ const float* frame_weights(const FeatureParams& p, int b, int f) {
-  if (p.att_src == 0) return nullptr;
-  if (f == 0 && p.att_tgt_ones) return nullptr;
-  if (p.att_src == 2) return p.static_w;
-  // slots of a unit: frontend.cuh unit_frame
-  if (p.unit_sample && p.fp.depth_split) return p.att_w + ((size_t)b * kAttFrames + 2 * (f - 1)) * kAttStride;   // (near, far) of src f-1
-  if (p.unit_sample) return p.att_w + ((size_t)b * kAttFrames + (f == 0 ? 2 : f - 1)) * kAttStride;
-  if (f == 0) return p.att_w + ((size_t)(2 * b) * kAttFrames + 1) * kAttStride;
-  return p.att_w + ((size_t)(2 * b + (f - 1)) * kAttFrames + 0) * kAttStride;
+  const int unit = p.unit_sample ? b : 2 * b + (f == 2 ? 1 : 0);
+  return unit_frame_weights(p.att_src, p.att_tgt_ones, p.unit_sample, p.fp.depth_split, p.att_w, p.static_w, unit, f);
+}
+
+// Attention of the 4 pixels p0.. of frame f (0 tgt, 1 src0, 2 src1) of view sample b, from the frame's table w (w_far:
+// the far table of a depth-split source) or all ones; lab / r / g / bl are the pixels' labels and [-1,1] colours.
+__device__ __forceinline__ void frame_attention4(const FrontParams& fp, int att_src, bool ones, const float* w,
+                                                 const float* w_far, int b, int f, int p0, int hw, const int (&lab)[4],
+                                                 const float (&r)[4], const float (&g)[4], const float (&bl)[4],
+                                                 float (&a)[4]) {
+  const bool need_depth = fp.depth_split || (fp.pixel_map && att_src == 5);
+  const bool need_flow = fp.pixel_map && (att_src == 6 || fp.pixel_map == 2);
+  const int plane = f == 0 ? 1 : f == 1 ? 0 : 2;        // position in the inputs: [src0, tgt, src1]
+  const InputView& in = fp.in;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    if (ones) { a[i] = 1.0f; continue; }
+    float ds = 0.f, dt = 0.f, sfx = se_in_x(0.f, fp), sfy = se_in_y(0.f, fp);   // the target's flow is zeros
+    if (need_depth) {
+      ds = __ldg(in.depth + frame_plane(in, b, plane, hw) + p0 + i);
+      dt = __ldg(in.depth + frame_plane(in, b, 1, hw) + p0 + i);
+    }
+    if (need_flow && f != 0) {
+      const float2 v = flow1_at(fp, b, f - 1, p0 + i, hw);
+      sfx = se_in_x(v.x, fp);
+      sfy = se_in_y(v.y, fp);
+    }
+    a[i] = frame_attention(fp, w, w_far, lab[i], r[i], g[i], bl[i], ds, dt, sfx, sfy);
+  }
 }
 
 // grid (blocks, B, 3 frames); a thread takes 4 consecutive pixels of a row
@@ -68,8 +104,6 @@ __global__ void __launch_bounds__(256) feature_frames_kernel(const FeatureParams
     s_wf[threadIdx.x] = (w && p.fp.depth_split) ? w[kAttStride + threadIdx.x] : 0.0f;   // slot 1 of the same pair
   }
   __syncthreads();
-  const bool need_depth = p.fp.depth_split || (p.fp.pixel_map && p.att_src == 5);
-  const bool need_flow = p.fp.pixel_map && (p.att_src == 6 || p.fp.pixel_map == 2);
   const bool ones = s_ones != 0;
   const int plane = f == 0 ? 1 : f == 1 ? 0 : 2;        // position in the inputs: [src0, tgt, src1]
   const InputView& in = p.fp.in;
@@ -87,21 +121,7 @@ __global__ void __launch_bounds__(256) feature_frames_kernel(const FeatureParams
       lab[0] = label_of(v.x); lab[1] = label_of(v.y); lab[2] = label_of(v.z); lab[3] = label_of(v.w);   // tf.cast truncates
     }
     float a[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      if (ones) { a[i] = 1.0f; continue; }
-      float ds = 0.f, dt = 0.f, sfx = se_in_x(0.f, p.fp), sfy = se_in_y(0.f, p.fp);   // the target's flow is zeros
-      if (need_depth) {
-        ds = __ldg(in.depth + frame_plane(in, b, plane, hw) + p0 + i);
-        dt = __ldg(in.depth + frame_plane(in, b, 1, hw) + p0 + i);
-      }
-      if (need_flow && f != 0) {
-        const float2 v = flow1_at(p.fp, b, f - 1, p0 + i, hw);
-        sfx = se_in_x(v.x, p.fp);
-        sfy = se_in_y(v.y, p.fp);
-      }
-      a[i] = frame_attention(p.fp, s_w, s_wf, lab[i], r[i], g[i], bl[i], ds, dt, sfx, sfy);
-    }
+    frame_attention4(p.fp, p.att_src, ones, s_w, s_wf, b, f, p0, hw, lab, r, g, bl, a);
     const size_t px0 = fb * hw + p0;
     if (p.attention) *reinterpret_cast<float4*>(p.attention + px0) = make_float4(a[0], a[1], a[2], a[3]);
     if (p.image) {
@@ -145,6 +165,75 @@ __global__ void __launch_bounds__(256) feature_frames_kernel(const FeatureParams
 #pragma unroll
       for (int j = 0; j < 3; ++j)
         o[j] = (uint32_t)c[4 * j] | ((uint32_t)c[4 * j + 1] << 8) | ((uint32_t)c[4 * j + 2] << 16) | ((uint32_t)c[4 * j + 3] << 24);
+    }
+  }
+}
+
+// ---- attention of odometry pushes ------------------------------------------------------------
+// One posed frame's outputs (include/davo_b200.h: davo_odometry_attention): its map [H][W] and its weight rows
+// [2][kAttStride]; either may be NULL.
+struct AttRow {
+  float* map;
+  float* weights;
+};
+
+struct AttentionOutParams {
+  FrontParams fp;         // the micro-batch's front end as launch_front ran it: the variant's flags, the view, att_w
+  const int4* units;      // per selection slot of the forward: the destination row of the unit's frame (x tgt, y src0,
+                          // z src1) or -1, and (w) the view sample; built by the host (davo_capi.cu: att_unit_table)
+  const AttRow* rows;
+  int width;              // entries of weight row 0 (and 1): davo_get_intermediate("att_weights:<k>")'s width
+};
+
+// grid (blocks, units of the micro-batch); a thread takes 4 consecutive pixels.  Unit u = pair0 + blockIdx.y of the
+// forward writes the maps of its frames that have a row -- the map its own pass masks the frame with, computed as
+// feature_frames_kernel computes it -- and block 0 the frame's table(s).  Reads att_w and the inputs only.
+__global__ void __launch_bounds__(256) attention_out_kernel(const AttentionOutParams p) {
+  const FrontParams& fp = p.fp;
+  const int4 e = p.units[fp.pair0 + blockIdx.y];
+  if (e.x < 0 && e.y < 0 && e.z < 0) return;
+  __shared__ float s_w[kAttStride], s_wf[kAttStride];
+  const int hw = fp.H * fp.W, groups = hw / 4, b = e.w;
+  const InputView& in = fp.in;
+  const bool need_rgb = fp.pixel_map && fp.att_src == 4;
+  const bool need_lab = !fp.pixel_map || fp.att_src == 6;
+#pragma unroll 1
+  for (int f = 0; f < 3; ++f) {
+    const int row = f == 0 ? e.x : f == 1 ? e.y : e.z;
+    if (row < 0) continue;
+    const float* w = unit_frame_weights(fp.att_src, fp.att_tgt_ones, fp.unit_sample, fp.depth_split, fp.att_w,
+                                        fp.static_w, blockIdx.y, f);
+    __syncthreads();                                      // the previous frame's tables have been read
+    if (threadIdx.x < kAttStride) {
+      const bool table = fp.att_src != 2 || threadIdx.x < kNumClasses;      // static_w holds 19 values
+      s_w[threadIdx.x] = (w && table) ? w[threadIdx.x] : 1.0f;
+      s_wf[threadIdx.x] = (w && fp.depth_split) ? w[kAttStride + threadIdx.x] : 0.0f;
+    }
+    const AttRow dst = p.rows[row];
+    if (blockIdx.x == 0 && dst.weights && threadIdx.x < 2 * kAttStride) {
+      const int slot = threadIdx.x / kAttStride, c = threadIdx.x - slot * kAttStride;
+      const bool has = w && c < p.width && (slot == 0 || (fp.depth_split && fp.att_src != 2));
+      dst.weights[threadIdx.x] = has ? w[slot * kAttStride + c] : 0.0f;
+    }
+    __syncthreads();
+    if (!dst.map) continue;
+    const bool ones = w == nullptr;
+    const int plane = f == 0 ? 1 : f == 1 ? 0 : 2;      // position in the inputs: [src0, tgt, src1]
+    const uint8_t* img_f = frame_img(in, b, plane);
+    const size_t lab_off = frame_plane(in, b, plane, hw);
+    for (int gi = blockIdx.x * blockDim.x + threadIdx.x; gi < groups; gi += gridDim.x * blockDim.x) {
+      const int p0 = gi * 4;
+      float r[4] = {0.f, 0.f, 0.f, 0.f}, g[4] = {0.f, 0.f, 0.f, 0.f}, bl[4] = {0.f, 0.f, 0.f, 0.f};
+      if (need_rgb && !ones) {
+        const int h = p0 / fp.W, x = p0 - h * fp.W;
+        const uint32_t* px = reinterpret_cast<const uint32_t*>(img_f + (size_t)h * in.img_row + x * 3);
+        unpack_rgb4(__ldg(px), __ldg(px + 1), __ldg(px + 2), r, g, bl);
+      }
+      int lab[4] = {-1, -1, -1, -1};
+      if (need_lab && !ones) labels4_at(fp, lab_off, p0, lab);
+      float a[4];
+      frame_attention4(fp, fp.att_src, ones, s_w, s_wf, b, f, p0, hw, lab, r, g, bl, a);
+      *reinterpret_cast<float4*>(dst.map + p0) = make_float4(a[0], a[1], a[2], a[3]);
     }
   }
 }

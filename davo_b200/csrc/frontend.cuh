@@ -30,7 +30,7 @@ constexpr int kPackBlocksPerPair = 104;
 //   1 trajectory:       s -> (s, 1)            tgt->src1 only: what test_kitti_pose.py:143-145 composes
 //   2 trajectory+first: 0 -> (0, 0), s -> (s - 1, 1)   plus the first sample's tgt->src0
 //   3 sample units:     s -> (s, 0)            the non-shared nets take (tgt, src0, src1) at once
-__device__ __forceinline__ void pair_of_slot(int mode, int s, int* b, int* k) {
+__host__ __device__ __forceinline__ void pair_of_slot(int mode, int s, int* b, int* k) {
   if (mode == 0) { *b = s >> 1; *k = s & 1; }
   else if (mode == 1 || mode == 3) { *b = s; *k = mode == 1 ? 1 : 0; }
   else if (s == 0) { *b = 0; *k = 0; }

@@ -267,10 +267,23 @@ class DAVO(object):
         import torch
         if flow is None or seg is None:
             raise ValueError("DAVO.inference: mode='feature' reads input_flow and input_seglabel")
+        img, flow, seg, depth = self._upload(img, torch.uint8), self._upload(flow), self._upload(seg), self._upload(depth)
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        return self._features(B, as_torch, "davo_forward_features", lambda pose, table, stream: self._lib.davo_forward_features(
+            self._h, B, ptr(img), ptr(flow), ptr(seg), ptr(depth), ptr(pose), table, stream))
+
+    def _upload(self, t, dt=None):
+        """A numpy array or tensor as a contiguous tensor of dtype ``dt`` (float32 by default) on this handle's GPU."""
+        import torch
+        if t is None:
+            return None
+        return (t if _is_torch(t) else torch.as_tensor(np.ascontiguousarray(t))).to(
+            device="cuda:%d" % self.device, dtype=torch.float32 if dt is None else dt).contiguous()
+
+    def _features(self, B, as_torch, what, call):
+        """The output tensors of mode='feature' for B samples, ``call(pose, table, stream)`` on them, and the dict."""
+        import torch
         dev = "cuda:%d" % self.device
-        up = lambda t, dt: None if t is None else (t if _is_torch(t) else torch.as_tensor(np.ascontiguousarray(t))).to(
-            device=dev, dtype=dt).contiguous()
-        img, flow, seg, depth = up(img, torch.uint8), up(flow, torch.float32), up(seg, torch.float32), up(depth, torch.float32)
         H, W, c6 = self.img_height, self.img_width, self.config.cnv6_out
         if self.config.posenn_se == V.PSE_REPLACE:
             c6 = 256                                     # "cnv6" is se_block(cnv5) there (reference posenn.py:234-236)
@@ -281,10 +294,8 @@ class DAVO(object):
         seg19, segc, flowc = f32(3, B, H, W, 19), u8(3, B, H, W, 3), u8(2, B, H, W, 3)
         rot, trans = f32(B, H, W, c6), f32(B, H, W, c6)
         table = _capi.DavoFeaturesC(*(C.c_void_p(t.data_ptr()) for t in (image, att, masked, seg19, segc, flowc, rot, trans)))
-        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        self._check(self._lib.davo_forward_features(self._h, B, ptr(img), ptr(flow), ptr(seg), ptr(depth), ptr(pose),
-                                                    C.byref(table), C.c_void_p(stream)), "davo_forward_features")
+        self._check(call(pose, C.byref(table), C.c_void_p(stream)), what)
         conv = (lambda t: t) if as_torch else (lambda t: t.cpu().numpy())
         squeeze = (lambda t: t.squeeze()) if as_torch else np.squeeze        # tf.squeeze drops every unit axis (davo.py:1115)
         return {
@@ -394,7 +405,7 @@ class DAVO(object):
                 raise ValueError("DAVO.%s: %s has shape %s, expected %s" % (who, name, tuple(t.shape), want[name]))
         return N, _capi.PAIRS[pairs], depth
 
-    def inference_sequence(self, img, flow_fwd, flow_bwd, seg, depth=None, pairs='all', as_torch=False):
+    def inference_sequence(self, img, flow_fwd, flow_bwd, seg, depth=None, pairs='all', as_torch=False, mode='pose'):
         """Poses of a frame sequence -> ``{'pose': [N-2,2,6]}`` (include/davo_b200.h: davo_forward_sequence).
 
         ``img`` uint8 [N,H,W,3]; ``flow_fwd`` / ``flow_bwd`` float32 [N-1,H,W,2], entry i the flow from frame i to i+1 /
@@ -402,8 +413,28 @@ class DAVO(object):
         (s, s+1, s+2); the poses equal ``inference`` on ``sequence_to_triplets`` of the same frames, bit for bit.
         ``flow_fwd`` may be None under ``pairs='trajectory'`` for the shared nets.  numpy arrays take the host path
         (each frame crosses PCIe once), CUDA tensors the device path; ``-batch_norm`` uploads and takes the device
-        path.  A long sequence continues with a call that starts two frames before the previous one ended."""
+        path.  A long sequence continues with a call that starts two frames before the previous one ended.
+
+        ``mode='feature'`` (include/davo_b200.h: davo_forward_sequence_features) returns the nested dict of
+        ``inference(mode='feature')`` for the N-2 samples, the same bits as that call on ``sequence_to_triplets`` of the
+        frames; it computes every pair (``pairs='all'``), reads both flows and the labels, and takes one pass (2(N-2),
+        or N-2 for the non-shared nets, <= micro_batch).  numpy inputs are uploaded."""
+        if mode not in ('pose', 'feature'):
+            raise NotImplementedError("davo_b200: inference_sequence mode %r is not built ('pose', 'feature')" % (mode,))
+        if mode == 'feature' and pairs != 'all':
+            raise ValueError("DAVO.inference_sequence: mode='feature' computes every pair (pairs='all')")
         N, sel, depth = self._sequence_args(img, flow_fwd, flow_bwd, seg, depth, pairs, "inference_sequence")
+        if mode == 'feature':
+            if flow_fwd is None or flow_bwd is None or seg is None:
+                raise ValueError("DAVO.inference_sequence: mode='feature' reads flow_fwd, flow_bwd and seg")
+            import torch
+            img, seg, depth = self._upload(img, torch.uint8), self._upload(seg), self._upload(depth)
+            flow_fwd, flow_bwd = self._upload(flow_fwd), self._upload(flow_bwd)
+            ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+            return self._features(N - 2, as_torch, "davo_forward_sequence_features",
+                                  lambda pose, table, stream: self._lib.davo_forward_sequence_features(
+                                      self._h, N, ptr(img), ptr(flow_fwd), ptr(flow_bwd), ptr(seg), ptr(depth), ptr(pose),
+                                      table, stream))
         if not _is_torch(img) and not self.config.batch_norm:
             return self.inference_sequence_async(img, flow_fwd, flow_bwd, seg, depth, pairs, _block=True).result()
         import torch
@@ -544,6 +575,24 @@ class DAVO(object):
                         "davo_odometry_load_many")
         return [Odometry._adopt(self, C.c_void_p(out[i]), h) for i, h in enumerate(hdrs)]
 
+    def _att_shape(self):
+        """(slots, width) of a frame's attention weights: the far table is slot 1 under -se_flow_on_depthseg_seplayers;
+        the width is that of get_intermediate('att_weights:<k>')."""
+        c = self.config
+        width = 19 if not c.pixel_map else 3 if c.pixel_map == 2 else 3 if c.att_src == 4 else 1 if c.att_src == 5 else 21
+        return (2 if c.depth_split else 1), width
+
+    def _att_host(self, n_t):
+        return (np.empty((n_t, self.img_height, self.img_width), np.float32), np.empty((n_t, 2, 24), np.float32))
+
+    def _result(self, pose, traj, frames, amap=None, aw=None):
+        """A push's dict; with attention, the maps and the weight rows trimmed to the variant's slots and width."""
+        out = {'pose': pose, 'trajectory': traj, 'frames': frames}
+        if amap is not None:
+            slots, width = self._att_shape()
+            out['attention'], out['att_weights'] = amap, aw[:, :slots, :width]
+        return out
+
     def _many_args(self, sessions, img, flow_fwd, flow_bwd, seg, depth, host, who):
         """The list and session checks of the batched pushes; returns the sessions, each entry's inputs and its
         (k, n_samples, n_traj)."""
@@ -574,12 +623,13 @@ class DAVO(object):
             counts.append((k,) + od._counts(k))
         return sessions, ins, counts
 
-    def odometry_push_many(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None):
+    def odometry_push_many(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None, attention=False):
         """One push on each of several device sessions of this handle, in one forward pass (include/davo_b200.h:
         davo_odometry_push_many).  ``img``, ``flow_fwd``, ``flow_bwd``, ``seg`` and ``depth`` are lists aligned with
         ``sessions``, entry i holding the CUDA tensors ``sessions[i].push`` takes (None, or a list of None, where no
         entry has one).  Returns the list of the dicts ``push`` returns; the results are the bits of pushing each
-        session alone, in list order.  Enqueued on the current stream."""
+        session alone, in list order.  Enqueued on the current stream.  ``attention=True`` adds each session's
+        ``'attention'`` and ``'att_weights'`` (``Odometry.push``), with one extra launch per micro-batch in all."""
         sessions, ins, counts = self._many_args(sessions, img, flow_fwd, flow_bwd, seg, depth, False, "odometry_push_many")
         n = len(sessions)
         for i, (od, x) in enumerate(zip(sessions, ins)):     # where the tensors live
@@ -594,25 +644,35 @@ class DAVO(object):
         cols = [arr([ptr(x[j]) for x in ins]) for j in range(5)]
         ns, nt = (C.c_int * n)(), (C.c_int * n)()
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        self._check(self._lib.davo_odometry_push_many(
-            n, arr([od._o.value for od in sessions]), (C.c_int * n)(*[c[0] for c in counts]), *cols,
-            arr([ptr(o[0]) for o in outs]), arr([ptr(o[1]) for o in outs]), ns, nt, vp(stream)),
-            "davo_odometry_push_many")
+        head = (n, arr([od._o.value for od in sessions]), (C.c_int * n)(*[c[0] for c in counts]), *cols,
+                arr([ptr(o[0]) for o in outs]), arr([ptr(o[1]) for o in outs]))
+        atts = [(None, None)] * n
+        if attention:
+            atts = [(torch.empty((c[2], self.img_height, self.img_width), dtype=torch.float32, device=dev),
+                     torch.empty((c[2], 2, 24), dtype=torch.float32, device=dev)) for c in counts]
+            table = (_capi.DavoOdometryAttentionC * n)(*[_capi.DavoOdometryAttentionC(ptr(a), ptr(w)) for a, w in atts])
+            self._check(self._lib.davo_odometry_push_many_attention(*head, table, ns, nt, vp(stream)),
+                        "davo_odometry_push_many_attention")
+        else:
+            self._check(self._lib.davo_odometry_push_many(*head, ns, nt, vp(stream)), "davo_odometry_push_many")
         res = []
-        for od, (k, _, _), (pose, traj), m in zip(sessions, counts, outs, nt):
-            res.append({'pose': pose, 'trajectory': traj, 'frames': range(od._posed, od._posed + m)})
+        for od, (k, _, _), (pose, traj), m, (a, w) in zip(sessions, counts, outs, nt, atts):
+            res.append(self._result(pose, traj, range(od._posed, od._posed + m), a, w))
             od._pushed += k
             od._posed += m
         return res
 
-    def odometry_push_many_host(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None):
+    def odometry_push_many_host(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None, attention=False):
         """One push on each of several host sessions of this handle, in one forward pass (include/davo_b200.h:
         davo_odometry_push_many_host): many cameras whose frames arrive in host memory.  The lists are those of
         ``odometry_push_many``, holding the numpy arrays ``sessions[i].push`` takes.  Returns the list of the dicts
-        ``push`` returns; the results are the bits of pushing each session alone, in list order."""
-        return self.odometry_push_many_host_async(sessions, img, flow_fwd, flow_bwd, seg, depth, _block=True).result()
+        ``push`` returns; the results are the bits of pushing each session alone, in list order.  ``attention`` as
+        for ``odometry_push_many``, as numpy arrays."""
+        return self.odometry_push_many_host_async(sessions, img, flow_fwd, flow_bwd, seg, depth, _block=True,
+                                                  attention=attention).result()
 
-    def odometry_push_many_host_async(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None, _block=False):
+    def odometry_push_many_host_async(self, sessions, img, flow_fwd, flow_bwd, seg=None, depth=None, _block=False,
+                                      attention=False):
         """``odometry_push_many_host`` without waiting: returns a handle whose ``.result()`` gives the list of dicts.
         The results land in each session's page-locked ring slot (as ``Odometry.push_async``); the inputs must stay
         unmodified until ``.result()``.  Up to 8 calls may be in flight."""
@@ -623,22 +683,28 @@ class DAVO(object):
         dts = (np.uint8, np.float32, np.float32, np.float32, np.float32)
         ins = [tuple(conv(a, dt) for a, dt in zip(x, dts)) for x in ins]
         if _block:
-            outs = [(np.zeros((ns, 2, 6), np.float32), np.empty((nt, 4, 4), np.float64)) for _, ns, nt in counts]
+            outs = [(np.zeros((ns, 2, 6), np.float32), np.empty((nt, 4, 4), np.float64))
+                    + (self._att_host(nt) if attention else (None, None)) for _, ns, nt in counts]
         else:
-            outs = [od._ring_slot(ns, nt) for od, (_, ns, nt) in zip(sessions, counts)]
+            outs = [od._ring_slot(ns, nt, attention) for od, (_, ns, nt) in zip(sessions, counts)]
         vp = C.c_void_p
         hp = lambda a: a.ctypes.data if a is not None and a.size else None
         arr = lambda vals: (vp * n)(*vals)
         cols = [arr([hp(x[j]) for x in ins]) for j in range(5)]
         ns, nt = (C.c_int * n)(), (C.c_int * n)()
         ticket = C.c_longlong(0)
-        self._check(self._lib.davo_odometry_push_many_host(
-            n, arr([od._o.value for od in sessions]), (C.c_int * n)(*[c[0] for c in counts]), *cols,
-            arr([hp(o[0]) for o in outs]), arr([hp(o[1]) for o in outs]), ns, nt, None,
-            None if _block else C.byref(ticket)), "davo_odometry_push_many_host")
+        head = (n, arr([od._o.value for od in sessions]), (C.c_int * n)(*[c[0] for c in counts]), *cols,
+                arr([hp(o[0]) for o in outs]), arr([hp(o[1]) for o in outs]))
+        tail = (ns, nt, None, None if _block else C.byref(ticket))
+        if attention:
+            table = (_capi.DavoOdometryAttentionC * n)(*[_capi.DavoOdometryAttentionC(hp(o[2]), hp(o[3])) for o in outs])
+            self._check(self._lib.davo_odometry_push_many_host_attention(*head, table, *tail),
+                        "davo_odometry_push_many_host_attention")
+        else:
+            self._check(self._lib.davo_odometry_push_many_host(*head, *tail), "davo_odometry_push_many_host")
         res = []
-        for od, (k, _, _), (pose, traj), m in zip(sessions, counts, outs, nt):
-            res.append(Odometry._Pending(None, {'pose': pose, 'trajectory': traj, 'frames': range(od._posed, od._posed + m)}))
+        for od, (k, _, _), o, m in zip(sessions, counts, outs, nt):
+            res.append(Odometry._Pending(None, self._result(o[0], o[1], range(od._posed, od._posed + m), o[2], o[3])))
             od._pushed += k
             od._posed += m
         return DAVO._PendingMany(self, None if _block else ticket.value, res, None if _block else ins)
@@ -655,8 +721,7 @@ class DAVO(object):
                 s._check(s._lib.davo_host_wait(s._h, self._ticket), "davo_host_wait")
                 self._ticket, self._keep = None, None
                 for p in self._pending:                      # own copies: the pinned ring slots are reused
-                    p._out = {'pose': np.array(p._out['pose']), 'trajectory': np.array(p._out['trajectory']),
-                              'frames': p._out['frames']}
+                    p._out = {k: (v if k == 'frames' else np.array(v)) for k, v in p._out.items()}
             return [p.result() for p in self._pending]
 
     def bind_host_numa(self):
@@ -814,55 +879,85 @@ class Odometry(object):
                                       and t.dtype == dt and t.is_contiguous()):
                 raise ValueError("%s: %s must be a contiguous %s tensor on %s" % (who, name, dt, dev))
 
-    def _call(self, k, ins, pose, traj, stream, ticket):
+    def _call(self, k, ins, pose, traj, stream, ticket, att=None):
         s = self._system
         ns, nt = C.c_int(0), C.c_int(0)
-        s._check(s._lib.davo_odometry_push(self._o, k, *ins, pose, traj, C.byref(ns), C.byref(nt), stream, ticket),
-                 "davo_odometry_push")
+        if att is None:
+            s._check(s._lib.davo_odometry_push(self._o, k, *ins, pose, traj, C.byref(ns), C.byref(nt), stream, ticket),
+                     "davo_odometry_push")
+        else:
+            s._check(s._lib.davo_odometry_push_attention(self._o, k, *ins, pose, traj, C.byref(att), C.byref(ns),
+                                                         C.byref(nt), stream, ticket), "davo_odometry_push_attention")
         frames = range(self._posed, self._posed + nt.value)
         self._pushed += k
         self._posed += nt.value
         return frames
 
-    def push_async(self, img, flow_fwd, flow_bwd, seg=None, depth=None, _block=False):
+    def push_async(self, img, flow_fwd, flow_bwd, seg=None, depth=None, _block=False, attention=False):
         k, depth = self._args(img, flow_fwd, flow_bwd, seg, depth)
         n_s, n_t = self._counts(k)
+        s = self._system
         if not self._host:
             import torch
-            dev = "cuda:%d" % self._system.device
+            dev = "cuda:%d" % s.device
             self._check_device(img, flow_fwd, flow_bwd, seg, depth)
             pose = torch.zeros((n_s, 2, 6), dtype=torch.float32, device=dev)
             traj = torch.empty((n_t, 4, 4), dtype=torch.float64, device=dev)
             ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None and t.numel() else None
-            stream = torch.cuda.current_stream(self._system.device).cuda_stream
+            amap = aw = att = None
+            if attention:
+                amap = torch.empty((n_t, s.img_height, s.img_width), dtype=torch.float32, device=dev)
+                aw = torch.empty((n_t, 2, 24), dtype=torch.float32, device=dev)
+                att = _capi.DavoOdometryAttentionC(ptr(amap), ptr(aw))
+            stream = torch.cuda.current_stream(s.device).cuda_stream
             frames = self._call(k, [ptr(t) for t in (img, flow_fwd, flow_bwd, seg, depth)], ptr(pose), ptr(traj),
-                                C.c_void_p(stream), None)
-            return Odometry._Pending(None, {'pose': pose, 'trajectory': traj, 'frames': frames}, None)
+                                C.c_void_p(stream), None, att)
+            return Odometry._Pending(None, s._result(pose, traj, frames, amap, aw), None)
         arr = lambda a, dt: None if a is None else np.ascontiguousarray(a, dtype=dt)
         ins = (arr(img, np.uint8), arr(flow_fwd, np.float32), arr(flow_bwd, np.float32), arr(seg, np.float32),
                arr(depth, np.float32))
         hp = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None and a.size else None
         if _block:
             pose, traj = np.zeros((n_s, 2, 6), np.float32), np.empty((n_t, 4, 4), np.float64)
-            frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, None)
-            return Odometry._Pending(None, {'pose': pose, 'trajectory': traj, 'frames': frames}, None)
-        pose, traj = self._ring_slot(n_s, n_t)
+            amap, aw = s._att_host(n_t) if attention else (None, None)
+        else:
+            pose, traj, amap, aw = self._ring_slot(n_s, n_t, attention)
+        att = _capi.DavoOdometryAttentionC(hp(amap), hp(aw)) if attention else None
         ticket = C.c_longlong(0)
-        frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, C.byref(ticket))
-        return Odometry._Pending(self._system, {'pose': pose, 'trajectory': traj, 'frames': frames}, ticket.value, ins)
+        frames = self._call(k, [hp(a) for a in ins], hp(pose), hp(traj), None, None if _block else C.byref(ticket), att)
+        out = s._result(pose, traj, frames, amap, aw)
+        if _block:
+            return Odometry._Pending(None, out, None)
+        return Odometry._Pending(s, out, ticket.value, ins)
 
-    def _ring_slot(self, n_s, n_t):
-        """The next page-locked (pose, trajectory) output pair of an asynchronous host push, single or batched."""
+    def _ring_slot(self, n_s, n_t, attention=False):
+        """The next page-locked (pose, trajectory, map, weights) outputs of an asynchronous host push, single or batched;
+        map and weights are None unless asked for.  The attention slots are allocated by the first push that asks
+        (a 128x416 map is 213 KB: a ring of them for every session would pin far more than the poses need)."""
         import torch
         if self._ring is None:                      # page-locked results, one slot per call that can be in flight
             self._ring = [(torch.empty((self.max_push, 2, 6), dtype=torch.float32).pin_memory(),
                            torch.empty((self.max_push + 2, 4, 4), dtype=torch.float64).pin_memory()) for _ in range(8)]
-        slot = self._ring[self._ring_n % 8]
+        i = self._ring_n % 8
         self._ring_n += 1
-        return slot[0][:n_s].numpy(), slot[1][:n_t].numpy()
+        slot = self._ring[i]
+        amap = aw = None
+        if attention:
+            s = self._system
+            if getattr(self, "_att_ring", None) is None:
+                self._att_ring = [(torch.empty((self.max_push + 2, s.img_height, s.img_width), dtype=torch.float32).pin_memory(),
+                                   torch.empty((self.max_push + 2, 2, 24), dtype=torch.float32).pin_memory())
+                                  for _ in range(8)]
+            amap, aw = self._att_ring[i][0][:n_t].numpy(), self._att_ring[i][1][:n_t].numpy()
+        return slot[0][:n_s].numpy(), slot[1][:n_t].numpy(), amap, aw
 
-    def push(self, img, flow_fwd, flow_bwd, seg=None, depth=None):
-        return self.push_async(img, flow_fwd, flow_bwd, seg, depth, _block=True).result()
+    def push(self, img, flow_fwd, flow_bwd, seg=None, depth=None, attention=False):
+        """See the class.  ``attention=True`` adds each posed frame's attention (include/davo_b200.h:
+        davo_odometry_push_attention): ``'attention'`` [n_t,H,W], the map of the frame of ``trajectory[i]`` as the pair
+        that placed it masks it, and ``'att_weights'`` [n_t,slots,width], the table(s) it was computed from (slots 2
+        under -se_flow_on_depthseg_seplayers, else 1; width that of ``get_intermediate('att_weights:<k>')``; zeros for
+        a map of ones).  CUDA tensors for device sessions, numpy for host sessions."""
+        return self.push_async(img, flow_fwd, flow_bwd, seg, depth, _block=True, attention=attention).result()
 
     class _Pending(object):
         def __init__(self, system, out, ticket=None, keep=None):
@@ -873,8 +968,8 @@ class Odometry(object):
                 s = self._system
                 s._check(s._lib.davo_host_wait(s._h, self._ticket), "davo_host_wait")
                 self._ticket, self._keep = None, None
-                self._out = {'pose': np.array(self._out['pose']), 'trajectory': np.array(self._out['trajectory']),
-                             'frames': self._out['frames']}           # own copies: the pinned ring slot is reused
+                # own copies: the pinned ring slot is reused
+                self._out = {k: (v if k == 'frames' else np.array(v)) for k, v in self._out.items()}
             return self._out
 
     def move_to(self, system):

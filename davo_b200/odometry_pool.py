@@ -72,11 +72,11 @@ class OdometryPool(object):
         """Camera ``cam``'s ``Odometry`` session."""
         return self._cams[cam]
 
-    def push(self, ids, img, flow_fwd, flow_bwd, seg=None, depth=None):
+    def push(self, ids, img, flow_fwd, flow_bwd, seg=None, depth=None, attention=False):
         """One push on each camera of ``ids``: the inputs are lists aligned with ``ids``, entry j holding what
         ``Odometry.push`` takes for camera ``ids[j]`` (None, or a list of None, where no camera has one).  One batched
         push per handle, all queued before any is waited for; returns the dicts ``Odometry.push`` returns, in ``ids``
-        order."""
+        order (with each posed frame's ``'attention'`` and ``'att_weights'`` when ``attention`` is true)."""
         ids = list(ids)
         n = len(ids)
         lists = {}
@@ -99,9 +99,9 @@ class OdometryPool(object):
             args = [[self._cams[ids[j]] for j in pos]] + [[lists[name][j] for j in pos] for name in _INPUTS]
             with torch.cuda.device(s.device):            # the library switches devices; torch's current one is restored
                 if self._host:
-                    pending.append((pos, s.odometry_push_many_host_async(*args)))
+                    pending.append((pos, s.odometry_push_many_host_async(*args, attention=attention)))
                 else:
-                    for j, r in zip(pos, s.odometry_push_many(*args)):
+                    for j, r in zip(pos, s.odometry_push_many(*args, attention=attention)):
                         out[j] = r
         for pos, p in pending:
             for j, r in zip(pos, p.result()):

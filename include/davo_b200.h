@@ -224,6 +224,16 @@ int davo_forward_sequence(davo_ctx*, int n_frames, int pairs, const uint8_t* img
 int davo_forward_sequence_host(davo_ctx*, int n_frames, int pairs, const uint8_t* img_u8, const float* flow_fwd,
                                const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
                                void* cuda_stream, long long* ticket);
+/* davo_forward_sequence_features: mode='feature' (davo_forward_features) on a frame sequence in the device layout of
+ *   davo_forward_sequence, always DAVO_PAIRS_ALL: B = n_frames - 2 samples, the same davo_features table and output
+ *   layouts as davo_forward_features with that B.  Every output is the same bits as davo_forward_features on
+ *   davo_b200.sequence_to_triplets of the same frames (the flow colouring's largest magnitude is over the same B
+ *   samples).  One pass, as davo_forward_features: 2B (B for posenn 2-5) <= micro_batch; a longer sequence is refused
+ *   naming the limit.  Argument errors are those of davo_forward_sequence plus the output table's (a NULL table, a
+ *   flow colouring without both flows, label outputs without seg). */
+int davo_forward_sequence_features(davo_ctx*, int n_frames, const uint8_t* img_u8, const float* flow_fwd,
+                                   const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                                   const davo_features* out, void* cuda_stream);
 
 /* --- online odometry sessions ---
  * A camera loop: push frames as they arrive, get each frame's absolute pose, composed on the device.  A session
@@ -305,6 +315,44 @@ int davo_odometry_push_many_host(int n, davo_odometry* const* sessions, const in
                                  const float* const* flow_fwd, const float* const* flow_bwd, const float* const* seg,
                                  const float* const* depth, float* const* pose_out, double* const* traj_out,
                                  int* n_samples, int* n_traj, void* cuda_stream, long long* ticket);
+/* --- each posed frame's attention ---
+ * The _attention forms of the three pushes return, next to traj_out, the attention of each frame whose pose became
+ * known.  Row i belongs to the frame of traj_out[i]:
+ *   map      float [n_traj,H,W]   the frame's attention map as the pair that placed it in the trajectory masks it:
+ *            frame 0 as src0 of sample 0, frame 1 as the target of sample 0 (after the target override; usually all
+ *            ones), frame s+2 as src1 of sample s.  Bit for bit the planes attention[1][0], attention[0][0] and
+ *            attention[2][s] of davo_forward_features on the triplets of the whole stream, in either pair mode.
+ *   weights  float [n_traj,2,24]  row 0: the table the map was computed from -- the 19 class weights, or a per-pixel
+ *            source's excitation (the width of davo_get_intermediate("att_weights:<k>"): 19, 3, 1, 3 or 21); row 1:
+ *            the far table under -se_flow_on_depthseg_seplayers; the static table for a static variant; entries past
+ *            the width are 0, and a frame whose map is all ones (no attention source, or the forced target map) has
+ *            all zeros.
+ * Either pointer may be NULL (not written), not both where rows are due; each is 16-byte aligned.  Device sessions take
+ * device buffers, host sessions host buffers (page-locked when a ticket is passed), like traj_out; a host push's
+ * davo_last_host_copy_bytes counts them in d2h.  The maps are written by one extra launch per micro-batch of the
+ * forward, from the pass's own attention weights and inputs: every pose, trajectory and count is the bits of the same
+ * push without attention, and pushes with and without attention mix freely on a session.  The plain entry points are
+ * the att == NULL case.  A refused call (a bad att entry is named with its session index) changes no session. */
+typedef struct davo_odometry_attention {
+  float* map;        /* [n_traj, H, W]; NULL: not written */
+  float* weights;    /* [n_traj, 2, 24]; NULL: not written */
+} davo_odometry_attention;
+int davo_odometry_push_attention(davo_odometry*, int k, const uint8_t* img, const float* flow_fwd,
+                                 const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                                 double* traj_out, const davo_odometry_attention* att, int* n_samples, int* n_traj,
+                                 void* cuda_stream, long long* ticket);
+/* att: n entries, a host array (NULL: none written) */
+int davo_odometry_push_many_attention(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
+                                      const float* const* flow_fwd, const float* const* flow_bwd,
+                                      const float* const* seg, const float* const* depth, float* const* pose_out,
+                                      double* const* traj_out, const davo_odometry_attention* att, int* n_samples,
+                                      int* n_traj, void* cuda_stream);
+int davo_odometry_push_many_host_attention(int n, davo_odometry* const* sessions, const int* k,
+                                           const uint8_t* const* img, const float* const* flow_fwd,
+                                           const float* const* flow_bwd, const float* const* seg,
+                                           const float* const* depth, float* const* pose_out,
+                                           double* const* traj_out, const davo_odometry_attention* att,
+                                           int* n_samples, int* n_traj, void* cuda_stream, long long* ticket);
 int davo_odometry_reset(davo_odometry*);
 int davo_odometry_frames(const davo_odometry*, long long* pushed, long long* posed);
 void davo_odometry_destroy(davo_odometry*);
