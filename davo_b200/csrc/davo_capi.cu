@@ -244,7 +244,8 @@ struct davo_ctx {
   float *d_bn_mean = nullptr, *d_bn_rstd = nullptr;
   void* d_traj_scratch = nullptr;         // davo_compose_trajectory / davo_kitti_errors: relative motions, distances, segments
   size_t traj_scratch_bytes = 0;
-  float flow16_frac = 0.75f;              // share of a chunk's samples converted on the CPU (the rest keeps the copy engine busy)
+  float flow16_frac = 0.75f;              // share of a chunk's samples (of a push's flow entries) converted on the CPU (the
+                                          // rest keeps the copy engine busy)
   HostPool* pool = nullptr;
   bool host_seg8 = true;
   int s_chunk = 0;                  // samples per staging buffer
@@ -264,9 +265,10 @@ struct davo_ctx {
   uint8_t* q_img[2] = {}; uint8_t* q_seg8[2] = {}; float *q_seg[2] = {}, *q_depth[2] = {};
   cudaEvent_t ev_q_done[2] = {};    // the call that last used set i has finished reading it
   long long q_calls = 0;
-  // davo_odometry_push_many: one stacked-triplet staging batch of max_batch samples (input_view.cuh: stacked_view) and
-  // its poses, allocated by the first batched push; the per-call session and sample descriptors go from a pinned ring
-  // slot to its device twin in one copy, and a slot is refilled once the call that used it has finished
+  // odometry pushes: one stacked-triplet staging batch of max_batch samples (input_view.cuh: stacked_view) and
+  // its poses, allocated by the first push of any kind; the per-call session and sample descriptors and the attention
+  // unit table and rows go from a pinned ring slot to its device twin in one copy, and a slot is refilled once the call
+  // that used it has finished
   uint8_t *m_img = nullptr, *m_lab = nullptr;
   float *m_depth = nullptr, *m_flow = nullptr, *m_pose = nullptr;
   static constexpr int kManyRing = 4;
@@ -274,11 +276,12 @@ struct davo_ctx {
   size_t m_desc_cap[kManyRing] = {};
   cudaEvent_t m_ev[kManyRing] = {};
   long long m_calls = 0;
-  // davo_odometry_push_many_host: two arrivals sets (device; pinned byte labels), the caller's frames and flow entries
-  // of a call at the indices the stage kernel reads them; set i is refilled once the stage and carry kernels of the call
-  // that last used it have finished (a_done[i]), so that the copies of call t+1 run under the forward of call t
-  uint8_t* a_dev[2] = {}; uint8_t* a_hlab[2] = {};
-  size_t a_dev_cap[2] = {}, a_hlab_cap[2] = {};
+  // host sessions' pushes: two arrivals sets (device; pinned byte labels and binary16 flow entries), the caller's
+  // frames and flow entries of a call at the indices the stage kernel reads them; set i is refilled once the stage and
+  // carry kernels of the call that last used it have finished (a_done[i]), so that the copies of call t+1 run under the
+  // forward of call t
+  uint8_t* a_dev[2] = {}; uint8_t* a_pin[2] = {};
+  size_t a_dev_cap[2] = {}, a_pin_cap[2] = {};
   cudaEvent_t a_copied[2] = {}, a_done[2] = {};
   long long a_calls = 0;
   float* m_hpose = nullptr;           // the pose rows of each session's push, [max_batch,2,6], copied to the host from here
@@ -295,16 +298,11 @@ struct davo_ctx {
   float* d_wheel = nullptr;         // Middlebury colour wheel / 255
   unsigned int* d_maxrad = nullptr; // largest flow magnitude per source frame
   // attention outputs of odometry pushes (features.cuh: attention_out_kernel).  While a push that asked for them runs
-  // its forward, att_units / att_rows are the device unit table of the forward (or of the host chunk) being launched
-  // and its destination rows; NULL otherwise.  The tables go from a pinned ring slot to its device twin in one copy, a
-  // slot refilled once the call that used it has finished.  Host sessions' maps and weights are written to att_stage
-  // and copied back on the caller's stream, like s_pose.
+  // its forward, att_units / att_rows are the device unit table of the forward being launched and its destination
+  // rows (in the call's m_ddesc slot); NULL otherwise.  Host sessions' maps and weights are written to att_stage and
+  // copied back on the caller's stream.
   const int4* att_units = nullptr;
   const AttRow* att_rows = nullptr;
-  void *att_hdesc[kManyRing] = {}, *att_ddesc[kManyRing] = {};
-  size_t att_desc_cap[kManyRing] = {};
-  cudaEvent_t att_ev[kManyRing] = {};
-  long long att_calls = 0;
   float* att_stage = nullptr;
   size_t att_stage_cap = 0;
   // pose all-gather (comm.cuh): the handle's own communicator, if davo_comm_create made one
@@ -1459,16 +1457,11 @@ extern "C" void davo_destroy(davo_ctx* ctx) {
     if (ctx->q_depth[i]) cudaFree(ctx->q_depth[i]);
     if (ctx->ev_q_done[i]) cudaEventDestroy(ctx->ev_q_done[i]);
     if (ctx->a_dev[i]) cudaFree(ctx->a_dev[i]);
-    if (ctx->a_hlab[i]) cudaFreeHost(ctx->a_hlab[i]);
+    if (ctx->a_pin[i]) cudaFreeHost(ctx->a_pin[i]);
     if (ctx->a_copied[i]) cudaEventDestroy(ctx->a_copied[i]);
     if (ctx->a_done[i]) cudaEventDestroy(ctx->a_done[i]);
   }
   cudaFree(ctx->m_hpose);
-  for (int i = 0; i < davo_ctx::kManyRing; ++i) {
-    if (ctx->att_hdesc[i]) cudaFreeHost(ctx->att_hdesc[i]);
-    if (ctx->att_ddesc[i]) cudaFree(ctx->att_ddesc[i]);
-    if (ctx->att_ev[i]) cudaEventDestroy(ctx->att_ev[i]);
-  }
   cudaFree(ctx->att_stage);
   cudaFree(ctx->b_stage); cudaFree(ctx->b_ddesc);
   if (ctx->b_hdesc) cudaFreeHost(ctx->b_hdesc);
@@ -2135,23 +2128,11 @@ int host_done(davo_ctx* ctx, cudaStream_t st, long long* ticket) {
   return 0;
 }
 
-// Poses of a host call back to the caller's memory, and an odometry push's n_traj absolute poses from traj_dev;
-// blocking, or the asynchronous form's ticket.
-// `att`: a push's maps and weights rows from the device staging (att_maps, att_weights) to the caller's host buffers.
-int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket, const double* traj_dev = nullptr,
-                double* traj_out = nullptr, int n_traj = 0, const davo_odometry_attention* att = nullptr,
-                const float* att_maps = nullptr, const float* att_weights = nullptr) {
+// Poses of a host call back to the caller's memory; blocking, or the asynchronous form's ticket.
+int host_finish(davo_ctx* ctx, int B, float* pose_out, cudaStream_t st, long long* ticket) {
   if (B > 0) CU_OK(cudaMemcpyAsync(pose_out, ctx->s_pose, (size_t)12 * 4 * B, cudaMemcpyDeviceToHost, st));
-  if (n_traj > 0) CU_OK(cudaMemcpyAsync(traj_out, traj_dev, (size_t)16 * 8 * n_traj, cudaMemcpyDeviceToHost, st));
-  long long att_bytes = 0;
-  if (att && n_traj > 0) {
-    const size_t mb = (size_t)ctx->cfg.H * ctx->cfg.W * 4 * n_traj, wb = (size_t)2 * 24 * 4 * n_traj;
-    if (att->map) CU_OK(cudaMemcpyAsync(att->map, att_maps, mb, cudaMemcpyDeviceToHost, st));
-    if (att->weights) CU_OK(cudaMemcpyAsync(att->weights, att_weights, wb, cudaMemcpyDeviceToHost, st));
-    att_bytes = (att->map ? (long long)mb : 0) + (att->weights ? (long long)wb : 0);
-  }
   if (int rc = host_done(ctx, st, ticket)) return rc;
-  ctx->last_d2h = (long long)12 * 4 * B + (long long)16 * 8 * n_traj + att_bytes;
+  ctx->last_d2h = (long long)12 * 4 * B;
   return 0;
 }
 
@@ -2298,26 +2279,20 @@ static int forward_host_impl(davo_ctx* ctx, int B, int pairs, const uint8_t* img
   return 0;
 }
 
-// An online odometry session (include/davo_b200.h: davo_odometry_*).  A push of k frames runs as a sequence call over
-// a virtual sequence: the session's last `head` (<= 2) frames, then the k new ones.  Virtual frame v is global frame
-// g0 + v, and every sample of that call is new.  The carried state lives in the session's own buffers, because other
-// calls on the handle reuse the handle's frame sets and staging slots.
+// An online odometry session (include/davo_b200.h: davo_odometry_*).  A push of k frames computes the samples of a
+// virtual sequence: the session's last `head` (<= 2) frames, then the k new ones.  Virtual frame v is global frame
+// g0 + v, and every sample of that push is new.  The carried state lives in the session's own buffers; the frames of a
+// push are staged in the handle's buffers (odometry_push_many_impl).
 struct davo_odometry {
   davo_ctx* ctx = nullptr;
   int max_push = 0, pairs = DAVO_PAIRS_TRAJECTORY;
   bool host = true;
   long long pushed = 0, posed = 0;               // frames pushed; frames whose absolute pose has been written
-  // frame sets of max_push + 2 frames, in the form the passes read (labels as bytes on the host path with byte labels);
-  // two, so that a host push's copies can run under the previous push
-  uint8_t* q_img[2] = {}; uint8_t* q_seg8[2] = {}; float *q_seg[2] = {}, *q_depth[2] = {};
-  cudaEvent_t ev_q_done[2] = {};
-  long long q_calls = 0;
-  // carried state: the last two frames (same forms as a set), the last flow_fwd entry when a later sample reads it, the
-  // last absolute pose
+  // carried state: the last two frames (labels as bytes in host sessions with byte labels, else as floats), the last
+  // flow_fwd entry when a later sample reads it, the last absolute pose
   uint8_t* c_img = nullptr; uint8_t* c_seg8 = nullptr; float *c_seg = nullptr, *c_depth = nullptr, *c_fwd = nullptr;
   double* d_P = nullptr;
   Mat4 *d_rel = nullptr, *d_traj = nullptr;      // this push's relative motions; a host push's absolute poses
-  float* d_fwd = nullptr;                        // device pushes: the carried flow_fwd entry followed by the pushed ones
   int head() const { return (int)std::min<long long>(pushed, 2); }
 };
 
@@ -2326,22 +2301,10 @@ namespace {
 std::mutex g_odo_mutex;
 std::set<davo_odometry*> g_odo_live;             // sessions not yet destroyed (a push on any other pointer is refused)
 
-// One push as a sequence call: n_frames virtual frames of which frames [0, head) are carried, flow entries e >= fe of
-// the caller's arrays are virtual entries e (fe = 1: virtual flow_fwd entry 0 is the carried one).
-struct OdoPush {
-  davo_odometry* o;
-  int head, fe;
-  long long g0;
-  double* traj_out;
-  int n_traj;
-  const davo_odometry_attention* att;   // each posed frame's map and weights, or NULL
-};
-
 // ---- each posed frame's attention (include/davo_b200.h: davo_odometry_attention) ----
 // Row r of a push's outputs is the frame of traj_out[r]: with sample 0 of the stream, frame 0 (src0 of sample 0) and
 // frame 1 (its target), then frame s+2, src1 of sample s.  attention_out_kernel writes the rows through a unit table:
-// the only code that knows how a single push, the chunks of a host push and the staging of a batched push order their
-// units.
+// the only code that knows how the staging of a push orders its units.
 
 // Where view sample b's frames go: the row of its src1 frame, and whether it opens its stream (its src0 and target then
 // take the two rows before), or row -1 when no frame of it has a row.
@@ -2365,37 +2328,6 @@ void att_unit_table(std::vector<int4>& out, int mode, int nsel, F sample_of) {
     }
     out.push_back(e);
   }
-}
-
-// The tables of a call to the device: one copy from a pinned ring slot (refilled once the call that last used it has
-// finished), recorded as done after the call's last use on st by att_tables_done.  Returns the slot.
-int att_tables_upload(davo_ctx* ctx, const std::vector<int4>& units, const std::vector<AttRow>& rows, cudaStream_t st,
-                      const int4** d_units, const AttRow** d_rows, int* slot_out) {
-  const int slot = (int)(ctx->att_calls++ % davo_ctx::kManyRing);
-  const size_t ub = sizeof(int4) * units.size(), bytes = ub + sizeof(AttRow) * rows.size();
-  if (ctx->att_ev[slot]) CU_OK(cudaEventSynchronize(ctx->att_ev[slot]));
-  else CU_OK(cudaEventCreateWithFlags(&ctx->att_ev[slot], cudaEventDisableTiming));
-  if (ctx->att_desc_cap[slot] < bytes) {
-    const size_t cap = std::max<size_t>(bytes, 2 * ctx->att_desc_cap[slot]);
-    if (ctx->att_hdesc[slot]) { CU_OK(cudaFreeHost(ctx->att_hdesc[slot])); ctx->att_hdesc[slot] = nullptr; }
-    if (ctx->att_ddesc[slot]) { CU_OK(cudaFree(ctx->att_ddesc[slot])); ctx->att_ddesc[slot] = nullptr; }
-    ctx->att_desc_cap[slot] = 0;
-    CU_OK(cudaHostAlloc(&ctx->att_hdesc[slot], cap, cudaHostAllocDefault));
-    CU_OK(cudaMalloc(&ctx->att_ddesc[slot], cap));
-    ctx->att_desc_cap[slot] = cap;
-  }
-  uint8_t* h = static_cast<uint8_t*>(ctx->att_hdesc[slot]);
-  if (ub) memcpy(h, units.data(), ub);
-  if (!rows.empty()) memcpy(h + ub, rows.data(), bytes - ub);
-  if (bytes) CU_OK(cudaMemcpyAsync(ctx->att_ddesc[slot], h, bytes, cudaMemcpyHostToDevice, st));
-  *d_units = static_cast<const int4*>(ctx->att_ddesc[slot]);
-  *d_rows = reinterpret_cast<const AttRow*>(static_cast<const uint8_t*>(ctx->att_ddesc[slot]) + ub);
-  *slot_out = slot;
-  return 0;
-}
-int att_tables_done(davo_ctx* ctx, int slot, cudaStream_t st) {
-  CU_OK(cudaEventRecord(ctx->att_ev[slot], st));
-  return 0;
 }
 
 // The unit table in use while a forward is launched; cleared on every way out.
@@ -2427,16 +2359,23 @@ int att_stage(davo_ctx* ctx, size_t n_rows, float** maps, float** weights) {
   return 0;
 }
 
+// An input's name in a push's messages: `name[idx]` for entry idx of a batched push, `name` for a single push (-1)
+struct EntryName {
+  char s[48];
+  EntryName(const char* name, int idx) {
+    if (idx >= 0) snprintf(s, sizeof s, "%s[%d]", name, idx);
+    else snprintf(s, sizeof s, "%s", name);
+  }
+};
+
 // A session's attention entry where `n_rows` rows are due: map / weights each NULL (not written) or 16-byte aligned,
-// not both NULL.  `idx` >= 0 names the entry of a batched push.
+// not both NULL.
 int att_check(davo_ctx* ctx, const char* who, const davo_odometry_attention& a, int n_rows, int idx) {
-  char name[32];
-  if (idx >= 0) snprintf(name, sizeof name, "att[%d]", idx);
-  else snprintf(name, sizeof name, "att");
+  const EntryName name("att", idx);
   if (n_rows > 0 && !a.map && !a.weights)
-    return fail(ctx, DAVO_ERR_ARG, "%s: %s has neither map nor weights; %d row(s) are due", who, name, n_rows);
+    return fail(ctx, DAVO_ERR_ARG, "%s: %s has neither map nor weights; %d row(s) are due", who, name.s, n_rows);
   if ((reinterpret_cast<uintptr_t>(a.map) | reinterpret_cast<uintptr_t>(a.weights)) & 15)
-    return fail(ctx, DAVO_ERR_ARG, "%s: %s.%s is not 16-byte aligned", who, name,
+    return fail(ctx, DAVO_ERR_ARG, "%s: %s.%s is not 16-byte aligned", who, name.s,
                 (reinterpret_cast<uintptr_t>(a.map) & 15) ? "map" : "weights");
   return 0;
 }
@@ -2455,24 +2394,18 @@ void att_rows_of(std::vector<AttRow>& rows, float* map, float* weights, int n, s
 // final place in one of two per-call frame sets: a chunk copies the frames that the call reads and that no earlier
 // chunk copied, and the chunk's passes read the set through a sequence view.  Every copied frame or flow crosses PCIe
 // once; those that no computed pair reads are not copied.
-// An odometry push (`op`) is the same call over its virtual sequence, on the session's frame sets: the carried frames
-// are copied device to device to the head of the set, frames [0, head) count as staged, and the carried flow_fwd entry
-// stands in for the first chunk's first fwd slot.  A frame or flow entry is copied when any sample of the whole stream
-// reads it, now or in a later push, which then finds it in the carried state.
 static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, const uint8_t* img, const float* flow_fwd,
                                       const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
-                                      void* stream, long long* ticket, const OdoPush* op = nullptr) {
-  const char* who = op ? "davo_odometry_push" : ticket ? "davo_forward_sequence_host_async" : "davo_forward_sequence_host";
-  if (!op) {
-    if (int rc = check_sequence(ctx, who, n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
-    if (ctx->cfg.batch_norm)
-      return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm needs the whole batch in one pass; the chunked host entry point does not take it (copy the frames to the device and call davo_forward_sequence)", who);
-  }
+                                      void* stream, long long* ticket) {
+  const char* who = ticket ? "davo_forward_sequence_host_async" : "davo_forward_sequence_host";
+  if (int rc = check_sequence(ctx, who, n_frames, pairs, img, flow_fwd, flow_bwd, seg, depth, pose_out)) return rc;
+  if (ctx->cfg.batch_norm)
+    return fail(ctx, DAVO_ERR_ARG, "%s: -batch_norm needs the whole batch in one pass; the chunked host entry point does not take it (copy the frames to the device and call davo_forward_sequence)", who);
   const davo_config& c = ctx->cfg;
   CU_OK(cudaSetDevice(ctx->device));
   const SeqReads r = seq_reads(ctx, pairs);
   pairs = r.pairs;
-  const int B = std::max(0, n_frames - 2);
+  const int B = n_frames - 2;
   const size_t hw = (size_t)c.H * c.W, fl = hw * 2;               // pixels per frame, floats per flow entry
   const int cs = host_setup(ctx, who);
   if (cs < 0) return cs;
@@ -2480,38 +2413,20 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
   cudaStream_t cp = ctx->copy_stream;
   if (int rc = host_order_first_call(ctx, st)) return rc;
   const bool seg8 = r.labels && ctx->host_seg8;
-  davo_odometry* o = op ? op->o : nullptr;
-  const int set = (int)((o ? o->q_calls : ctx->q_calls)++ & 1);
-  uint8_t*& q_img = o ? o->q_img[set] : ctx->q_img[set];
-  uint8_t*& q_seg8 = o ? o->q_seg8[set] : ctx->q_seg8[set];
-  float*& q_seg = o ? o->q_seg[set] : ctx->q_seg[set];
-  float*& q_depth = o ? o->q_depth[set] : ctx->q_depth[set];
-  cudaEvent_t& ev_q_done = o ? o->ev_q_done[set] : ctx->ev_q_done[set];
-  if (!q_img) {
-    const size_t nf = (size_t)(o ? o->max_push : c.max_batch) + 2;
-    CU_OK(cudaMalloc((void**)&q_img, nf * hw * 3));
-    if (c.att_src != 0 && ctx->host_seg8) CU_OK(cudaMalloc((void**)&q_seg8, nf * hw));
-    if (c.att_src != 0 && !ctx->host_seg8) CU_OK(cudaMalloc((void**)&q_seg, nf * hw * 4));
-    if (r.depth) CU_OK(cudaMalloc((void**)&q_depth, nf * hw * 4));
-    CU_OK(cudaEventCreateWithFlags(&ev_q_done, cudaEventDisableTiming));
+  const int set = (int)(ctx->q_calls++ & 1);
+  if (!ctx->q_img[set]) {
+    const size_t nf = (size_t)c.max_batch + 2;
+    CU_OK(cudaMalloc((void**)&ctx->q_img[set], nf * hw * 3));
+    if (c.att_src != 0 && ctx->host_seg8) CU_OK(cudaMalloc((void**)&ctx->q_seg8[set], nf * hw));
+    if (c.att_src != 0 && !ctx->host_seg8) CU_OK(cudaMalloc((void**)&ctx->q_seg[set], nf * hw * 4));
+    if (r.depth) CU_OK(cudaMalloc((void**)&ctx->q_depth[set], nf * hw * 4));
+    CU_OK(cudaEventCreateWithFlags(&ctx->ev_q_done[set], cudaEventDisableTiming));
   } else {
-    CU_OK(cudaStreamWaitEvent(cp, ev_q_done, 0));                   // the call before the previous one has read this set
-  }
-  const int head = op ? op->head : 0, fe = op ? op->fe : 0;
-  // which frames and flow_fwd entries some pair reads: this call's, or for a push the whole stream's (global index
-  // g0 + f; every read predicate is true from frame 2 on, hence the clamp)
-  const SeqReads rg = o ? seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST) : r;
-  const int n_rd = o ? INT_MAX : n_frames;
-  auto glob = [&](int f) { return o ? (int)std::min<long long>(op->g0 + f, 2) : f; };
-  if (head > 0) {                                                  // the carried frames to the head of the set
-    CU_OK(cudaMemcpyAsync(q_img, o->c_img, hw * 3 * head, cudaMemcpyDeviceToDevice, cp));
-    if (seg8) CU_OK(cudaMemcpyAsync(q_seg8, o->c_seg8, hw * head, cudaMemcpyDeviceToDevice, cp));
-    else if (r.labels) CU_OK(cudaMemcpyAsync(q_seg, o->c_seg, hw * 4 * head, cudaMemcpyDeviceToDevice, cp));
-    if (r.depth) CU_OK(cudaMemcpyAsync(q_depth, o->c_depth, hw * 4 * head, cudaMemcpyDeviceToDevice, cp));
+    CU_OK(cudaStreamWaitEvent(cp, ctx->ev_q_done[set], 0));         // the call before the previous one has read this set
   }
   size_t h2d = 0;
   int launches = 0, last_n = 0, chunk = 0, ns = 0, last_ns = 0;
-  int staged = head;                                               // frames [0, staged) are on the device (or never read)
+  int staged = 0;                                                  // frames [0, staged) are on the device (or never read)
   if (pairs == DAVO_PAIRS_TRAJECTORY || pairs == DAVO_PAIRS_TRAJECTORY_FIRST)
     CU_OK(cudaMemsetAsync(ctx->s_pose, 0, (size_t)B * 12 * sizeof(float), st));
   // copies runs of consecutive frames in [f0, f1) that `read` selects: copy(first frame, frame count)
@@ -2526,53 +2441,29 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
     return 0;
   };
   InputView in{};
-  // a push's attention outputs: rows staged on the device, one unit table per chunk (the chunks' own pair modes)
-  const davo_odometry_attention* att = op && op->att && B > 0 ? op->att : nullptr;
-  float *att_maps = nullptr, *att_wts = nullptr;
-  const int4* att_units = nullptr;
-  const AttRow* att_rows = nullptr;
-  std::vector<int> att_off;
-  int att_slot = -1;
-  if (att) {
-    if (int rc = att_stage(ctx, (size_t)op->n_traj, &att_maps, &att_wts)) return rc;
-    std::vector<int4> units;
-    std::vector<AttRow> rows;
-    const bool opens = op->g0 == 0;
-    for (int a0 = 0; a0 < B; a0 += cs) {
-      const int an = std::min(cs, B - a0);
-      const int cp_ = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && a0 > 0) ? DAVO_PAIRS_TRAJECTORY : pairs;
-      att_off.push_back((int)units.size());
-      att_unit_table(units, cp_, pairs_selected(cp_, an),
-                     [&](int b) { const int sm = a0 + b; return AttSample{sm + 2 * opens, opens && sm == 0}; });
-    }
-    att_rows_of(rows, att->map ? att_maps : nullptr, att->weights ? att_wts : nullptr, op->n_traj, hw);
-    if (int rc = att_tables_upload(ctx, units, rows, st, &att_units, &att_rows, &att_slot)) return rc;
-  }
-  // a push too short to hold a sample still stages its frames: one chunk of no samples
-  for (int s0 = 0; s0 < B || (o && chunk == 0); s0 += ns, ++chunk) {
+  for (int s0 = 0; s0 < B; s0 += ns, ++chunk) {
     ns = std::min(cs, B - s0);
     last_ns = ns;
     const int buf = chunk % davo_ctx::kStage;
-    const int f0 = staged, f1 = s0 + ns < B ? s0 + ns + 2 : n_frames;   // frames this chunk stages
+    const int f0 = staged, f1 = s0 + ns + 2;                       // frames this chunk stages
     CU_OK(cudaStreamWaitEvent(cp, ctx->ev_consumed[buf], 0));       // whoever read this staging slot last is done
-    auto img_rd = [&](int f) { return rg.img(glob(f), n_rd); };
-    auto lab_rd = [&](int f) { return rg.lab(glob(f), n_rd); };
-    auto dep_rd = [&](int f) { return r.depth && img_rd(f); };
+    auto img_rd = [&](int f) { return r.img(f, n_frames); };
+    auto lab_rd = [&](int f) { return r.lab(f, n_frames); };
+    auto dep_rd = [&](int f) { return r.depth && r.img(f, n_frames); };
     if (int rc = runs(f0, f1, img_rd, [&](int f, int n) -> int {
-          CU_OK(cudaMemcpyAsync(q_img + hw * 3 * f, img + hw * 3 * (f - head), hw * 3 * n, cudaMemcpyHostToDevice, cp));
+          CU_OK(cudaMemcpyAsync(ctx->q_img[set] + hw * 3 * f, img + hw * 3 * f, hw * 3 * n, cudaMemcpyHostToDevice, cp));
           h2d += hw * 3 * n;
           return 0;
         })) return rc;
     if (int rc = runs(f0, f1, dep_rd, [&](int f, int n) -> int {
-          CU_OK(cudaMemcpyAsync(q_depth + hw * f, depth + hw * (f - head), hw * 4 * n, cudaMemcpyHostToDevice, cp));
+          CU_OK(cudaMemcpyAsync(ctx->q_depth[set] + hw * f, depth + hw * f, hw * 4 * n, cudaMemcpyHostToDevice, cp));
           h2d += hw * 4 * n;
           return 0;
         })) return rc;
     // flow entries of the chunk: flow_fwd[s0 + i] at slot entry i, flow_bwd[s0 + 1 + i] at slot entry cs + i
-    const int nfwd = ns > 0 && r.fwd(s0) ? (r.k0(s0 + ns - 1) ? ns : 1) : 0;   // fwd entries read: all, the first one (FIRST), none
+    const int nfwd = r.fwd(s0) ? (r.k0(s0 + ns - 1) ? ns : 1) : 0;    // fwd entries read: all, the first one (FIRST), none
     const bool need_bwd = r.flow;
-    const int carried = s0 < fe && nfwd > 0 ? 1 : 0;              // the session's flow_fwd entry takes slot entry 0
-    int n16 = (r.flow && ctx->host_flow16 && !carried) ? std::min(ns, (int)std::lround(ctx->flow16_frac * ns)) : 0;
+    int n16 = (r.flow && ctx->host_flow16) ? std::min(ns, (int)std::lround(ctx->flow16_frac * ns)) : 0;
     const bool conv_flow = n16 > 0;
     bool flow_ok = true;
     if (seg8 || conv_flow) {
@@ -2580,11 +2471,11 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
       std::vector<NarrowJob> jobs;
       uint16_t* h16 = ctx->h_flow16[buf];
       for (int i = 0; conv_flow && i < n16; ++i) {
-        if (i < nfwd) jobs.push_back({flow_fwd + fl * (s0 + i - fe), h16 + fl * i, fl, true});
-        jobs.push_back({flow_bwd + fl * (s0 + 1 + i - fe), h16 + fl * (cs + i), fl, true});
+        if (i < nfwd) jobs.push_back({flow_fwd + fl * (s0 + i), h16 + fl * i, fl, true});
+        jobs.push_back({flow_bwd + fl * (s0 + 1 + i), h16 + fl * (cs + i), fl, true});
       }
       for (int f = f0; seg8 && f < f1; ++f)                         // pinned label staging: frame f at f - f0
-        if (lab_rd(f)) jobs.push_back({seg + hw * (f - head), ctx->h_seg8[buf] + hw * (f - f0), hw, false});
+        if (lab_rd(f)) jobs.push_back({seg + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw, false});
       flow_ok = host_narrow(ctx, jobs);
     }
     if (conv_flow && !flow_ok) n16 = 0;                            // a value with no finite half: the whole chunk as float32
@@ -2597,25 +2488,23 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
       h2d += fl * 2 * (n16_fwd + n16);
     }
     float* dflow = ctx->s_flow[buf];
-    if (carried) CU_OK(cudaMemcpyAsync(dflow, o->c_fwd, fl * 4, cudaMemcpyDeviceToDevice, cp));
-    const int fwd0 = std::max(n16_fwd, carried);                   // first fwd slot entry copied as float32
-    if (nfwd > fwd0) {
-      CU_OK(cudaMemcpyAsync(dflow + fl * fwd0, flow_fwd + fl * (s0 + fwd0 - fe), fl * 4 * (nfwd - fwd0), cudaMemcpyHostToDevice, cp));
-      h2d += fl * 4 * (nfwd - fwd0);
+    if (nfwd > n16_fwd) {
+      CU_OK(cudaMemcpyAsync(dflow + fl * n16_fwd, flow_fwd + fl * (s0 + n16_fwd), fl * 4 * (nfwd - n16_fwd), cudaMemcpyHostToDevice, cp));
+      h2d += fl * 4 * (nfwd - n16_fwd);
     }
     if (need_bwd && ns > n16) {
-      CU_OK(cudaMemcpyAsync(dflow + fl * (cs + n16), flow_bwd + fl * (s0 + 1 + n16 - fe), fl * 4 * (ns - n16), cudaMemcpyHostToDevice, cp));
+      CU_OK(cudaMemcpyAsync(dflow + fl * (cs + n16), flow_bwd + fl * (s0 + 1 + n16), fl * 4 * (ns - n16), cudaMemcpyHostToDevice, cp));
       h2d += fl * 4 * (ns - n16);
     }
     if (seg8) {
       if (int rc = runs(f0, f1, lab_rd, [&](int f, int n) -> int {
-            CU_OK(cudaMemcpyAsync(q_seg8 + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw * n, cudaMemcpyHostToDevice, cp));
+            CU_OK(cudaMemcpyAsync(ctx->q_seg8[set] + hw * f, ctx->h_seg8[buf] + hw * (f - f0), hw * n, cudaMemcpyHostToDevice, cp));
             h2d += hw * n;
             return 0;
           })) return rc;
     } else if (r.labels) {
       if (int rc = runs(f0, f1, lab_rd, [&](int f, int n) -> int {
-            CU_OK(cudaMemcpyAsync(q_seg + hw * f, seg + hw * (f - head), hw * 4 * n, cudaMemcpyHostToDevice, cp));
+            CU_OK(cudaMemcpyAsync(ctx->q_seg[set] + hw * f, seg + hw * f, hw * 4 * n, cudaMemcpyHostToDevice, cp));
             h2d += hw * 4 * n;
             return 0;
           })) return rc;
@@ -2626,52 +2515,23 @@ static int forward_sequence_host_impl(davo_ctx* ctx, int n_frames, int pairs, co
     CU_OK(cudaStreamWaitEvent(st, ctx->ev_copied[buf], 0));
     // the chunk's view: sample 0 is sequence sample s0; a flow_fwd the chunk does not read stands in as its flow_bwd
     // (davo_profile_layers re-runs every pair of the last chunk)
-    in = sequence_view(c.H, c.W, q_img + hw * 3 * s0, nfwd ? dflow : dflow + fl * cs, dflow + fl * cs,
-                       seg8 ? nullptr : (q_seg ? q_seg + hw * s0 : nullptr),
-                       seg8 ? q_seg8 + hw * s0 : nullptr, q_depth ? q_depth + hw * s0 : nullptr,
+    in = sequence_view(c.H, c.W, ctx->q_img[set] + hw * 3 * s0, nfwd ? dflow : dflow + fl * cs, dflow + fl * cs,
+                       seg8 ? nullptr : (ctx->q_seg[set] ? ctx->q_seg[set] + hw * s0 : nullptr),
+                       seg8 ? ctx->q_seg8[set] + hw * s0 : nullptr, ctx->q_depth[set] ? ctx->q_depth[set] + hw * s0 : nullptr,
                        n16 > 0 ? (n16_fwd > 0 ? ctx->s_flow16[buf] : ctx->s_flow16[buf] + fl * cs) : nullptr,
                        n16 > 0 ? ctx->s_flow16[buf] + fl * cs : nullptr, n16);
     const int chunk_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && s0 > 0) ? DAVO_PAIRS_TRAJECTORY : pairs;
-    if (ns > 0) {
-      AttScope scope(ctx, att ? att_units + att_off[chunk] : nullptr, att_rows);
-      if (int rc = host_run_chunk(ctx, chunk_pairs, s0, ns, in, st, &launches, &last_n)) return rc;
-    }
+    if (int rc = host_run_chunk(ctx, chunk_pairs, s0, ns, in, st, &launches, &last_n)) return rc;
     CU_OK(cudaEventRecord(ctx->ev_consumed[buf], st));
   }
-  if (o) {
-    // carried state for the next push: the last two frames from the set, and the last flow_fwd entry (virtual entry
-    // n_frames - 2, which no sample of this push reads) when the sample that reads it is computed later
-    const int nc = std::min(n_frames, 2), fc = n_frames - nc;
-    CU_OK(cudaMemcpyAsync(o->c_img, q_img + hw * 3 * fc, hw * 3 * nc, cudaMemcpyDeviceToDevice, cp));
-    if (seg8) CU_OK(cudaMemcpyAsync(o->c_seg8, q_seg8 + hw * fc, hw * nc, cudaMemcpyDeviceToDevice, cp));
-    else if (r.labels) CU_OK(cudaMemcpyAsync(o->c_seg, q_seg + hw * fc, hw * 4 * nc, cudaMemcpyDeviceToDevice, cp));
-    if (r.depth) CU_OK(cudaMemcpyAsync(o->c_depth, q_depth + hw * fc, hw * 4 * nc, cudaMemcpyDeviceToDevice, cp));
-    const int e = n_frames - 2;
-    if (e >= fe && rg.fwd(glob(e))) {
-      CU_OK(cudaMemcpyAsync(o->c_fwd, flow_fwd + fl * (e - fe), fl * 4, cudaMemcpyHostToDevice, cp));
-      h2d += fl * 4;
-    }
-  }
-  CU_OK(cudaEventRecord(ev_q_done, st));
-  if (o && B > 0) {                                                // this push's absolute poses, after the last pass
-    const int first = op->g0 == 0, m = B + first;
-    pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(ctx->s_pose, B, first, o->d_rel);
-    CU_OK(cudaGetLastError());
-    traj_extend_kernel<<<1, 32, 0, st>>>(o->d_rel, m, first, o->d_P, o->d_traj);
-    CU_OK(cudaGetLastError());
-  }
-  if (att)
-    if (int rc = att_tables_done(ctx, att_slot, st)) return rc;
-  if (int rc = host_finish(ctx, B, pose_out, st, ticket, o ? reinterpret_cast<double*>(o->d_traj) : nullptr,
-                           op ? op->traj_out : nullptr, op ? op->n_traj : 0, att, att_maps, att_wts)) return rc;
+  CU_OK(cudaEventRecord(ctx->ev_q_done[set], st));
+  if (int rc = host_finish(ctx, B, pose_out, st, ticket)) return rc;
+  ctx->last_launches = launches;
+  ctx->last_npairs_mb = last_n;
   ctx->last_h2d = (long long)h2d;
-  if (B > 0) {                                                     // a push without samples ran no forward
-    ctx->last_launches = launches;
-    ctx->last_npairs_mb = last_n;
-    ctx->last_in = in;
-    ctx->last_pose = ctx->s_pose; ctx->last_B = last_ns;
-    ctx->last_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && chunk > 1) ? DAVO_PAIRS_TRAJECTORY : pairs;
-  }
+  ctx->last_in = in;
+  ctx->last_pose = ctx->s_pose; ctx->last_B = last_ns;
+  ctx->last_pairs = (pairs == DAVO_PAIRS_TRAJECTORY_FIRST && chunk > 1) ? DAVO_PAIRS_TRAJECTORY : pairs;
   return 0;
 }
 
@@ -2685,24 +2545,20 @@ extern "C" int davo_forward_sequence_host(davo_ctx* ctx, int n_frames, int pairs
 // ---- online odometry sessions (include/davo_b200.h: davo_odometry_*) ----
 static void odometry_free(davo_odometry* o) {
   cudaSetDevice(o->ctx->device);
-  for (int i = 0; i < 2; ++i) {
-    cudaFree(o->q_img[i]); cudaFree(o->q_seg8[i]); cudaFree(o->q_seg[i]); cudaFree(o->q_depth[i]);
-    if (o->ev_q_done[i]) cudaEventDestroy(o->ev_q_done[i]);
-  }
   cudaFree(o->c_img); cudaFree(o->c_seg8); cudaFree(o->c_seg); cudaFree(o->c_depth); cudaFree(o->c_fwd);
-  cudaFree(o->d_P); cudaFree(o->d_rel); cudaFree(o->d_traj); cudaFree(o->d_fwd);
+  cudaFree(o->d_P); cudaFree(o->d_rel); cudaFree(o->d_traj);
   delete o;
 }
 
 // A session's buffers on its handle's device (o->ctx): the carried state, the relative motions, a host session's
-// absolute poses, a device session's frame set.  A host session's frame sets come with its first push.
+// absolute poses.
 static int odometry_alloc(davo_odometry* o) {
   davo_ctx* ctx = o->ctx;
   CU_OK(cudaSetDevice(ctx->device));
   const davo_config& c = ctx->cfg;
   const SeqReads r = seq_reads(ctx, o->pairs);
-  const size_t hw = (size_t)c.H * c.W, nf = (size_t)o->max_push + 2;
-  const bool seg8 = o->host && ctx->host_seg8;                     // the form the passes read the labels in
+  const size_t hw = (size_t)c.H * c.W;
+  const bool seg8 = o->host && ctx->host_seg8;                     // the form the session carries its labels in
   auto alloc = [&](void** p, size_t bytes) -> int {
     CU_OK(cudaMalloc(p, bytes));
     return 0;
@@ -2714,12 +2570,6 @@ static int odometry_alloc(davo_odometry* o) {
   if (!rc) rc = alloc((void**)&o->d_P, 16 * sizeof(double));
   if (!rc) rc = alloc((void**)&o->d_rel, (size_t)(o->max_push + 1) * sizeof(Mat4));
   if (!rc && o->host) rc = alloc((void**)&o->d_traj, (size_t)(o->max_push + 2) * sizeof(Mat4));
-  if (!rc && !o->host) {                                           // one frame set, filled on the caller's stream
-    rc = alloc((void**)&o->q_img[0], nf * hw * 3);
-    if (!rc && c.att_src != 0) rc = alloc((void**)&o->q_seg[0], nf * hw * 4);
-    if (!rc && r.depth) rc = alloc((void**)&o->q_depth[0], nf * hw * 4);
-    if (!rc && r.flow) rc = alloc((void**)&o->d_fwd, (size_t)(o->max_push + 1) * hw * 2 * 4);
-  }
   return rc;
 }
 
@@ -2746,140 +2596,20 @@ extern "C" int davo_odometry_create(davo_ctx* ctx, int max_push, int pairs, int 
   return 0;
 }
 
-static int odometry_push_impl(const char* who, davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd,
-                              const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
-                              double* traj_out, const davo_odometry_attention* att, int* n_samples, int* n_traj,
-                              void* stream, long long* ticket) {
-  {
-    std::lock_guard<std::mutex> lk(g_odo_mutex);
-    if (!o || !g_odo_live.count(o)) return fail(nullptr, DAVO_ERR_ARG, "%s: the session is NULL or was destroyed", who);
-  }
-  davo_ctx* ctx = o->ctx;
-  const davo_config& c = ctx->cfg;
-  if (k < 1 || k > o->max_push) return fail(ctx, DAVO_ERR_ARG, "%s: k=%d new frames outside 1..max_push %d", who, k, o->max_push);
-  if (ticket && !o->host) return fail(ctx, DAVO_ERR_ARG, "%s: ticket: a device session runs on the caller's stream; only host sessions take a ticket", who);
-  const long long f0 = o->pushed;
-  const int head = o->head(), fe = head == 2 ? 1 : 0, n = head + k, ns = std::max(0, n - 2);
-  const long long g0 = f0 - head;
-  const int first = g0 == 0 && ns > 0, nt = ns + 2 * first;
-  const int vpairs = o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : first ? DAVO_PAIRS_TRAJECTORY_FIRST : DAVO_PAIRS_TRAJECTORY;
-  // what the stream reads of this push's flow entries: flow_fwd global entry e is read by sample e (as its plane 0)
-  // now or later, flow_bwd entry e by sample e - 1 (plane 1), which is computed now when it exists
-  const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
-  const long long e0 = std::max(f0 - 1, 0LL), e1 = f0 + k - 1;    // global flow entries [e0, e1) arrive with this push
-  const bool fwd_read = rg.flow && e1 > e0 && rg.k0((int)std::min(e0, 2LL));
-  const bool bwd_read = rg.flow && ns > 0;
-  struct { const void* p; bool needed; const char* name; } in[] = {
-      {img, true, "img"}, {pose_out, ns > 0, "pose_out"}, {traj_out, nt > 0, "traj_out"}, {seg, c.att_src != 0, "seg"},
-      {depth, rg.depth, "depth"}, {flow_bwd, bwd_read, "flow_bwd"}, {flow_fwd, fwd_read, "flow_fwd"}};
-  for (const auto& x : in) {
-    if (x.needed && !x.p) return fail(ctx, DAVO_ERR_ARG, "%s: %s is NULL; this variant and pair selection read it", who, x.name);
-    if (x.p && (reinterpret_cast<uintptr_t>(x.p) & 15)) return fail(ctx, DAVO_ERR_ARG, "%s: %s is not 16-byte aligned", who, x.name);
-  }
-  if (att)
-    if (int rc = att_check(ctx, who, *att, nt, -1)) return rc;
-  CU_OK(cudaSetDevice(ctx->device));
-  if (o->host) {
-    OdoPush op{o, head, fe, g0, traj_out, nt, att};
-    if (int rc = forward_sequence_host_impl(ctx, n, vpairs, img, flow_fwd, flow_bwd, seg, depth, pose_out, stream, ticket, &op))
-      return rc;
-  } else {
-    // the carried frames and the pushed ones into the session's set, the carried flow_fwd entry in front of the pushed
-    // ones, all on the caller's stream (which orders the caller's buffers); then the passes of davo_forward_sequence
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    const SeqReads r = seq_reads(ctx, vpairs);
-    const size_t hw = (size_t)c.H * c.W, fl = hw * 2;
-    auto d2d = [&](void* dst, const void* src, size_t bytes) -> int {
-      if (bytes) CU_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st));
-      return 0;
-    };
-    const bool labels = c.att_src != 0;
-    int rc = d2d(o->q_img[0], o->c_img, hw * 3 * head);
-    if (!rc) rc = d2d(o->q_img[0] + hw * 3 * head, img, hw * 3 * k);
-    if (!rc && labels) rc = d2d(o->q_seg[0], o->c_seg, hw * 4 * head);
-    if (!rc && labels) rc = d2d(o->q_seg[0] + hw * head, seg, hw * 4 * k);
-    if (!rc && r.depth) rc = d2d(o->q_depth[0], o->c_depth, hw * 4 * head);
-    if (!rc && r.depth) rc = d2d(o->q_depth[0] + hw * head, depth, hw * 4 * k);
-    // virtual flow entry v is the caller's entry v - fe; plane 1 of sample s is virtual flow_bwd entry s + 1
-    const float* fwd = flow_fwd;
-    if (!rc && fe && ns > 0 && r.fwd(0)) {
-      const int nfwd = r.k0(ns - 1) ? ns : 1;
-      rc = d2d(o->d_fwd, o->c_fwd, fl * 4);
-      if (!rc) rc = d2d(o->d_fwd + fl, flow_fwd, fl * 4 * (nfwd - 1));
-      fwd = o->d_fwd;
-    }
-    const float* bwd1 = flow_bwd ? flow_bwd + fl * (1 - fe) : nullptr;
-    if (!rc && ns > 0) {
-      const InputView v = sequence_view(c.H, c.W, o->q_img[0], fwd ? fwd : bwd1, bwd1, labels ? o->q_seg[0] : nullptr, nullptr,
-                                        o->q_depth[0], nullptr, nullptr, 0);
-      if (att) {                                                   // the frames' maps and weights: one unit table
-        const int mode = ctx->unit_sample ? kUnitsAreSamples : vpairs;
-        std::vector<int4> units;
-        std::vector<AttRow> rows;
-        att_unit_table(units, mode, pairs_selected(mode, ns), [&](int b) { return AttSample{b + 2 * first, first && b == 0}; });
-        att_rows_of(rows, att->map, att->weights, nt, hw);
-        const int4* du = nullptr;
-        const AttRow* dr = nullptr;
-        int slot = -1;
-        rc = att_tables_upload(ctx, units, rows, st, &du, &dr, &slot);
-        if (!rc) {
-          AttScope scope(ctx, du, dr);
-          rc = forward_device(ctx, who, ns, vpairs, v, pose_out, st);
-        }
-        if (!rc) rc = att_tables_done(ctx, slot, st);
-      } else {
-        rc = forward_device(ctx, who, ns, vpairs, v, pose_out, st);
-      }
-    }
-    const int nc = std::min(n, 2), fc = n - nc;
-    if (!rc) rc = d2d(o->c_img, o->q_img[0] + hw * 3 * fc, hw * 3 * nc);
-    if (!rc && labels) rc = d2d(o->c_seg, o->q_seg[0] + hw * fc, hw * 4 * nc);
-    if (!rc && r.depth) rc = d2d(o->c_depth, o->q_depth[0] + hw * fc, hw * 4 * nc);
-    const int e = n - 2;                                           // the last flow_fwd entry, read by a later sample
-    if (!rc && e >= fe && rg.fwd((int)std::min(g0 + e, 2LL))) rc = d2d(o->c_fwd, flow_fwd + fl * (e - fe), fl * 4);
-    if (rc) return rc;
-    if (ns > 0) {
-      const int m = ns + first;
-      pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(pose_out, ns, first, o->d_rel);
-      CU_OK(cudaGetLastError());
-      traj_extend_kernel<<<1, 32, 0, st>>>(o->d_rel, m, first, o->d_P, reinterpret_cast<Mat4*>(traj_out));
-      CU_OK(cudaGetLastError());
-    }
-  }
-  o->pushed += k;
-  o->posed += nt;
-  if (n_samples) *n_samples = ns;
-  if (n_traj) *n_traj = nt;
-  return 0;
-}
-
-extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
-                                  const float* seg, const float* depth, float* pose_out, double* traj_out, int* n_samples,
-                                  int* n_traj, void* stream, long long* ticket) {
-  return odometry_push_impl("davo_odometry_push", o, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, nullptr,
-                            n_samples, n_traj, stream, ticket);
-}
-
-extern "C" int davo_odometry_push_attention(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd,
-                                            const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
-                                            double* traj_out, const davo_odometry_attention* att, int* n_samples,
-                                            int* n_traj, void* stream, long long* ticket) {
-  return odometry_push_impl("davo_odometry_push_attention", o, k, img, flow_fwd, flow_bwd, seg, depth, pose_out,
-                            traj_out, att, n_samples, n_traj, stream, ticket);
-}
-
 namespace {
 
-// davo_odometry_push_many_host: each session's new frames, label planes, depth planes and flow entries that some
-// computed pair of its stream reads, now or in a later push (the rule of a single host push:
-// forward_sequence_host_impl's img_rd / lab_rd / dep_rd and its carried flow_fwd entry), copied on the copy stream into
-// one of the two arrivals sets.  Session i's part of the set holds its caller frame u and caller flow entry u at index
-// u, so that the stage and carry kernels read it as they read a device session's buffers; ds[i]'s caller pointers are
-// replaced by pointers into the set.  Labels are narrowed to bytes on the CPU for all sessions in one pool pass into the
-// set's pinned area (float labels with DAVO_B200_HOST_SEG8=0); the label planes of consecutive sessions sit back to back
-// there and on the device, so one copy sends them all, except where a plane no pair reads (global frame 1 in trajectory
-// mode when the target's labels are not read) breaks the run.  The flow goes as float32: with flow_f16 = 1 the front
-// end rounds it when read (frontend.cuh: flow_q), so the bits are those of a single push either way.
+// Host sessions' pushes: each session's new frames, label planes, depth planes and flow entries that some computed pair
+// of its stream reads, now or in a later push, copied on the copy stream into one of the two arrivals sets.  Session
+// i's part of the set holds its caller frame u and caller flow entry u at index u, so that the stage and carry kernels
+// read it as they read a device session's buffers; ds[i]'s caller pointers are replaced by pointers into the set.
+// Labels are narrowed to bytes on the CPU for all sessions in one pool pass into the set's pinned area (float labels
+// with DAVO_B200_HOST_SEG8=0); the label planes of consecutive sessions sit back to back there and on the device, so
+// one copy sends them all, except where a plane no pair reads (global frame 1 in trajectory mode when the target's
+// labels are not read) breaks the run.  With the binary16 transport (host_flow16), the first flow16_frac of the flow
+// entries the call sends (rounded up) are narrowed in the same pass, cross PCIe as binary16 in one copy with their
+// destination table, and odo_widen_kernel writes them into the set's float32 flow areas; a call with a value that has
+// no finite binary16 sends those entries as float32.  The front end reads the flow through flow_q, which rounds it to
+// binary16 when flow_f16 = 1, so either way the bits are the same.
 int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, OdoManySession* ds,
                        cudaStream_t st, int set, size_t* h2d_out) {
   const davo_config& c = ctx->cfg;
@@ -2887,19 +2617,29 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
   const size_t hw = (size_t)c.H * c.W, fl = hw * 2;
   const bool seg8 = rv.labels && ctx->host_seg8;
   cudaStream_t cp = ctx->copy_stream;
-  // the set's regions: session i's k[i] frames (or flow entries) at its running offset in each
-  size_t kt = 0;
-  for (int i = 0; i < n; ++i) kt += (size_t)ds[i].k;
+  // flow_fwd entry u is read as plane 0 of sample u + fe when that sample computes both pairs, or carried; flow_bwd
+  // entry u as plane 1 of sample u + fe - 1, for every sample
+  auto fwd_rd = [](const OdoManySession& d, int u) { return u + d.fe < d.na || u == d.carry_fwd; };
+  // the set's regions: session i's k[i] frames (or flow entries) at its running offset in each; ne flow entries sent
+  size_t kt = 0, ne = 0;
+  for (int i = 0; i < n; ++i) {
+    kt += (size_t)ds[i].k;
+    for (int u = 0; rv.flow && u < ds[i].k; ++u) ne += fwd_rd(ds[i], u);
+    if (rv.flow) ne += (size_t)ds[i].ns;
+  }
+  // the first ceil(flow16_frac * ne) of them go as binary16
+  const size_t n16 = rv.flow && ctx->host_flow16 ? std::min(ne, (size_t)std::ceil(ctx->flow16_frac * ne)) : 0;
   auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
   const size_t b_img = up(kt * hw * 3), b_lab = seg8 ? up(kt * hw) : 0, b_seg = rv.labels && !seg8 ? up(kt * hw * 4) : 0;
   const size_t b_dep = rv.depth ? up(kt * hw * 4) : 0, b_fl = rv.flow ? up(kt * fl * 4) : 0;
-  const size_t total = b_img + b_lab + b_seg + b_dep + 2 * b_fl;
+  const size_t b_16 = n16 * (fl * 2 + sizeof(int));                 // binary16 entries, then their destinations
+  const size_t total = b_img + b_lab + b_seg + b_dep + 2 * b_fl + b_16, pinned = b_lab + b_16;
   cudaEvent_t& done = ctx->a_done[set];
   if (!done) {
     CU_OK(cudaEventCreateWithFlags(&done, cudaEventDisableTiming));
     CU_OK(cudaEventCreateWithFlags(&ctx->a_copied[set], cudaEventDisableTiming));
   }
-  if (ctx->a_dev_cap[set] < total || (seg8 && ctx->a_hlab_cap[set] < kt * hw)) {
+  if (ctx->a_dev_cap[set] < total || ctx->a_pin_cap[set] < pinned) {
     CU_OK(cudaEventSynchronize(done));                             // the call that last used the set has read it
     if (ctx->a_dev_cap[set] < total) {
       const size_t cap = std::max(total, 2 * ctx->a_dev_cap[set]);
@@ -2908,12 +2648,12 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
       CU_OK(cudaMalloc((void**)&ctx->a_dev[set], cap));
       ctx->a_dev_cap[set] = cap;
     }
-    if (seg8 && ctx->a_hlab_cap[set] < kt * hw) {
-      const size_t cap = std::max(kt * hw, 2 * ctx->a_hlab_cap[set]);
-      if (ctx->a_hlab[set]) { CU_OK(cudaFreeHost(ctx->a_hlab[set])); ctx->a_hlab[set] = nullptr; }
-      ctx->a_hlab_cap[set] = 0;
-      CU_OK(cudaHostAlloc((void**)&ctx->a_hlab[set], cap, cudaHostAllocDefault));
-      ctx->a_hlab_cap[set] = cap;
+    if (ctx->a_pin_cap[set] < pinned) {
+      const size_t cap = std::max(pinned, 2 * ctx->a_pin_cap[set]);
+      if (ctx->a_pin[set]) { CU_OK(cudaFreeHost(ctx->a_pin[set])); ctx->a_pin[set] = nullptr; }
+      ctx->a_pin_cap[set] = 0;
+      CU_OK(cudaHostAlloc((void**)&ctx->a_pin[set], cap, cudaHostAllocDefault));
+      ctx->a_pin_cap[set] = cap;
     }
   }
   uint8_t* a_img = ctx->a_dev[set];
@@ -2922,6 +2662,9 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
   float* a_dep = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(a_seg) + b_seg);
   float* a_fwd = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(a_dep) + b_dep);
   float* a_bwd = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(a_fwd) + b_fl);
+  uint8_t* a_16 = reinterpret_cast<uint8_t*>(a_bwd) + b_fl;
+  uint16_t* h16 = reinterpret_cast<uint16_t*>(ctx->a_pin[set] + b_lab);
+  int* h16_dst = reinterpret_cast<int*>(h16 + n16 * fl);              // entry j's destination: fwd entry e < kt, else bwd e - kt
   CU_OK(cudaStreamWaitEvent(cp, done, 0));                         // the device part of the set is free
   size_t h2d = 0;
   auto h2d_copy = [&](void* dst, const void* src, size_t bytes) -> int {
@@ -2942,6 +2685,16 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
   };
   std::vector<NarrowJob> jobs;
   std::vector<std::pair<size_t, size_t>> lab_runs;                  // byte label planes read: [begin, end) in the area
+  std::vector<std::pair<int, const float*>> e16;                    // the entries narrowed: destination, source
+  auto flow_at = [&](size_t e) { return e < kt ? a_fwd + e * fl : a_bwd + (e - kt) * fl; };
+  // m flow entries from src to the set's entries e on (fwd e < kt, else bwd e - kt): the call's first n16 as binary16
+  auto send_flow = [&](size_t e, const float* src, int m) -> int {
+    for (; m > 0 && e16.size() < n16; --m, ++e, src += fl) {
+      jobs.push_back({src, h16 + e16.size() * fl, fl, true});
+      e16.push_back({(int)e, src});
+    }
+    return m > 0 ? h2d_copy(flow_at(e), src, fl * 4 * m) : 0;
+  };
   size_t off = 0;
   for (int i = 0; i < n; off += (size_t)ds[i].k, ++i) {
     OdoManySession& d = ds[i];
@@ -2971,7 +2724,7 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
       for (int u = 0; u < k; ++u) {
         if (!lab_rd(u)) continue;
         const size_t b = (off + u) * hw;
-        jobs.push_back({seg + u * hw, ctx->a_hlab[set] + b, hw, false});
+        jobs.push_back({seg + u * hw, ctx->a_pin[set] + b, hw, false});
         if (!lab_runs.empty() && lab_runs.back().second == b) lab_runs.back().second = b + hw;
         else lab_runs.push_back({b, b + hw});
       }
@@ -2982,26 +2735,33 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
       if (int rc = runs(k, lab_rd, [&](int u, int m) { return h2d_copy(as + u * hw, seg + u * hw, hw * 4 * m); })) return rc;
     }
     if (rv.flow) {
-      // flow_fwd entry u is read as plane 0 of sample u + fe when that sample computes both pairs, or carried; flow_bwd
-      // entry u as plane 1 of sample u + fe - 1, for every sample
-      float *af = a_fwd + off * fl, *ab = a_bwd + off * fl;
-      d.fwd = af;
-      d.bwd = ab;
-      auto fwd_rd = [&](int u) { return u + d.fe < d.na || u == d.carry_fwd; };
-      if (int rc = runs(k, fwd_rd, [&](int u, int m) { return h2d_copy(af + u * fl, fwd + u * fl, fl * 4 * m); })) return rc;
+      d.fwd = a_fwd + off * fl;
+      d.bwd = a_bwd + off * fl;
+      if (int rc = runs(k, [&](int u) { return fwd_rd(d, u); },
+                        [&](int u, int m) { return send_flow(off + u, fwd + u * fl, m); })) return rc;
       if (d.ns > 0)
-        if (int rc = h2d_copy(ab + (1 - d.fe) * fl, bwd + (1 - d.fe) * fl, fl * 4 * d.ns)) return rc;
+        if (int rc = send_flow(kt + off + 1 - d.fe, bwd + (1 - d.fe) * fl, d.ns)) return rc;
     }
   }
   if (!jobs.empty()) {
     CU_OK(cudaEventSynchronize(done));                             // the pinned area has been copied out by that call
-    host_narrow(ctx, jobs);
+    const bool flow_ok = host_narrow(ctx, jobs);
     for (const auto& r : lab_runs)
-      if (int rc = h2d_copy(a_lab + r.first, ctx->a_hlab[set] + r.first, r.second - r.first)) return rc;
+      if (int rc = h2d_copy(a_lab + r.first, ctx->a_pin[set] + r.first, r.second - r.first)) return rc;
+    if (!e16.empty() && flow_ok) {
+      for (size_t j = 0; j < e16.size(); ++j) h16_dst[j] = e16[j].first;
+      CU_OK(cudaMemcpyAsync(a_16, h16, b_16, cudaMemcpyHostToDevice, cp));
+      h2d += n16 * fl * 2;                                         // the flow's bytes (descriptors are not counted)
+      const int ny = (int)std::min<size_t>(n16, 65535);
+      odo_widen_kernel<<<dim3(std::max(1, 4 * 148 / ny), ny), 256, 0, cp>>>(
+          reinterpret_cast<const uint16_t*>(a_16), reinterpret_cast<const int*>(a_16 + n16 * fl * 2), (int)n16,
+          a_fwd, a_bwd, (long long)kt, (long long)fl);
+      CU_OK(cudaGetLastError());
+    } else {
+      for (const auto& x : e16)                                    // a value with no finite binary16: as float32
+        if (int rc = h2d_copy(flow_at(x.first), x.second, fl * 4)) return rc;
+    }
   }
-  // The stage kernel reads the carried state, which a single host push writes on the copy stream (the carried frames
-  // at the tail of forward_sequence_host_impl, the c_fwd upload).  Recorded after this call's copies, the event also
-  // follows that earlier work, so the wait orders the stage kernel behind it.
   CU_OK(cudaEventRecord(ctx->a_copied[set], cp));
   CU_OK(cudaStreamWaitEvent(st, ctx->a_copied[set], 0));
   *h2d_out = h2d;
@@ -3010,26 +2770,29 @@ int many_host_arrivals(davo_ctx* ctx, int n, davo_odometry* const* sessions, Odo
 
 }  // namespace
 
-// A batched push (include/davo_b200.h: davo_odometry_push_many, davo_odometry_push_many_host): entry i is
-// davo_odometry_push(sessions[i], k[i], ...), and all of them share one forward.  The samples are staged as stacked
-// triplets, those that compute both pairs (all-mode sessions, sample 0 of a trajectory session that opens its sequence,
-// every sample of the non-shared nets) first, so that the forward is at most one DAVO_PAIRS_ALL and one
-// DAVO_PAIRS_TRAJECTORY call.  A pair's result does not depend on which pairs share its pass, so every pose is the bits
-// of the single push; the trajectory is chained by the single push's code (traj_chain).  Launches: stage, carry, the
-// forward's, compose -- none per session.  Host sessions (`host`) first copy what the call reads into an arrivals set
-// (many_host_arrivals); their pose rows and absolute poses go back to the caller's host buffers at the end.
+// A push (include/davo_b200.h: davo_odometry_push, davo_odometry_push_many, davo_odometry_push_many_host): entry i is
+// the push of sessions[i], k[i] new frames, and all of them share one forward; a single push is the call with n = 1.
+// The samples are staged as stacked triplets, those that compute both pairs (all-mode sessions, sample 0 of a
+// trajectory session that opens its sequence, every sample of the non-shared nets) first, so that the forward is one
+// DAVO_PAIRS_TRAJECTORY_FIRST call when only the first sample computes both pairs, else at most one DAVO_PAIRS_ALL and
+// one DAVO_PAIRS_TRAJECTORY call.  A pair's result does not depend on which pairs share its pass, so every pose is
+// the bits of the session's push alone; the trajectory is chained by one code for every push (traj_chain).  Launches:
+// stage, carry, the forward's, compose -- none per session.  Host sessions (`host`) first copy what the call reads
+// into an arrivals set (many_host_arrivals); their pose rows and absolute poses go back to the caller's host buffers
+// at the end.  `single`: the messages name the inputs of davo_odometry_push, without an index.
 static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
                                    const float* const* flow_fwd, const float* const* flow_bwd,
                                    const float* const* seg, const float* const* depth, float* const* pose_out,
                                    double* const* traj_out, const davo_odometry_attention* att, int* n_samples,
-                                   int* n_traj, void* stream, long long* ticket, const char* who) {
+                                   int* n_traj, void* stream, long long* ticket, const char* who, bool single = false) {
   if (n < 1) return fail(nullptr, DAVO_ERR_ARG, "%s: n=%d: at least one session", who, n);
   if (!sessions) return fail(nullptr, DAVO_ERR_ARG, "%s: sessions is NULL", who);
   {
     std::lock_guard<std::mutex> lk(g_odo_mutex);
     for (int i = 0; i < n; ++i)
       if (!sessions[i] || !g_odo_live.count(sessions[i]))
-        return fail(nullptr, DAVO_ERR_ARG, "%s: sessions[%d] is NULL or was destroyed", who, i);
+        return fail(nullptr, DAVO_ERR_ARG, "%s: %s is NULL or was destroyed", who,
+                    single ? "the session" : EntryName("sessions", i).s);
   }
   davo_ctx* ctx = sessions[0]->ctx;
   const davo_config& c = ctx->cfg;
@@ -3049,14 +2812,17 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
   const size_t hw = (size_t)c.H * c.W;
   std::vector<OdoManySession> ds(n);
   int B = 0, nA = 0;
-  for (int i = 0; i < n; ++i) {                                           // the checks and counts of davo_odometry_push
+  for (int i = 0; i < n; ++i) {
     davo_odometry* o = sessions[i];
+    const int idx = single ? -1 : i;
     if (k[i] < 1 || k[i] > o->max_push)
-      return fail(ctx, DAVO_ERR_ARG, "%s: k[%d]=%d new frames outside 1..max_push %d", who, i, k[i], o->max_push);
+      return fail(ctx, DAVO_ERR_ARG, "%s: %s=%d new frames outside 1..max_push %d", who, EntryName("k", idx).s, k[i], o->max_push);
     const long long f0 = o->pushed;
     const int head = o->head(), fe = head == 2 ? 1 : 0, nn = head + k[i], ns = std::max(0, nn - 2);
     const long long g0 = f0 - head;
     const int first = g0 == 0 && ns > 0;
+    // what the stream reads of this push's flow entries: flow_fwd global entry e is read by sample e (as its plane 0)
+    // now or later, flow_bwd entry e by sample e - 1 (plane 1), which is computed now when it exists
     const SeqReads rg = seq_reads(ctx, o->pairs == DAVO_PAIRS_ALL ? DAVO_PAIRS_ALL : DAVO_PAIRS_TRAJECTORY_FIRST);
     const long long e0 = std::max(f0 - 1, 0LL), e1 = f0 + k[i] - 1;
     const bool fwd_read = rg.flow && e1 > e0 && rg.k0((int)std::min(e0, 2LL));
@@ -3070,8 +2836,10 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
         {d.seg, c.att_src != 0, "seg"}, {d.depth, rg.depth, "depth"}, {d.bwd, bwd_read, "flow_bwd"},
         {d.fwd, fwd_read, "flow_fwd"}};
     for (const auto& x : in) {
-      if (x.needed && !x.p) return fail(ctx, DAVO_ERR_ARG, "%s: %s[%d] is NULL; this variant and pair selection read it", who, x.name, i);
-      if (x.p && (reinterpret_cast<uintptr_t>(x.p) & 15)) return fail(ctx, DAVO_ERR_ARG, "%s: %s[%d] is not 16-byte aligned", who, x.name, i);
+      if (x.needed && !x.p)
+        return fail(ctx, DAVO_ERR_ARG, "%s: %s is NULL; this variant and pair selection read it", who, EntryName(x.name, idx).s);
+      if (x.p && (reinterpret_cast<uintptr_t>(x.p) & 15))
+        return fail(ctx, DAVO_ERR_ARG, "%s: %s is not 16-byte aligned", who, EntryName(x.name, idx).s);
     }
     d.c_img = o->c_img; d.c_seg = o->c_seg; d.c_depth = rv.depth ? o->c_depth : nullptr; d.c_fwd = o->c_fwd;
     d.P = o->d_P; d.rel = o->d_rel;
@@ -3080,7 +2848,7 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
     const int e = nn - 2;                                                 // the last flow_fwd entry, read by a later sample
     d.carry_fwd = e >= fe && rg.fwd((int)std::min(g0 + e, 2LL)) ? e - fe : -1;
     if (att)
-      if (int rc = att_check(ctx, who, att[i], ns + 2 * first, i)) return rc;
+      if (int rc = att_check(ctx, who, att[i], ns + 2 * first, idx)) return rc;
     B += ns;
     nA += d.na;
   }
@@ -3090,6 +2858,16 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
     OdoManySession& d = ds[i];
     d.ba = a; d.bt = t;
     for (int s = 0; s < d.ns; ++s) smp[s < d.na ? a++ : t++] = make_int2(i, s);
+  }
+  // the forwards over the staging batch: one pass when only staging sample 0 computes both pairs (the opening push of a
+  // trajectory session; the non-shared nets stage every sample as both-pair, nA == B)
+  struct Pass { int mode, b0, nb; };
+  std::vector<Pass> passes;
+  if (nA == 1 && B > 1) {
+    passes.push_back({DAVO_PAIRS_TRAJECTORY_FIRST, 0, B});
+  } else {
+    if (nA > 0) passes.push_back({DAVO_PAIRS_ALL, 0, nA});
+    if (B > nA) passes.push_back({DAVO_PAIRS_TRAJECTORY, nA, B - nA});
   }
   CU_OK(cudaSetDevice(ctx->device));
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -3114,9 +2892,40 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
     set = (int)(ctx->a_calls++ & 1);
     if (int rc = many_host_arrivals(ctx, n, sessions, ds.data(), st, set, &h2d)) return rc;
   }
-  // the descriptors: one copy from a pinned ring slot, refilled only after the call that last used it has finished
+  // each posed frame's attention: session i's rows from rb[i] on, one unit table per pass; host sessions' rows are
+  // staged on the device
+  std::vector<int> rb(n + 1, 0);
+  for (int i = 0; i < n; ++i) rb[i + 1] = rb[i] + ds[i].ns + 2 * ds[i].first;
+  const bool want_att = att && B > 0;
+  float *att_maps = nullptr, *att_wts = nullptr;
+  std::vector<int4> units;
+  std::vector<AttRow> rows;
+  std::vector<size_t> unit0;                                              // each pass's first unit
+  if (want_att) {
+    if (host)
+      if (int rc = att_stage(ctx, (size_t)rb[n], &att_maps, &att_wts)) return rc;
+    for (int i = 0; i < n; ++i) {
+      const int nt = rb[i + 1] - rb[i];
+      if (host) att_rows_of(rows, att[i].map ? att_maps + hw * rb[i] : nullptr,
+                            att[i].weights ? att_wts + kAttWeightFloats * rb[i] : nullptr, nt, hw);
+      else att_rows_of(rows, att[i].map, att[i].weights, nt, hw);
+    }
+    for (const Pass& p : passes) {
+      const int mode = ctx->unit_sample ? kUnitsAreSamples : p.mode;
+      unit0.push_back(units.size());
+      att_unit_table(units, mode, pairs_selected(mode, p.nb), [&](int b) {
+        const int2 m = smp[p.b0 + b];
+        const OdoManySession& d = ds[m.x];
+        return AttSample{rb[m.x] + m.y + 2 * d.first, d.first && m.y == 0};
+      });
+    }
+  }
+  // the descriptors (sessions, staging samples, unit table, rows): one copy from a pinned ring slot, refilled only
+  // after the call that last used it has finished
   const int slot = (int)(ctx->m_calls++ % davo_ctx::kManyRing);
-  const size_t sess_bytes = sizeof(OdoManySession) * n, bytes = sess_bytes + sizeof(int2) * B;
+  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+  const size_t o_smp = up16(sizeof(OdoManySession) * n), o_units = up16(o_smp + sizeof(int2) * B);
+  const size_t o_rows = o_units + sizeof(int4) * units.size(), bytes = o_rows + sizeof(AttRow) * rows.size();
   if (ctx->m_ev[slot]) CU_OK(cudaEventSynchronize(ctx->m_ev[slot]));
   else CU_OK(cudaEventCreateWithFlags(&ctx->m_ev[slot], cudaEventDisableTiming));
   if (ctx->m_desc_cap[slot] < bytes) {
@@ -3129,46 +2938,18 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
     ctx->m_desc_cap[slot] = cap;
   }
   uint8_t* h = static_cast<uint8_t*>(ctx->m_hdesc[slot]);
-  memcpy(h, ds.data(), sess_bytes);
-  if (B) memcpy(h + sess_bytes, smp.data(), sizeof(int2) * B);
+  memcpy(h, ds.data(), sizeof(OdoManySession) * n);
+  if (B) memcpy(h + o_smp, smp.data(), sizeof(int2) * B);
+  if (!units.empty()) memcpy(h + o_units, units.data(), sizeof(int4) * units.size());
+  if (!rows.empty()) memcpy(h + o_rows, rows.data(), sizeof(AttRow) * rows.size());
   CU_OK(cudaMemcpyAsync(ctx->m_ddesc[slot], h, bytes, cudaMemcpyHostToDevice, st));
-  const OdoManySession* dsess = static_cast<const OdoManySession*>(ctx->m_ddesc[slot]);
-  // each posed frame's attention: session i's rows from rb[i] on, one unit table per forward (staging order: the
-  // both-pair samples, then the trajectory samples); host sessions' rows are staged on the device
-  std::vector<int> rb(n + 1, 0);
-  for (int i = 0; i < n; ++i) rb[i + 1] = rb[i] + ds[i].ns + 2 * ds[i].first;
-  const bool want_att = att && B > 0;
-  float *att_maps = nullptr, *att_wts = nullptr;
-  const int4* att_units = nullptr;
-  const AttRow* att_rows = nullptr;
-  int att_slot = -1, nsel_a = 0;
-  if (want_att) {
-    if (host)
-      if (int rc = att_stage(ctx, (size_t)rb[n], &att_maps, &att_wts)) return rc;
-    std::vector<AttRow> rows;
-    for (int i = 0; i < n; ++i) {
-      const int nt = rb[i + 1] - rb[i];
-      if (host) att_rows_of(rows, att[i].map ? att_maps + hw * rb[i] : nullptr,
-                            att[i].weights ? att_wts + kAttWeightFloats * rb[i] : nullptr, nt, hw);
-      else att_rows_of(rows, att[i].map, att[i].weights, nt, hw);
-    }
-    auto sample_at = [&](int b) {
-      const int2 m = smp[b];
-      const OdoManySession& d = ds[m.x];
-      return AttSample{rb[m.x] + m.y + 2 * d.first, d.first && m.y == 0};
-    };
-    std::vector<int4> units;
-    const int mode_a = ctx->unit_sample ? kUnitsAreSamples : DAVO_PAIRS_ALL;
-    nsel_a = pairs_selected(mode_a, nA);
-    att_unit_table(units, mode_a, nsel_a, sample_at);
-    att_unit_table(units, DAVO_PAIRS_TRAJECTORY, B - nA, [&](int b) { return sample_at(nA + b); });
-    if (int rc = att_tables_upload(ctx, units, rows, st, &att_units, &att_rows, &att_slot)) return rc;
-  }
+  const uint8_t* dd = static_cast<const uint8_t*>(ctx->m_ddesc[slot]);
+  const OdoManySession* dsess = reinterpret_cast<const OdoManySession*>(dd);
   constexpr int kCopyBlocks = 4 * 148;                                     // blocks of a copy launch, over its rows
   if (B > 0) {
     OdoStageParams sp;
     sp.sess = dsess;
-    sp.smp = reinterpret_cast<const int2*>(static_cast<const uint8_t*>(ctx->m_ddesc[slot]) + sess_bytes);
+    sp.smp = reinterpret_cast<const int2*>(dd + o_smp);
     sp.hw = (long long)hw; sp.na = nA;
     sp.flow = rv.flow; sp.labels = rv.labels; sp.tgt_labels = rv.tgt_labels; sp.depth = rv.depth;
     sp.lab8 = host && ctx->host_seg8;
@@ -3180,26 +2961,22 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
   odo_carry_kernel<<<dim3(std::min(16, std::max(1, kCopyBlocks / n)), n), 256, 0, st>>>(dsess, (long long)hw, rv.depth);
   CU_OK(cudaGetLastError());
   if (host) {
-    // the arrivals set is free again, and a single host push, which reads and writes the carried state on the copy
-    // stream, must not start before the carry kernel has written it
+    // the arrivals set is free again; the next call's copies also wait for this point, which measured faster for host
+    // pushes of 128 frames than letting them start under this call's staging (DESIGN section 8.5)
     CU_OK(cudaEventRecord(ctx->a_done[set], st));
     CU_OK(cudaStreamWaitEvent(ctx->copy_stream, ctx->a_done[set], 0));
   }
   if (B > 0) {
-    auto view = [&](int b0) {
-      return stacked_view(c.H, c.W, ctx->m_img + hw * 9 * b0, ctx->m_flow ? ctx->m_flow + hw * 4 * b0 : nullptr,
-                          ctx->m_lab ? ctx->m_lab + hw * 3 * b0 : nullptr, ctx->m_depth ? ctx->m_depth + hw * 3 * b0 : nullptr);
-    };
-    if (nA > 0) {
-      AttScope scope(ctx, want_att ? att_units : nullptr, att_rows);
-      if (int rc = forward_device(ctx, who, nA, DAVO_PAIRS_ALL, view(0), ctx->m_pose, st)) return rc;
+    for (size_t q = 0; q < passes.size(); ++q) {
+      const Pass& p = passes[q];
+      const size_t b0 = (size_t)p.b0;
+      const InputView v = stacked_view(c.H, c.W, ctx->m_img + hw * 9 * b0, ctx->m_flow ? ctx->m_flow + hw * 4 * b0 : nullptr,
+                                       ctx->m_lab ? ctx->m_lab + hw * 3 * b0 : nullptr,
+                                       ctx->m_depth ? ctx->m_depth + hw * 3 * b0 : nullptr);
+      AttScope scope(ctx, want_att ? reinterpret_cast<const int4*>(dd + o_units) + unit0[q] : nullptr,
+                     want_att ? reinterpret_cast<const AttRow*>(dd + o_rows) : nullptr);
+      if (int rc = forward_device(ctx, who, p.nb, p.mode, v, ctx->m_pose + 12 * b0, st)) return rc;
     }
-    if (B > nA) {
-      AttScope scope(ctx, want_att ? att_units + nsel_a : nullptr, att_rows);
-      if (int rc = forward_device(ctx, who, B - nA, DAVO_PAIRS_TRAJECTORY, view(nA), ctx->m_pose + 12 * nA, st)) return rc;
-    }
-    if (want_att)
-      if (int rc = att_tables_done(ctx, att_slot, st)) return rc;
     odo_compose_many_kernel<<<(n + 3) / 4, 128, 0, st>>>(dsess, n, ctx->m_pose);
     CU_OK(cudaGetLastError());
   }
@@ -3231,6 +3008,37 @@ static int odometry_push_many_impl(bool host, int n, davo_odometry* const* sessi
     if (n_traj) n_traj[i] = nt;
   }
   return 0;
+}
+
+// The single push: the push of one session, with the messages of the single form.  Only host sessions take a ticket.
+static int odometry_push_one(const char* who, davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd,
+                             const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                             double* traj_out, const davo_odometry_attention* att, int* n_samples, int* n_traj,
+                             void* stream, long long* ticket) {
+  bool host;
+  {
+    std::lock_guard<std::mutex> lk(g_odo_mutex);
+    if (!o || !g_odo_live.count(o)) return fail(nullptr, DAVO_ERR_ARG, "%s: the session is NULL or was destroyed", who);
+    host = o->host;
+  }
+  if (ticket && !host) return fail(o->ctx, DAVO_ERR_ARG, "%s: ticket: a device session runs on the caller's stream; only host sessions take a ticket", who);
+  return odometry_push_many_impl(host, 1, &o, &k, &img, &flow_fwd, &flow_bwd, &seg, &depth, &pose_out, &traj_out, att,
+                                 n_samples, n_traj, stream, ticket, who, true);
+}
+
+extern "C" int davo_odometry_push(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd, const float* flow_bwd,
+                                  const float* seg, const float* depth, float* pose_out, double* traj_out, int* n_samples,
+                                  int* n_traj, void* stream, long long* ticket) {
+  return odometry_push_one("davo_odometry_push", o, k, img, flow_fwd, flow_bwd, seg, depth, pose_out, traj_out, nullptr,
+                           n_samples, n_traj, stream, ticket);
+}
+
+extern "C" int davo_odometry_push_attention(davo_odometry* o, int k, const uint8_t* img, const float* flow_fwd,
+                                            const float* flow_bwd, const float* seg, const float* depth, float* pose_out,
+                                            double* traj_out, const davo_odometry_attention* att, int* n_samples,
+                                            int* n_traj, void* stream, long long* ticket) {
+  return odometry_push_one("davo_odometry_push_attention", o, k, img, flow_fwd, flow_bwd, seg, depth, pose_out,
+                           traj_out, att, n_samples, n_traj, stream, ticket);
 }
 
 extern "C" int davo_odometry_push_many(int n, davo_odometry* const* sessions, const int* k, const uint8_t* const* img,
@@ -3321,7 +3129,7 @@ int label_form(const davo_ctx* ctx, bool host) { return ctx->cfg.att_src == 0 ? 
 // them) and depth planes, the flow_fwd entry a later sample reads (global entry pushed - 2, there when the push that
 // ended at frame `pushed` kept it) and the last absolute pose.  The sizes follow from the handle's configuration, the
 // session's kind and its counts, so they hold for a session whose buffers are not allocated yet; p[] are its buffers.
-// Frame sets, events, per-push buffers and q_calls are not state: a push writes them before it reads them.
+// Per-push buffers are not state: a push writes them before it reads them.
 enum { kSecImg, kSecSeg8, kSecSeg, kSecDepth, kSecFwd, kSecPose };
 struct Carried {
   void* p[kOdoSections];
@@ -4159,7 +3967,7 @@ extern "C" int davo_compose_trajectory(davo_ctx* ctx, const float* poses, int n,
   const int m = n + 1;                                   // relative motions
   if (int rc = traj_scratch(ctx, (size_t)m * sizeof(Mat4))) return rc;
   Mat4* rel = reinterpret_cast<Mat4*>(ctx->d_traj_scratch);
-  pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(poses, n, 1, rel);
+  pose_rel_kernel<<<(m + 127) / 128, 128, 0, st>>>(poses, n, rel);
   CU_OK(cudaGetLastError());
   const int threads = 256, chunk = (m + threads - 1) / threads;
   traj_scan_kernel<<<1, threads, threads * 16 * sizeof(double), st>>>(rel, m, chunk, reinterpret_cast<Mat4*>(traj));

@@ -1,4 +1,4 @@
-// Batched odometry pushes (include/davo_b200.h: davo_odometry_push_many): the kernels around the forward.
+// Odometry pushes (include/davo_b200.h: davo_odometry_push, davo_odometry_push_many): the kernels around the forward.
 //
 //   odo_stage_kernel        : every sample of the call into one stacked-triplet staging batch (input_view.cuh:
 //                             stacked_view), each frame slot from the session's carried state or the caller's buffer,
@@ -7,13 +7,16 @@
 //   odo_carry_kernel        : each session's new carried state (last two frames, the flow_fwd entry a later sample
 //                             reads) from its old carried state and the caller's buffers
 //   odo_compose_many_kernel : one warp per session: its pose rows out of the staging poses, its relative motions and
-//                             its absolute poses, chained with the code of a single push (trajectory.cuh: traj_chain)
+//                             its absolute poses (trajectory.cuh: traj_chain)
+//   odo_widen_kernel        : host sessions' flow entries sent as binary16, widened into the arrivals set's float32
+//                             flow areas before the stage kernel reads them
 // A push of session i is the virtual sequence of davo_odometry_push: its last `head` carried frames, then its k new
 // ones; virtual frame v < head is carried frame v, else the caller's frame v - head; virtual flow entry v < fe is the
 // carried flow_fwd entry, else the caller's entry v - fe.  Sample s is virtual frames (s, s+1, s+2).  For host sessions
 // "the caller's buffers" are the call's arrivals set on the device, which holds the caller's frames and entries at
 // the same indices (davo_capi.cu: many_host_arrivals).
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -199,6 +202,19 @@ __global__ void __launch_bounds__(128) odo_compose_many_kernel(const OdoManySess
   }
   __syncwarp();                                             // every lane's motions are visible to the chain
   traj_chain(d.rel, ns + first, first, d.P, d.traj_out);
+}
+
+// grid (x, y): entry j of the n binary16 entries of `fl` values each goes to fwd entry dst[j] when dst[j] < kt, else
+// to bwd entry dst[j] - kt.  Exact: every binary16 is a float32.
+__global__ void __launch_bounds__(256) odo_widen_kernel(const uint16_t* __restrict__ h16, const int* __restrict__ dst,
+                                                        int n, float* fwd, float* bwd, long long kt, long long fl) {
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
+  for (int j = blockIdx.y; j < n; j += gridDim.y) {
+    const long long e = dst[j];
+    const __half2* s = reinterpret_cast<const __half2*>(h16 + (size_t)j * fl);
+    float2* d = reinterpret_cast<float2*>(e < kt ? fwd + e * fl : bwd + (e - kt) * fl);
+    for (size_t i = t; i < (size_t)fl / 2; i += stride) d[i] = __half22float2(s[i]);
+  }
 }
 
 }  // namespace davo

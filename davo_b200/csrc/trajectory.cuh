@@ -5,7 +5,6 @@
 //                          the inverse of tgt->src1 in fp64)
 //   traj_scan_kernel     : P_0 = I, P_{i+1} = P_i . rel_i (test_kitti_pose.py:147-149) as a three-phase blocked
 //                          prefix product in fp64 (chunk-local products, a scan of the chunk totals, fix-up)
-//   traj_extend_kernel   : the same chain continued from a carried P, sequentially in frame order (online sessions)
 //   kitti_dist_kernel    : trajectoryDistances (kitti_benchmark/cpp/test_odometry_all.cpp:44-56): the devkit
 //                          accumulates in FLOAT, sequentially -- one thread does exactly that, so that
 //                          lastFrameFromSegmentLength picks the same frames
@@ -98,16 +97,16 @@ __device__ __forceinline__ void pose_vec2mat_f32(const float* v, double* out) {
   out[12] = 0.0; out[13] = 0.0; out[14] = 0.0; out[15] = 1.0;
 }
 
-// rel[0] = T(pose[0,0]) when `first` (the poses start at sample 0 of a sequence), then rel[first + s] = inv(T(pose[s,1]))
+// rel[0] = T(pose[0,0]) (the poses start at sample 0 of a sequence), then rel[1 + s] = inv(T(pose[s,1]))
 // (test_kitti_pose.py:143-145, batch_size 1)
-__global__ void __launch_bounds__(128) pose_rel_kernel(const float* __restrict__ poses, int n, int first, Mat4* __restrict__ rel) {
+__global__ void __launch_bounds__(128) pose_rel_kernel(const float* __restrict__ poses, int n, Mat4* __restrict__ rel) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n + first) return;
+  if (i >= n + 1) return;
   double t[16];
-  if (first && i == 0) {
+  if (i == 0) {
     pose_vec2mat_f32(poses, rel[0].m);
   } else {
-    pose_vec2mat_f32(poses + (size_t)(i - first) * 12 + 6, t);
+    pose_vec2mat_f32(poses + (size_t)(i - 1) * 12 + 6, t);
     mat4_inv(t, rel[i].m);
   }
 }
@@ -116,8 +115,7 @@ __global__ void __launch_bounds__(128) pose_rel_kernel(const float* __restrict__
 // `first` the chain starts from P_0 = I (also written to traj[0]) instead of the carried *P, which receives the last P.
 // One whole warp: lane l < 16 owns element l of P and sums its row-by-column product in k = 0..3 order, as mat4_mul
 // does, so that the result does not depend on how the frames were cut into pushes; P[r][k] comes from its owner by
-// shuffle.  A single push (traj_extend_kernel) and a batched one (odo_compose_many_kernel) both run this code, so a
-// session's trajectory is the same bits whichever way it was pushed.
+// shuffle.  Every push runs this code (odometry_many.cuh: odo_compose_many_kernel).
 __device__ __forceinline__ void traj_chain(const Mat4* rel, int m, int first, double* P, Mat4* traj) {
   const int lane = threadIdx.x & 31, l = lane & 15, r = l >> 2, c = l & 3;
   const bool owner = lane < 16;
@@ -131,11 +129,6 @@ __device__ __forceinline__ void traj_chain(const Mat4* rel, int m, int first, do
     if (owner) traj[first + i].m[l] = p;
   }
   if (owner) P[l] = p;
-}
-
-__global__ void __launch_bounds__(32) traj_extend_kernel(const Mat4* __restrict__ rel, int m, int first, double* __restrict__ P,
-                                                         Mat4* __restrict__ traj) {
-  traj_chain(rel, m, first, P, traj);
 }
 
 // traj[0] = I, traj[i + 1] = traj[i] . rel[i], i < m.  One block; thread t owns elements [t*chunk, (t+1)*chunk).

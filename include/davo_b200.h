@@ -258,9 +258,11 @@ int davo_forward_sequence_features(davo_ctx*, int n_frames, const uint8_t* img_u
  * handle are independent, and other calls on the handle may run between pushes.
  *
  * davo_odometry_create: max_push = most frames per push (1..max_batch); pairs = DAVO_PAIRS_TRAJECTORY or
- *   DAVO_PAIRS_ALL; host_inputs = 1: pushes pass host buffers and get host results (chunked, copies under compute,
- *   CPU narrowing, as davo_forward_sequence_host); 0: device buffers in, device results out, asynchronous on
- *   cuda_stream.  -batch_norm is refused (its poses depend on which samples share a call).
+ *   DAVO_PAIRS_ALL; host_inputs = 1: pushes pass host buffers and get host results (the push's copies run on a copy
+ *   stream, under the forward of the push before, with CPU narrowing as in davo_odometry_push_many_host); 0: device
+ *   buffers in, device results out, asynchronous on cuda_stream.  -batch_norm is refused (its poses depend on which
+ *   samples share a call).  A push is the batched push of one session (davo_odometry_push_many, _many_host): the
+ *   first push of any kind on a handle allocates its staging batch of max_batch samples.
  * davo_odometry_push: *n_samples / *n_traj (either may be NULL) receive the counts.  Host sessions: ticket == NULL
  *   blocks until the results are in pose_out / traj_out; otherwise they must be page-locked, the call returns once
  *   queued, and davo_host_wait(ctx, *ticket) waits for it.  Argument errors (k outside 1..max_push, a NULL input the
@@ -284,7 +286,7 @@ int davo_odometry_push(davo_odometry*, int k, const uint8_t* img, const float* f
  *   (with the zero rows of trajectory mode), traj_out, the counts and every later push on those sessions, single or
  *   batched.  Sessions may be in any state (first push, mid-stream, just reset), and trajectory and all-mode sessions
  *   may be mixed; the handle's other sessions are untouched.  Asynchronous on cuda_stream, no synchronisation; the
- *   number of kernel launches does not depend on n.  The first batched push on a handle allocates a staging batch of
+ *   number of kernel launches does not depend on n.  The first push on a handle allocates a staging batch of
  *   max_batch samples, freed with the handle.
  *   Argument errors return DAVO_ERR_ARG with a message naming the input and the session index: n < 1; a NULL or
  *   destroyed session (davo_last_error(NULL)); a session given twice; a host session; sessions of two handles; k[i]
@@ -304,8 +306,9 @@ int davo_odometry_push_many(int n, davo_odometry* const* sessions, const int* k,
  *   otherwise the outputs must be page-locked, the call returns once everything is queued, davo_host_wait(ctx, *ticket)
  *   waits for it, and the inputs must not be written before then.  Each new frame, label plane, depth plane and flow
  *   entry that some computed pair of its stream reads is copied once, as by the single push (labels narrowed to bytes
- *   on the CPU unless DAVO_B200_HOST_SEG8=0; the flow as float32); davo_last_host_copy_bytes reports the call's data
- *   bytes, with the default configuration the sum of what the same pushes made one by one report.  The kernel launches
+ *   on the CPU unless DAVO_B200_HOST_SEG8=0; with flow_f16 = 1 a share of the call's flow entries as binary16, see
+ *   DAVO_B200_HOST_FLOW16_FRAC, the rest as float32); davo_last_host_copy_bytes reports the call's data bytes, with
+ *   flow_f16 = 0 the sum of what the same pushes made one by one report.  The kernel launches
  *   do not depend on n; the copies are per session.  The first call allocates two arrivals sets that grow on demand,
  *   freed with the handle.
  *   Argument errors return DAVO_ERR_ARG with a message naming the input and the session index, as for

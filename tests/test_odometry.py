@@ -199,10 +199,11 @@ def test_sessions_on_one_handle_are_independent(host):
     ob.close()
 
 
-def _expected_stream_h2d(sysm, n, pairs):
+def _expected_stream_h2d(sysm, n, pairs, flow_entry_bytes=H * W * 8):
     """Bytes a host session moves over a whole n-frame stream: every frame, label plane, depth plane and flow entry some
     pair of the stream reads, once -- and the last flow_fwd entry of the stream when the sample after the last one
-    would read it (a push copies that entry for the next push, which the session cannot know will not come)."""
+    would read it (a push copies that entry for the next push, which the session cannot know will not come).  A flow
+    entry is `flow_entry_bytes`: H*W*8 as float32, H*W*4 as binary16."""
     c, hw = sysm.config, H * W
     unit = c.posenn not in (V.POSENN_DECOUPLE_SHARED_DIL, V.POSENN_COUPLE_SHARED_DIL)
     k0 = lambda s: unit or pairs == "all" or s == 0
@@ -212,15 +213,21 @@ def _expected_stream_h2d(sysm, n, pairs):
     lab = [f for f in range(n) if labels and (f >= 2 or k0(f) or (not c.att_tgt_ones and f >= 1))]
     depth = c.att_src == V.ATT_SE_DEPTH_SEG or c.depth_split
     fwd = sum(k0(s) for s in range(n - 1))                 # flow_fwd entry s is read by sample s (plane 0)
-    fl = (fwd + b) * hw * 8 if flow else 0
+    fl = (fwd + b) * flow_entry_bytes if flow else 0
     return n * hw * 3 + len(lab) * hw + (n * hw * 4 if depth else 0) + fl
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("key", ["headline", "se_seg", "decouple_net", "se_depth", "no_segmask"])
-def test_host_session_sends_each_read_plane_once(key):
+@pytest.mark.parametrize("key,f16", [pytest.param(k, False, id=k) for k in
+                                     ["headline", "se_seg", "decouple_net", "se_depth", "no_segmask"]] +
+                                    [pytest.param("headline", True, id="headline-flow16")])
+def test_host_session_sends_each_read_plane_once(key, f16, monkeypatch):
+    """f16: flow_f16 with every flow entry a push sends narrowed on the CPU, so every one crosses as binary16."""
     _need_gpu()
-    sysm = _system(G.CASES[key], 7, micro_batch=4)
+    flow_bytes = H * W * (4 if f16 else 8)
+    if f16:
+        monkeypatch.setenv("DAVO_B200_HOST_FLOW16_FRAC", "1")
+    sysm = _system(G.CASES[key], 7, micro_batch=4, flow_f16=f16)
     n = 20
     seq = _seq(n, seed=11)
     for pairs in ("trajectory", "all"):
@@ -232,7 +239,7 @@ def test_host_session_sends_each_read_plane_once(key):
                     h2d, d2h = sysm.last_host_copy_bytes()
                     assert d2h == out["pose"].nbytes + out["trajectory"].nbytes
                     total += h2d
-            assert total == _expected_stream_h2d(sysm, n, pairs), (key, pairs, cut)
+            assert total == _expected_stream_h2d(sysm, n, pairs, flow_bytes), (key, pairs, cut)
     # against the same stream as 3-frame sequence calls, one per new frame
     img, fwd, bwd, seg, depth = seq
     triples = 0
@@ -240,7 +247,7 @@ def test_host_session_sends_each_read_plane_once(key):
         sysm.inference_sequence(img[s:s + 3], fwd[s:s + 2], bwd[s:s + 2], seg[s:s + 3], depth[s:s + 3],
                                 pairs="trajectory_first" if s == 0 else "trajectory")
         triples += sysm.last_host_copy_bytes()[0]
-    assert _expected_stream_h2d(sysm, n, "trajectory") < triples
+    assert _expected_stream_h2d(sysm, n, "trajectory", flow_bytes) < triples
 
 
 @pytest.mark.gpu
@@ -314,9 +321,10 @@ def _ptxas(text):
     return out
 
 
-def test_forward_kernels_keep_their_registers_and_traj_extend_does_not_spill():
+def test_forward_kernels_keep_their_registers_and_push_kernels_do_not_spill():
     """The build's ptxas report (davo_b200/csrc/build.log) against profiles/odometry_ptxas.txt: pack8_kernel and every
-    conv kernel as recorded, traj_extend_kernel without spills."""
+    conv kernel as recorded; odo_compose_many_kernel (its stack frame holds a matrix) and odo_widen_kernel without
+    spills, odo_widen_kernel without a stack frame."""
     log = os.path.join(ROOT, "davo_b200", "csrc", "build.log")
     if not os.path.exists(log):
         pytest.skip("the library was not built by davo_b200/build.py here")
@@ -330,5 +338,6 @@ def test_forward_kernels_keep_their_registers_and_traj_extend_does_not_spill():
     assert len(names) >= 10
     for k in names:
         assert got[k] == rec[k], (k, got[k], rec[k])
-    ext = [k for k in got if "traj_extend_kernel" in k]
-    assert len(ext) == 1 and got[ext[0]][1:] == (0, 0, 0), got[ext[0]]
+    for name, tail in (("odo_compose_many_kernel", 2), ("odo_widen_kernel", 1)):
+        ext = [k for k in got if name in k]
+        assert len(ext) == 1 and got[ext[0]][tail:] == (0,) * (4 - tail), (name, got[ext[0]])

@@ -370,7 +370,7 @@ def test_ptxas_record_shows_no_spills_in_the_new_kernels():
         m = re.match(r"(\S+) regs=(\d+) stack=(\d+) spill=\((\d+), (\d+)\)$", line.strip())
         if m:
             rec[m.group(1)] = tuple(int(x) for x in m.groups()[1:])
-    for name in ("odo_stage_kernel", "odo_carry_kernel", "odo_compose_many_kernel", "traj_extend_kernel"):
+    for name in ("odo_stage_kernel", "odo_carry_kernel", "odo_compose_many_kernel"):
         got = [v for k, v in rec.items() if name in k]
         assert len(got) == 1 and got[0][2:] == (0, 0), (name, got)
     pack8 = [v for k, v in rec.items() if "pack8_kernel" in k]

@@ -8,7 +8,9 @@ Headline version, 128x416, a seeded frame stream (synthetic.make_sequence) in pi
   with the composition step on the host (T = pose_vec2mat, its inverse, one fp64 product).
 * Bulk rate: a host session fed pushes of 1, 16 and 128 frames with two pushes in flight, alternated in the same run
   with inference_sequence_async calls of 130 frames starting every 128 frames (two in flight) on the same frames.
-* Host-to-device bytes per frame for both (davo_last_host_copy_bytes).
+* Host-to-device bytes per frame for both (davo_last_host_copy_bytes), and for host sessions of a flow_f16 handle
+  (whose flow entries may cross as binary16; the share depends on the host's threads, DAVO_B200_HOST_FLOW16_FRAC).
+* Bulk rate of a device session fed pushes of 128 frames from HBM, synchronised at the end.
 
     python tools/odometry_stream.py [--frames 1026] [--reps 3] [--latency-frames 2000] [--log profiles/odometry_stream.log]
 
@@ -107,6 +109,25 @@ def latency(system, seq, n_lat, warm):
     return out
 
 
+def bulk_device(system, dev_seq, k):
+    """Frames per second of a device session fed pushes of k frames already on the GPU."""
+    import torch
+    n = dev_seq[0].shape[0]
+    cut = [k] * (n // k) + ([n % k] if n % k else [])
+    with system.odometry(max_push=k, host=False) as od:
+        for p in pieces(dev_seq, [k, k]):                       # warm: staging batch, pass shapes
+            od.push(*p)
+        od.reset()
+        torch.cuda.synchronize()
+        poses = []
+        t0 = time.perf_counter()
+        for p in pieces(dev_seq, cut):
+            poses.append(od.push(*p)["pose"])
+        torch.cuda.synchronize()
+        dt = time.perf_counter() - t0
+    return n / dt, torch.cat(poses).cpu().numpy()
+
+
 def bulk_session(system, seq, k, in_flight=2):
     """Frames per second and H2D bytes per frame of a host session fed pushes of k frames."""
     n = seq[0].shape[0]
@@ -166,7 +187,8 @@ def main(argv=None):
     res = {"workload": "host-fed online odometry, headline version, %dx%d, %d-frame seeded stream, trajectory mode"
                        % (H, W, a.frames), "gpus": 1, "card": card()}
     # bulk first (it warms every pass shape), alternating session and sequence calls rep by rep
-    rates = {k: [] for k in ("push_1", "push_16", "push_128", "sequence_calls_130")}
+    rates = {k: [] for k in ("push_1", "push_16", "push_128", "sequence_calls_130", "device_push_128")}
+    dev_seq = tuple(torch.as_tensor(x).cuda() for x in seq)
     ref = None
     identical = True
     for _ in range(a.reps):
@@ -180,10 +202,19 @@ def main(argv=None):
         rates["sequence_calls_130"].append(r)
         res["sequence_calls_h2d_bytes_per_frame"] = b
         identical &= np.array_equal(p, ref)
+        r, p = bulk_device(system, dev_seq, 128)
+        rates["device_push_128"].append(r)
+        identical &= np.array_equal(p, ref)
     res["bulk_frames_per_s"] = {k: {"median": float(np.median(v)), "all": [float(x) for x in v]} for k, v in rates.items()}
     res["push_128_over_sequence_calls"] = (res["bulk_frames_per_s"]["push_128"]["median"]
                                            / res["bulk_frames_per_s"]["sequence_calls_130"]["median"])
     res["poses_identical"] = bool(identical)
+    f16 = DAVO(version=ver)
+    f16.setup_inference(H, W, "davo", 3, PER_CALL, device=0, flow_f16=True)
+    f16.load_weights(S.init_weights(ver, seed=1, random_bias=True))
+    for k in (1, 16, 128):
+        res["flow_f16_push_%d_h2d_bytes_per_frame" % k] = bulk_session(f16, seq, k)[1]
+    f16.close()
     n_lat = a.latency_frames
     res["latency"] = latency(system, tuple(x[:min(a.frames, 514)] for x in seq), n_lat, a.warm)
     res["latency"]["note"] = "wall time from push of one frame to its absolute pose in host memory"
